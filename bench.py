@@ -2,6 +2,7 @@
 """bench.py -- lattice candidates evaluated / s (BASELINE.json metric) on N B200s of one node.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload c4]
+                    [--dump-outputs DIR]
 
 A step = one pass of the hot path (sampler -> spiral generation -> fused cost + collision ->
 argmin -> tracker) over one batch of synthetic planning scenarios (SURVEY.md 8d, config 4):
@@ -14,6 +15,10 @@ barrier and the max-over-ranks of the step time).
 through the public Python API (LatticePlanner.plan_batch) with pinned HOST buffers, H2D and D2H
 inside the timed region.  `--impl reference` times the CPU oracle port (the reference's lattice
 path cannot execute: SURVEY.md section 0) on all host cores on a bounded sample of the workload.
+
+`--dump-outputs DIR` writes what the last timed step of the device-resident arm returned (rank 0)
+as DIR/<name>.npy (dump_outputs).  The scenarios are seeded, so two builds run with the same
+arguments can be compared output for output.
 """
 import argparse
 import json
@@ -54,7 +59,14 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--quick", action="store_true",
                     help="kernel A/B runs: device-resident arm only, prints a short JSON line")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to the CUDA path (--impl ours)")
+    return args
 
 
 # ------------------------------------------------------------------------------------------------
@@ -505,6 +517,45 @@ class DeviceArm:
                                 steer_speed=self.o_ss)
 
 
+DUMP_BYTES = 60 * 10**6   # with the .npy headers and file-system blocks, under 64 MB
+
+
+def dump_outputs(torch, arm, out_dir):
+    """Every output of DeviceArm.step() as out_dir/<name>.npy in float32 / float64 (indices and
+    flags converted exactly), DUMP_BYTES in all.  Every value written is finite: a non-finite
+    entry (the +inf cost of an invalid or collided candidate, the +inf best_cost of a scenario
+    without a feasible candidate) is written as 0, and <name>_finite.npy holds 1 where the value
+    is finite (per scenario for best_traj).  The per-scenario outputs cover every scenario while
+    they fit in 2/3 of the budget (the default size does), else a seeded sample of scenarios;
+    best_traj [S, M, 4] (160 MB at the default size) a seeded sample in the rest.  scenarios.npy
+    and best_traj_scenarios.npy give the scenario index of each row."""
+    S, M, C = arm.S, arm.o_traj.shape[1], arm.o_costs.shape[1]
+    rng = np.random.default_rng(0)
+
+    def rows(budget, row_bytes):
+        n = max(0, budget // row_bytes)
+        return np.arange(S) if n >= S else np.sort(rng.choice(S, n, replace=False))
+
+    def finite(v, per_scenario):
+        ok = torch.isfinite(v)
+        return torch.where(ok, v, torch.zeros_like(v)), (ok.flatten(1).all(1) if per_scenario else ok).float()
+
+    # index, best_idx, best_cost + mask, costs + mask, flags, steer_speed + mask
+    row_bytes = 8 + 8 + 8 + C * 12 + 24
+    r = rows(DUMP_BYTES * 2 // 3, row_bytes)
+    t = rows(DUMP_BYTES - len(r) * row_bytes - (16 << 10), 8 + M * 16 + 4)   # 16 KB: .npy headers
+    ri = torch.from_numpy(r).to(arm.o_costs.device)
+    ti = torch.from_numpy(t).to(arm.o_costs.device)
+    out = {"scenarios": r.astype(np.float64), "best_idx": arm.o_idx[ri].double(),
+           "flags": arm.o_flags[ri].float(), "best_traj_scenarios": t.astype(np.float64)}
+    for name, v, per_scenario in (("best_cost", arm.o_cost[ri], False), ("costs", arm.o_costs[ri], False),
+                                  ("steer_speed", arm.o_ss[ri], False), ("best_traj", arm.o_traj[ti], True)):
+        out[name], out[name + "_finite"] = finite(v, per_scenario)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), v.cpu().numpy() if torch.is_tensor(v) else v)
+
+
 class HostArm:
     """the public API with pinned HOST buffers: every output the device-resident arm writes"""
 
@@ -641,6 +692,8 @@ def run_ours(args):
     eval_shape = eng.last_eval_shape()   # the template instance the timed steps launched
     eng.set_timing(False)
     value = world_size * S * C * args.steps / (ms_total * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(torch, arm, args.dump_outputs)   # before any later step overwrites them
 
     if args.quick:
         if rank == 0:

@@ -1,18 +1,7 @@
 """Loaders for the reference's on-disk formats (raceline CSV, ROS map yaml + image)."""
-import os
-
 import numpy as np
-import pytest
 
 from f1tenth_planning_b200 import io
-
-REF = "/root/reference/examples/control"
-GOLDEN = os.path.join(os.path.dirname(__file__), "golden")
-
-
-def _unpack(g, name):
-    h, w = g[name + "_shape"]
-    return np.unpackbits(g[name + "_bits"], axis=1)[:, :w]
 
 
 def test_map_round_trip(tmp_path):
@@ -43,18 +32,3 @@ def test_raceline_layouts(tmp_path):
     p7.write_text("# id\n# hash\n# s_m; x_m; y_m; psi_rad; kappa_radpm; vx_mps; ax_mps2\n" +
                   "\n".join("; ".join("%.7f" % v for v in r) for r in b))
     assert np.array_equal(io.load_raceline(str(p7)), b[:, [1, 2, 5, 3, 4]])
-
-
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference fixtures only exist in the build container")
-def test_reference_fixtures_match_committed_golden(golden_spielberg):
-    g = np.load(os.path.join(GOLDEN, "maps.npz"))
-    wp = io.load_raceline(os.path.join(REF, "Spielberg_raceline.csv"))
-    assert np.array_equal(wp, golden_spielberg["waypoints"])
-    occ, origin, res = io.load_map(os.path.join(REF, "Spielberg_map.yaml"))
-    assert np.array_equal(occ, _unpack(g, "spielberg"))
-    assert tuple(g["spielberg_origin"]) == origin and float(g["spielberg_res"]) == res
-    # the raceline runs through free cells of its own map
-    col = np.floor((wp[:, 0] - origin[0]) / res).astype(int)
-    row = np.floor((wp[:, 1] - origin[1]) / res).astype(int)
-    assert not occ[row, col].any()
-    assert np.array_equal(io.load_raceline(os.path.join(REF, "levine_raceline.csv")), g["levine_raceline"])

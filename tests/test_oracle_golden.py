@@ -1,16 +1,11 @@
 """Pins the CPU oracle to the reference: golden vectors minted by tests/golden/make_golden.py from
-the UNMODIFIED reference functions (utils/utils.py, pure_pursuit.py), the SURVEY appendix-C known
-answers, and -- when /root/reference is present (build container only) -- the live functions."""
+the UNMODIFIED reference functions (utils/utils.py, pure_pursuit.py) and the SURVEY appendix-C
+known answers."""
 import os
-import sys
 
 import numpy as np
-import pytest
 
-from f1tenth_planning_b200 import synth
 from oracle import c_oracle as co
-
-REF = "/root/reference"
 
 
 def _check_pp(g, wp):
@@ -77,26 +72,6 @@ def test_argmin_and_length_cost_semantics(golden_misc):
     assert int(golden_misc["select"][0]) == 1                 # LatticePlanner.select([3,1,1,2])
     assert golden_misc["length_cost"].tolist() == [0.5, 0.25]  # get_length_cost
     assert int(np.argmin([3.0, 1.0, 1.0, 2.0])) == 1
-
-
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout only exists in the build container")
-def test_live_reference_functions(ellipse):
-    sys.path.insert(0, REF)
-    try:
-        from f1tenth_planning.utils.utils import nearest_point, intersect_point
-    finally:
-        sys.path.remove(REF)
-    rng = np.random.default_rng(99)
-    poses, _ = synth.random_poses(ellipse, 60, rng)
-    xy = np.ascontiguousarray(ellipse[:, :2])
-    for q in poses:
-        pos = np.array([q[0], q[1]])
-        rp, rd, rt, ri = nearest_point(pos, xy)
-        p, d, t, i = co.nearest_point(pos, xy)
-        assert i == ri and abs(d - rd) < 1e-12 and abs(t - rt) < 1e-12
-        rq, ri2, rt2 = intersect_point(pos, 1.7, xy, float(ri + rt), wrap=True)
-        q2, i2, t2 = co.intersect_point(pos, 1.7, xy, i + t, wrap=True)
-        assert i2 == ri2 and abs(t2 - rt2) < 1e-9
 
 
 def test_front_axle_errors_match_stanley_and_lqr(golden_spielberg):
