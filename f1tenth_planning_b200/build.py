@@ -39,7 +39,7 @@ def _compile(OUT, verbose, defs):
            "-std=c++17", "-Xcompiler", "-fPIC", "-shared", "-diag-suppress", "177",
            "-o", OUT] + [os.path.join(SRC_DIR, s) for s in SOURCES]
     for d in list(defs) + os.environ.get("F1L_NVCC_DEFS", "").split():
-        cmd.insert(1, "-D" + d)   # e.g. F1L_NVCC_DEFS="EVAL_MIN_BLOCKS=4" for build-time experiments
+        cmd.insert(1, "-D" + d)   # e.g. F1L_NVCC_DEFS="PP_UNROLL=4" for build-time experiments
     if verbose:
         cmd.insert(1, "-Xptxas")
         cmd.insert(2, "-v")

@@ -85,8 +85,6 @@ struct f1l_ctx {
     DevBuf q_res, q_in, q_goals, q_ctx, q_centres, q_best, q_states, q_headings, q_params, q_flags;
     // pinned staging for the single query
     void* h_in = nullptr;   // pose + opponents
-    void* h_in_dev = nullptr;   // the same block as the device sees it (mapped): the sampler of a single
-                                // query reads its 416 bytes of input straight from it
     void* h_out = nullptr;  // header + best trajectory
     void* h_out_dev = nullptr;  // the same block as the device sees it (mapped pinned memory): the
                                 // select kernel of a single query writes its results straight into it
@@ -267,106 +265,81 @@ int check_config(const f1l_config* c) {
     return F1L_OK;
 }
 
-// ---- kernel dispatch on the sample count -------------------------------------------------
-struct EvalShape {
-    int ipl, s, sg;
-};
-
-// deviation-pass shape of the M <= 104 kernels: S samples per lane x SG sample groups (A/B switch)
-#ifndef EVAL_S104
-#define EVAL_S104 13
-#define EVAL_SG104 8
-#endif
-EvalShape eval_shape(int M) {
-    if (M <= 32) return {1, 4, 8};
-    if (M <= 64) return {2, 8, 8};
-    if (M <= 104) return {4, EVAL_S104, EVAL_SG104};
-    if (M <= 128) return {4, 16, 8};
-    if (M <= 208) return {7, 13, 16};
-    return {8, 16, 16};
-}
-
+// ---- kernel instances per sample count ---------------------------------------------------------
 typedef void (*eval_fn)(EvalArgs);
 typedef void (*select_fn)(SelectArgs);
 typedef void (*generate_fn)(LutView, EvalParams, const float4*, int, float4*, float4*, uint8_t*);
 
+// One compiled eval_kernel: the resident CTAs per SM its register budget is built for (MINB), and
+// its shared memory in front of the window table (EvalSmem::C_TAB).
+struct EvalBuild {
+    eval_fn fn;   // null: not built
+    int minb;
+    uint32_t smem_fixed;
+    size_t smem_bytes(int nseg_pad) const {
+        return smem_fixed + (size_t)(nseg_pad + EVAL_SEG_PAD) * (2 * sizeof(float4));
+    }
+};
+
+// The kernels that serve sample counts M <= m_max: the deviation-pass shape (IPL samples per lane;
+// S samples per lane x SG sample groups in the loop), one eval build per warp count, and the select
+// and generate kernels of the same IPL.
+struct EvalBucket {
+    int m_max, ipl, s, sg;
+    EvalBuild nw4, nw7, nw8;
+    EvalBuild wide;   // 8 warps at two CTAs per SM (128 registers), large dense queries
+    select_fn select;
+    generate_fn generate;
+    const EvalBuild& build(int nw) const { return nw == 4 ? nw4 : (nw == 7 ? nw7 : nw8); }
+};
+
+template <int IPL, int S, int SG, int NW, int MINB>
+EvalBuild eval_build() {
+    if constexpr (MINB == 0) return {nullptr, 0, 0};
+    else return {eval_kernel<IPL, S, SG, NW, MINB>, MINB, EvalSmem<S, SG, NW>::C_TAB};
+}
+template <int M_MAX, int IPL, int S, int SG, int MINB4, int MINB7, int MINB8, int MINB_WIDE>
+EvalBucket eval_bucket() {
+    return {M_MAX, IPL, S, SG,
+            eval_build<IPL, S, SG, 4, MINB4>(), eval_build<IPL, S, SG, 7, MINB7>(),
+            eval_build<IPL, S, SG, 8, MINB8>(), eval_build<IPL, S, SG, 8, MINB_WIDE>(),
+            select_kernel<IPL>, generate_kernel<IPL>};
+}
+
+// Every eval_kernel instance and its residency, one row per bucket (MINB 0: no such build).
 // NW = 7 (four resident CTAs of 7 warps at <= 72 registers) serves candidate counts that are a
-// small multiple of 7 -- the default 4x7 goal grid; everything else runs 8-warp CTAs.
-#ifndef EVAL_MINB8
-#define EVAL_MINB8 3
-#endif
-#ifndef EVAL_MINB7
-#define EVAL_MINB7 4
-#endif
-#ifndef EVAL_MINB4
-#define EVAL_MINB4 7
-#endif
-// The M <= 104 shape on 4-warp CTAs (the batch regime of the 4x7 grid): FOUR CTAs per SM at 125
-// registers instead of seven at 72 -- the deviation loop gets the schedule it wants (no spill, 8.2
-// instead of 9.6 sub-partition cycles per (sample, segment) in isolation) and sixteen warps per SM
-// still cover the latency-bound stages: 11.10 -> 10.84 ms on the bench workload (five CTAs at 96
-// registers: 11.16, six at 80: 11.26, three at 161: 11.69; profiles/r2_microbench.md).
-#ifndef EVAL_MINB4_104
-#define EVAL_MINB4_104 4
-#endif
-static inline int eval_minb(int nw, int M) {
-    if (nw == 4) return (M > 64 && M <= 104) ? EVAL_MINB4_104 : EVAL_MINB4;
-    return nw == 7 ? EVAL_MINB7 : EVAL_MINB8;
-}
-eval_fn eval_entry(int M, int nw) {
-    if (nw == 4) {
-        if (M <= 32) return eval_kernel<1, 4, 8, 4, EVAL_MINB4>;
-        if (M <= 64) return eval_kernel<2, 8, 8, 4, EVAL_MINB4>;
-        if (M <= 104) return eval_kernel<4, EVAL_S104, EVAL_SG104, 4, EVAL_MINB4_104>;
-        if (M <= 128) return eval_kernel<4, 16, 8, 4, EVAL_MINB4>;
-        if (M <= 208) return eval_kernel<7, 13, 16, 4, EVAL_MINB4>;
-        return eval_kernel<8, 16, 16, 4, EVAL_MINB4>;
-    }
-    if (nw == 7) {
-        if (M <= 32) return eval_kernel<1, 4, 8, 7, EVAL_MINB7>;
-        if (M <= 64) return eval_kernel<2, 8, 8, 7, EVAL_MINB7>;
-        if (M <= 104) return eval_kernel<4, EVAL_S104, EVAL_SG104, 7, EVAL_MINB7>;
-        if (M <= 128) return eval_kernel<4, 16, 8, 7, EVAL_MINB7>;
-        if (M <= 208) return eval_kernel<7, 13, 16, 7, EVAL_MINB7>;
-        return eval_kernel<8, 16, 16, 7, EVAL_MINB7>;
-    }
-    if (M <= 32) return eval_kernel<1, 4, 8, 8, EVAL_MINB8>;
-    if (M <= 64) return eval_kernel<2, 8, 8, 8, EVAL_MINB8>;
-    if (M <= 104) return eval_kernel<4, EVAL_S104, EVAL_SG104, 8, EVAL_MINB8>;
-    if (M <= 128) return eval_kernel<4, 16, 8, 8, EVAL_MINB8>;
-    if (M <= 208) return eval_kernel<7, 13, 16, 8, EVAL_MINB8>;
-    return eval_kernel<8, 16, 16, 8, EVAL_MINB8>;
-}
-// M > 128 shapes at two 8-warp CTAs per SM (128 registers): the deviation loop gets the registers
-// it wants (tools/microbench/devloop_bench.cu), at the price of a third fewer resident warps.  Pays
-// for a dense query with many candidates per warp slot (the unsharded 65 536), not for its shards.
-#define EVAL_MINB8_WIDE 2
-eval_fn eval_entry_wide(int M) {
-    if (M <= 208) return eval_kernel<7, 13, 16, 8, EVAL_MINB8_WIDE>;
-    return eval_kernel<8, 16, 16, 8, EVAL_MINB8_WIDE>;
-}
-select_fn select_entry(int M) {
-    if (M <= 32) return select_kernel<1>;
-    if (M <= 64) return select_kernel<2>;
-    if (M <= 128) return select_kernel<4>;
-    if (M <= 208) return select_kernel<7>;
-    return select_kernel<8>;
-}
-generate_fn generate_entry(int M) {
-    if (M <= 32) return generate_kernel<1>;
-    if (M <= 64) return generate_kernel<2>;
-    if (M <= 128) return generate_kernel<4>;
-    if (M <= 208) return generate_kernel<7>;
-    return generate_kernel<8>;
+// small multiple of 7 -- the default 4x7 goal grid; everything else runs 8-warp CTAs (three at 80).
+// The M <= 104 shape on 4-warp CTAs (the batch regime of the 4x7 grid) runs FOUR CTAs per SM at
+// 125 registers instead of seven at 72 -- the deviation loop gets the schedule it wants (no spill,
+// 8.2 instead of 9.6 sub-partition cycles per (sample, segment) in isolation) and sixteen warps per
+// SM still cover the latency-bound stages: 11.10 -> 10.84 ms on the bench workload (five CTAs at
+// 96 registers: 11.16, six at 80: 11.26, three at 161: 11.69; S = 7 x SG = 16 instead of 13 x 8:
+// 11.53; profiles/r2_microbench.md).  The wide build of the M > 128 shapes, two 8-warp CTAs per SM
+// at 128 registers, gives the deviation loop the registers it wants
+// (tools/microbench/devloop_bench.cu) at the price of a third fewer resident warps: it pays for a
+// dense query with many candidates per warp slot (the unsharded 65 536), not for its shards.
+//
+//                  M <=  IPL   S  SG   MINB at NW = 4, 7, 8, 8 (wide)
+const EvalBucket kEvalBuckets[] = {
+    eval_bucket<      32,   1,  4,  8,   7, 4, 3, 0>(),
+    eval_bucket<      64,   2,  8,  8,   7, 4, 3, 0>(),
+    eval_bucket<     104,   4, 13,  8,   4, 4, 3, 0>(),
+    eval_bucket<     128,   4, 16,  8,   7, 4, 3, 0>(),
+    eval_bucket<     208,   7, 13, 16,   7, 4, 3, 2>(),
+    eval_bucket<F1L_MAX_M,  8, 16, 16,   7, 4, 3, 2>(),
+};
+
+const EvalBucket& eval_bucket_of(int M) {
+    for (const EvalBucket& b : kEvalBuckets)
+        if (M <= b.m_max) return b;
+    return kEvalBuckets[sizeof(kEvalBuckets) / sizeof(kEvalBuckets[0]) - 1];
 }
 
 // CTA plan of the eval kernel: NW warps per CTA, `chunk` candidates per CTA.  NW = 7 runs four
 // resident CTAs per SM (72 registers, 28 warps), NW = 8 three (80 registers, 24 warps); besides
 // exact divisibility (no idle warp in the last round of a CTA) the choice minimises the number
 // of CTA waves, which is what decides the latency of one dense query.
-#ifndef EVAL_ITEM
-#define EVAL_ITEM 4
-#endif
+constexpr int EVAL_ITEM = 4;   // candidates a warp takes at a time to share their Newton solves
 struct CtaPlan {
     int nw, chunk, ctas_per_scn;
 };
@@ -388,18 +361,13 @@ CtaPlan plan_ctas(int n_cand, int S, int M, int sm_count, bool cubic) {
     {
         const int full4 = ((n_cand + 3) / 4) * 4;
         if (cubic && M <= 128 && full4 >= 4 * EVAL_ITEM && n_cand <= 256 &&
-            (long long)S >= 8LL * eval_minb(4, M) * sm_count)
+            (long long)S >= 8LL * eval_bucket_of(M).nw4.minb * sm_count)
             return CtaPlan{4, full4, 1};
     }
     const int nws[3] = {4, 7, 8};
     for (int nw : nws) {
-#ifdef F1L_FORCE_NW
-        if (nw != F1L_FORCE_NW) continue;
-#endif
-#ifndef F1L_ALLOW_SMALL_NW_BIG_M
         if (nw != 8 && M > 128) continue;   // the 72-register builds of the M = 200 shapes spill
-#endif
-        const int resident = eval_minb(nw, M) * sm_count;
+        const int resident = eval_bucket_of(M).build(nw).minb * sm_count;
         const int full = ((n_cand + nw - 1) / nw) * nw;   // one CTA per scenario
         // chunk sizes worth a look: enough CTAs for ~8 waves (dense single queries), the smallest
         // chunk whose warps share Newton solves, and the whole scenario in one CTA
@@ -492,16 +460,6 @@ void launch_pp(const TrackView& tv, cudaStream_t stream, const double* poses, in
         tv, poses, pose_stride, n_poses, L, wb, max_reacquire, front_axle, k_path, key, o);
 }
 
-size_t eval_smem_bytes(int nseg_pad, int warps, int M) {   // mirrors EvalSmem (f1l_lattice.cuh)
-    const EvalShape sh = eval_shape(M);
-    const size_t pcap = (size_t)sh.s * sh.sg, slab = (size_t)((sh.s + 1) / 2) * sh.sg * 2;
-    size_t b = (size_t)warps * (pcap * 32 + 128 + 2 * slab * 4);               // per-warp blocks
-    b += F1L_MAX_OPP * sizeof(float4) + 48;                                    // opponents, grid constants
-    b += (size_t)F1L_MAX_M * sizeof(float);                                    // previous path
-    b += (size_t)(nseg_pad + EVAL_SEG_PAD) * (2 * sizeof(float4));             // window table
-    return b;
-}
-
 struct BatchOut {
     int32_t* best_idx = nullptr;
     float* best_cost = nullptr;
@@ -591,13 +549,13 @@ int launch_pipeline(f1l_handle h, cudaStream_t stream, const double* poses, cons
     const int n_cand = o.empty_shard ? 1 : c_end - c_begin;
     const CtaPlan cp = plan_ctas(n_cand, S, M, h->sm_count, ep.generator == 0);
     const int wpc = cp.nw;
-    const size_t smem = eval_smem_bytes(nseg_pad, wpc, M);
-    if (smem > 226 * 1024) return F1L_ERR_TOO_LARGE;
+    const EvalBucket& bucket = eval_bucket_of(M);
+    const EvalBuild* build = &bucket.build(wpc);
     // A lone dense query that needs more than one wave of CTAs runs on a PERSISTENT grid instead: one
     // wave of CTAs whose warps pull single candidates from a device-wide counter, far lookahead rows
     // (the expensive candidates) first.  No wave quantisation, one window-table prologue per
     // resident CTA, and the cheap early-exit candidates fill the tail.
-    int resident_ctas = eval_minb(wpc, M) * h->sm_count;
+    int resident_ctas = build->minb * h->sm_count;
     // F1L_EVAL_DYNAMIC: 0 = never, 2 = whenever the query has more than one CTA (sanitizer runs at
     // small sizes), default = when it needs more than one wave
     static const int dyn_mode = getenv("F1L_EVAL_DYNAMIC") ? atoi(getenv("F1L_EVAL_DYNAMIC")) : 1;
@@ -607,9 +565,14 @@ int launch_pipeline(f1l_handle h, cudaStream_t stream, const double* poses, cons
     // 128-register build of the M > 128 shapes on two CTAs per SM (measured on config 5: 65 536
     // candidates 471 -> 431 us, 32 768: 247 -> 234, 16 384: 134 -> 128, 8 192: 76 -> 100)
     static const int wide_min = getenv("F1L_EVAL_WIDE_MIN") ? atoi(getenv("F1L_EVAL_WIDE_MIN")) : 4;
-    const bool wide = dyn && wpc == 8 && M > 128 && wide_min > 0 &&
+    const bool wide = dyn && wpc == 8 && bucket.wide.fn && wide_min > 0 &&
                       (long long)n_cand >= (long long)wide_min * resident_ctas * wpc;
-    if (wide) resident_ctas = EVAL_MINB8_WIDE * h->sm_count;
+    if (wide) {
+        build = &bucket.wide;
+        resident_ctas = build->minb * h->sm_count;
+    }
+    const size_t smem = build->smem_bytes(nseg_pad);
+    if (smem > 226 * 1024) return F1L_ERR_TOO_LARGE;
 
     SampleArgs sa;
     sa.tr = track_view(h);
@@ -704,19 +667,16 @@ int launch_pipeline(f1l_handle h, cudaStream_t stream, const double* poses, cons
     ea.stats = h->stats_on ? (unsigned long long*)h->stats.p : nullptr;
     const long long n_ctas = (long long)S * ea.ctas_per_scn;
     if (n_ctas > 0x7fffffffLL) return F1L_ERR_TOO_LARGE;
-    if (!o.empty_shard) (wide ? eval_entry_wide(M) : eval_entry(M, wpc))<<<(unsigned)n_ctas, wpc * 32, smem, stream>>>(ea);
+    if (!o.empty_shard) build->fn<<<(unsigned)n_ctas, wpc * 32, smem, stream>>>(ea);
     {
-        const EvalShape sh = eval_shape(M);
-        const int info[8] = {sh.ipl, sh.s, sh.sg, wpc,
-                             wide ? EVAL_MINB8_WIDE : eval_minb(wpc, M),
-                             ea.chunk, ea.ctas_per_scn, ea.item};
+        const int info[8] = {bucket.ipl, bucket.s, bucket.sg, wpc, build->minb, ea.chunk, ea.ctas_per_scn, ea.item};
         for (int i = 0; i < 8; ++i) h->eval_info[i] = info[i];
     }
     if (time_it) cudaEventRecord(ev[2], stream);
 
     const SelectArgs se = select_args(h, sa.tr, ea.lut, ep, ctx, centres, goals, C,
                                       o.row_step > 1 ? c_begin + o.row0 * h->nW : c_begin, best, S, o);
-    select_entry(M)<<<S, SELECT_THREADS, 0, stream>>>(se);
+    bucket.select<<<S, SELECT_THREADS, 0, stream>>>(se);
     if (time_it) {
         cudaEventRecord(ev[3], stream);
         h->timed = 1;
@@ -948,15 +908,8 @@ int f1l_create(f1l_handle* out, int device, const f1l_config* cfg) {
         e = cudaStreamCreateWithFlags(&h->pipe[i].stream, cudaStreamNonBlocking);
         if (e == cudaSuccess) e = cudaEventCreateWithFlags(&h->pipe[i].done, cudaEventDisableTiming);
     }
-    if (e == cudaSuccess) e = cudaHostAlloc(&h->h_in, 1024, cudaHostAllocMapped);
-    if (e == cudaSuccess) {
-        memset(h->h_in, 0, 1024);
-        static const bool in_off = !getenv("F1L_DIRECT_IN") || atoi(getenv("F1L_DIRECT_IN")) == 0;
-        if (in_off || cudaHostGetDevicePointer(&h->h_in_dev, h->h_in, 0) != cudaSuccess) {
-            h->h_in_dev = nullptr;
-            cudaGetLastError();
-        }
-    }
+    if (e == cudaSuccess) e = cudaHostAlloc(&h->h_in, 1024, cudaHostAllocDefault);
+    if (e == cudaSuccess) memset(h->h_in, 0, 1024);
     if (e == cudaSuccess) {
         h->h_out_cap = Q_RES_BYTES;
         e = cudaHostAlloc(&h->h_out, h->h_out_cap, cudaHostAllocMapped);
@@ -973,20 +926,14 @@ int f1l_create(f1l_handle* out, int device, const f1l_config* cfg) {
         int sm = 0;
         cudaDeviceGetAttribute(&sm, cudaDevAttrMultiProcessorCount, device);
         if (sm > 0) h->sm_count = sm;
-        // opt in to large dynamic shared memory for every eval instantiation + the scan kernel
+        // opt in to large dynamic shared memory for every eval instantiation
         const int big = 226 * 1024;  // opt-in maximum is 227 KB per block INCLUDING static shared memory
-        const int nws[3] = {4, 7, 8};
-        for (int nw : nws) {
-            const int ms[] = {32, 64, 100, 128, 200, 256};
-            for (int m : ms) {
-                cudaError_t e2 = cudaFuncSetAttribute(
-                    eval_entry(m, nw), cudaFuncAttributeMaxDynamicSharedMemorySize, big);
+        for (const EvalBucket& b : kEvalBuckets) {
+            for (const EvalBuild* eb : {&b.nw4, &b.nw7, &b.nw8, &b.wide}) {
+                if (!eb->fn) continue;
+                cudaError_t e2 = cudaFuncSetAttribute(eb->fn, cudaFuncAttributeMaxDynamicSharedMemorySize, big);
                 if (e2 != cudaSuccess && e == cudaSuccess) e = e2;
             }
-        }
-        for (int m : {200, 256}) {
-            cudaError_t e2 = cudaFuncSetAttribute(eval_entry_wide(m), cudaFuncAttributeMaxDynamicSharedMemorySize, big);
-            if (e2 != cudaSuccess && e == cudaSuccess) e = e2;
         }
     }
     if (e != cudaSuccess) {
@@ -1354,13 +1301,12 @@ static int plan_internal(f1l_handle h, const double pose[4], const double* opp, 
     const bool sharded = exchange || row_step > 1 || c_begin != 0 || (c_end > 0 && c_end < C);
     QHeader* hd = (QHeader*)h->h_out;
     float* htraj = (float*)((char*)h->h_out + sizeof(QHeader));
-    const bool direct_in = h->h_in_dev != nullptr;
-    const QInput* din = direct_in ? (const QInput*)h->h_in_dev : (const QInput*)h->q_in.p;
+    const QInput* din = (const QInput*)h->q_in.p;
     // H2D of the input block, the three kernels, D2H of header + best trajectory.  The
     // similarity term reads the previous path while select overwrites it: eval reads it before
     // select runs (stream order), so one buffer suffices.
     auto enqueue = [&](bool time_it) -> int {
-        if (!direct_in) CK(cudaMemcpyAsync(h->q_in.p, hin, sizeof(QInput), cudaMemcpyHostToDevice, st));
+        CK(cudaMemcpyAsync(h->q_in.p, hin, sizeof(QInput), cudaMemcpyHostToDevice, st));
         if (sharded && want_detail) {
             // sharded evaluation: untouched candidates keep +inf / zero flags (only when the
             // per-candidate arrays travel back at all)
@@ -1502,7 +1448,7 @@ int f1l_select_candidate(f1l_handle h, int idx, float cost, int update_prev, f1l
                                       (const QueryCtx*)h->q_ctx.p, (const Centre*)h->q_centres.p,
                                       h->lastq_goals ? (const float4*)h->q_goals.p : nullptr, C, 0,
                                       (const unsigned long long*)h->q_best.p, 1, o);
-    select_entry(M)<<<1, SELECT_THREADS, 0, st>>>(se);
+    eval_bucket_of(M).select<<<1, SELECT_THREADS, 0, st>>>(se);
     h->launches += 1;
     CK(cudaGetLastError());
     CK(cudaMemcpyAsync(h->h_out, dres, Q_OFF_TRAJ + (size_t)M * 16, cudaMemcpyDeviceToHost, st));
@@ -1605,7 +1551,7 @@ int f1l_generate(f1l_handle h, const double* goals, int n_goals, float* states, 
     cudaStream_t st = h->stream;
     CK(cudaMemcpyAsync(h->q_goals.p, g4.data(), (size_t)C * 16, cudaMemcpyHostToDevice, st));
     const int wpc = 8;
-    generate_entry(M)<<<(C + wpc - 1) / wpc, wpc * 32, 0, st>>>(
+    eval_bucket_of(M).generate<<<(C + wpc - 1) / wpc, wpc * 32, 0, st>>>(
         lut_view(h), eval_params(h), (const float4*)h->q_goals.p, C, (float4*)h->q_states.p,
         (float4*)h->q_params.p, (uint8_t*)h->q_flags.p);
     h->launches += 1;

@@ -482,23 +482,13 @@ __device__ __forceinline__ f32x2 ffma2(f32x2 a, f32x2 b, f32x2 c) {
     asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(d) : "l"(a), "l"(b), "l"(c));
     return d;
 }
-__device__ __forceinline__ f32x2 fadd2(f32x2 a, f32x2 b) {
-    f32x2 d;
-    asm("add.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b));
-    return d;
-}
 __device__ __forceinline__ f32x2 fmul2(f32x2 a, f32x2 b) {
     f32x2 d;
     asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b));
     return d;
 }
 
-// three-input max / min (sm_100 FMNMX3, one ALU-pipe instruction)
-__device__ __forceinline__ float fmax3(float a, float b, float c) {
-    float r;
-    asm("max.f32 %0, %1, %2, %3;" : "=f"(r) : "f"(a), "f"(b), "f"(c));
-    return r;
-}
+// three-input min (sm_100 FMNMX3, one ALU-pipe instruction)
 __device__ __forceinline__ float fmin3(float a, float b, float c) {
     float r;
     asm("min.f32 %0, %1, %2, %3;" : "=f"(r) : "f"(a), "f"(b), "f"(c));

@@ -747,101 +747,48 @@ __device__ __forceinline__ float fast_sqrt(float x) {
     return r;
 }
 
-// deviation-loop variant: how |e| = |q - clamp(q, 0, len)| is formed
-//   0  e = q - sat(q / len) * len        FMUL.SAT + FFMA2: 8 FMA-pipe cycles per sample x segment
-//   1  e = q - min(max(q, 0), len)       two FMNMX + FADD2: 7 FMA-pipe, 3 ALU instructions
-//   2  e = max(-q, q - len, 0)           FADD2 + one three-input FMNMX3 (sm_100): 7 FMA-pipe, 2 ALU
-//   3  e = sat(|q - h| - h), h = len/2   one FADD.SAT with an |.| operand modifier: 7 FMA-pipe, no
-//                                        ALU instruction and the fewest register-operand reads.
-//                                        The table holds q's constant with h folded in, and all
-//                                        lengths in units of EVAL_DEV_UNIT metres so that the
-//                                        saturation (clamp to [0, 1]) only ever acts at 0.
+// Raceline deviation: distance of a sample to one window segment in line form.  The segment's
+// table entry is T0 = (ux, uy, -uy, 1/len), T1 = (-(a.u + h), -a.n, -h, 0) with h = len / 2, so
+// that q = p.u - (a.u + h) is measured from the segment's midpoint and n = p.n - a.n; the
+// distance beyond the segment's ends is
+//   e = sat(|q| - h)
+// and d^2 = e^2 + n^2 (nearest_point, utils.py:53-65, without the division and the square root).
+// (Nothing reads T0.w; the entry keeps it.)  e is one FADD.SAT with an |.| operand modifier: no ALU instruction and the fewest
+// register-operand reads of the formulations measured (DESIGN §8, profiles/r2_microbench.md).
 // The loop is bound by register-file operand bandwidth (about two 32-bit operands per lane per
 // clock, measured: tools/microbench/rf_bench.cu), not by the FMA pipe, so operand reads count.
-#ifndef EVAL_DEV_MODE
-#define EVAL_DEV_MODE 3
-#endif
-// order of the packed instructions of one segment step: 0 = sample pair after sample pair,
-// 1 = operation-major over groups of EVAL_DEV_GROUP pairs (consecutive instructions share their segment
-// constants, which then come from the operand reuse cache instead of the register file)
-#ifndef EVAL_DEV_ORDER
-#define EVAL_DEV_ORDER 1
-#endif
-#define EVAL_DEV_UNIT 16384.0f   // metres per table unit (a power of two: the scaling is exact)
-#if EVAL_DEV_MODE == 3
-#define EVAL_DEV_SCALE (1.0f / EVAL_DEV_UNIT)
-#else
-#define EVAL_DEV_SCALE 1.0f
-#endif
-// segments per trip of the deviation loop: 0 = one (FMNMX per sample), 1 / 2 = two, the running
-// minimum taking both distances in one FMNMX3 (1: next trip's table entries prefetched into
-// registers, 2: loaded at the end of the trip -- fewer live registers, measured faster)
-#ifndef EVAL_DEV_MIN3
-#define EVAL_DEV_MIN3 2
-#endif
-#ifndef EVAL_SEG_UNROLL
-#define EVAL_SEG_UNROLL 2
-#endif
+// Samples and table hold all lengths in units of EVAL_DEV_UNIT metres so that the saturation
+// (clamp to [0, 1]) only ever acts at 0.
+constexpr float EVAL_DEV_UNIT = 16384.0f;   // metres per table unit (a power of two: the scaling is exact)
+constexpr float EVAL_DEV_SCALE = 1.0f / EVAL_DEV_UNIT;
 #define EVAL_SEG_PAD 32   // readable slack behind the window tables (software-pipelined loads)
 
-// |e| of a packed pair from its q (see the mode table above)
-__device__ __forceinline__ f32x2 seg_axis_excess(f32x2 q2, const float4& T0, const float4& T1) {
+// e of a packed pair from its q
+__device__ __forceinline__ f32x2 seg_axis_excess(f32x2 q2, const float4& T1) {
     float qa, qb;
     unpack2(q2, qa, qb);
-#if EVAL_DEV_MODE == 3
     return pack2(__saturatef(fabsf(qa) + T1.z), __saturatef(fabsf(qb) + T1.z));
-#elif EVAL_DEV_MODE == 2
-    float ra, rb;
-    unpack2(fadd2(q2, pack2(T1.z, T1.z)), ra, rb);
-    return pack2(fmax3(-qa, ra, 0.0f), fmax3(-qb, rb, 0.0f));
-#elif EVAL_DEV_MODE == 1
-    return fadd2(q2, pack2(-fminf(fmaxf(qa, 0.0f), -T1.z), -fminf(fmaxf(qb, 0.0f), -T1.z)));
-#else
-    return ffma2(pack2(__saturatef(qa * T0.w), __saturatef(qb * T0.w)), pack2(T1.z, T1.z), q2);
-#endif
 }
 
-// squared distance of a packed pair of samples (sx, sy) to one window segment in line form
-// T0 = (ux, uy, -uy, 1/len), T1 = (-a.u, -a.n, -len, 0):  q = p.u - a.u, n = p.n - a.n,
-// e = distance of q to [0, len], d^2 = e^2 + n^2  (nearest_point, utils.py:53-65, without the
-// division and the square root).  Segment constants enter FFMA2 as scalar-broadcast operands.
-// Mode 3: T1 = (-(a.u + h), -a.n, -h, 0) with h = len / 2, samples and T1 in table units.
-__device__ __forceinline__ f32x2 seg_dist2_pair(f32x2 sx, f32x2 sy, const float4& T0,
-                                                const float4& T1) {
-    const f32x2 ux = pack2(T0.x, T0.x), uy = pack2(T0.y, T0.y);
-    const f32x2 nuy = pack2(T0.z, T0.z), nc = pack2(T1.x, T1.x);
-    const f32x2 ne = pack2(T1.y, T1.y);
-    const f32x2 q2 = ffma2(sx, ux, ffma2(sy, uy, nc));
-    const f32x2 n2 = ffma2(sy, ux, ffma2(sx, nuy, ne));
-    const f32x2 e2 = seg_axis_excess(q2, T0, T1);
-    return ffma2(e2, e2, fmul2(n2, n2));
-}
+// squared distance of one sample (sx, sy) to one window segment (table units)
 __device__ __forceinline__ float seg_dist2(float sx, float sy, const float4& T0, const float4& T1) {
     const float qq = fmaf(sx, T0.x, fmaf(sy, T0.y, T1.x));
     const float nn = fmaf(sy, T0.x, fmaf(sx, T0.z, T1.y));
-#if EVAL_DEV_MODE == 3
     const float e = __saturatef(fabsf(qq) + T1.z);
-#elif EVAL_DEV_MODE == 2
-    const float e = fmax3(-qq, qq + T1.z, 0.0f);
-#elif EVAL_DEV_MODE == 1
-    const float e = qq - fminf(fmaxf(qq, 0.0f), -T1.z);
-#else
-    const float e = fmaf(__saturatef(qq * T0.w), T1.z, qq);
-#endif
     return fmaf(e, e, nn * nn);
 }
 
-// squared distances of the sample pairs [J0, J0 + EVAL_DEV_GROUP) of a lane to one segment
-// (pairs per operation-major group, re-measured with the batch shape at 125 registers: 2 gives
-//  10.76 ms against 10.83 on the full scan but 6.50 against 6.35 with prune_window = 1; 6: 10.88)
-#ifndef EVAL_DEV_GROUP
-#define EVAL_DEV_GROUP 3
-#endif
+// Squared distances of the sample pairs [J0, J0 + EVAL_DEV_GROUP) of a lane to one segment, on
+// packed FP32x2 instructions whose segment constants enter as scalar-broadcast operands, in
+// operation-major order: consecutive instructions share their segment constants, which then come
+// from the operand reuse cache instead of the register file.  (Pairs per group, re-measured with
+// the batch shape at 125 registers: 2 gives 10.76 ms against 10.83 on the full scan but 6.50
+// against 6.35 with prune_window = 1; 6: 10.88.)
+constexpr int EVAL_DEV_GROUP = 3;
 template <int SP, int J0>
 __device__ __forceinline__ void seg_group(const f32x2 (&sx2)[SP], const f32x2 (&sy2)[SP],
                                           const float4& T0, const float4& T1,
                                           f32x2 (&d)[EVAL_DEV_GROUP]) {
-#if EVAL_DEV_ORDER == 1
     const f32x2 ux = pack2(T0.x, T0.x), uy = pack2(T0.y, T0.y);
     const f32x2 nuy = pack2(T0.z, T0.z), nc = pack2(T1.x, T1.x), ne = pack2(T1.y, T1.y);
     f32x2 q[EVAL_DEV_GROUP], n[EVAL_DEV_GROUP], e[EVAL_DEV_GROUP];
@@ -854,38 +801,15 @@ __device__ __forceinline__ void seg_group(const f32x2 (&sx2)[SP], const f32x2 (&
 #pragma unroll
     for (int j = 0; j < EVAL_DEV_GROUP; ++j) if (J0 + j < SP) n[j] = ffma2(sy2[J0 + j], ux, n[j]);
 #pragma unroll
-    for (int j = 0; j < EVAL_DEV_GROUP; ++j) if (J0 + j < SP) e[j] = seg_axis_excess(q[j], T0, T1);
+    for (int j = 0; j < EVAL_DEV_GROUP; ++j) if (J0 + j < SP) e[j] = seg_axis_excess(q[j], T1);
 #pragma unroll
     for (int j = 0; j < EVAL_DEV_GROUP; ++j) if (J0 + j < SP) n[j] = fmul2(n[j], n[j]);
 #pragma unroll
     for (int j = 0; j < EVAL_DEV_GROUP; ++j) if (J0 + j < SP) d[j] = ffma2(e[j], e[j], n[j]);
-#else
-#pragma unroll
-    for (int j = 0; j < EVAL_DEV_GROUP; ++j)
-        if (J0 + j < SP) d[j] = seg_dist2_pair(sx2[J0 + j], sy2[J0 + j], T0, T1);
-#endif
 }
 
-// running minima of all SP sample pairs of a lane over one segment (A) or two (A and B: the
-// minimum takes both distances in one three-input FMNMX3)
-template <int SP, int J0 = 0>
-__device__ __forceinline__ void seg_min1(const f32x2 (&sx2)[SP], const f32x2 (&sy2)[SP],
-                                         const float4& A0, const float4& A1, float (&bdx)[SP],
-                                         float (&bdy)[SP]) {
-    if constexpr (J0 < SP) {
-        f32x2 dA[EVAL_DEV_GROUP];
-        seg_group<SP, J0>(sx2, sy2, A0, A1, dA);
-#pragma unroll
-        for (int j = 0; j < EVAL_DEV_GROUP; ++j)
-            if (J0 + j < SP) {
-                float da, db;
-                unpack2(dA[j], da, db);
-                bdx[J0 + j] = fminf(bdx[J0 + j], da);
-                bdy[J0 + j] = fminf(bdy[J0 + j], db);
-            }
-        seg_min1<SP, J0 + EVAL_DEV_GROUP>(sx2, sy2, A0, A1, bdx, bdy);
-    }
-}
+// running minima of all SP sample pairs of a lane over two segments A and B: the minimum takes
+// both distances in one three-input FMNMX3
 template <int SP, int J0 = 0>
 __device__ __forceinline__ void seg_min2(const f32x2 (&sx2)[SP], const f32x2 (&sy2)[SP],
                                          const float4& A0, const float4& A1, const float4& B0,
@@ -937,8 +861,8 @@ __device__ __forceinline__ float halve_min_sqrt_sum(float (&v)[N], int lane_in_g
     }
 }
 
-// Shared-memory layout of eval_kernel (bytes; the host's eval_smem_bytes mirrors it).  Per warp one
-// contiguous block -- list of the footprints that need their nine grid probes (centre and half-axes
+// Shared-memory layout of eval_kernel (bytes; the host sizes a launch as C_TAB plus the window
+// table's (nseg_pad + EVAL_SEG_PAD) x 32 bytes).  Per warp one contiguous block -- list of the footprints that need their nine grid probes (centre and half-axes
 // in grid-cell coordinates, two float4 per entry) | solutions of the four candidates of an item
 // ((gx, gy, gth, p3), (p1, p2, sf, have | passes)) | sample slab x | sample slab y, in the pair
 // layout of the deviation pass: element (j, sg, half) holds sample (2j + half) * SG + sg, so that
@@ -968,7 +892,6 @@ struct EvalSmem {
 template <int IPL, int S, int SG, int NW, int MINB>
 __global__ void __launch_bounds__(NW * 32, MINB) eval_kernel(EvalArgs a) {
     constexpr int GG = 32 / SG;
-    constexpr int kSegUnroll = EVAL_SEG_UNROLL;
     using L = EvalSmem<S, SG, NW>;
     extern __shared__ __align__(16) unsigned char ev_smem[];
     __shared__ int s_next;
@@ -1010,11 +933,7 @@ __global__ void __launch_bounds__(NW * 32, MINB) eval_kernel(EvalArgs a) {
         const int seg0 = q->seg0, nseg = q->nseg, ns = a.tr.n - 1;
         for (int k = tid; k < ntab; k += NW * 32) {
             float4 T0 = make_float4(1.0f, 0.0f, -0.0f, 1.0f);      // padding: far away, finite
-#if EVAL_DEV_MODE == 3
             float4 T1 = make_float4(-1e9f, -1e9f, -1.0f, 0.0f);    // (table units) d^2 = 1e18
-#else
-            float4 T1 = make_float4(-1e15f, -1e15f, -1.0f, 0.0f);
-#endif
             if (k < nseg) {
                 int sg = seg0 + k;
                 if (sg >= ns) sg -= ns;
@@ -1027,13 +946,9 @@ __global__ void __launch_bounds__(NW * 32, MINB) eval_kernel(EvalArgs a) {
                 const float il = rsqrtf(l2);
                 const float ux = dx * il, uy = dy * il;
                 T0 = make_float4(ux, uy, -uy, il);
-#if EVAL_DEV_MODE == 3
                 const float hh = 0.5f * (l2 * il);
                 T1 = make_float4(-(fmaf(avx, ux, avy * uy) + hh) * EVAL_DEV_SCALE,
                                  -fmaf(avy, ux, -avx * uy) * EVAL_DEV_SCALE, -hh * EVAL_DEV_SCALE, 0.0f);
-#else
-                T1 = make_float4(-fmaf(avx, ux, avy * uy), -fmaf(avy, ux, -avx * uy), -(l2 * il), 0.0f);
-#endif
             }
             sts128(cbase + L::C_TAB + k * 32, T0);
             sts128(cbase + L::C_TAB + k * 32 + 16, T1);
@@ -1388,10 +1303,7 @@ __global__ void __launch_bounds__(NW * 32, MINB) eval_kernel(EvalArgs a) {
                 // the upper half segment B, each from its own table address (one extra LDS.128
                 // pair per trip instead of a second 7-instruction scalar chain), and the two
                 // halves' minima meet in one shuffle after the loop.
-#ifndef EVAL_SPLIT_ODD
-#define EVAL_SPLIT_ODD 1
-#endif
-                const bool split_odd = EVAL_SPLIT_ODD && ODD && EVAL_DEV_MIN3 && (M - (S - 1) * SG) <= SG / 2;   // uniform
+                const bool split_odd = ODD && (M - (S - 1) * SG) <= SG / 2;   // uniform
                 if (ODD) {
                     const uint32_t ro = split_odd ? wbase + L::W_SLABX + (sgi & (SG / 2 - 1)) * 8 : ra;
                     sxl = lds32(ro + SP * SG * 8);
@@ -1439,9 +1351,10 @@ __global__ void __launch_bounds__(NW * 32, MINB) eval_kernel(EvalArgs a) {
                 // warp-uniform and lives in a uniform register
                 uint32_t ta = cbase + L::C_TAB + (k_begin + ggi) * 32;
                 float4 T0 = lds128(ta), T1 = lds128(ta + 16);
-#if EVAL_DEV_MIN3
                 // two segments per trip: the running minimum takes both distances in one
-                // three-input FMNMX3 (nseg_pad / GG is a multiple of 8)
+                // three-input FMNMX3 (nseg_pad / GG is a multiple of 8).  The next trip's entries
+                // are loaded at the end of the trip (fewer live registers than a prefetch into
+                // registers at its start, measured faster).
                 if (split_odd) {
                     const uint32_t off = (sgi >= SG / 2) ? GG * 32 : 0;   // this lane's segment of the trip
                     for (int n = (k_end - k_begin) / (2 * GG); n > 0; --n) {
@@ -1454,27 +1367,16 @@ __global__ void __launch_bounds__(NW * 32, MINB) eval_kernel(EvalArgs a) {
                         T1 = lds128(ta + 16);
                     }
                     bdl = fminf(bdl, __shfl_xor_sync(F1L_FULL, bdl, (SG / 2) * GG));
-                } else
-                for (int n = (k_end - k_begin) / (2 * GG); n > 0; --n) {
-                    const float4 B0 = lds128(ta + GG * 32), B1 = lds128(ta + GG * 32 + 16);
-                    seg_min2<SP>(sx2, sy2, T0, T1, B0, B1, bdx, bdy);
-                    if (ODD) bdl = fmin3(bdl, seg_dist2(sxl, syl, T0, T1), seg_dist2(sxl, syl, B0, B1));
-                    ta += 2 * GG * 32;
-                    T0 = lds128(ta);   // EVAL_SEG_PAD entries of slack
-                    T1 = lds128(ta + 16);
+                } else {
+                    for (int n = (k_end - k_begin) / (2 * GG); n > 0; --n) {
+                        const float4 B0 = lds128(ta + GG * 32), B1 = lds128(ta + GG * 32 + 16);
+                        seg_min2<SP>(sx2, sy2, T0, T1, B0, B1, bdx, bdy);
+                        if (ODD) bdl = fmin3(bdl, seg_dist2(sxl, syl, T0, T1), seg_dist2(sxl, syl, B0, B1));
+                        ta += 2 * GG * 32;
+                        T0 = lds128(ta);   // EVAL_SEG_PAD entries of slack
+                        T1 = lds128(ta + 16);
+                    }
                 }
-#else
-#pragma unroll kSegUnroll
-                for (int n = (k_end - k_begin) / GG; n > 0; --n) {
-                    const float4 N0 = lds128(ta + GG * 32);       // EVAL_SEG_PAD entries of slack
-                    const float4 N1 = lds128(ta + GG * 32 + 16);
-                    seg_min1<SP>(sx2, sy2, T0, T1, bdx, bdy);
-                    if (ODD) bdl = fminf(bdl, seg_dist2(sxl, syl, T0, T1));
-                    ta += GG * 32;
-                    T0 = N0;
-                    T1 = N1;
-                }
-#endif
                 // Minima over the GG lanes of a sample group, by halving: at every step a lane keeps
                 // one half of its rows and hands the other half to its partner, so it ends with S / GG
                 // fully reduced rows of its own (7 + 4 shuffles and 4 square roots for S = 13, GG = 4,
