@@ -79,6 +79,10 @@ SIGNATURES = {
                                      _vp, _vp, _vp]),
     "f1l_plan_batch": (C.c_int, [_vp, _vp, _vp, _vp, C.c_int, C.c_int, _vp, _vp, _vp, _vp, _vp,
                                  _vp]),
+    "f1l_plan_batch_prev_dev": (C.c_int, [_vp, _vp, _vp, _vp, C.c_int, C.c_int, _vp, _vp, C.c_int,
+                                          _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "f1l_plan_batch_prev": (C.c_int, [_vp, _vp, _vp, _vp, C.c_int, C.c_int, _vp, _vp, C.c_int,
+                                      _vp, _vp, _vp, _vp, _vp, _vp]),
     "f1l_pure_pursuit_batch_dev": (C.c_int, [_vp, _vp, C.c_int, C.c_double, _vp, _vp, _vp, _vp,
                                              _vp, _vp, _vp]),
     "f1l_pure_pursuit_batch": (C.c_int, [_vp, _vp, C.c_int, C.c_double, _vp, _vp, _vp, _vp, _vp,

@@ -41,6 +41,7 @@ struct PipeSlot {
     cudaStream_t stream = nullptr;
     cudaEvent_t done = nullptr;
     DevBuf poses, opp, nopp, ctx, centres, best, idx, cost, traj, costs, flags, ss, near_i, near4;
+    DevBuf prev, pvalid;   // the chunk's previous paths [n,M] f32 and their flags [n] u8
 };
 
 }  // namespace
@@ -474,7 +475,8 @@ struct BatchOut {
     float4* params = nullptr;
     float4* states = nullptr;
     float2* headings = nullptr;
-    float* prev_out = nullptr;
+    float* prev_out = nullptr;         // [S,M] theta column of each best trajectory (update_prev)
+    uint8_t* prev_valid_out = nullptr; // [S] set to 1 with it (per-scenario previous paths)
     int row0 = 0, row_step = 1;        // row-interleaved shard (c_begin / c_end are shard-local)
     const XchgView* xc = nullptr;      // sharded single query: exchange the argmin with the peers
     int32_t* xchg_status = nullptr;
@@ -516,15 +518,19 @@ SelectArgs select_args(f1l_handle h, const TrackView& tv, const LutView& lut, co
     se.best_traj = o.best_traj;
     se.best_traj_map = o.best_traj_map;
     se.prev_theta_out = o.prev_out;
+    se.prev_valid_out = o.prev_valid_out;
     return se;
 }
 
-// sampler -> eval -> select for S scenarios on `stream`; all pointers are device pointers
+// sampler -> eval -> select for S scenarios on `stream`; all pointers are device pointers.
+// Previous paths: scenario s reads prev_theta + s * prev_stride (stride 0: one path for all) when
+// prev_valid is null or prev_valid[s] != 0; prev_theta null: no similarity term.
 int launch_pipeline(f1l_handle h, cudaStream_t stream, const double* poses, const double* opp,
                     const int32_t* n_opp, int S, int max_opp, const float4* goals, int n_goals,
                     int c_begin, int c_end, QueryCtx* ctx, Centre* centres,
                     unsigned long long* best, int32_t* near_i, double* near4,
-                    const float* prev_theta, const BatchOut& o, bool time_it) {
+                    const float* prev_theta, int prev_stride, const uint8_t* prev_valid,
+                    const BatchOut& o, bool time_it) {
     if (h->n < 2) return F1L_ERR_NO_TRACK;
     const int C = goals ? n_goals : h->nL * h->nW;
     if (C <= 0) return F1L_ERR_NO_GOALS;
@@ -635,6 +641,8 @@ int launch_pipeline(f1l_handle h, cudaStream_t stream, const double* poses, cons
     ea.nW = h->nW;
     ea.goals = goals;
     ea.prev_theta = prev_theta;
+    ea.prev_stride = prev_stride;
+    ea.prev_valid = prev_valid;
     ea.C = C;
     ea.c_begin = c_begin;
     ea.c_end = c_end;
@@ -968,7 +976,7 @@ int f1l_destroy(f1l_handle h) {
     for (int i = 0; i < N_PIPE; ++i) {
         PipeSlot& p = h->pipe[i];
         DevBuf* pb[] = {&p.poses, &p.opp, &p.nopp, &p.ctx, &p.centres, &p.best, &p.idx, &p.cost,
-                        &p.traj, &p.costs, &p.flags, &p.ss, &p.near_i, &p.near4};
+                        &p.traj, &p.costs, &p.flags, &p.ss, &p.near_i, &p.near4, &p.prev, &p.pvalid};
         for (DevBuf* b : pb) release(*b);
         if (p.done) cudaEventDestroy(p.done);
         if (p.stream) cudaStreamDestroy(p.stream);
@@ -1317,7 +1325,7 @@ static int plan_internal(f1l_handle h, const double pose[4], const double* opp, 
         int r = launch_pipeline(h, st, din->pose, din->opp, &din->n_opp, 1, F1L_MAX_OPP, d_goals, C,
                                 c_begin, c_end, (QueryCtx*)h->q_ctx.p, (Centre*)h->q_centres.p,
                                 (unsigned long long*)h->q_best.p, nullptr, nullptr,
-                                h->has_prev ? (const float*)h->prev.p : nullptr, o, time_it);
+                                h->has_prev ? (const float*)h->prev.p : nullptr, 0, nullptr, o, time_it);
         if (r != F1L_OK) return r;
         if (!direct) {
             CK(cudaMemcpyAsync(hd, h->q_res.p, sizeof(QHeader) + (size_t)M * 16, cudaMemcpyDeviceToHost, st));
@@ -1564,12 +1572,18 @@ int f1l_generate(f1l_handle h, const double* goals, int n_goals, float* states, 
 }
 
 // ---- batch --------------------------------------------------------------------------------
-int f1l_plan_batch_dev(f1l_handle h, const double* poses_dev, const double* opp_dev,
-                       const int32_t* n_opp_dev, int S, int max_opp, int32_t* best_idx_dev,
-                       float* best_cost_dev, float* best_traj_dev, float* costs_dev,
-                       uint8_t* flags_dev, double* steer_speed_dev, void* stream) {
+// prev_theta [S,M] / has_prev [S] (nullable): per-scenario previous paths.  With update_prev the
+// select kernel overwrites them in place with each scenario's best trajectory.  That is safe:
+// eval_kernel reads a scenario's path in its prologue, and select_kernel writes it in a later
+// kernel on the same stream.
+static int plan_batch_dev_internal(f1l_handle h, const double* poses_dev, const double* opp_dev,
+                                   const int32_t* n_opp_dev, int S, int max_opp, float* prev_theta_dev,
+                                   uint8_t* has_prev_dev, int update_prev, int32_t* best_idx_dev,
+                                   float* best_cost_dev, float* best_traj_dev, float* costs_dev,
+                                   uint8_t* flags_dev, double* steer_speed_dev, void* stream) {
     if (!h || !poses_dev || S <= 0) return F1L_ERR_INVALID_ARG;
     if (max_opp > 0 && !opp_dev) return F1L_ERR_INVALID_ARG;
+    if ((update_prev || has_prev_dev) && !prev_theta_dev) return F1L_ERR_INVALID_ARG;
     CK(cudaSetDevice(h->device));
     if (h->nL * h->nW <= 0) return F1L_ERR_NO_GOALS;
     ENS(h->b_ctx, sizeof(QueryCtx) * (size_t)S);
@@ -1584,18 +1598,41 @@ int f1l_plan_batch_dev(f1l_handle h, const double* poses_dev, const double* opp_
     o.costs = costs_dev;
     o.flags = flags_dev;
     o.steer_speed = steer_speed_dev;
+    o.prev_out = update_prev ? prev_theta_dev : nullptr;
+    o.prev_valid_out = update_prev ? has_prev_dev : nullptr;
     return launch_pipeline(h, (cudaStream_t)stream, poses_dev, max_opp > 0 ? opp_dev : nullptr,
                            n_opp_dev, S, max_opp, nullptr, 0, 0, 0, (QueryCtx*)h->b_ctx.p,
                            (Centre*)h->b_centres.p, (unsigned long long*)h->b_best.p,
-                           (int32_t*)h->b_near_i.p, (double*)h->b_near4.p, nullptr, o,
-                           h->timing != 0);
+                           (int32_t*)h->b_near_i.p, (double*)h->b_near4.p, prev_theta_dev,
+                           h->cfg.n_samples, has_prev_dev, o, h->timing != 0);
 }
 
-int f1l_plan_batch(f1l_handle h, const double* poses, const double* opp, const int32_t* n_opp,
-                   int S, int max_opp, int32_t* best_idx, float* best_cost, float* best_traj,
-                   float* costs, uint8_t* flags, double* steer_speed) {
+int f1l_plan_batch_dev(f1l_handle h, const double* poses_dev, const double* opp_dev,
+                       const int32_t* n_opp_dev, int S, int max_opp, int32_t* best_idx_dev,
+                       float* best_cost_dev, float* best_traj_dev, float* costs_dev,
+                       uint8_t* flags_dev, double* steer_speed_dev, void* stream) {
+    return plan_batch_dev_internal(h, poses_dev, opp_dev, n_opp_dev, S, max_opp, nullptr, nullptr, 0,
+                                   best_idx_dev, best_cost_dev, best_traj_dev, costs_dev, flags_dev,
+                                   steer_speed_dev, stream);
+}
+
+int f1l_plan_batch_prev_dev(f1l_handle h, const double* poses_dev, const double* opp_dev,
+                            const int32_t* n_opp_dev, int S, int max_opp, float* prev_theta_dev,
+                            uint8_t* has_prev_dev, int update_prev, int32_t* best_idx_dev,
+                            float* best_cost_dev, float* best_traj_dev, float* costs_dev,
+                            uint8_t* flags_dev, double* steer_speed_dev, void* stream) {
+    return plan_batch_dev_internal(h, poses_dev, opp_dev, n_opp_dev, S, max_opp, prev_theta_dev,
+                                   has_prev_dev, update_prev, best_idx_dev, best_cost_dev, best_traj_dev,
+                                   costs_dev, flags_dev, steer_speed_dev, stream);
+}
+
+static int plan_batch_internal(f1l_handle h, const double* poses, const double* opp, const int32_t* n_opp,
+                               int S, int max_opp, float* prev_theta, uint8_t* has_prev, int update_prev,
+                               int32_t* best_idx, float* best_cost, float* best_traj, float* costs,
+                               uint8_t* flags, double* steer_speed) {
     if (!h || !poses || S <= 0) return F1L_ERR_INVALID_ARG;
     if (max_opp > 0 && !opp) return F1L_ERR_INVALID_ARG;
+    if ((update_prev || has_prev) && !prev_theta) return F1L_ERR_INVALID_ARG;
     CK(cudaSetDevice(h->device));
     const int C = h->nL * h->nW;
     if (C <= 0) return F1L_ERR_NO_GOALS;
@@ -1636,11 +1673,16 @@ int f1l_plan_batch(f1l_handle h, const double* poses, const double* opp, const i
         if (costs) ENS(p.costs, (size_t)n * C * 4);
         if (flags) ENS(p.flags, (size_t)n * C);
         if (steer_speed) ENS(p.ss, (size_t)n * 16);
+        if (prev_theta) ENS(p.prev, (size_t)n * M * 4);
+        if (has_prev) ENS(p.pvalid, (size_t)n);
         CK(cudaMemcpyAsync(p.poses.p, poses + 4 * (size_t)s0, (size_t)n * 32, cudaMemcpyHostToDevice, st));
         if (max_opp > 0)
             CK(cudaMemcpyAsync(p.opp.p, opp + 3 * (size_t)max_opp * s0, (size_t)n * max_opp * 24,
                                cudaMemcpyHostToDevice, st));
         if (n_opp) CK(cudaMemcpyAsync(p.nopp.p, n_opp + s0, (size_t)n * 4, cudaMemcpyHostToDevice, st));
+        if (prev_theta)
+            CK(cudaMemcpyAsync(p.prev.p, prev_theta + (size_t)M * s0, (size_t)n * M * 4, cudaMemcpyHostToDevice, st));
+        if (has_prev) CK(cudaMemcpyAsync(p.pvalid.p, has_prev + s0, (size_t)n, cudaMemcpyHostToDevice, st));
         BatchOut o;
         o.best_idx = best_idx ? (int32_t*)p.idx.p : nullptr;
         o.best_cost = best_cost ? (float*)p.cost.p : nullptr;
@@ -1648,12 +1690,16 @@ int f1l_plan_batch(f1l_handle h, const double* poses, const double* opp, const i
         o.costs = costs ? (float*)p.costs.p : nullptr;
         o.flags = flags ? (uint8_t*)p.flags.p : nullptr;
         o.steer_speed = steer_speed ? (double*)p.ss.p : nullptr;
+        // in place on the slot's copies, as in plan_batch_dev_internal
+        o.prev_out = update_prev ? (float*)p.prev.p : nullptr;
+        o.prev_valid_out = update_prev && has_prev ? (uint8_t*)p.pvalid.p : nullptr;
         int r = launch_pipeline(h, st, (const double*)p.poses.p,
                                 max_opp > 0 ? (const double*)p.opp.p : nullptr,
                                 n_opp ? (const int32_t*)p.nopp.p : nullptr, n, max_opp, nullptr, 0,
                                 0, 0, (QueryCtx*)p.ctx.p, (Centre*)p.centres.p,
                                 (unsigned long long*)p.best.p, (int32_t*)p.near_i.p,
-                                (double*)p.near4.p, nullptr, o, false);
+                                (double*)p.near4.p, prev_theta ? (const float*)p.prev.p : nullptr, M,
+                                has_prev ? (const uint8_t*)p.pvalid.p : nullptr, o, false);
         if (r != F1L_OK) return r;
         if (best_idx) CK(cudaMemcpyAsync(best_idx + s0, p.idx.p, (size_t)n * 4, cudaMemcpyDeviceToHost, st));
         if (best_cost) CK(cudaMemcpyAsync(best_cost + s0, p.cost.p, (size_t)n * 4, cudaMemcpyDeviceToHost, st));
@@ -1663,9 +1709,28 @@ int f1l_plan_batch(f1l_handle h, const double* poses, const double* opp, const i
         if (costs) CK(cudaMemcpyAsync(costs + (size_t)C * s0, p.costs.p, (size_t)n * C * 4, cudaMemcpyDeviceToHost, st));
         if (flags) CK(cudaMemcpyAsync(flags + (size_t)C * s0, p.flags.p, (size_t)n * C, cudaMemcpyDeviceToHost, st));
         if (steer_speed) CK(cudaMemcpyAsync(steer_speed + 2 * (size_t)s0, p.ss.p, (size_t)n * 16, cudaMemcpyDeviceToHost, st));
+        if (update_prev) {
+            CK(cudaMemcpyAsync(prev_theta + (size_t)M * s0, p.prev.p, (size_t)n * M * 4, cudaMemcpyDeviceToHost, st));
+            if (has_prev) CK(cudaMemcpyAsync(has_prev + s0, p.pvalid.p, (size_t)n, cudaMemcpyDeviceToHost, st));
+        }
     }
     for (int i = 0; i < N_PIPE; ++i) CK(cudaStreamSynchronize(h->pipe[i].stream));
     return F1L_OK;
+}
+
+int f1l_plan_batch(f1l_handle h, const double* poses, const double* opp, const int32_t* n_opp,
+                   int S, int max_opp, int32_t* best_idx, float* best_cost, float* best_traj,
+                   float* costs, uint8_t* flags, double* steer_speed) {
+    return plan_batch_internal(h, poses, opp, n_opp, S, max_opp, nullptr, nullptr, 0, best_idx, best_cost,
+                               best_traj, costs, flags, steer_speed);
+}
+
+int f1l_plan_batch_prev(f1l_handle h, const double* poses, const double* opp, const int32_t* n_opp,
+                        int S, int max_opp, float* prev_theta, uint8_t* has_prev, int update_prev,
+                        int32_t* best_idx, float* best_cost, float* best_traj, float* costs,
+                        uint8_t* flags, double* steer_speed) {
+    return plan_batch_internal(h, poses, opp, n_opp, S, max_opp, prev_theta, has_prev, update_prev, best_idx,
+                               best_cost, best_traj, costs, flags, steer_speed);
 }
 
 // ---- pure pursuit -------------------------------------------------------------------------

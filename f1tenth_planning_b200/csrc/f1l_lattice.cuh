@@ -340,7 +340,9 @@ struct EvalArgs {
     const float* widths;     // [nW] device
     int nL, nW;
     const float4* goals;     // explicit goals [S,C] (gx, gy, gth, p3) or null
-    const float* prev_theta; // [M] or null
+    const float* prev_theta; // previous path of scenario s at prev_theta + s * prev_stride, or null
+    int prev_stride;         // 0: one [M] path for every scenario (single query), M: [S,M]
+    const uint8_t* prev_valid; // [S]: scenario s has a previous path iff != 0 (null: every one has)
     int C;                   // candidates per scenario
     int c_begin, c_end;      // evaluated range (of shard-local indices when row_step > 1)
     int row0, row_step;      // row-interleaved shard: local index v -> lookahead row
@@ -472,7 +474,8 @@ struct SelectArgs {
     double* steer_speed;    // [S,2]
     float4* best_traj;      // [S,M]
     double* best_traj_map;  // [S,M,4] map frame (X, Y, v, Theta): SURVEY B.8, closed-loop tracking
-    float* prev_theta_out;  // [M] (single query, update_prev)
+    float* prev_theta_out;  // [S,M] theta column of best_traj (update_prev)
+    uint8_t* prev_valid_out; // [S] set to 1 (update_prev with per-scenario flags)
 };
 
 // Candidate index of shard-local index v.  A row-interleaved shard (rank r of W takes lookahead
@@ -880,7 +883,7 @@ struct EvalSmem {
     static constexpr uint32_t W_SLABY = W_SLABX + SLAB * 4;
     static constexpr uint32_t W_BYTES = W_SLABY + SLAB * 4;
     static constexpr uint32_t C_OPP = NW * W_BYTES;                // [F1L_MAX_OPP] float4
-    static constexpr uint32_t C_GRID = C_OPP + F1L_MAX_OPP * 16;   // 3 float4: A, (fx, fy, ix0, iy0), (n_opp, has_grid)
+    static constexpr uint32_t C_GRID = C_OPP + F1L_MAX_OPP * 16;   // 3 float4: A, (fx, fy, ix0, iy0), (n_opp, has_grid, use_prev)
     static constexpr uint32_t C_PREV = C_GRID + 48;                // [F1L_MAX_M] float
     static constexpr uint32_t C_TAB = C_PREV + F1L_MAX_M * 4;      // [ntab][2] float4
     static_assert(W_BYTES % 16 == 0, "per-warp block keeps 16-byte alignment");
@@ -953,9 +956,12 @@ __global__ void __launch_bounds__(NW * 32, MINB) eval_kernel(EvalArgs a) {
             sts128(cbase + L::C_TAB + k * 32, T0);
             sts128(cbase + L::C_TAB + k * 32 + 16, T1);
         }
-        if (a.prev_theta) {
+        // the scenario's previous path (every CTA of a scenario loads its own copy)
+        const bool use_prev = a.prev_theta && (!a.prev_valid || a.prev_valid[s]);
+        if (use_prev) {
+            const float* pt = a.prev_theta + (size_t)s * a.prev_stride;
 #pragma unroll 1
-            for (int i = tid; i < M; i += NW * 32) sts32(cbase + L::C_PREV + i * 4, a.prev_theta[i]);
+            for (int i = tid; i < M; i += NW * 32) sts32(cbase + L::C_PREV + i * 4, pt[i]);
         }
         if (tid < F1L_MAX_OPP)   // unused slots: an opponent far away
             sts128(cbase + L::C_OPP + tid * 16,
@@ -966,7 +972,8 @@ __global__ void __launch_bounds__(NW * 32, MINB) eval_kernel(EvalArgs a) {
         if (tid == 32 % (NW * 32)) {
             sts128(cbase + L::C_GRID, make_float4(q->gA00, q->gA01, q->gA10, q->gA11));
             sts128(cbase + L::C_GRID + 16, make_float4(q->gfx, q->gfy, __int_as_float(q->gix), __int_as_float(q->giy)));
-            sts128(cbase + L::C_GRID + 32, make_float4(__int_as_float(q->n_opp), __int_as_float(q->has_grid), 0.0f, 0.0f));
+            sts128(cbase + L::C_GRID + 32, make_float4(__int_as_float(q->n_opp), __int_as_float(q->has_grid),
+                                                       __int_as_float((int)use_prev), 0.0f));
         }
     }
     __syncthreads();
@@ -1127,6 +1134,7 @@ __global__ void __launch_bounds__(NW * 32, MINB) eval_kernel(EvalArgs a) {
             const float4 GC = lds128(cbase + L::C_GRID + 32);
             const int n_opp = __float_as_int(GC.x);
             const bool has_grid = __float_as_int(GC.y) != 0;
+            const bool use_prev = __float_as_int(GC.z) != 0;
             const float hl = a.ep.half_l, hw = a.ep.half_w;
             const float A00 = GA.x, A01 = GA.y, A10 = GA.z, A11 = GA.w;
             const float gfx = GB.x, gfy = GB.y;
@@ -1160,7 +1168,7 @@ __global__ void __launch_bounds__(NW * 32, MINB) eval_kernel(EvalArgs a) {
                 const float reach = 0.5f * sp.sf + a.ep.reach_pad;
                 opp_mask = __ballot_sync(F1L_FULL, lane < n_opp && fmaf(mx, mx, my * my) <= reach * reach);
             }
-            if (a.prev_theta) {   // uniform
+            if (use_prev) {   // uniform
                 const int lim = M - a.ep.n_shift - a.ep.n_cull;
 #pragma unroll
                 for (int j = 0; j < IPL; ++j) {
@@ -1263,7 +1271,7 @@ __global__ void __launch_bounds__(NW * 32, MINB) eval_kernel(EvalArgs a) {
                     __syncwarp();
                 }
             }
-            if (a.prev_theta) t_sim = warp_sum(sim);
+            if (use_prev) t_sim = warp_sum(sim);
             hit_opp = __any_sync(F1L_FULL, hit_opp);
             hit_map = __any_sync(F1L_FULL, hit_map);
             if (hit_opp) flags |= F1L_FLAG_COLLIDE_OPP;
@@ -1487,9 +1495,10 @@ __global__ void __launch_bounds__(SELECT_THREADS) select_kernel(SelectArgs a) {
             const float4 st = make_float4(x[j], y[j], th[j], kp[j]);
             s_traj[i] = st;
             if (a.best_traj) a.best_traj[(size_t)s * M + i] = st;
-            if (a.prev_theta_out) a.prev_theta_out[i] = th[j];
+            if (a.prev_theta_out) a.prev_theta_out[(size_t)s * M + i] = th[j];
         }
     }
+    if (a.prev_valid_out && lane == 0) a.prev_valid_out[s] = 1;
     if (a.best_traj_map) {   // warp-uniform
         // map-frame copy with a speed column, what a tracker in the map frame consumes (SURVEY B.8):
         // X = pose + R(theta_pose) (x, y), Theta = theta + theta_pose, v = raceline speed at the

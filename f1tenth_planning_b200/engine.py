@@ -268,12 +268,57 @@ class Engine:
         return states, params, (flags & FLAG_VALID) != 0
 
     # -- batch ------------------------------------------------------------------------------
+    def _check_prev(self, S, prev_theta, has_prev, update_prev, is_dev):
+        """Validates the per-scenario previous paths of plan_batch / plan_batch_dev.  They are
+        read and, with update_prev, written in place, so anything that would need a copy (wrong
+        type, shape, dtype, layout or device) is a ValueError rather than a silent conversion."""
+        if prev_theta is None:
+            if has_prev is not None or update_prev:
+                raise ValueError("has_prev / update_prev need prev_theta")
+            return
+        shape = (S, self.n_samples)
+        if is_dev:
+            import torch
+            ok_type = isinstance(prev_theta, torch.Tensor) and prev_theta.is_cuda
+            if not (ok_type and prev_theta.dtype == torch.float32 and tuple(prev_theta.shape) == shape
+                    and prev_theta.is_contiguous() and prev_theta.device.index == self.device):
+                raise ValueError("prev_theta must be a contiguous float32 CUDA tensor [%d, %d] on "
+                                 "cuda:%d" % (S, self.n_samples, self.device))
+            if has_prev is not None and not (
+                    isinstance(has_prev, torch.Tensor) and has_prev.is_cuda
+                    and has_prev.dtype in (torch.uint8, torch.bool) and tuple(has_prev.shape) == (S,)
+                    and has_prev.is_contiguous() and has_prev.device == prev_theta.device):
+                raise ValueError("has_prev must be a contiguous uint8 / bool CUDA tensor [%d] on "
+                                 "prev_theta's device" % S)
+            return
+        if not (isinstance(prev_theta, np.ndarray) and prev_theta.dtype == np.float32
+                and prev_theta.shape == shape and prev_theta.flags.c_contiguous):
+            raise ValueError("prev_theta must be a C-contiguous float32 numpy array [%d, %d]"
+                             % (S, self.n_samples))
+        if has_prev is not None and not (
+                isinstance(has_prev, np.ndarray) and has_prev.dtype in (np.uint8, np.bool_)
+                and has_prev.shape == (S,) and has_prev.flags.c_contiguous):
+            raise ValueError("has_prev must be a contiguous uint8 / bool numpy array [%d]" % S)
+        if update_prev and not (prev_theta.flags.writeable
+                                and (has_prev is None or has_prev.flags.writeable)):
+            raise ValueError("update_prev writes prev_theta / has_prev in place: they must be writeable")
+
     def plan_batch(self, poses, opponents=None, n_opp=None, out=None, want_traj=True,
-                   want_costs=True, want_flags=False):
+                   want_costs=True, want_flags=False, prev_theta=None, has_prev=None,
+                   update_prev=False):
         """S independent scenarios with HOST buffers (numpy; pinned if allocated through
-        ``pinned_empty``).  poses [S,4], opponents [S,K,3], n_opp [S]."""
+        ``pinned_empty``).  poses [S,4], opponents [S,K,3], n_opp [S].
+
+        Previous paths of the similarity cost, one per scenario (f1l_plan_batch_prev):
+        prev_theta [S, n_samples] C-contiguous float32, the theta column of each scenario's
+        previous best trajectory; has_prev [S] bool / uint8 (None: every scenario has one).
+        Scenario s then plans exactly as plan() after set_prev_path(prev_theta[s]) (or
+        set_prev_path(None) where has_prev[s] is 0).  update_prev=True overwrites both arrays in
+        place with this call's best trajectories' theta columns and ones, ready for the next
+        step.  The engine's own previous path (set_prev_path) is not used."""
         poses = _f64(poses).reshape(-1, 4)
         S = poses.shape[0]
+        self._check_prev(S, prev_theta, has_prev, update_prev, False)
         K = 0
         if opponents is not None:
             opponents = _f64(opponents)
@@ -299,23 +344,42 @@ class Engine:
             flags = np.zeros((S, Cn), np.uint8)
         if S == 0:   # an empty batch is a valid (empty) answer, not an error
             return BatchPlan(best_idx, best_cost, best_traj, costs, flags, steer_speed)
-        self._ck(self._L.f1l_plan_batch(self._h, _vp(poses), _vp(opponents), _vp(n_opp), S, K,
-                                        _vp(best_idx), _vp(best_cost), _vp(best_traj), _vp(costs),
-                                        _vp(flags), _vp(steer_speed)))
+        if prev_theta is None:
+            self._ck(self._L.f1l_plan_batch(self._h, _vp(poses), _vp(opponents), _vp(n_opp), S, K,
+                                            _vp(best_idx), _vp(best_cost), _vp(best_traj),
+                                            _vp(costs), _vp(flags), _vp(steer_speed)))
+        else:
+            self._ck(self._L.f1l_plan_batch_prev(self._h, _vp(poses), _vp(opponents), _vp(n_opp),
+                                                 S, K, _vp(prev_theta), _vp(has_prev),
+                                                 int(bool(update_prev)), _vp(best_idx),
+                                                 _vp(best_cost), _vp(best_traj), _vp(costs),
+                                                 _vp(flags), _vp(steer_speed)))
         return BatchPlan(best_idx, best_cost, best_traj, costs, flags, steer_speed)
 
     def plan_batch_dev(self, poses, opponents=None, n_opp=None, best_idx=None, best_cost=None,
-                       best_traj=None, costs=None, flags=None, steer_speed=None, stream=None):
+                       best_traj=None, costs=None, flags=None, steer_speed=None, stream=None,
+                       prev_theta=None, has_prev=None, update_prev=False):
         """Same with torch CUDA tensors; enqueues on `stream` (default: torch's current stream)
-        and does not synchronise."""
+        and does not synchronise.  prev_theta / has_prev / update_prev as for plan_batch, as
+        contiguous CUDA tensors (float32 [S, n_samples], uint8 / bool [S]) updated in place on
+        the stream (f1l_plan_batch_prev_dev)."""
         import torch
         S = poses.shape[0]
         K = 0 if opponents is None else opponents.shape[1]
+        self._check_prev(S, prev_theta, has_prev, update_prev, True)
         st = stream if stream is not None else torch.cuda.current_stream(poses.device).cuda_stream
-        self._ck(self._L.f1l_plan_batch_dev(self._h, _vp(poses), _vp(opponents), _vp(n_opp), S, K,
-                                            _vp(best_idx), _vp(best_cost), _vp(best_traj),
-                                            _vp(costs), _vp(flags), _vp(steer_speed),
-                                            C.c_void_p(st)))
+        if prev_theta is None:
+            self._ck(self._L.f1l_plan_batch_dev(self._h, _vp(poses), _vp(opponents), _vp(n_opp), S,
+                                                K, _vp(best_idx), _vp(best_cost), _vp(best_traj),
+                                                _vp(costs), _vp(flags), _vp(steer_speed),
+                                                C.c_void_p(st)))
+        else:
+            self._ck(self._L.f1l_plan_batch_prev_dev(self._h, _vp(poses), _vp(opponents),
+                                                     _vp(n_opp), S, K, _vp(prev_theta),
+                                                     _vp(has_prev), int(bool(update_prev)),
+                                                     _vp(best_idx), _vp(best_cost),
+                                                     _vp(best_traj), _vp(costs), _vp(flags),
+                                                     _vp(steer_speed), C.c_void_p(st)))
 
     # -- candidate sharding over peer memory -------------------------------------------------
     def export_peer_handle(self):

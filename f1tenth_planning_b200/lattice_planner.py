@@ -19,7 +19,8 @@ Reference-compatible surface
 Additive (north-star) surface
     .plan(..., opponent_poses=[K,3])      opponents in the map frame
     .plan_detailed(...) / .last           PlanDetail: best_idx, costs[C], terms[C,5], flags[C] ...
-    .plan_batch(poses[S,4], opponents[S,K,3], n_opp[S])
+    .plan_batch(poses[S,4], opponents[S,K,3], n_opp[S][, prev_theta=[S,M], has_prev=[S],
+                update_prev=True])  per-scenario previous paths, carried in place step to step
     .set_map(occupancy, origin, resolution), .set_goal_grid(lookaheads, widths)
 
 With no plug-ins registered every stage runs on the GPU.  A registered ``sample_func`` replaces
@@ -245,7 +246,13 @@ class LatticePlanner():
 
     def plan_batch(self, poses, opponents=None, n_opp=None, **kw):
         """S independent scenarios: poses [S,4], opponents [S,K,3], n_opp [S] -> BatchPlan
-        (best_idx [S], best_cost [S], best_traj [S,M,4], costs [S,C], flags, steer_speed [S,2])."""
+        (best_idx [S], best_cost [S], best_traj [S,M,4], costs [S,C], flags, steer_speed [S,2]).
+
+        Each scenario may carry its own previous path for the similarity cost, the batched form
+        of what plan() keeps from call to call: prev_theta [S,M] float32 (C-contiguous) and
+        has_prev [S] bool / uint8.  With update_prev=True both are overwritten in place with this
+        step's best trajectories' theta columns and ones, so a loop of S cars passes them back
+        unchanged on the next step.  Keywords go to Engine.plan_batch."""
         return self._sync().plan_batch(poses, opponents, n_opp, **kw)
 
 

@@ -276,6 +276,35 @@ int f1l_plan_batch(f1l_handle h, const double* poses, const double* opp,
                    float* costs, uint8_t* flags, double* steer_speed);
 
 /*
+ * Batch with a previous path per scenario: the batched form of `prev_path` of
+ * get_similarity_cost (lattice_planner.py:287-296), which f1l_plan keeps on the handle for a
+ * single query.  Scenario s gives bit-identically the answer of f1l_plan on this handle after
+ * f1l_set_prev_path(prev_theta[s]), or after f1l_clear_prev_path when has_prev[s] == 0.
+ *   prev_theta [S,M] f32 (M = n_samples, as for f1l_set_prev_path): theta column of each
+ *       scenario's previous best trajectory, read; with update_prev != 0 overwritten in place with
+ *       the theta column of best_traj[s] -- what f1l_plan(..., update_prev = 1) stores, also for
+ *       a scenario without a feasible candidate.
+ *   has_prev [S] u8 or NULL (every scenario has a path): read; with update_prev != 0 set to 1.
+ * The handle's own previous path is neither read nor written.  F1L_ERR_INVALID_ARG when
+ * update_prev or has_prev is given without prev_theta.  Other arguments as f1l_plan_batch_dev.
+ */
+int f1l_plan_batch_prev_dev(f1l_handle h, const double* poses_dev, const double* opp_dev,
+                            const int32_t* n_opp_dev, int n_scenarios, int max_opp,
+                            float* prev_theta_dev, uint8_t* has_prev_dev, int update_prev,
+                            int32_t* best_idx_dev, float* best_cost_dev, float* best_traj_dev,
+                            float* costs_dev, uint8_t* flags_dev, double* steer_speed_dev,
+                            void* stream);
+
+/* Same with HOST buffers, through the chunked pipeline of f1l_plan_batch: each chunk's paths and
+ * flags travel with its other inputs and, with update_prev, come back with its other outputs.
+ * Synchronised before returning. */
+int f1l_plan_batch_prev(f1l_handle h, const double* poses, const double* opp,
+                        const int32_t* n_opp, int n_scenarios, int max_opp,
+                        float* prev_theta, uint8_t* has_prev, int update_prev,
+                        int32_t* best_idx, float* best_cost, float* best_traj,
+                        float* costs, uint8_t* flags, double* steer_speed);
+
+/*
  * Batched nearest_point + pure-pursuit lookahead over B poses on the uploaded track.
  * Replaces nearest_point (utils/utils.py:37-67), intersect_point (:69-151), get_actuation
  * (:153-161) and PurePursuitPlanner._get_current_waypoint / plan (pure_pursuit.py:56-122).
