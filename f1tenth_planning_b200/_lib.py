@@ -10,6 +10,8 @@ N_TERMS = 5
 MAX_OPP = 16
 MAX_M = 256
 FLAG_VALID, FLAG_COLLIDE_OPP, FLAG_COLLIDE_MAP, FLAG_NO_CENTRE = 1, 2, 4, 8
+CAR_HIT_MAP, CAR_HIT_CAR, CAR_NO_FEASIBLE = 1, 2, 4
+MAX_GROUP = 1 + MAX_OPP
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 # F1L_LIB selects another build of the same library (A/B builds of kernel variants)
@@ -49,6 +51,24 @@ class PlanResult(C.Structure):
                 ("best_traj_map", _vp)]
 
 
+class RolloutConfig(C.Structure):
+    """f1l_rollout_config (include/f1l.h)."""
+    _fields_ = [("dt", C.c_double), ("substeps", C.c_int32), ("group", C.c_int32),
+                ("max_steer", C.c_double), ("max_accel", C.c_double), ("v_max", C.c_double)]
+
+
+class FleetBuffers(C.Structure):
+    """f1l_fleet (include/f1l.h): device pointers."""
+    _fields_ = [("state", _vp), ("prev_theta", _vp), ("has_prev", _vp), ("status", _vp),
+                ("progress", _vp), ("track_i", _vp), ("track_s", _vp)]
+
+
+class RolloutTraceBuffers(C.Structure):
+    """f1l_rollout_trace (include/f1l.h): device pointers, each nullable."""
+    _fields_ = [("state", _vp), ("steer_speed", _vp), ("best_idx", _vp), ("status", _vp),
+                ("progress", _vp)]
+
+
 # name -> (restype, argtypes); must list every symbol include/f1l.h declares
 SIGNATURES = {
     "f1l_default_config": (C.c_int, [C.POINTER(Config)]),
@@ -83,6 +103,9 @@ SIGNATURES = {
                                           _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "f1l_plan_batch_prev": (C.c_int, [_vp, _vp, _vp, _vp, C.c_int, C.c_int, _vp, _vp, C.c_int,
                                       _vp, _vp, _vp, _vp, _vp, _vp]),
+    "f1l_default_rollout_config": (C.c_int, [C.POINTER(RolloutConfig)]),
+    "f1l_rollout_dev": (C.c_int, [_vp, C.POINTER(RolloutConfig), C.POINTER(FleetBuffers), C.c_int,
+                                  C.c_int, C.POINTER(RolloutTraceBuffers), _vp]),
     "f1l_pure_pursuit_batch_dev": (C.c_int, [_vp, _vp, C.c_int, C.c_double, _vp, _vp, _vp, _vp,
                                              _vp, _vp, _vp]),
     "f1l_pure_pursuit_batch": (C.c_int, [_vp, _vp, C.c_int, C.c_double, _vp, _vp, _vp, _vp, _vp,

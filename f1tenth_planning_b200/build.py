@@ -8,7 +8,7 @@ SRC_DIR = os.path.join(HERE, "csrc")
 OUT_DIR = os.path.join(HERE, "lib")
 OUT = os.path.join(OUT_DIR, "libf1l.so")
 SOURCES = ["f1l_api.cu"]
-DEPS = ["f1l_api.cu", "f1l_common.cuh", "f1l_lattice.cuh", "f1l_pp.cuh", "f1l_peaks.cuh",
+DEPS = ["f1l_api.cu", "f1l_common.cuh", "f1l_lattice.cuh", "f1l_pp.cuh", "f1l_peaks.cuh", "f1l_rollout.cuh",
         os.path.join("..", "..", "include", "f1l.h")]
 
 

@@ -25,6 +25,7 @@ struct NvtxRange {
 #include "f1l_lattice.cuh"
 #include "f1l_peaks.cuh"
 #include "f1l_pp.cuh"
+#include "f1l_rollout.cuh"
 
 #ifndef N_PIPE
 #define N_PIPE 3  // streams of the host-buffer batch pipeline
@@ -67,6 +68,8 @@ struct f1l_ctx {
     // track
     int n = 0, ncols = 0;
     DevBuf xy, v, psi, kappa, segA, segB, blk;
+    DevBuf seg_s;      // [n-1] double2 (cumulative length at the segment's start, length): rollout progress
+    double lap = 0.0;  // cumulative length of the n-1 segments plus the closing gap p_{n-1} -> p_0
     // grid
     DevBuf grid, clear, clear_tmp, edt;
     int use_clearance = 1;
@@ -100,6 +103,8 @@ struct f1l_ctx {
     int stats_on = 0;
     // batch (device-pointer API) scratch
     DevBuf b_ctx, b_centres, b_best, b_near_i, b_near4;
+    // rollout (f1l_rollout_dev) scratch: command, cost, the races' opponent table, re-acquisition
+    DevBuf r_ss, r_cost, r_opp, r_nopp, r_key, r_near_i, r_near4;
     // batch pipeline (host-pointer API)
     PipeSlot pipe[N_PIPE];
     // misc scratch for the pure-pursuit / intersect host APIs
@@ -971,7 +976,8 @@ int f1l_destroy(f1l_handle h) {
                       &h->lut, &h->lookaheads, &h->widths, &h->prev, &h->q_res, &h->q_in, &h->q_goals,
                       &h->q_ctx, &h->q_centres, &h->q_best, &h->q_detail, &h->q_params, &h->q_flags, &h->q_states, &h->q_headings, &h->b_ctx, &h->b_centres,
                       &h->b_best, &h->b_near_i, &h->b_near4, &h->stats, &h->m_in, &h->m_in2, &h->m_o0, &h->m_o1, &h->m_o2, &h->m_o3,
-                      &h->m_o4, &h->m_o5, &h->pp_key};
+                      &h->m_o4, &h->m_o5, &h->pp_key, &h->seg_s, &h->r_ss, &h->r_cost, &h->r_opp,
+                      &h->r_nopp, &h->r_key, &h->r_near_i, &h->r_near4};
     for (DevBuf* b : bufs) release(*b);
     for (int i = 0; i < N_PIPE; ++i) {
         PipeSlot& p = h->pipe[i];
@@ -1006,7 +1012,7 @@ int f1l_set_track(f1l_handle h, const double* wpts, int n, int ncols) {
         if (ncols > 4) kap[i] = wpts[(size_t)i * ncols + 4];
     }
     std::vector<float> segA(4 * (size_t)nseg), segB(2 * (size_t)nseg);
-    std::vector<double> blk(2 * (size_t)nblk);
+    std::vector<double> blk(2 * (size_t)nblk), seg_s(2 * (size_t)nseg);
     for (int b = 0; b < nblk; ++b) {
         blk[2 * b] = xy[2 * (size_t)(32 * b)];
         blk[2 * b + 1] = xy[2 * (size_t)(32 * b) + 1];
@@ -1016,6 +1022,8 @@ int f1l_set_track(f1l_handle h, const double* wpts, int n, int ncols) {
         const double ax = xy[2 * k] - ox, ay = xy[2 * k + 1] - oy;
         const double dx = xy[2 * k + 2] - xy[2 * k], dy = xy[2 * k + 3] - xy[2 * k + 1];
         const double len = std::sqrt(dx * dx + dy * dy);
+        seg_s[2 * k] = k ? seg_s[2 * k - 2] + seg_s[2 * k - 1] : 0.0;
+        seg_s[2 * k + 1] = len;
         const double ux = dx / len, uy = dy / len;
         const double sc = (double)TRACK_SCALE, hh = 0.5 * len;   // table units (track_seg_d2)
         segA[4 * k] = (float)ux;
@@ -1032,6 +1040,7 @@ int f1l_set_track(f1l_handle h, const double* wpts, int n, int ncols) {
     ENS(h->segA, segA.size() * 4);
     ENS(h->segB, segB.size() * 4);
     ENS(h->blk, blk.size() * 8);
+    ENS(h->seg_s, seg_s.size() * 8);
     CK(cudaStreamSynchronize(h->stream));
     CK(cudaMemcpy(h->xy.p, xy.data(), xy.size() * 8, cudaMemcpyHostToDevice));
     CK(cudaMemcpy(h->v.p, v.data(), v.size() * 8, cudaMemcpyHostToDevice));
@@ -1040,6 +1049,11 @@ int f1l_set_track(f1l_handle h, const double* wpts, int n, int ncols) {
     CK(cudaMemcpy(h->segA.p, segA.data(), segA.size() * 4, cudaMemcpyHostToDevice));
     CK(cudaMemcpy(h->segB.p, segB.data(), segB.size() * 4, cudaMemcpyHostToDevice));
     CK(cudaMemcpy(h->blk.p, blk.data(), blk.size() * 8, cudaMemcpyHostToDevice));
+    CK(cudaMemcpy(h->seg_s.p, seg_s.data(), seg_s.size() * 8, cudaMemcpyHostToDevice));
+    {
+        const double gx = xy[0] - xy[2 * (size_t)nseg], gy = xy[1] - xy[2 * (size_t)nseg + 1];
+        h->lap = seg_s[2 * (size_t)nseg - 2] + seg_s[2 * (size_t)nseg - 1] + std::sqrt(gx * gx + gy * gy);
+    }
     // the scan's constant-memory copy: one table per device, taken over by the latest upload (no
     // kernel of another handle may still be reading it: device-wide sync, this is the slow path)
     h->ctab_key = 0;
@@ -1731,6 +1745,106 @@ int f1l_plan_batch_prev(f1l_handle h, const double* poses, const double* opp, co
                         uint8_t* flags, double* steer_speed) {
     return plan_batch_internal(h, poses, opp, n_opp, S, max_opp, prev_theta, has_prev, update_prev, best_idx,
                                best_cost, best_traj, costs, flags, steer_speed);
+}
+
+// ---- closed-loop rollouts -----------------------------------------------------------------
+int f1l_default_rollout_config(f1l_rollout_config* rc) {
+    if (!rc) return F1L_ERR_INVALID_ARG;
+    rc->dt = 0.01;
+    rc->substeps = 1;
+    rc->group = 1;
+    rc->max_steer = 0.4189;
+    rc->max_accel = 9.51;
+    rc->v_max = INFINITY;
+    return F1L_OK;
+}
+
+int f1l_rollout_dev(f1l_handle h, const f1l_rollout_config* rc, const f1l_fleet* fl, int S,
+                    int n_steps, const f1l_rollout_trace* trace, void* stream) {
+    if (!h || !rc || !fl) return F1L_ERR_INVALID_ARG;
+    if (!fl->state || !fl->prev_theta || !fl->has_prev || !fl->status || !fl->progress ||
+        !fl->track_i || !fl->track_s)
+        return F1L_ERR_INVALID_ARG;
+    if (rc->group < 1 || rc->group > F1L_MAX_GROUP || S <= 0 || S % rc->group != 0) return F1L_ERR_INVALID_ARG;
+    if (rc->substeps < 1 || n_steps < 0) return F1L_ERR_INVALID_ARG;
+    if (!(rc->dt > 0) || !(rc->max_steer > 0) || !(rc->max_accel > 0) || !(rc->v_max > 0))
+        return F1L_ERR_INVALID_ARG;
+    if (n_steps == 0) return F1L_OK;
+    if (h->n < 2) return F1L_ERR_NO_TRACK;
+    if (h->nL * h->nW <= 0) return F1L_ERR_NO_GOALS;
+    CK(cudaSetDevice(h->device));
+    ENS(h->r_ss, (size_t)S * 16);
+    ENS(h->r_cost, (size_t)S * 4);
+    ENS(h->r_opp, (size_t)S * F1L_MAX_OPP * 24);
+    ENS(h->r_nopp, (size_t)S * 4);
+    ENS(h->r_key, (size_t)S * 8);
+    ENS(h->r_near_i, (size_t)S * 4);
+    ENS(h->r_near4, (size_t)S * 32);
+    cudaStream_t st = (cudaStream_t)stream;
+    NvtxRange nvtx_rollout("f1l.rollout");
+
+    RolloutArgs a;
+    memset(&a, 0, sizeof(a));
+    a.tr = track_view(h);
+    a.grid = grid_view(h);
+    a.seg_s = (const double2*)h->seg_s.p;
+    a.lap = h->lap;
+    a.res = h->gres;
+    a.has_grid = h->grid.p != nullptr;
+    a.collision_mode = h->cfg.collision_mode;
+    a.hl = 0.5 * h->cfg.car_length;
+    a.hw = 0.5 * h->cfg.car_width;
+    a.disc_off = h->cfg.car_length / 3.0;
+    a.wheelbase = h->cfg.wheelbase;
+    a.dt = rc->dt;
+    a.max_steer = rc->max_steer;
+    a.max_accel = rc->max_accel;
+    a.v_max = rc->v_max;
+    a.substeps = rc->substeps;
+    a.group = rc->group;
+    a.n_races = S / rc->group;
+    a.state = fl->state;
+    a.status = fl->status;
+    a.progress = fl->progress;
+    a.track_i = fl->track_i;
+    a.track_s = fl->track_s;
+    a.opp = (double*)h->r_opp.p;
+    a.n_opp = (int32_t*)h->r_nopp.p;
+    const unsigned blocks = (unsigned)((a.n_races + ROLLOUT_WARPS - 1) / ROLLOUT_WARPS);
+
+    // once per call: global nearest_point of every car (K1) for the cars to re-acquire, then the
+    // initial pass of the step kernel (no integration) builds step 0's opponent table
+    PPOut po;
+    memset(&po, 0, sizeof(po));
+    po.nearest = (double*)h->r_near4.p;
+    po.nearest_i = (int32_t*)h->r_near_i.p;
+    launch_pp(a.tr, st, fl->state, 4, S, -1.0, h->cfg.wheelbase, 0.0, 0, 0.0,
+              (unsigned long long*)h->r_key.p, pp_slots(h), po, ctab_valid(h), h);
+    a.near_i = po.nearest_i;
+    a.near4 = po.nearest;
+    rollout_step_kernel<<<blocks, ROLLOUT_WARPS * 32, 0, st>>>(a);
+    h->launches += 3;
+    CK(cudaGetLastError());
+    a.near_i = nullptr;
+    a.near4 = nullptr;
+    a.steer_speed = (const double*)h->r_ss.p;
+    a.best_cost = (const float*)h->r_cost.p;
+    for (int k = 0; k < n_steps; ++k) {
+        const size_t row = (size_t)k * S;
+        int32_t* best_idx = trace && trace->best_idx ? trace->best_idx + row : nullptr;
+        const int r = plan_batch_dev_internal(h, fl->state, a.opp, a.n_opp, S, F1L_MAX_OPP, fl->prev_theta,
+                                              fl->has_prev, 1, best_idx, (float*)h->r_cost.p, nullptr,
+                                              nullptr, nullptr, (double*)h->r_ss.p, stream);
+        if (r != F1L_OK) return r;
+        a.tr_state = trace && trace->state ? trace->state + 4 * row : nullptr;
+        a.tr_ss = trace && trace->steer_speed ? trace->steer_speed + 2 * row : nullptr;
+        a.tr_status = trace && trace->status ? trace->status + row : nullptr;
+        a.tr_progress = trace && trace->progress ? trace->progress + row : nullptr;
+        rollout_step_kernel<<<blocks, ROLLOUT_WARPS * 32, 0, st>>>(a);
+        h->launches += 1;
+        CK(cudaGetLastError());
+    }
+    return F1L_OK;
 }
 
 // ---- pure pursuit -------------------------------------------------------------------------

@@ -721,25 +721,35 @@ __device__ __forceinline__ float ffm(float a, float b, float c) { return __fmaf_
 __device__ __forceinline__ float fm(float a, float b) { return __fmul_rn(a, b); }
 __device__ __forceinline__ float fa(float a, float b) { return __fadd_rn(a, b); }
 __device__ __forceinline__ float fs(float a, float b) { return __fsub_rn(a, b); }
+// the same in float64: the rollout kernel (f1l_rollout.cuh) runs the predicates below in the map frame
+__device__ __forceinline__ double fm(double a, double b) { return __dmul_rn(a, b); }
+__device__ __forceinline__ double fa(double a, double b) { return __dadd_rn(a, b); }
+__device__ __forceinline__ double fs(double a, double b) { return __dsub_rn(a, b); }
+__device__ __forceinline__ float vabs(float a) { return fabsf(a); }
+__device__ __forceinline__ double vabs(double a) { return fabs(a); }
+__device__ __forceinline__ int floor_int(float a) { return __float2int_rd(a); }
+__device__ __forceinline__ int floor_int(double a) { return __double2int_rd(a); }
 
 // SAT of two equal rectangles; ego axes (c, s), opponent axes (oc, os), T = opp - ego.
 // collide iff every axis overlaps strictly (touching = no collision).
-__device__ __forceinline__ bool sat_collide(float tx, float ty, float c, float s, float oc,
-                                            float os, float hl, float hw) {
-    const float cc = fabsf(fa(fm(c, oc), fm(s, os)));
-    const float ss = fabsf(fs(fm(s, oc), fm(c, os)));
-    const float rl = fa(hl, fa(fm(hl, cc), fm(hw, ss)));
-    const float rw = fa(hw, fa(fm(hl, ss), fm(hw, cc)));
-    const float e0 = fabsf(fa(fm(tx, c), fm(ty, s)));
-    const float e1 = fabsf(fs(fm(ty, c), fm(tx, s)));
-    const float e2 = fabsf(fa(fm(tx, oc), fm(ty, os)));
-    const float e3 = fabsf(fs(fm(ty, oc), fm(tx, os)));
+template <class T>
+__device__ __forceinline__ bool sat_collide(T tx, T ty, T c, T s, T oc, T os, T hl, T hw) {
+    const T cc = vabs(fa(fm(c, oc), fm(s, os)));
+    const T ss = vabs(fs(fm(s, oc), fm(c, os)));
+    const T rl = fa(hl, fa(fm(hl, cc), fm(hw, ss)));
+    const T rw = fa(hw, fa(fm(hl, ss), fm(hw, cc)));
+    const T e0 = vabs(fa(fm(tx, c), fm(ty, s)));
+    const T e1 = vabs(fs(fm(ty, c), fm(tx, s)));
+    const T e2 = vabs(fa(fm(tx, oc), fm(ty, os)));
+    const T e3 = vabs(fs(fm(ty, oc), fm(tx, os)));
     return e0 < rl && e1 < rw && e2 < rl && e3 < rw;
 }
 
+// occupancy probe at cell (ix0 + floor(cx), iy0 + floor(cy)); out of bounds counts as occupied
+template <class T>
 __device__ __forceinline__ bool grid_hit(const uint8_t* __restrict__ occ, int gw, int gh, int ix0,
-                                         int iy0, float cx, float cy) {
-    const int col = ix0 + __float2int_rd(cx), row = iy0 + __float2int_rd(cy);
+                                         int iy0, T cx, T cy) {
+    const int col = ix0 + floor_int(cx), row = iy0 + floor_int(cy);
     if ((unsigned)col >= (unsigned)gw || (unsigned)row >= (unsigned)gh) return true;
     return __ldg(occ + (size_t)row * gw + col) != 0;
 }

@@ -381,6 +381,13 @@ class Engine:
                                                      _vp(best_traj), _vp(costs), _vp(flags),
                                                      _vp(steer_speed), C.c_void_p(st)))
 
+    # -- closed-loop rollouts ----------------------------------------------------------------
+    def fleet(self, poses, group=1):
+        """A fleet of kinematic-bicycle cars at `poses` [S,4] (x, y, theta, v) on this engine's
+        device, raced in groups of `group` consecutive cars (rollout.Fleet, f1l_rollout_dev)."""
+        from .rollout import Fleet
+        return Fleet(self, poses, group)
+
     # -- candidate sharding over peer memory -------------------------------------------------
     def export_peer_handle(self):
         """64-byte CUDA IPC handle of this engine's exchange block (f1l_xchg_export)."""

@@ -21,6 +21,7 @@ Additive (north-star) surface
     .plan_detailed(...) / .last           PlanDetail: best_idx, costs[C], terms[C,5], flags[C] ...
     .plan_batch(poses[S,4], opponents[S,K,3], n_opp[S][, prev_theta=[S,M], has_prev=[S],
                 update_prev=True])  per-scenario previous paths, carried in place step to step
+    .rollout(poses[S,4], n_steps, group=1, **kw)  closed-loop rollouts of a fleet on the device
     .set_map(occupancy, origin, resolution), .set_goal_grid(lookaheads, widths)
 
 With no plug-ins registered every stage runs on the GPU.  A registered ``sample_func`` replaces
@@ -232,6 +233,16 @@ class LatticePlanner():
                            best_traj_map=t.best_traj_map)
         self.last = d
         return d
+
+    def rollout(self, poses, n_steps, group=1, **kw):
+        """Closed-loop rollouts on the device for host users: the cars at `poses` [S,4] (x, y,
+        theta, v), raced in groups of `group` consecutive cars, advanced n_steps planning steps
+        (keywords as rollout.Fleet.run).  Returns the per-step RolloutTrace as numpy arrays and the
+        final (state [S,4], status [S], progress [S])."""
+        fleet = self._sync().fleet(poses, group)
+        tr = fleet.run(n_steps, trace=True, **kw)
+        trace = type(tr)(*(t.cpu().numpy() for t in tr))
+        return trace, (fleet.state.cpu().numpy(), fleet.status.cpu().numpy(), fleet.progress.cpu().numpy())
 
     def plan(self, pose_x, pose_y, pose_theta, velocity, waypoints=None, opponent_poses=None):
         """lattice_planner.py:174-214 -> (steering_angle, speed, selected_traj [M,4]).

@@ -305,6 +305,84 @@ int f1l_plan_batch_prev(f1l_handle h, const double* poses, const double* opp,
                         float* costs, uint8_t* flags, double* steer_speed);
 
 /*
+ * Closed-loop rollouts on the device: a fleet of S kinematic-bicycle cars advanced n_steps planning
+ * steps.  Replaces the user loop around the planner -- plan, then step the vehicle
+ * (lattice_planner.py:204-214 plus the gym step of examples/control/pure_pursuit.py:47-57, which
+ * is not part of the reference checkout) -- with no host synchronisation and no host copy inside
+ * the steps.  Device buffers, caller's stream, no sync.
+ *
+ * Cars form races of `group` consecutive scenarios [g*group, (g+1)*group); group = 1: independent
+ * cars without opponents.  Planning step k, for every car:
+ *   1. plan from (x, y, theta, v) exactly as f1l_plan_batch_prev_dev with update_prev = 1 on the
+ *      fleet's prev_theta / has_prev; the opponents are the other group-1 cars of the race at their
+ *      step-k poses, in race order without the car itself (crashed cars included);
+ *   2. steer = clamp(steer_cmd, +-max_steer); target = min(speed_cmd, v_max), or 0 when the plan
+ *      had no feasible candidate (best_cost = +inf; sets F1L_CAR_NO_FEASIBLE for this step);
+ *   3. `substeps` times, float64: v += clamp(target - v, +-max_accel*dt), x += v cos(theta) dt,
+ *      y += v sin(theta) dt, theta += v / wheelbase * tan(steer) dt (wheelbase of the f1l_config;
+ *      theta is not wrapped);
+ *   4. after every substep, at the new poses: the footprint (car_length x car_width) against the
+ *      map with the configured collision_mode (nine probes, or three discs on the distance
+ *      transform; out of bounds = occupied; float64, cell = floor((p - origin) / res)) sets
+ *      F1L_CAR_HIT_MAP, a float64 SAT against every other car of the race (touching = free) sets
+ *      F1L_CAR_HIT_CAR on both.  The hit bits are sticky and freeze the car: it keeps its pose at
+ *      v = 0, is still planned and is still an opponent of the others;
+ *   5. progress: the nearest raceline segment in a window of 32 segments starting 4 behind the
+ *      tracked one (cyclic over the n-1 segments, nearest_point's float64 operations, first
+ *      minimum); s = cum[i] + t * len[i]; progress += (s - s_prev) wrapped into [-lap/2, lap/2),
+ *      lap = cum[n-1] + |p_0 - p_{n-1}|, so counting continues across the raceline's seam.
+ * A car with track_i < 0 at the start of a call is re-acquired by a global nearest_point (its
+ * progress stays as given).  All state lives in the fleet buffers: run(30) + run(30) is
+ * bit-identical to run(60).  A reset is a caller write: new pose, has_prev = 0, status = 0,
+ * track_i = -1.
+ */
+#define F1L_CAR_HIT_MAP 1u
+#define F1L_CAR_HIT_CAR 2u
+#define F1L_CAR_NO_FEASIBLE 4u
+#define F1L_MAX_GROUP (1 + F1L_MAX_OPP)   /* cars per race */
+
+/* Defaults: dt 0.01, substeps 1, group 1, max_steer 0.4189, max_accel 9.51 (the steering and
+ * acceleration limits the closed-loop tests of the batch planner use), v_max +inf. */
+typedef struct {
+    double dt;           /* integration step (s), > 0 */
+    int32_t substeps;    /* integration steps per planning step, >= 1 */
+    int32_t group;       /* cars per race, 1..F1L_MAX_GROUP, divides n_scenarios */
+    double max_steer;    /* steering limit (rad), > 0 */
+    double max_accel;    /* acceleration limit (m/s^2), > 0 */
+    double v_max;        /* speed cap (m/s), > 0, may be +inf */
+} f1l_rollout_config;
+
+/* The fleet, device buffers read and written in place (S cars, M = n_samples). */
+typedef struct {
+    double* state;        /* [S,4] x, y, theta, v */
+    float* prev_theta;    /* [S,M] previous paths, as f1l_plan_batch_prev_dev */
+    uint8_t* has_prev;    /* [S] */
+    uint8_t* status;      /* [S] F1L_CAR_* */
+    double* progress;     /* [S] metres along the raceline */
+    int32_t* track_i;     /* [S] tracked raceline segment, < 0: re-acquire */
+    double* track_s;      /* [S] arc length at the tracked point */
+} f1l_fleet;
+
+/* Optional per-step record (T = n_steps), each buffer nullable. */
+typedef struct {
+    double* state;        /* [T,S,4] state at the START of step k */
+    double* steer_speed;  /* [T,S,2] raw planner command of step k */
+    int32_t* best_idx;    /* [T,S] chosen candidate of step k */
+    uint8_t* status;      /* [T,S] status after step k */
+    double* progress;     /* [T,S] progress after step k */
+} f1l_rollout_trace;
+
+int f1l_default_rollout_config(f1l_rollout_config* rc);
+
+/* F1L_ERR_INVALID_ARG for a null handle, config or fleet pointer, group outside 1..F1L_MAX_GROUP,
+ * n_scenarios not a positive multiple of group, substeps < 1, a dt / max_steer / max_accel / v_max
+ * that is not positive (NaN included) or n_steps < 0.  n_steps = 0 does nothing.  The handle owns
+ * the opponent table ([S,16,3] f64 + [S] i32) and the command scratch; one call in flight per
+ * handle.  Numpy users go through the Python layer (Fleet), which copies once per call. */
+int f1l_rollout_dev(f1l_handle h, const f1l_rollout_config* rc, const f1l_fleet* fleet,
+                    int n_scenarios, int n_steps, const f1l_rollout_trace* trace, void* stream);
+
+/*
  * Batched nearest_point + pure-pursuit lookahead over B poses on the uploaded track.
  * Replaces nearest_point (utils/utils.py:37-67), intersect_point (:69-151), get_actuation
  * (:153-161) and PurePursuitPlanner._get_current_waypoint / plan (pure_pursuit.py:56-122).
