@@ -3,7 +3,6 @@
 #include <cmath>
 #include <cstddef>
 #include <cstdio>
-#include <cstdlib>
 #include <cstring>
 #include <mutex>
 #include <new>
@@ -33,15 +32,38 @@ struct NvtxRange {
 
 namespace {
 
-struct DevBuf {
+// An allocation the handle owns: freed by its destructor, i.e. at f1l_destroy's `delete h`, after
+// the device synchronise.  DevBuf: device memory (grown by ensure); HostBuf: pinned host memory.
+template <cudaError_t (*FREE)(void*)>
+struct OwnedBuf {
     void* p = nullptr;
     size_t cap = 0;
+    OwnedBuf() = default;
+    OwnedBuf(const OwnedBuf&) = delete;
+    OwnedBuf& operator=(const OwnedBuf&) = delete;
+    ~OwnedBuf() { reset(); }
+    void reset() {
+        if (p) FREE(p);
+        p = nullptr;
+        cap = 0;
+    }
+};
+using DevBuf = OwnedBuf<cudaFree>;
+using HostBuf = OwnedBuf<cudaFreeHost>;
+
+// Per-scenario scratch of a sampler -> eval -> select pipeline: the sampler context, the goal
+// centres, the argmin keys (which double as K1's key scratch) and K1's nearest points.  `best` has
+// one 8-byte word behind the S keys: the persistent-grid work counter of a single query.
+struct PipeScratch {
+    DevBuf ctx, centres, best, near_i, near4;
+    int reserve(f1l_handle h, int S);
 };
 
 struct PipeSlot {
     cudaStream_t stream = nullptr;
     cudaEvent_t done = nullptr;
-    DevBuf poses, opp, nopp, ctx, centres, best, idx, cost, traj, costs, flags, ss, near_i, near4;
+    PipeScratch scratch;
+    DevBuf poses, opp, nopp, idx, cost, traj, costs, flags, ss;
     DevBuf prev, pvalid;   // the chunk's previous paths [n,M] f32 and their flags [n] u8
 };
 
@@ -86,25 +108,24 @@ struct f1l_ctx {
     DevBuf prev;
     int has_prev = 0, prev_m = 0;
     // single-query device buffers
-    DevBuf q_res, q_in, q_goals, q_ctx, q_centres, q_best, q_states, q_headings, q_params, q_flags;
+    PipeScratch q_scratch;
+    DevBuf q_in, q_goals, q_states, q_headings, q_params, q_flags;
     // pinned staging for the single query
-    void* h_in = nullptr;   // pose + opponents
-    void* h_out = nullptr;  // header + best trajectory
+    HostBuf h_in;   // pose + opponents
+    HostBuf h_out;  // result block (QHeader | best trajectory | map-frame trajectory)
     void* h_out_dev = nullptr;  // the same block as the device sees it (mapped pinned memory): the
                                 // select kernel of a single query writes its results straight into it
-    size_t h_out_cap = 0;
     // per-candidate detail block of a single query (costs | terms | goals | params | flags): one
     // device block, one D2H into pinned staging, then plain copies into the caller's arrays
     DevBuf q_detail;
-    void* h_detail = nullptr;
-    size_t h_detail_cap = 0;
+    HostBuf h_detail;
     // deviation-pass work counters (f1l_set_stats / f1l_get_stats)
     DevBuf stats;
     int stats_on = 0;
-    // batch (device-pointer API) scratch
-    DevBuf b_ctx, b_centres, b_best, b_near_i, b_near4;
-    // rollout (f1l_rollout_dev) scratch: command, cost, the races' opponent table, re-acquisition
-    DevBuf r_ss, r_cost, r_opp, r_nopp, r_key, r_near_i, r_near4;
+    // batch (device-pointer API) scratch, also the scratch of every rollout step
+    PipeScratch b_scratch;
+    // rollout (f1l_rollout_dev) scratch: command, cost, the races' opponent table
+    DevBuf r_ss, r_cost, r_opp, r_nopp;
     // batch pipeline (host-pointer API)
     PipeSlot pipe[N_PIPE];
     // misc scratch for the pure-pursuit / intersect host APIs
@@ -153,17 +174,20 @@ int ensure(f1l_handle h, DevBuf& b, size_t bytes) {
     return F1L_OK;
 }
 
-void release(DevBuf& b) {
-    if (b.p) cudaFree(b.p);
-    b.p = nullptr;
-    b.cap = 0;
-}
-
 #define ENS(buf, bytes)                          \
     do {                                         \
         int r__ = ensure(h, (buf), (bytes));     \
         if (r__ != F1L_OK) return r__;           \
     } while (0)
+
+int PipeScratch::reserve(f1l_handle h, int S) {
+    ENS(ctx, sizeof(QueryCtx) * (size_t)S);
+    ENS(centres, sizeof(Centre) * (size_t)S * (h->nL > 0 ? h->nL : 1));
+    ENS(best, 8 * (size_t)S + 8);
+    ENS(near_i, 4 * (size_t)S);
+    ENS(near4, 32 * (size_t)S);
+    return F1L_OK;
+}
 
 TrackView track_view(f1l_handle h) {
     TrackView t;
@@ -353,13 +377,6 @@ struct CtaPlan {
 CtaPlan plan_ctas(int n_cand, int S, int M, int sm_count, bool cubic) {
     CtaPlan best{8, 8, 1};
     double best_cost = 1e300;
-    // tuning hook for experiments: F1L_EVAL_PLAN="<warps>,<candidates per CTA>"
-    if (const char* e = getenv("F1L_EVAL_PLAN")) {
-        int nw = 0, chunk = 0;
-        if (sscanf(e, "%d,%d", &nw, &chunk) == 2 && (nw == 4 || nw == 7 || nw == 8) && chunk >= nw &&
-            chunk % nw == 0 && !(nw != 8 && M > 128))
-            return CtaPlan{nw, chunk, (n_cand + chunk - 1) / chunk};
-    }
     // Throughput regime -- many waves of small scenarios (the 4x7 grid: 28 candidates) with shared
     // Newton solves: one 4-warp CTA per scenario whose warps pull the scenario's 4-candidate items.
     // Measured, not modelled (the wave model below counts CTAs and would always prefer the CTA with
@@ -443,11 +460,7 @@ void launch_pp(const TrackView& tv, cudaStream_t stream, const double* poses, in
                unsigned long long* key, int slots, const PPOut& o, bool ctab, f1l_handle owner = nullptr) {
     const int n_groups = (n_poses + PP_CTA_POSES - 1) / PP_CTA_POSES;
     const int nblk = (tv.n - 1 + 31) >> 5;
-    int n_parts = pp_task_parts(n_groups, nblk, slots, ctab ? 16 : 6);
-    if (const char* e = getenv("F1L_PP_PARTS")) {   // tuning hook
-        const int v = atoi(e);
-        if (v >= 1 && v <= PP_MAX_PARTS && v <= nblk) n_parts = v;
-    }
+    const int n_parts = pp_task_parts(n_groups, nblk, slots, ctab ? 16 : 6);
     cudaMemsetAsync(key, 0xff, (size_t)n_poses * 8, stream);
     PPParts parts;
     parts.n = n_parts;
@@ -527,25 +540,40 @@ SelectArgs select_args(f1l_handle h, const TrackView& tv, const LutView& lut, co
     return se;
 }
 
-// sampler -> eval -> select for S scenarios on `stream`; all pointers are device pointers.
-// Previous paths: scenario s reads prev_theta + s * prev_stride (stride 0: one path for all) when
-// prev_valid is null or prev_valid[s] != 0; prev_theta null: no similarity term.
-int launch_pipeline(f1l_handle h, cudaStream_t stream, const double* poses, const double* opp,
-                    const int32_t* n_opp, int S, int max_opp, const float4* goals, int n_goals,
-                    int c_begin, int c_end, QueryCtx* ctx, Centre* centres,
-                    unsigned long long* best, int32_t* near_i, double* near4,
-                    const float* prev_theta, int prev_stride, const uint8_t* prev_valid,
+// Inputs of a pipeline over S scenarios; all pointers are device pointers.
+struct PipeIn {
+    const double* poses = nullptr;     // [S,4]
+    const double* opp = nullptr;       // [S,max_opp,3] (null: no opponents)
+    const int32_t* n_opp = nullptr;    // [S] (null: max_opp each)
+    int S = 0, max_opp = 0;
+    const float4* goals = nullptr;     // [n_goals] explicit goals (null: the goal grid)
+    int n_goals = 0;
+    int c_begin = 0, c_end = 0;        // evaluated candidates (c_end <= 0: to the last)
+    // previous paths: scenario s reads prev_theta + s * prev_stride (stride 0: one path for all)
+    // when prev_valid is null or prev_valid[s] != 0; prev_theta null: no similarity term
+    const float* prev_theta = nullptr;
+    int prev_stride = 0;
+    const uint8_t* prev_valid = nullptr;
+};
+
+// sampler -> eval -> select on `stream`, with `sc` reserved for in.S scenarios
+int launch_pipeline(f1l_handle h, cudaStream_t stream, const PipeIn& in, PipeScratch& sc,
                     const BatchOut& o, bool time_it) {
     if (h->n < 2) return F1L_ERR_NO_TRACK;
-    const int C = goals ? n_goals : h->nL * h->nW;
+    const int S = in.S;
+    const float4* goals = in.goals;
+    const int C = goals ? in.n_goals : h->nL * h->nW;
     if (C <= 0) return F1L_ERR_NO_GOALS;
-    if (c_begin < 0) c_begin = 0;
+    int c_begin = in.c_begin > 0 ? in.c_begin : 0, c_end = in.c_end;
     if (o.empty_shard) { c_begin = 0; c_end = 0; }
     else {
         if (c_end <= 0 || c_end > C) c_end = C;
         if (c_begin >= c_end) return F1L_ERR_INVALID_ARG;
     }
-    if (max_opp > F1L_MAX_OPP || max_opp < 0) return F1L_ERR_INVALID_ARG;
+    if (in.max_opp > F1L_MAX_OPP || in.max_opp < 0) return F1L_ERR_INVALID_ARG;
+    QueryCtx* ctx = (QueryCtx*)sc.ctx.p;
+    Centre* centres = (Centre*)sc.centres.p;
+    unsigned long long* best = (unsigned long long*)sc.best.p;
     const int M = h->cfg.n_samples;
     const EvalParams ep = eval_params(h);
     if (ep.collision_mode == 1 && h->grid.p) {
@@ -567,17 +595,14 @@ int launch_pipeline(f1l_handle h, cudaStream_t stream, const double* poses, cons
     // (the expensive candidates) first.  No wave quantisation, one window-table prologue per
     // resident CTA, and the cheap early-exit candidates fill the tail.
     int resident_ctas = build->minb * h->sm_count;
-    // F1L_EVAL_DYNAMIC: 0 = never, 2 = whenever the query has more than one CTA (sanitizer runs at
-    // small sizes), default = when it needs more than one wave
-    static const int dyn_mode = getenv("F1L_EVAL_DYNAMIC") ? atoi(getenv("F1L_EVAL_DYNAMIC")) : 1;
-    const bool dyn = S == 1 && wpc != 4 && o.work_next && !o.empty_shard && dyn_mode != 0 &&
-                     ((long long)cp.ctas_per_scn > resident_ctas || (dyn_mode == 2 && cp.ctas_per_scn > 1));
-    // ... and with at least F1L_EVAL_WIDE_MIN (default 4) candidates per resident warp it runs the
-    // 128-register build of the M > 128 shapes on two CTAs per SM (measured on config 5: 65 536
-    // candidates 471 -> 431 us, 32 768: 247 -> 234, 16 384: 134 -> 128, 8 192: 76 -> 100)
-    static const int wide_min = getenv("F1L_EVAL_WIDE_MIN") ? atoi(getenv("F1L_EVAL_WIDE_MIN")) : 4;
-    const bool wide = dyn && wpc == 8 && bucket.wide.fn && wide_min > 0 &&
-                      (long long)n_cand >= (long long)wide_min * resident_ctas * wpc;
+    const bool dyn = S == 1 && wpc != 4 && o.work_next && !o.empty_shard &&
+                     (long long)cp.ctas_per_scn > resident_ctas;
+    // ... and with at least EVAL_WIDE_MIN candidates per resident warp it runs the 128-register
+    // build of the M > 128 shapes on two CTAs per SM (measured on config 5: 65 536 candidates
+    // 471 -> 431 us, 32 768: 247 -> 234, 16 384: 134 -> 128, 8 192: 76 -> 100)
+    constexpr int EVAL_WIDE_MIN = 4;
+    const bool wide = dyn && wpc == 8 && bucket.wide.fn &&
+                      (long long)n_cand >= (long long)EVAL_WIDE_MIN * resident_ctas * wpc;
     if (wide) {
         build = &bucket.wide;
         resident_ctas = build->minb * h->sm_count;
@@ -589,10 +614,10 @@ int launch_pipeline(f1l_handle h, cudaStream_t stream, const double* poses, cons
     sa.tr = track_view(h);
     sa.grid = grid_view(h);
     sa.ep = ep;
-    sa.poses = poses;
-    sa.opp = opp;
-    sa.n_opp = n_opp;
-    sa.max_opp = max_opp;
+    sa.poses = in.poses;
+    sa.opp = in.opp;
+    sa.n_opp = in.n_opp;
+    sa.max_opp = in.max_opp;
     sa.lookaheads = (const double*)h->lookaheads.p;
     sa.nL = goals ? 0 : h->nL;
     sa.row0 = o.s_rows >= 0 ? o.s_row0 : 0;
@@ -605,20 +630,15 @@ int launch_pipeline(f1l_handle h, cudaStream_t stream, const double* poses, cons
     cudaEvent_t* ev = h->ev + 4 * h->ev_next;
     if (time_it) cudaEventRecord(ev[0], stream);
     nvtxRangePushA("f1l.sample");
-    if (near_i && near4 && S >= 32) {
+    if (S >= 32) {
         // batch: nearest_point of all scenarios by the thread-per-pose scan kernel (K1), then one
         // warp per scenario for the lookahead intersections / context
-        PPOut po;
-        po.nearest = near4;
-        po.nearest_i = near_i;
-        po.lookahead = nullptr;
-        po.lookahead_i = nullptr;
-        po.actuation = nullptr;
-        po.status = nullptr;
-        po.front = nullptr;
-        launch_pp(sa.tr, stream, poses, 4, S, -1.0, 0.33, 0.0, 0, 0.0, best, pp_slots(h), po, ctab_valid(h), h);   // `best` doubles as K1's key scratch: the sampler resets it
+        PPOut po{};
+        po.nearest = (double*)sc.near4.p;
+        po.nearest_i = (int32_t*)sc.near_i.p;
+        launch_pp(sa.tr, stream, in.poses, 4, S, -1.0, 0.33, 0.0, 0, 0.0, best, pp_slots(h), po, ctab_valid(h), h);   // `best` doubles as K1's key scratch: the sampler resets it
         sample_warp_kernel<<<(S + SAMPLE_WARPS - 1) / SAMPLE_WARPS, SAMPLE_WARPS * 32, 0, stream>>>(
-            sa, near_i, near4, S);
+            sa, po.nearest_i, po.nearest, S);
         h->launches += 2;
     } else {
         // a lone dense query: one warp per ~2 lookahead rows; small batches: 8 warps each
@@ -645,9 +665,9 @@ int launch_pipeline(f1l_handle h, cudaStream_t stream, const double* poses, cons
     ea.nL = h->nL;
     ea.nW = h->nW;
     ea.goals = goals;
-    ea.prev_theta = prev_theta;
-    ea.prev_stride = prev_stride;
-    ea.prev_valid = prev_valid;
+    ea.prev_theta = in.prev_theta;
+    ea.prev_stride = in.prev_stride;
+    ea.prev_valid = in.prev_valid;
     ea.C = C;
     ea.c_begin = c_begin;
     ea.c_end = c_end;
@@ -702,8 +722,8 @@ int launch_pipeline(f1l_handle h, cudaStream_t stream, const double* poses, cons
     return F1L_OK;
 }
 
-// device / pinned-host result block of a single query: header then the best trajectory, so
-// that one D2H copy brings everything a plain plan() call returns
+// result block of a single query (h_out, mapped pinned memory that select_kernel writes): header
+// then the best trajectory, everything a plain plan() call returns
 struct QHeader {
     double steer, speed;                 // +0
     int32_t best_idx;                    // +16
@@ -717,6 +737,35 @@ static_assert(sizeof(QHeader) == 48, "QHeader layout");
 #define Q_OFF_TRAJ (sizeof(QHeader))
 #define Q_OFF_MAP (Q_OFF_TRAJ + F1L_MAX_M * sizeof(float4))
 #define Q_RES_BYTES (Q_OFF_MAP + F1L_MAX_M * 4 * sizeof(double))
+
+// select_kernel's outputs of a single query: the result block as the device sees it
+BatchOut q_result_out(f1l_handle h, bool want_map) {
+    char* dres = (char*)h->h_out_dev;
+    BatchOut o;
+    o.steer_speed = (double*)(dres + offsetof(QHeader, steer));
+    o.best_idx = (int32_t*)(dres + offsetof(QHeader, best_idx));
+    o.status = (int32_t*)(dres + offsetof(QHeader, no_feasible));
+    o.best_cost = (float*)(dres + offsetof(QHeader, best_cost));
+    o.best_traj = (float4*)(dres + Q_OFF_TRAJ);
+    o.best_traj_map = want_map ? (double*)(dres + Q_OFF_MAP) : nullptr;
+    return o;
+}
+
+// the result block into the caller's f1l_plan_result (after the stream synchronise)
+void q_copy_result(f1l_handle h, int C, f1l_plan_result* out) {
+    const int M = h->cfg.n_samples;
+    const char* res = (const char*)h->h_out.p;
+    const QHeader* hd = (const QHeader*)res;
+    out->steer = hd->steer;
+    out->speed = hd->speed;
+    out->best_idx = hd->best_idx;
+    out->no_feasible = hd->no_feasible;
+    out->tracker_found = hd->tracker_found;
+    out->n_candidates = C;
+    out->best_cost = hd->best_cost;
+    if (out->best_traj) memcpy(out->best_traj, res + Q_OFF_TRAJ, (size_t)M * 16);
+    if (out->best_traj_map) memcpy(out->best_traj_map, res + Q_OFF_MAP, (size_t)M * 32);
+}
 
 // pinned-host / device input block of a single query (fixed size, so that the copy is a constant
 // node of the CUDA graph): the opponent count travels in the block, not as a kernel argument
@@ -921,19 +970,13 @@ int f1l_create(f1l_handle* out, int device, const f1l_config* cfg) {
         e = cudaStreamCreateWithFlags(&h->pipe[i].stream, cudaStreamNonBlocking);
         if (e == cudaSuccess) e = cudaEventCreateWithFlags(&h->pipe[i].done, cudaEventDisableTiming);
     }
-    if (e == cudaSuccess) e = cudaHostAlloc(&h->h_in, 1024, cudaHostAllocDefault);
-    if (e == cudaSuccess) memset(h->h_in, 0, 1024);
+    if (e == cudaSuccess) e = cudaHostAlloc(&h->h_in.p, 1024, cudaHostAllocDefault);
+    if (e == cudaSuccess) e = cudaHostAlloc(&h->h_out.p, Q_RES_BYTES, cudaHostAllocMapped);
+    // single queries write their results straight into h_out: no mapping, no handle
+    if (e == cudaSuccess) e = cudaHostGetDevicePointer(&h->h_out_dev, h->h_out.p, 0);
     if (e == cudaSuccess) {
-        h->h_out_cap = Q_RES_BYTES;
-        e = cudaHostAlloc(&h->h_out, h->h_out_cap, cudaHostAllocMapped);
-        if (e == cudaSuccess) {
-            memset(h->h_out, 0, h->h_out_cap);
-            static const bool direct_off = getenv("F1L_DIRECT_OUT") && atoi(getenv("F1L_DIRECT_OUT")) == 0;
-            if (direct_off || cudaHostGetDevicePointer(&h->h_out_dev, h->h_out, 0) != cudaSuccess) {
-                h->h_out_dev = nullptr;   // fall back to the device block + D2H copy
-                cudaGetLastError();
-            }
-        }
+        memset(h->h_in.p, 0, 1024);
+        memset(h->h_out.p, 0, Q_RES_BYTES);
     }
     if (e == cudaSuccess) {
         int sm = 0;
@@ -971,30 +1014,16 @@ int f1l_destroy(f1l_handle h) {
     cudaSetDevice(h->device);
     cudaDeviceSynchronize();
     f1l_xchg_detach(h);
-    release(h->xchg);
-    DevBuf* bufs[] = {&h->xy, &h->v, &h->psi, &h->kappa, &h->segA, &h->segB, &h->blk, &h->grid, &h->clear, &h->clear_tmp, &h->edt,
-                      &h->lut, &h->lookaheads, &h->widths, &h->prev, &h->q_res, &h->q_in, &h->q_goals,
-                      &h->q_ctx, &h->q_centres, &h->q_best, &h->q_detail, &h->q_params, &h->q_flags, &h->q_states, &h->q_headings, &h->b_ctx, &h->b_centres,
-                      &h->b_best, &h->b_near_i, &h->b_near4, &h->stats, &h->m_in, &h->m_in2, &h->m_o0, &h->m_o1, &h->m_o2, &h->m_o3,
-                      &h->m_o4, &h->m_o5, &h->pp_key, &h->seg_s, &h->r_ss, &h->r_cost, &h->r_opp,
-                      &h->r_nopp, &h->r_key, &h->r_near_i, &h->r_near4};
-    for (DevBuf* b : bufs) release(*b);
     for (int i = 0; i < N_PIPE; ++i) {
         PipeSlot& p = h->pipe[i];
-        DevBuf* pb[] = {&p.poses, &p.opp, &p.nopp, &p.ctx, &p.centres, &p.best, &p.idx, &p.cost,
-                        &p.traj, &p.costs, &p.flags, &p.ss, &p.near_i, &p.near4, &p.prev, &p.pvalid};
-        for (DevBuf* b : pb) release(*b);
         if (p.done) cudaEventDestroy(p.done);
         if (p.stream) cudaStreamDestroy(p.stream);
     }
     if (h->gexec) cudaGraphExecDestroy(h->gexec);
     for (int i = 0; i < 4 * F1L_EV_SLOTS; ++i)
         if (h->ev[i]) cudaEventDestroy(h->ev[i]);
-    if (h->h_in) cudaFreeHost(h->h_in);
-    if (h->h_out) cudaFreeHost(h->h_out);
-    if (h->h_detail) cudaFreeHost(h->h_detail);
     if (h->stream) cudaStreamDestroy(h->stream);
-    delete h;
+    delete h;   // frees every device and pinned buffer
     return F1L_OK;
 }
 
@@ -1057,8 +1086,7 @@ int f1l_set_track(f1l_handle h, const double* wpts, int n, int ncols) {
     // the scan's constant-memory copy: one table per device, taken over by the latest upload (no
     // kernel of another handle may still be reading it: device-wide sync, this is the slow path)
     h->ctab_key = 0;
-    static const bool ctab_off = getenv("F1L_CTAB") && atoi(getenv("F1L_CTAB")) == 0;
-    if (nblk * 32 <= F1L_CTAB_SEGS && h->device >= 0 && h->device < 64 && !ctab_off) {
+    if (nblk * 32 <= F1L_CTAB_SEGS && h->device >= 0 && h->device < 64) {
         {   // withdraw the table from whoever owns it, then wait for the scans already enqueued on it
             std::lock_guard<std::mutex> lk(g_ctab_mu);
             g_ctab_owner[h->device] = 0;
@@ -1121,10 +1149,10 @@ int f1l_clear_grid(f1l_handle h) {
     if (!h) return F1L_ERR_INVALID_ARG;
     cudaSetDevice(h->device);
     cudaStreamSynchronize(h->stream);
-    release(h->grid);
-    release(h->clear);
-    release(h->clear_tmp);
-    release(h->edt);
+    h->grid.reset();
+    h->clear.reset();
+    h->clear_tmp.reset();
+    h->edt.reset();
     h->epoch++;
     h->gh = h->gw = 0;
     return F1L_OK;
@@ -1219,15 +1247,13 @@ static int plan_internal(f1l_handle h, const double pose[4], const double* opp, 
 
     NvtxRange nvtx_plan("f1l.plan (single query)");
     // stage inputs (pinned)
-    QInput* hin = (QInput*)h->h_in;
+    QInput* hin = (QInput*)h->h_in.p;
     memcpy(hin->pose, pose, 4 * sizeof(double));
     hin->n_opp = n_opp;
     hin->pad = 0;
     if (n_opp) memcpy(hin->opp, opp, (size_t)n_opp * 3 * sizeof(double));
     ENS(h->q_in, sizeof(QInput));
-    ENS(h->q_ctx, sizeof(QueryCtx));
-    ENS(h->q_centres, sizeof(Centre) * (size_t)(h->nL > 0 ? h->nL : 1));
-    ENS(h->q_best, 16);   // argmin key | work counter of the persistent-grid schedule
+    if (const int r = h->q_scratch.reserve(h, 1); r != F1L_OK) return r;
     ENS(h->prev, F1L_MAX_M * sizeof(float));
     // detail block layout (every region 16-byte aligned)
     const size_t c16 = ((size_t)C + 3) & ~(size_t)3;
@@ -1236,13 +1262,11 @@ static int plan_internal(f1l_handle h, const double pose[4], const double* opp, 
     const size_t detail_bytes = off_flags + c16;
     ENS(h->q_detail, detail_bytes);
     const bool want_detail = out->costs || out->terms || out->flags || out->goals || out->params;
-    if (want_detail && h->h_detail_cap < detail_bytes) {
+    if (want_detail && h->h_detail.cap < detail_bytes) {
         CK(cudaStreamSynchronize(st));
-        if (h->h_detail) cudaFreeHost(h->h_detail);
-        h->h_detail = nullptr;
-        h->h_detail_cap = 0;
-        CK(cudaHostAlloc(&h->h_detail, detail_bytes, cudaHostAllocDefault));
-        h->h_detail_cap = detail_bytes;
+        h->h_detail.reset();
+        CK(cudaHostAlloc(&h->h_detail.p, detail_bytes, cudaHostAllocDefault));
+        h->h_detail.cap = detail_bytes;
         h->epoch++;   // the captured graph holds the old staging address
     }
     char* ddet = (char*)h->q_detail.p;
@@ -1263,23 +1287,10 @@ static int plan_internal(f1l_handle h, const double pose[4], const double* opp, 
         d_goals = (const float4*)h->q_goals.p;
     }
 
-    if (!h->q_res.p) {
-        ENS(h->q_res, Q_RES_BYTES);
-        // the header's padding words travel with the D2H copy: defined bytes (initcheck-clean)
-        CK(cudaMemsetAsync(h->q_res.p, 0, sizeof(QHeader), st));
-    }
     // Results of a single query: the select kernel writes header and best trajectory straight into
     // the mapped pinned block (posted writes over the host link, 3-10 KB) -- no D2H copy node on the
-    // latency path; without a mapping they go to the device block and one D2H copy.
-    const bool direct = h->h_out_dev != nullptr;
-    char* dres = direct ? (char*)h->h_out_dev : (char*)h->q_res.p;
-    BatchOut o;
-    o.steer_speed = (double*)(dres + offsetof(QHeader, steer));
-    o.best_idx = (int32_t*)(dres + offsetof(QHeader, best_idx));
-    o.status = (int32_t*)(dres + offsetof(QHeader, no_feasible));
-    o.best_cost = (float*)(dres + offsetof(QHeader, best_cost));
-    o.best_traj = (float4*)(dres + Q_OFF_TRAJ);
-    o.best_traj_map = out->best_traj_map ? (double*)(dres + Q_OFF_MAP) : nullptr;
+    // latency path.
+    BatchOut o = q_result_out(h, out->best_traj_map != nullptr);
     o.costs = (float*)(ddet + off_costs);
     o.terms = out->terms ? (float*)(ddet + off_terms) : nullptr;
     o.flags = out->flags ? (uint8_t*)(ddet + off_flags) : nullptr;
@@ -1314,19 +1325,28 @@ static int plan_internal(f1l_handle h, const double pose[4], const double* opp, 
             o.s_rows = (ce - 1) / h->nW - o.s_row0 + 1;
         }
     }
-    o.work_next = (int*)((char*)h->q_best.p + 8);
+    o.work_next = (int*)((char*)h->q_scratch.best.p + 8);   // behind the one argmin key
     exchange = exchange && h->xview.world > 1;
     if (exchange) {   // the ranks' minima meet inside select_kernel (peer memory over NVLink)
         o.xc = &h->xview;
-        o.xchg_status = (int32_t*)(dres + offsetof(QHeader, pad));
+        o.xchg_status = (int32_t*)((char*)h->h_out_dev + offsetof(QHeader, pad));
     }
     const bool sharded = exchange || row_step > 1 || c_begin != 0 || (c_end > 0 && c_end < C);
-    QHeader* hd = (QHeader*)h->h_out;
-    float* htraj = (float*)((char*)h->h_out + sizeof(QHeader));
     const QInput* din = (const QInput*)h->q_in.p;
-    // H2D of the input block, the three kernels, D2H of header + best trajectory.  The
-    // similarity term reads the previous path while select overwrites it: eval reads it before
-    // select runs (stream order), so one buffer suffices.
+    PipeIn in;
+    in.poses = din->pose;
+    in.opp = din->opp;
+    in.n_opp = &din->n_opp;
+    in.S = 1;
+    in.max_opp = F1L_MAX_OPP;
+    in.goals = d_goals;
+    in.n_goals = C;
+    in.c_begin = c_begin;
+    in.c_end = c_end;
+    in.prev_theta = h->has_prev ? (const float*)h->prev.p : nullptr;
+    // H2D of the input block, the three kernels, D2H of the detail block.  The similarity term
+    // reads the previous path while select overwrites it: eval reads it before select runs
+    // (stream order), so one buffer suffices.
     auto enqueue = [&](bool time_it) -> int {
         CK(cudaMemcpyAsync(h->q_in.p, hin, sizeof(QInput), cudaMemcpyHostToDevice, st));
         if (sharded && want_detail) {
@@ -1336,19 +1356,10 @@ static int plan_internal(f1l_handle h, const double pose[4], const double* opp, 
             h->launches += 1;
             if (o.flags) CK(cudaMemsetAsync(o.flags, 0, (size_t)C, st));
         }
-        int r = launch_pipeline(h, st, din->pose, din->opp, &din->n_opp, 1, F1L_MAX_OPP, d_goals, C,
-                                c_begin, c_end, (QueryCtx*)h->q_ctx.p, (Centre*)h->q_centres.p,
-                                (unsigned long long*)h->q_best.p, nullptr, nullptr,
-                                h->has_prev ? (const float*)h->prev.p : nullptr, 0, nullptr, o, time_it);
+        int r = launch_pipeline(h, st, in, h->q_scratch, o, time_it);
         if (r != F1L_OK) return r;
-        if (!direct) {
-            CK(cudaMemcpyAsync(hd, h->q_res.p, sizeof(QHeader) + (size_t)M * 16, cudaMemcpyDeviceToHost, st));
-            if (o.best_traj_map)
-                CK(cudaMemcpyAsync((char*)h->h_out + Q_OFF_MAP, dres + Q_OFF_MAP, (size_t)M * 32,
-                                   cudaMemcpyDeviceToHost, st));
-        }
         if (want_detail)
-            CK(cudaMemcpyAsync(h->h_detail, ddet, detail_bytes, cudaMemcpyDeviceToHost, st));
+            CK(cudaMemcpyAsync(h->h_detail.p, ddet, detail_bytes, cudaMemcpyDeviceToHost, st));
         return F1L_OK;
     };
     if (h->use_graph && !goals && !h->timing) {
@@ -1396,24 +1407,16 @@ static int plan_internal(f1l_handle h, const double pose[4], const double* opp, 
         h->has_prev = 1;
         h->prev_m = M;
     }
-    if (exchange && hd->pad != 0) return F1L_ERR_PEER_TIMEOUT;
+    if (exchange && ((const QHeader*)h->h_out.p)->pad != 0) return F1L_ERR_PEER_TIMEOUT;
     h->lastq_C = C;
     h->lastq_goals = goals != nullptr;
     h->lastq_rows[0] = o.s_row0;
     h->lastq_rows[1] = o.s_step;
     h->lastq_rows[2] = o.s_rows;
     h->lastq_epoch = h->epoch;
-    out->steer = hd->steer;
-    out->speed = hd->speed;
-    out->best_idx = hd->best_idx;
-    out->no_feasible = hd->no_feasible;
-    out->tracker_found = hd->tracker_found;
-    out->n_candidates = C;
-    out->best_cost = hd->best_cost;
-    if (out->best_traj) memcpy(out->best_traj, htraj, (size_t)M * 16);
-    if (out->best_traj_map) memcpy(out->best_traj_map, (char*)h->h_out + Q_OFF_MAP, (size_t)M * 32);
+    q_copy_result(h, C, out);
     if (want_detail) {
-        const char* hdet = (const char*)h->h_detail;
+        const char* hdet = (const char*)h->h_detail.p;
         if (out->costs) memcpy(out->costs, hdet + off_costs, (size_t)C * 4);
         if (out->terms) memcpy(out->terms, hdet + off_terms, (size_t)C * F1L_N_TERMS * 4);
         if (out->flags) memcpy(out->flags, hdet + off_flags, (size_t)C);
@@ -1448,47 +1451,28 @@ int f1l_select_candidate(f1l_handle h, int idx, float cost, int update_prev, f1l
     CK(cudaSetDevice(h->device));
     cudaStream_t st = h->stream;
     const int M = h->cfg.n_samples, C = h->lastq_C;
-    unsigned long long* hkey = (unsigned long long*)h->h_in;   // pinned staging
+    unsigned long long* hkey = (unsigned long long*)h->h_in.p;   // pinned staging
     uint32_t cb;
     memcpy(&cb, &cost, 4);
     const uint32_t ord = (cb & 0x80000000u) ? ~cb : (cb | 0x80000000u);   // float_orderable
     *hkey = ((unsigned long long)ord << 32) | (unsigned)idx;
-    CK(cudaMemcpyAsync(h->q_best.p, hkey, 8, cudaMemcpyHostToDevice, st));
-    char* dres = (char*)h->q_res.p;
-    BatchOut o;
-    o.steer_speed = (double*)(dres + offsetof(QHeader, steer));
-    o.best_idx = (int32_t*)(dres + offsetof(QHeader, best_idx));
-    o.status = (int32_t*)(dres + offsetof(QHeader, no_feasible));
-    o.best_cost = (float*)(dres + offsetof(QHeader, best_cost));
-    o.best_traj = (float4*)(dres + Q_OFF_TRAJ);
-    o.best_traj_map = out->best_traj_map ? (double*)(dres + Q_OFF_MAP) : nullptr;
+    const PipeScratch& sc = h->q_scratch;
+    CK(cudaMemcpyAsync(sc.best.p, hkey, 8, cudaMemcpyHostToDevice, st));
+    BatchOut o = q_result_out(h, out->best_traj_map != nullptr);
     o.prev_out = update_prev ? (float*)h->prev.p : nullptr;
     o.s_row0 = h->lastq_rows[0];
     o.s_step = h->lastq_rows[1];
     o.s_rows = h->lastq_rows[2];
     const SelectArgs se = select_args(h, track_view(h), lut_view(h), eval_params(h),
-                                      (const QueryCtx*)h->q_ctx.p, (const Centre*)h->q_centres.p,
+                                      (const QueryCtx*)sc.ctx.p, (const Centre*)sc.centres.p,
                                       h->lastq_goals ? (const float4*)h->q_goals.p : nullptr, C, 0,
-                                      (const unsigned long long*)h->q_best.p, 1, o);
+                                      (const unsigned long long*)sc.best.p, 1, o);
     eval_bucket_of(M).select<<<1, SELECT_THREADS, 0, st>>>(se);
     h->launches += 1;
     CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(h->h_out, dres, Q_OFF_TRAJ + (size_t)M * 16, cudaMemcpyDeviceToHost, st));
-    if (o.best_traj_map)
-        CK(cudaMemcpyAsync((char*)h->h_out + Q_OFF_MAP, dres + Q_OFF_MAP, (size_t)M * 32,
-                           cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
     if (update_prev) { h->has_prev = 1; h->prev_m = M; }
-    const QHeader* hd = (const QHeader*)h->h_out;
-    out->steer = hd->steer;
-    out->speed = hd->speed;
-    out->best_idx = hd->best_idx;
-    out->no_feasible = hd->no_feasible;
-    out->tracker_found = hd->tracker_found;
-    out->n_candidates = C;
-    out->best_cost = hd->best_cost;
-    if (out->best_traj) memcpy(out->best_traj, (char*)h->h_out + Q_OFF_TRAJ, (size_t)M * 16);
-    if (out->best_traj_map) memcpy(out->best_traj_map, (char*)h->h_out + Q_OFF_MAP, (size_t)M * 32);
+    q_copy_result(h, C, out);
     return F1L_OK;
 }
 
@@ -1600,11 +1584,16 @@ static int plan_batch_dev_internal(f1l_handle h, const double* poses_dev, const 
     if ((update_prev || has_prev_dev) && !prev_theta_dev) return F1L_ERR_INVALID_ARG;
     CK(cudaSetDevice(h->device));
     if (h->nL * h->nW <= 0) return F1L_ERR_NO_GOALS;
-    ENS(h->b_ctx, sizeof(QueryCtx) * (size_t)S);
-    ENS(h->b_centres, sizeof(Centre) * (size_t)S * h->nL);
-    ENS(h->b_best, 8 * (size_t)S);
-    ENS(h->b_near_i, 4 * (size_t)S);
-    ENS(h->b_near4, 32 * (size_t)S);
+    if (const int r = h->b_scratch.reserve(h, S); r != F1L_OK) return r;
+    PipeIn in;
+    in.poses = poses_dev;
+    in.opp = max_opp > 0 ? opp_dev : nullptr;
+    in.n_opp = n_opp_dev;
+    in.S = S;
+    in.max_opp = max_opp;
+    in.prev_theta = prev_theta_dev;
+    in.prev_stride = h->cfg.n_samples;
+    in.prev_valid = has_prev_dev;
     BatchOut o;
     o.best_idx = best_idx_dev;
     o.best_cost = best_cost_dev;
@@ -1614,11 +1603,7 @@ static int plan_batch_dev_internal(f1l_handle h, const double* poses_dev, const 
     o.steer_speed = steer_speed_dev;
     o.prev_out = update_prev ? prev_theta_dev : nullptr;
     o.prev_valid_out = update_prev ? has_prev_dev : nullptr;
-    return launch_pipeline(h, (cudaStream_t)stream, poses_dev, max_opp > 0 ? opp_dev : nullptr,
-                           n_opp_dev, S, max_opp, nullptr, 0, 0, 0, (QueryCtx*)h->b_ctx.p,
-                           (Centre*)h->b_centres.p, (unsigned long long*)h->b_best.p,
-                           (int32_t*)h->b_near_i.p, (double*)h->b_near4.p, prev_theta_dev,
-                           h->cfg.n_samples, has_prev_dev, o, h->timing != 0);
+    return launch_pipeline(h, (cudaStream_t)stream, in, h->b_scratch, o, h->timing != 0);
 }
 
 int f1l_plan_batch_dev(f1l_handle h, const double* poses_dev, const double* opp_dev,
@@ -1657,18 +1642,14 @@ static int plan_batch_internal(f1l_handle h, const double* poses, const double* 
     // last chunks taper (half, quarter, ... of a chunk, down to 1024): the result copy of the final
     // chunk is the one transfer nothing overlaps, 14 MB at full size but under 2 MB tapered.
     int chunk = 8192;
-    bool taper = true;
-    if (const char* e = getenv("F1L_PIPE_CHUNK")) { const int v = atoi(e); if (v > 0) { chunk = v; taper = false; } }
-    else if (S < 8 * chunk) { chunk = (S + 7) / 8; if (chunk < 1024) chunk = 1024; }
+    if (S < 8 * chunk) { chunk = (S + 7) / 8; if (chunk < 1024) chunk = 1024; }
     if (chunk > S) chunk = S;
     int slot = 0;
     for (int s0 = 0, n = 0; s0 < S; s0 += n, slot = (slot + 1) % N_PIPE) {
         n = (S - s0 < chunk) ? (S - s0) : chunk;
-        if (taper) {
-            // rest = what is left after this chunk: keep halving while the tail is short
-            const int rest = S - s0;
-            if (rest < 2 * chunk && rest > 1024) { n = rest / 2; if (n < 1024) n = 1024; if (n > rest) n = rest; }
-        }
+        // rest = what is left after this chunk: keep halving while the tail is short
+        const int rest = S - s0;
+        if (rest < 2 * chunk && rest > 1024) { n = rest / 2; if (n < 1024) n = 1024; if (n > rest) n = rest; }
         NvtxRange nvtx_chunk("f1l.plan_batch.chunk (H2D, kernels, D2H)");
         PipeSlot& p = h->pipe[slot];
         cudaStream_t st = p.stream;
@@ -1676,11 +1657,7 @@ static int plan_batch_internal(f1l_handle h, const double* poses, const double* 
         ENS(p.poses, (size_t)n * 32);
         if (max_opp > 0) ENS(p.opp, (size_t)n * max_opp * 24);
         if (n_opp) ENS(p.nopp, (size_t)n * 4);
-        ENS(p.ctx, sizeof(QueryCtx) * (size_t)n);
-        ENS(p.centres, sizeof(Centre) * (size_t)n * h->nL);
-        ENS(p.best, 8 * (size_t)n);
-        ENS(p.near_i, 4 * (size_t)n);
-        ENS(p.near4, 32 * (size_t)n);
+        if (const int r = p.scratch.reserve(h, n); r != F1L_OK) return r;
         if (best_idx) ENS(p.idx, (size_t)n * 4);
         if (best_cost) ENS(p.cost, (size_t)n * 4);
         if (best_traj) ENS(p.traj, (size_t)n * M * 16);
@@ -1707,13 +1684,16 @@ static int plan_batch_internal(f1l_handle h, const double* poses, const double* 
         // in place on the slot's copies, as in plan_batch_dev_internal
         o.prev_out = update_prev ? (float*)p.prev.p : nullptr;
         o.prev_valid_out = update_prev && has_prev ? (uint8_t*)p.pvalid.p : nullptr;
-        int r = launch_pipeline(h, st, (const double*)p.poses.p,
-                                max_opp > 0 ? (const double*)p.opp.p : nullptr,
-                                n_opp ? (const int32_t*)p.nopp.p : nullptr, n, max_opp, nullptr, 0,
-                                0, 0, (QueryCtx*)p.ctx.p, (Centre*)p.centres.p,
-                                (unsigned long long*)p.best.p, (int32_t*)p.near_i.p,
-                                (double*)p.near4.p, prev_theta ? (const float*)p.prev.p : nullptr, M,
-                                has_prev ? (const uint8_t*)p.pvalid.p : nullptr, o, false);
+        PipeIn in;
+        in.poses = (const double*)p.poses.p;
+        in.opp = max_opp > 0 ? (const double*)p.opp.p : nullptr;
+        in.n_opp = n_opp ? (const int32_t*)p.nopp.p : nullptr;
+        in.S = n;
+        in.max_opp = max_opp;
+        in.prev_theta = prev_theta ? (const float*)p.prev.p : nullptr;
+        in.prev_stride = M;
+        in.prev_valid = has_prev ? (const uint8_t*)p.pvalid.p : nullptr;
+        int r = launch_pipeline(h, st, in, p.scratch, o, false);
         if (r != F1L_OK) return r;
         if (best_idx) CK(cudaMemcpyAsync(best_idx + s0, p.idx.p, (size_t)n * 4, cudaMemcpyDeviceToHost, st));
         if (best_cost) CK(cudaMemcpyAsync(best_cost + s0, p.cost.p, (size_t)n * 4, cudaMemcpyDeviceToHost, st));
@@ -1777,9 +1757,8 @@ int f1l_rollout_dev(f1l_handle h, const f1l_rollout_config* rc, const f1l_fleet*
     ENS(h->r_cost, (size_t)S * 4);
     ENS(h->r_opp, (size_t)S * F1L_MAX_OPP * 24);
     ENS(h->r_nopp, (size_t)S * 4);
-    ENS(h->r_key, (size_t)S * 8);
-    ENS(h->r_near_i, (size_t)S * 4);
-    ENS(h->r_near4, (size_t)S * 32);
+    PipeScratch& sc = h->b_scratch;   // every step's pipeline reserves it for the same S: no realloc
+    if (const int r = sc.reserve(h, S); r != F1L_OK) return r;
     cudaStream_t st = (cudaStream_t)stream;
     NvtxRange nvtx_rollout("f1l.rollout");
 
@@ -1813,13 +1792,13 @@ int f1l_rollout_dev(f1l_handle h, const f1l_rollout_config* rc, const f1l_fleet*
     const unsigned blocks = (unsigned)((a.n_races + ROLLOUT_WARPS - 1) / ROLLOUT_WARPS);
 
     // once per call: global nearest_point of every car (K1) for the cars to re-acquire, then the
-    // initial pass of the step kernel (no integration) builds step 0's opponent table
-    PPOut po;
-    memset(&po, 0, sizeof(po));
-    po.nearest = (double*)h->r_near4.p;
-    po.nearest_i = (int32_t*)h->r_near_i.p;
+    // initial pass of the step kernel (no integration) builds step 0's opponent table.  Both run
+    // in the batch scratch: they are enqueued before the first step's pipeline overwrites it.
+    PPOut po{};
+    po.nearest = (double*)sc.near4.p;
+    po.nearest_i = (int32_t*)sc.near_i.p;
     launch_pp(a.tr, st, fl->state, 4, S, -1.0, h->cfg.wheelbase, 0.0, 0, 0.0,
-              (unsigned long long*)h->r_key.p, pp_slots(h), po, ctab_valid(h), h);
+              (unsigned long long*)sc.best.p, pp_slots(h), po, ctab_valid(h), h);
     a.near_i = po.nearest_i;
     a.near4 = po.nearest;
     rollout_step_kernel<<<blocks, ROLLOUT_WARPS * 32, 0, st>>>(a);
@@ -1856,14 +1835,13 @@ int f1l_pure_pursuit_batch_dev(f1l_handle h, const double* poses_dev, int n_pose
     if (h->n < 2) return F1L_ERR_NO_TRACK;
     CK(cudaSetDevice(h->device));
     NvtxRange nvtx_pp("f1l.pure_pursuit_batch (K1 scan + finish)");
-    PPOut o;
+    PPOut o{};
     o.nearest = nearest_dev;
     o.nearest_i = nearest_i_dev;
     o.lookahead = lookahead_dev;
     o.lookahead_i = lookahead_i_dev;
     o.actuation = actuation_dev;
     o.status = status_dev;
-    o.front = nullptr;
     ENS(h->pp_key, (size_t)n_poses * 8);   // scan scratch (one call in flight per handle)
     launch_pp(track_view(h), (cudaStream_t)stream, poses_dev, 3, n_poses, L, h->cfg.wheelbase,
               h->cfg.max_reacquire, 0, 0.0, (unsigned long long*)h->pp_key.p, pp_slots(h), o, ctab_valid(h), h);
@@ -1908,13 +1886,8 @@ int f1l_front_axle_batch_dev(f1l_handle h, const double* poses_dev, int n_poses,
     if (!h || !poses_dev || n_poses <= 0 || !front_dev) return F1L_ERR_INVALID_ARG;
     if (h->n < 2) return F1L_ERR_NO_TRACK;
     CK(cudaSetDevice(h->device));
-    PPOut o;
-    o.nearest = nullptr;
+    PPOut o{};
     o.nearest_i = nearest_i_dev;
-    o.lookahead = nullptr;
-    o.lookahead_i = nullptr;
-    o.actuation = nullptr;
-    o.status = nullptr;
     o.front = front_dev;
     ENS(h->pp_key, (size_t)n_poses * 8);
     launch_pp(track_view(h), (cudaStream_t)stream, poses_dev, 4, n_poses, 0.0, wheelbase, 0.0, 1,
@@ -1989,11 +1962,11 @@ int f1l_get_actuation_batch(f1l_handle h, const double* in, int n, double wheelb
 // out[0..1] cos/sin pose, [2..7] grid A00 A01 A10 A11 fx fy, [8..9] gix giy (as float bits via
 // int copy), [10..] opponents 16 x (x, y, cos, sin)
 int f1l_debug_query_ctx(f1l_handle h, float* out_f, int32_t* out_i) {
-    if (!h || !out_f || !out_i || !h->q_ctx.p) return F1L_ERR_INVALID_ARG;
+    if (!h || !out_f || !out_i || !h->q_scratch.ctx.p) return F1L_ERR_INVALID_ARG;
     CK(cudaSetDevice(h->device));
     QueryCtx q;
     CK(cudaStreamSynchronize(h->stream));
-    CK(cudaMemcpy(&q, h->q_ctx.p, sizeof(q), cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(&q, h->q_scratch.ctx.p, sizeof(q), cudaMemcpyDeviceToHost));
     out_f[0] = q.cth; out_f[1] = q.sth;
     out_f[2] = q.gA00; out_f[3] = q.gA01; out_f[4] = q.gA10; out_f[5] = q.gA11;
     out_f[6] = q.gfx; out_f[7] = q.gfy;

@@ -104,7 +104,9 @@ int f1l_default_config(f1l_config* cfg);
 
 /* Create / destroy the per-device planner state.  Replaces LatticePlanner.__init__
  * (lattice_planner.py:44-55) and PurePursuitPlanner.__init__ (pure_pursuit.py:51-54).
- * Builds the cubic-spiral seed LUT on the device (see f1l_get_lut). */
+ * Builds the cubic-spiral seed LUT on the device (see f1l_get_lut).  Single queries write their
+ * results straight into a mapped pinned host block: if the device cannot map it
+ * (cudaHostGetDevicePointer fails), f1l_create returns F1L_ERR_CUDA and creates no handle. */
 int f1l_create(f1l_handle* out, int device, const f1l_config* cfg);
 int f1l_destroy(f1l_handle h);
 const char* f1l_strerror(int code);

@@ -76,6 +76,9 @@ def test_config5_dense_sweep(ellipse, corridor):
     eng, cfg, world = H.make_pair(ellipse, la, wd, grid=corridor, n_samples=200, use_device_lut=False)
     pose, opp = H.scenario(ellipse, 1005, 8)
     d = eng.plan(pose, opp, update_prev=False)
+    # 32-candidate chunks, 2048 CTAs against 444 resident: the persistent grid on the wide build
+    shape = eng.last_eval_shape()
+    assert shape["nw"] == 8 and shape["minb"] == 2, shape
     C = 65536
     assert d.costs.shape == (C,)
     assert d.best_idx == int(np.argmin(d.costs)) and d.best_cost == d.costs[d.best_idx]

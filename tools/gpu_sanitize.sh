@@ -5,9 +5,3 @@ for tool in memcheck racecheck synccheck initcheck; do
   timeout 600 compute-sanitizer --tool $tool --print-limit 20 python tools/sanitize_driver.py > gpurun_out/sanitize_$tool.log 2>&1
   echo "$tool rc=$? : $(grep -E 'ERROR SUMMARY|RACECHECK SUMMARY|sanitize driver ok' gpurun_out/sanitize_$tool.log | tr '\n' ' ')"
 done
-# the same driver with every multi-CTA single query forced onto the persistent grid (device-wide work
-# counter), which the default policy only uses beyond one wave of CTAs
-for tool in memcheck racecheck; do
-  F1L_EVAL_DYNAMIC=2 timeout 600 compute-sanitizer --tool $tool --print-limit 20 python tools/sanitize_driver.py > gpurun_out/sanitize_${tool}_dyn.log 2>&1
-  echo "$tool (persistent grid forced) rc=$? : $(grep -E 'ERROR SUMMARY|RACECHECK SUMMARY|sanitize driver ok' gpurun_out/sanitize_${tool}_dyn.log | tr '\n' ' ')"
-done

@@ -1,6 +1,6 @@
 """Small-size pass over every kernel of the library, for compute-sanitizer (tools/gpu_sanitize.sh):
-single queries (4x7 grid, a dense 16x16 grid with M = 200, user goals, G1 clothoid, pruned
-window), a 96-scenario batch (batch sampler + K1 + pipeline), K1 with ragged sizes, front-axle
+single queries (4x7 grid, a dense 16x16 grid with M = 200, the 256x256 grid of config 5 on the
+persistent grid and the wide build, user goals, G1 clothoid, pruned window), a 96-scenario batch (batch sampler + K1 + pipeline), K1 with ragged sizes, front-axle
 mode, the intersect / actuation batches, generate, a shard.  No torch: host buffers only."""
 import os
 import sys
@@ -78,6 +78,10 @@ eng.close()
 eng = fresh(M=200)                                              # the 8-warp M = 200 shapes
 eng.set_goal_grid(np.linspace(0.5, 4.0, 16), np.linspace(-1.2, 1.2, 16))
 check(eng.plan(poses[8], opp[8, :n_opp[8]]))
+eng.set_goal_grid(*synth.goal_grid(5))                          # config 5: 65 536 candidates
+check(eng.plan(poses[8], opp[8, :n_opp[8]]))
+shape = eng.last_eval_shape()                                   # persistent grid, wide build
+assert shape["nw"] == 8 and shape["minb"] == 2, shape
 eng.close()
 eng = fresh(M=30)
 eng.set_goal_grid(la, wd)
