@@ -59,12 +59,35 @@ struct PipeScratch {
     int reserve(f1l_handle h, int S);
 };
 
+// The per-scenario arrays of a host-buffer batch chunk, in the order they are copied
+enum { B_POSES, B_OPP, B_NOPP, B_IDX, B_COST, B_TRAJ, B_COSTS, B_FLAGS, B_SS, B_PREV, B_PVALID, B_ARRAYS };
+
 struct PipeSlot {
     cudaStream_t stream = nullptr;
-    cudaEvent_t done = nullptr;
     PipeScratch scratch;
-    DevBuf poses, opp, nopp, idx, cost, traj, costs, flags, ss;
-    DevBuf prev, pvalid;   // the chunk's previous paths [n,M] f32 and their flags [n] u8
+    DevBuf buf[B_ARRAYS];   // the chunk's device copies of those arrays
+};
+
+// A single query's choice of candidates as the caller gives it: the contiguous block
+// [c_begin, c_end) (c_end <= 0: to the last), or with row_step > 1 the lookahead rows
+// row0, row0 + row_step, ... of the goal grid
+struct Shard {
+    int c_begin = 0, c_end = 0, row0 = 0, row_step = 1;
+};
+
+// What a query covers, resolved (make_span): the evaluated shard-local candidates [c_begin, c_end),
+// whose local index v maps to the candidate of lookahead row row0 + (v / nW) * row_step in the
+// same column (row_step 1: v itself); the lookahead rows the sampler fills, s_row0 + k * s_step for
+// k < s_rows; the candidate select returns when nothing at all was evaluated; and whether this rank
+// evaluates nothing (it still takes part in the exchange, with key ~0).  All int: no padding,
+// spans compare with memcmp.
+struct Span {
+    int C = 0;   // candidates per scenario
+    int c_begin = 0, c_end = 0;
+    int row0 = 0, row_step = 1;
+    int s_row0 = 0, s_step = 1, s_rows = 0;
+    int first = 0;
+    int empty = 0;
 };
 
 }  // namespace
@@ -80,7 +103,8 @@ struct f1l_ctx {
     int use_graph = 1;
     unsigned long long epoch = 0;   // bumped by every upload / config change
     cudaGraphExec_t gexec = nullptr;
-    unsigned long long gkey[4] = {~0ull, ~0ull, ~0ull, ~0ull};
+    unsigned long long gkey[2] = {~0ull, ~0ull};   // epoch and output mask of the captured graph
+    Span gspan;                                    // ... and its span
     int timed = 0;  // events of the last pipeline launch are valid
 #define F1L_EV_SLOTS 64
     cudaEvent_t ev[4 * F1L_EV_SLOTS] = {nullptr};
@@ -128,8 +152,9 @@ struct f1l_ctx {
     DevBuf r_ss, r_cost, r_opp, r_nopp;
     // batch pipeline (host-pointer API)
     PipeSlot pipe[N_PIPE];
-    // misc scratch for the pure-pursuit / intersect host APIs
-    DevBuf m_in, m_in2, m_o0, m_o1, m_o2, m_o3, m_o4, m_o5, pp_key;
+    // device copies of the arrays of the one-shot host-buffer calls (pure pursuit, intersect, ...)
+    DevBuf m[7];
+    DevBuf pp_key;   // K1's key scratch of the pure-pursuit / front-axle device calls
     // peer-memory exchange of candidate-sharded queries (f1l_xchg_*): the local block, the peers'
     // blocks as mapped by cudaIpcOpenMemHandle (own rank: the local pointer)
     int pp_per_sm = 0, pp_per_sm_ct = 0;   // resident pp_scan_kernel CTAs per SM (pp_slots): global / constant table
@@ -139,9 +164,9 @@ struct f1l_ctx {
     XchgView xview = {0, 0, {nullptr}};
     // template instance / CTA plan of the last eval_kernel launch (f1l_last_eval_shape)
     int eval_info[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-    // the last single query, for f1l_select_candidate: candidate count, explicit goals?, epoch
-    int lastq_C = 0, lastq_goals = 0;
-    int lastq_rows[3] = {0, 1, -1};   // lookahead rows its sampler filled (row0, step, count; -1: all)
+    // the last single query, for f1l_select_candidate: its span, explicit goals?, epoch
+    Span lastq_span;
+    int lastq_goals = 0;
     unsigned long long lastq_epoch = ~0ull;
 };
 
@@ -186,6 +211,50 @@ int PipeScratch::reserve(f1l_handle h, int S) {
     ENS(best, 8 * (size_t)S + 8);
     ENS(near_i, 4 * (size_t)S);
     ENS(near4, 32 * (size_t)S);
+    return F1L_OK;
+}
+
+// One per-item host array of a host-buffer call and its device copy.  A null source and
+// destination: the call has no such array, and the device sees a null pointer.
+struct Stage {
+    DevBuf* buf;
+    const void* src;   // copied in (nullable)
+    void* dst;         // copied back (nullable)
+    size_t bytes;      // per item
+    void* dev() const { return src || dst ? buf->p : nullptr; }
+};
+
+// ensures the device copies of items [i0, i0 + n), then enqueues the inputs' H2D copies
+template <int K>
+int stage_in(f1l_handle h, cudaStream_t st, const Stage (&t)[K], size_t i0, size_t n) {
+    for (const Stage& e : t)
+        if (e.src || e.dst) ENS(*e.buf, n * e.bytes);
+    for (const Stage& e : t)
+        if (e.src)
+            CK(cudaMemcpyAsync(e.buf->p, (const char*)e.src + i0 * e.bytes, n * e.bytes, cudaMemcpyHostToDevice, st));
+    return F1L_OK;
+}
+
+// enqueues the outputs' D2H copies of items [i0, i0 + n)
+template <int K>
+int stage_out(f1l_handle h, cudaStream_t st, const Stage (&t)[K], size_t i0, size_t n) {
+    for (const Stage& e : t)
+        if (e.dst)
+            CK(cudaMemcpyAsync((char*)e.dst + i0 * e.bytes, e.buf->p, n * e.bytes, cudaMemcpyDeviceToHost, st));
+    return F1L_OK;
+}
+
+// explicit goals [C,3] f64 -> float4 (x, y, theta, 0) in q_goals, by way of the caller's `g4`
+// (which must outlive the copy)
+int upload_goals(f1l_handle h, const double* goals, int C, std::vector<float>& g4, cudaStream_t st) {
+    g4.assign(4 * (size_t)C, 0.0f);
+    for (size_t c = 0; c < (size_t)C; ++c) {
+        g4[4 * c] = (float)goals[3 * c];
+        g4[4 * c + 1] = (float)goals[3 * c + 1];
+        g4[4 * c + 2] = (float)goals[3 * c + 2];
+    }
+    ENS(h->q_goals, (size_t)C * 16);
+    CK(cudaMemcpyAsync(h->q_goals.p, g4.data(), (size_t)C * 16, cudaMemcpyHostToDevice, st));
     return F1L_OK;
 }
 
@@ -453,14 +522,16 @@ int pp_slots(f1l_handle h) {
     return per_sm * h->sm_count;
 }
 
-// K1 = key preset + scan + finish on one stream.  key: 8 bytes of scratch per pose; slots: one-warp
-// scan CTAs resident on the device (pp_slots)
-void launch_pp(const TrackView& tv, cudaStream_t stream, const double* poses, int pose_stride,
-               int n_poses, double L, double wb, double max_reacquire, int front_axle, double k_path,
-               unsigned long long* key, int slots, const PPOut& o, bool ctab, f1l_handle owner = nullptr) {
+// K1 = key preset + scan + finish on one stream over the handle's track.  key: 8 bytes of scratch
+// per pose
+void launch_pp(f1l_handle h, cudaStream_t stream, const double* poses, int pose_stride, int n_poses,
+               double L, double wb, double max_reacquire, int front_axle, double k_path,
+               unsigned long long* key, const PPOut& o) {
+    const TrackView tv = track_view(h);
+    bool ctab = ctab_valid(h);
     const int n_groups = (n_poses + PP_CTA_POSES - 1) / PP_CTA_POSES;
     const int nblk = (tv.n - 1 + 31) >> 5;
-    const int n_parts = pp_task_parts(n_groups, nblk, slots, ctab ? 16 : 6);
+    const int n_parts = pp_task_parts(n_groups, nblk, pp_slots(h), ctab ? 16 : 6);
     cudaMemsetAsync(key, 0xff, (size_t)n_poses * 8, stream);
     PPParts parts;
     parts.n = n_parts;
@@ -469,7 +540,7 @@ void launch_pp(const TrackView& tv, cudaStream_t stream, const double* poses, in
     const dim3 grid((unsigned)n_groups, (unsigned)n_parts);
     if (ctab) {
         std::lock_guard<std::mutex> lk(g_ctab_mu);
-        ctab = owner && ctab_valid(owner);   // still ours?  (checked and enqueued under the mutex)
+        ctab = ctab_valid(h);   // still ours?  (checked and enqueued under the mutex)
         if (ctab)
             pp_scan_kernel<true><<<grid, 32, 0, stream>>>(tv, poses, pose_stride, n_poses, front_axle, wb, parts, key);
     }
@@ -495,40 +566,85 @@ struct BatchOut {
     float2* headings = nullptr;
     float* prev_out = nullptr;         // [S,M] theta column of each best trajectory (update_prev)
     uint8_t* prev_valid_out = nullptr; // [S] set to 1 with it (per-scenario previous paths)
-    int row0 = 0, row_step = 1;        // row-interleaved shard (c_begin / c_end are shard-local)
+    int32_t* xchg_status = nullptr;    // sharded single query: != 0 when a peer did not arrive
+};
+
+// Inputs of a pipeline over S scenarios: device pointers (host ones in a host-buffer batch call)
+struct PipeIn {
+    const double* poses = nullptr;     // [S,4]
+    const double* opp = nullptr;       // [S,max_opp,3] (null: no opponents)
+    const int32_t* n_opp = nullptr;    // [S] (null: max_opp each)
+    int S = 0, max_opp = 0;
+    const float4* goals = nullptr;     // [span.C] explicit goals (null: the goal grid)
+    Span span;
+    // previous paths: scenario s reads prev_theta + s * prev_stride (stride 0: one path for all)
+    // when prev_valid is null or prev_valid[s] != 0; prev_theta null: no similarity term
+    const float* prev_theta = nullptr;
+    int prev_stride = 0;
+    const uint8_t* prev_valid = nullptr;
     const XchgView* xc = nullptr;      // sharded single query: exchange the argmin with the peers
-    int32_t* xchg_status = nullptr;
-    int s_row0 = 0, s_step = 1, s_rows = -1;   // lookahead rows the sampler must fill (-1: all)
-    bool empty_shard = false;          // this rank owns no candidate of the query: it evaluates nothing
-                                       // but still takes part in the exchange (key = ~0)
     int* work_next = nullptr;          // single query: device counter for the persistent-grid schedule
 };
 
-// select_kernel arguments of a pipeline over S scenarios (first_cand: the first evaluated candidate,
-// returned when nothing at all was evaluated)
-SelectArgs select_args(f1l_handle h, const TrackView& tv, const LutView& lut, const EvalParams& ep,
-                       const QueryCtx* ctx, const Centre* centres, const float4* goals, int C,
-                       int first_cand, const unsigned long long* best, int S, const BatchOut& o) {
+// The span of a query over the explicit goals (n_goals > 0) or the goal grid (n_goals 0), with the
+// peers' exchange taking place or not: every check of the candidate and row arguments
+int make_span(f1l_handle h, int n_goals, const Shard& q, bool exchange, Span& sp) {
+    sp = Span{};
+    sp.C = n_goals > 0 ? n_goals : h->nL * h->nW;
+    if (sp.C <= 0) return F1L_ERR_NO_GOALS;
+    sp.s_rows = h->nL;
+    if (q.row_step > 1) {   // row-interleaved shard: rows row0, row0 + row_step, ... of the goal grid
+        if (n_goals > 0 || q.row0 < 0 || q.row0 >= q.row_step) return F1L_ERR_INVALID_ARG;
+        const int n_rows = q.row0 < h->nL ? (h->nL - q.row0 + q.row_step - 1) / q.row_step : 0;
+        // More ranks than lookahead rows: with peers attached the call is collective, so a rank
+        // without rows must still arrive at the exchange (it contributes key = ~0 and returns the
+        // global winner like everybody else); alone there is nothing to answer.
+        if (n_rows == 0) {
+            if (!exchange) return F1L_ERR_INVALID_ARG;
+            sp.empty = 1;
+        }
+        sp.c_end = n_rows * h->nW;
+        sp.row0 = q.row0;
+        sp.row_step = sp.s_step = q.row_step;
+        sp.s_row0 = sp.empty ? 0 : q.row0;   // the sampler fills this shard's rows only
+        sp.s_rows = n_rows;
+        sp.first = sp.empty ? 0 : q.row0 * h->nW;
+        return F1L_OK;
+    }
+    sp.c_begin = q.c_begin > 0 ? q.c_begin : 0;
+    sp.c_end = q.c_end > 0 && q.c_end < sp.C ? q.c_end : sp.C;
+    if (sp.c_begin >= sp.c_end) return F1L_ERR_INVALID_ARG;
+    sp.first = sp.c_begin;
+    if (n_goals == 0 && (sp.c_begin > 0 || sp.c_end < sp.C)) {
+        // contiguous candidate block: the lookahead rows it touches
+        sp.s_row0 = sp.c_begin / h->nW;
+        sp.s_rows = (sp.c_end - 1) / h->nW - sp.s_row0 + 1;
+    }
+    return F1L_OK;
+}
+
+// select_kernel arguments of a pipeline
+SelectArgs select_args(f1l_handle h, const PipeIn& in, const PipeScratch& sc, const BatchOut& o) {
     SelectArgs se;
-    if (o.xc && S == 1) se.xc = *o.xc;
+    if (in.xc && in.S == 1) se.xc = *in.xc;
     else { se.xc.world = 0; se.xc.rank = 0; }
     se.xchg_status = o.xchg_status;
-    se.tr = tv;
-    se.lut = lut;
-    se.ep = ep;
-    se.ctx = ctx;
-    se.centres = centres;
+    se.tr = track_view(h);
+    se.lut = lut_view(h);
+    se.ep = eval_params(h);
+    se.ctx = (const QueryCtx*)sc.ctx.p;
+    se.centres = (const Centre*)sc.centres.p;
     se.widths = (const float*)h->widths.p;
     se.nL = h->nL;
     se.nW = h->nW;
     se.inv_nW = 1.0f / (float)(h->nW > 0 ? h->nW : 1);
-    se.row0 = o.s_rows >= 0 ? o.s_row0 : 0;
-    se.row_step = o.s_rows >= 0 ? o.s_step : 1;
-    se.n_rows = o.s_rows >= 0 ? o.s_rows : h->nL;
-    se.goals = goals;
-    se.C = C;
-    se.c_begin = first_cand < C ? first_cand : 0;   // (a rank without rows)
-    se.best = best;
+    se.row0 = in.span.s_row0;
+    se.row_step = in.span.s_step;
+    se.n_rows = in.span.s_rows;
+    se.goals = in.goals;
+    se.C = in.span.C;
+    se.c_begin = in.span.first;
+    se.best = (const unsigned long long*)sc.best.p;
     se.best_idx = o.best_idx;
     se.best_cost = o.best_cost;
     se.status = o.status;
@@ -540,36 +656,12 @@ SelectArgs select_args(f1l_handle h, const TrackView& tv, const LutView& lut, co
     return se;
 }
 
-// Inputs of a pipeline over S scenarios; all pointers are device pointers.
-struct PipeIn {
-    const double* poses = nullptr;     // [S,4]
-    const double* opp = nullptr;       // [S,max_opp,3] (null: no opponents)
-    const int32_t* n_opp = nullptr;    // [S] (null: max_opp each)
-    int S = 0, max_opp = 0;
-    const float4* goals = nullptr;     // [n_goals] explicit goals (null: the goal grid)
-    int n_goals = 0;
-    int c_begin = 0, c_end = 0;        // evaluated candidates (c_end <= 0: to the last)
-    // previous paths: scenario s reads prev_theta + s * prev_stride (stride 0: one path for all)
-    // when prev_valid is null or prev_valid[s] != 0; prev_theta null: no similarity term
-    const float* prev_theta = nullptr;
-    int prev_stride = 0;
-    const uint8_t* prev_valid = nullptr;
-};
-
 // sampler -> eval -> select on `stream`, with `sc` reserved for in.S scenarios
 int launch_pipeline(f1l_handle h, cudaStream_t stream, const PipeIn& in, PipeScratch& sc,
                     const BatchOut& o, bool time_it) {
     if (h->n < 2) return F1L_ERR_NO_TRACK;
     const int S = in.S;
-    const float4* goals = in.goals;
-    const int C = goals ? in.n_goals : h->nL * h->nW;
-    if (C <= 0) return F1L_ERR_NO_GOALS;
-    int c_begin = in.c_begin > 0 ? in.c_begin : 0, c_end = in.c_end;
-    if (o.empty_shard) { c_begin = 0; c_end = 0; }
-    else {
-        if (c_end <= 0 || c_end > C) c_end = C;
-        if (c_begin >= c_end) return F1L_ERR_INVALID_ARG;
-    }
+    const Span& sp = in.span;
     if (in.max_opp > F1L_MAX_OPP || in.max_opp < 0) return F1L_ERR_INVALID_ARG;
     QueryCtx* ctx = (QueryCtx*)sc.ctx.p;
     Centre* centres = (Centre*)sc.centres.p;
@@ -585,7 +677,7 @@ int launch_pipeline(f1l_handle h, cudaStream_t stream, const PipeIn& in, PipeScr
     int nseg = h->cfg.window;
     if (nseg <= 0 || nseg > nsegs) nseg = nsegs;
     const int nseg_pad = (nseg + 31) & ~31;
-    const int n_cand = o.empty_shard ? 1 : c_end - c_begin;
+    const int n_cand = sp.empty ? 1 : sp.c_end - sp.c_begin;
     const CtaPlan cp = plan_ctas(n_cand, S, M, h->sm_count, ep.generator == 0);
     const int wpc = cp.nw;
     const EvalBucket& bucket = eval_bucket_of(M);
@@ -595,7 +687,7 @@ int launch_pipeline(f1l_handle h, cudaStream_t stream, const PipeIn& in, PipeScr
     // (the expensive candidates) first.  No wave quantisation, one window-table prologue per
     // resident CTA, and the cheap early-exit candidates fill the tail.
     int resident_ctas = build->minb * h->sm_count;
-    const bool dyn = S == 1 && wpc != 4 && o.work_next && !o.empty_shard &&
+    const bool dyn = S == 1 && wpc != 4 && in.work_next && !sp.empty &&
                      (long long)cp.ctas_per_scn > resident_ctas;
     // ... and with at least EVAL_WIDE_MIN candidates per resident warp it runs the 128-register
     // build of the M > 128 shapes on two CTAs per SM (measured on config 5: 65 536 candidates
@@ -619,14 +711,14 @@ int launch_pipeline(f1l_handle h, cudaStream_t stream, const PipeIn& in, PipeScr
     sa.n_opp = in.n_opp;
     sa.max_opp = in.max_opp;
     sa.lookaheads = (const double*)h->lookaheads.p;
-    sa.nL = goals ? 0 : h->nL;
-    sa.row0 = o.s_rows >= 0 ? o.s_row0 : 0;
-    sa.row_step = o.s_rows >= 0 ? o.s_step : 1;
-    sa.n_rows = o.s_rows >= 0 ? o.s_rows : h->nL;
+    sa.nL = in.goals ? 0 : h->nL;
+    sa.row0 = sp.s_row0;
+    sa.row_step = sp.s_step;
+    sa.n_rows = sp.s_rows;
     sa.ctx = ctx;
     sa.centres = centres;
     sa.best = best;
-    sa.work_next = dyn ? o.work_next : nullptr;
+    sa.work_next = dyn ? in.work_next : nullptr;
     cudaEvent_t* ev = h->ev + 4 * h->ev_next;
     if (time_it) cudaEventRecord(ev[0], stream);
     nvtxRangePushA("f1l.sample");
@@ -636,7 +728,7 @@ int launch_pipeline(f1l_handle h, cudaStream_t stream, const PipeIn& in, PipeScr
         PPOut po{};
         po.nearest = (double*)sc.near4.p;
         po.nearest_i = (int32_t*)sc.near_i.p;
-        launch_pp(sa.tr, stream, in.poses, 4, S, -1.0, 0.33, 0.0, 0, 0.0, best, pp_slots(h), po, ctab_valid(h), h);   // `best` doubles as K1's key scratch: the sampler resets it
+        launch_pp(h, stream, in.poses, 4, S, -1.0, 0.33, 0.0, 0, 0.0, best, po);   // `best` doubles as K1's key scratch: the sampler resets it
         sample_warp_kernel<<<(S + SAMPLE_WARPS - 1) / SAMPLE_WARPS, SAMPLE_WARPS * 32, 0, stream>>>(
             sa, po.nearest_i, po.nearest, S);
         h->launches += 2;
@@ -664,15 +756,15 @@ int launch_pipeline(f1l_handle h, cudaStream_t stream, const PipeIn& in, PipeScr
     ea.widths = (const float*)h->widths.p;
     ea.nL = h->nL;
     ea.nW = h->nW;
-    ea.goals = goals;
+    ea.goals = in.goals;
     ea.prev_theta = in.prev_theta;
     ea.prev_stride = in.prev_stride;
     ea.prev_valid = in.prev_valid;
-    ea.C = C;
-    ea.c_begin = c_begin;
-    ea.c_end = c_end;
-    ea.row0 = o.row0;
-    ea.row_step = o.row_step > 1 ? o.row_step : 1;
+    ea.C = sp.C;
+    ea.c_begin = sp.c_begin;
+    ea.c_end = sp.c_end;
+    ea.row0 = sp.row0;
+    ea.row_step = sp.row_step;
     ea.chunk = cp.chunk;
     ea.ctas_per_scn = cp.ctas_per_scn;
     // four candidates per warp at a time (shared Newton) when every warp has at least four
@@ -680,8 +772,8 @@ int launch_pipeline(f1l_handle h, cudaStream_t stream, const PipeIn& in, PipeScr
     ea.work_next = nullptr;
     ea.v_last = 0;
     if (dyn) {
-        ea.work_next = o.work_next;
-        ea.v_last = c_begin + c_end - 1;
+        ea.work_next = in.work_next;
+        ea.v_last = sp.c_begin + sp.c_end - 1;
         // single candidates per pull, unless every warp has at least four 4-candidate items to go
         // through: then the shared Newton solve pays more than the coarser tail costs
         ea.item = (ep.generator == 0 && (long long)n_cand >= 16LL * resident_ctas * wpc) ? EVAL_ITEM : 1;
@@ -700,16 +792,14 @@ int launch_pipeline(f1l_handle h, cudaStream_t stream, const PipeIn& in, PipeScr
     ea.stats = h->stats_on ? (unsigned long long*)h->stats.p : nullptr;
     const long long n_ctas = (long long)S * ea.ctas_per_scn;
     if (n_ctas > 0x7fffffffLL) return F1L_ERR_TOO_LARGE;
-    if (!o.empty_shard) build->fn<<<(unsigned)n_ctas, wpc * 32, smem, stream>>>(ea);
+    if (!sp.empty) build->fn<<<(unsigned)n_ctas, wpc * 32, smem, stream>>>(ea);
     {
         const int info[8] = {bucket.ipl, bucket.s, bucket.sg, wpc, build->minb, ea.chunk, ea.ctas_per_scn, ea.item};
         for (int i = 0; i < 8; ++i) h->eval_info[i] = info[i];
     }
     if (time_it) cudaEventRecord(ev[2], stream);
 
-    const SelectArgs se = select_args(h, sa.tr, ea.lut, ep, ctx, centres, goals, C,
-                                      o.row_step > 1 ? c_begin + o.row0 * h->nW : c_begin, best, S, o);
-    bucket.select<<<S, SELECT_THREADS, 0, stream>>>(se);
+    bucket.select<<<S, SELECT_THREADS, 0, stream>>>(select_args(h, in, sc, o));
     if (time_it) {
         cudaEventRecord(ev[3], stream);
         h->timed = 1;
@@ -728,7 +818,7 @@ struct QHeader {
     double steer, speed;                 // +0
     int32_t best_idx;                    // +16
     int32_t no_feasible, tracker_found;  // +20
-    int32_t pad;                         // +28
+    int32_t xchg_status;                 // +28 sharded query: != 0 when a peer did not arrive
     float best_cost;                     // +32
     float pad2[3];                       // -> 48 bytes, keeps the float4 trajectory 16-aligned
 };
@@ -966,10 +1056,8 @@ int f1l_create(f1l_handle* out, int device, const f1l_config* cfg) {
     cudaError_t e = cudaSetDevice(device);
     if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking);
     for (int i = 0; i < 4 * F1L_EV_SLOTS && e == cudaSuccess; ++i) e = cudaEventCreate(&h->ev[i]);
-    for (int i = 0; i < N_PIPE && e == cudaSuccess; ++i) {
+    for (int i = 0; i < N_PIPE && e == cudaSuccess; ++i)
         e = cudaStreamCreateWithFlags(&h->pipe[i].stream, cudaStreamNonBlocking);
-        if (e == cudaSuccess) e = cudaEventCreateWithFlags(&h->pipe[i].done, cudaEventDisableTiming);
-    }
     if (e == cudaSuccess) e = cudaHostAlloc(&h->h_in.p, 1024, cudaHostAllocDefault);
     if (e == cudaSuccess) e = cudaHostAlloc(&h->h_out.p, Q_RES_BYTES, cudaHostAllocMapped);
     // single queries write their results straight into h_out: no mapping, no handle
@@ -1014,11 +1102,8 @@ int f1l_destroy(f1l_handle h) {
     cudaSetDevice(h->device);
     cudaDeviceSynchronize();
     f1l_xchg_detach(h);
-    for (int i = 0; i < N_PIPE; ++i) {
-        PipeSlot& p = h->pipe[i];
-        if (p.done) cudaEventDestroy(p.done);
-        if (p.stream) cudaStreamDestroy(p.stream);
-    }
+    for (int i = 0; i < N_PIPE; ++i)
+        if (h->pipe[i].stream) cudaStreamDestroy(h->pipe[i].stream);
     if (h->gexec) cudaGraphExecDestroy(h->gexec);
     for (int i = 0; i < 4 * F1L_EV_SLOTS; ++i)
         if (h->ev[i]) cudaEventDestroy(h->ev[i]);
@@ -1233,16 +1318,17 @@ int f1l_clear_prev_path(f1l_handle h) {
 
 // ---- single query -------------------------------------------------------------------------
 static int plan_internal(f1l_handle h, const double pose[4], const double* opp, int n_opp,
-                         const double* goals, int n_goals, int c_begin, int c_end,
-                         int update_prev, f1l_plan_result* out, bool exchange = false,
-                         int row0 = 0, int row_step = 1) {
+                         const double* goals, int n_goals, const Shard& shard, bool exchange,
+                         int update_prev, f1l_plan_result* out) {
     if (!h || !pose || !out) return F1L_ERR_INVALID_ARG;
     if (n_opp < 0 || n_opp > F1L_MAX_OPP || (n_opp > 0 && !opp)) return F1L_ERR_INVALID_ARG;
     if (h->n < 2) return F1L_ERR_NO_TRACK;
     CK(cudaSetDevice(h->device));
-    const int C = goals ? n_goals : h->nL * h->nW;
-    if (C <= 0) return F1L_ERR_NO_GOALS;
-    const int M = h->cfg.n_samples;
+    exchange = exchange && h->xview.world > 1;
+    PipeIn in;
+    if (const int r = make_span(h, n_goals, shard, exchange, in.span); r != F1L_OK) return r;
+    const Span& sp = in.span;
+    const int C = sp.C, M = h->cfg.n_samples;
     cudaStream_t st = h->stream;
 
     NvtxRange nvtx_plan("f1l.plan (single query)");
@@ -1270,21 +1356,15 @@ static int plan_internal(f1l_handle h, const double pose[4], const double* opp, 
         h->epoch++;   // the captured graph holds the old staging address
     }
     char* ddet = (char*)h->q_detail.p;
-    if (out->states) ENS(h->q_states, (size_t)C * M * 16);
-    if (out->headings) ENS(h->q_headings, (size_t)C * M * 8);
-    const float4* d_goals = nullptr;
+    // the big optional arrays go straight into the caller's buffers
+    const Stage big[] = {{&h->q_states, nullptr, out->states, (size_t)M * 16},
+                         {&h->q_headings, nullptr, out->headings, (size_t)M * 8}};
+    if (const int r = stage_in(h, st, big, 0, C); r != F1L_OK) return r;
+    std::vector<float> g4;
     if (goals) {
-        std::vector<float> g4(4 * (size_t)C);
-        for (int c = 0; c < C; ++c) {
-            g4[4 * c] = (float)goals[3 * c];
-            g4[4 * c + 1] = (float)goals[3 * c + 1];
-            g4[4 * c + 2] = (float)goals[3 * c + 2];
-            g4[4 * c + 3] = 0.0f;
-        }
-        ENS(h->q_goals, (size_t)C * 16);
-        CK(cudaMemcpyAsync(h->q_goals.p, g4.data(), (size_t)C * 16, cudaMemcpyHostToDevice, st));
+        if (const int r = upload_goals(h, goals, C, g4, st); r != F1L_OK) return r;
         CK(cudaStreamSynchronize(st));  // g4 is a stack-lifetime staging buffer
-        d_goals = (const float4*)h->q_goals.p;
+        in.goals = (const float4*)h->q_goals.p;
     }
 
     // Results of a single query: the select kernel writes header and best trajectory straight into
@@ -1296,54 +1376,22 @@ static int plan_internal(f1l_handle h, const double pose[4], const double* opp, 
     o.flags = out->flags ? (uint8_t*)(ddet + off_flags) : nullptr;
     o.goals_out = out->goals ? (float*)(ddet + off_goals) : nullptr;
     o.params = out->params ? (float4*)(ddet + off_params) : nullptr;
-    o.states = out->states ? (float4*)h->q_states.p : nullptr;
-    o.headings = out->headings ? (float2*)h->q_headings.p : nullptr;
+    o.states = (float4*)big[0].dev();
+    o.headings = (float2*)big[1].dev();
     o.prev_out = update_prev ? (float*)h->prev.p : nullptr;
-    if (row_step > 1) {   // row-interleaved shard: rows row0, row0 + row_step, ... of the goal grid
-        if (goals || row0 < 0 || row0 >= row_step) return F1L_ERR_INVALID_ARG;
-        const int n_rows = row0 < h->nL ? (h->nL - row0 + row_step - 1) / row_step : 0;
-        // More ranks than lookahead rows: with peers attached the call is collective, so a rank
-        // without rows must still arrive at the exchange (it contributes key = ~0 and returns the
-        // global winner like everybody else); alone there is nothing to answer.
-        if (n_rows <= 0) {
-            if (!(exchange && h->xview.world > 1)) return F1L_ERR_INVALID_ARG;
-            o.empty_shard = true;
-        }
-        o.row0 = row0;
-        o.row_step = row_step;
-        c_begin = 0;
-        c_end = n_rows * h->nW;
-        o.s_row0 = row0 < h->nL ? row0 : 0;   // the sampler fills this shard's rows only
-        o.s_step = row_step;
-        o.s_rows = n_rows > 0 ? n_rows : 0;
-    } else if (!goals && h->nW > 0 && (c_begin > 0 || (c_end > 0 && c_end < C))) {
-        // contiguous candidate block: the lookahead rows it touches
-        const int cb = c_begin > 0 ? c_begin : 0, ce = (c_end > 0 && c_end < C) ? c_end : C;
-        if (cb < ce) {
-            o.s_row0 = cb / h->nW;
-            o.s_step = 1;
-            o.s_rows = (ce - 1) / h->nW - o.s_row0 + 1;
-        }
-    }
-    o.work_next = (int*)((char*)h->q_scratch.best.p + 8);   // behind the one argmin key
-    exchange = exchange && h->xview.world > 1;
     if (exchange) {   // the ranks' minima meet inside select_kernel (peer memory over NVLink)
-        o.xc = &h->xview;
-        o.xchg_status = (int32_t*)((char*)h->h_out_dev + offsetof(QHeader, pad));
+        in.xc = &h->xview;
+        o.xchg_status = (int32_t*)((char*)h->h_out_dev + offsetof(QHeader, xchg_status));
     }
-    const bool sharded = exchange || row_step > 1 || c_begin != 0 || (c_end > 0 && c_end < C);
+    const bool sharded = exchange || sp.row_step > 1 || sp.c_begin > 0 || sp.c_end < C;
     const QInput* din = (const QInput*)h->q_in.p;
-    PipeIn in;
     in.poses = din->pose;
     in.opp = din->opp;
     in.n_opp = &din->n_opp;
     in.S = 1;
     in.max_opp = F1L_MAX_OPP;
-    in.goals = d_goals;
-    in.n_goals = C;
-    in.c_begin = c_begin;
-    in.c_end = c_end;
     in.prev_theta = h->has_prev ? (const float*)h->prev.p : nullptr;
+    in.work_next = (int*)((char*)h->q_scratch.best.p + 8);   // behind the one argmin key
     // H2D of the input block, the three kernels, D2H of the detail block.  The similarity term
     // reads the previous path while select overwrites it: eval reads it before select runs
     // (stream order), so one buffer suffices.
@@ -1363,18 +1411,15 @@ static int plan_internal(f1l_handle h, const double pose[4], const double* opp, 
         return F1L_OK;
     };
     if (h->use_graph && !goals && !h->timing) {
-        // the whole chain as one CUDA graph, re-captured only when an upload / config change or
-        // the set of requested outputs alters a kernel argument
+        // the whole chain as one CUDA graph, re-captured only when an upload / config change, the
+        // set of requested outputs or the span (a constant of the captured kernels too) alters a
+        // kernel argument
         const unsigned long long mask = (want_detail ? 256u : 0u) | (out->terms ? 1u : 0u) | (out->flags ? 2u : 0u) |
                                         (out->goals ? 4u : 0u) | (out->params ? 8u : 0u) |
                                         (out->states ? 16u : 0u) | (out->headings ? 32u : 0u) |
                                         (update_prev ? 64u : 0u) | (h->has_prev ? 128u : 0u) |
                                         (exchange ? 512u : 0u) | (out->best_traj_map ? 1024u : 0u);
-        // a candidate shard is a constant of the captured kernels too
-        const unsigned long long shard_key = ((unsigned long long)(unsigned)c_begin << 32) | (unsigned)c_end;
-        const unsigned long long rows_key = ((unsigned long long)(unsigned)row_step << 32) | (unsigned)row0;
-        if (!h->gexec || h->gkey[0] != h->epoch || h->gkey[1] != mask || h->gkey[2] != shard_key ||
-            h->gkey[3] != rows_key) {
+        if (!h->gexec || h->gkey[0] != h->epoch || h->gkey[1] != mask || memcmp(&h->gspan, &sp, sizeof(Span))) {
             if (h->gexec) { cudaGraphExecDestroy(h->gexec); h->gexec = nullptr; }
             const int64_t launches0 = h->launches;
             cudaGraph_t graph = nullptr;
@@ -1389,8 +1434,7 @@ static int plan_internal(f1l_handle h, const double pose[4], const double* opp, 
             if (ce != cudaSuccess) { h->gexec = nullptr; return fail(h, ce, "cudaGraphInstantiate"); }
             h->gkey[0] = h->epoch;
             h->gkey[1] = mask;
-            h->gkey[2] = shard_key;
-            h->gkey[3] = rows_key;
+            h->gspan = sp;
         }
         CK(cudaGraphLaunch(h->gexec, st));
         h->launches += 3;
@@ -1399,20 +1443,15 @@ static int plan_internal(f1l_handle h, const double pose[4], const double* opp, 
         if (r != F1L_OK) return r;
     }
 
-    // the big optional arrays go straight into the caller's buffers
-    if (out->states) CK(cudaMemcpyAsync(out->states, h->q_states.p, (size_t)C * M * 16, cudaMemcpyDeviceToHost, st));
-    if (out->headings) CK(cudaMemcpyAsync(out->headings, h->q_headings.p, (size_t)C * M * 8, cudaMemcpyDeviceToHost, st));
+    if (const int r = stage_out(h, st, big, 0, C); r != F1L_OK) return r;
     CK(cudaStreamSynchronize(st));
     if (update_prev) {
         h->has_prev = 1;
         h->prev_m = M;
     }
-    if (exchange && ((const QHeader*)h->h_out.p)->pad != 0) return F1L_ERR_PEER_TIMEOUT;
-    h->lastq_C = C;
+    if (exchange && ((const QHeader*)h->h_out.p)->xchg_status != 0) return F1L_ERR_PEER_TIMEOUT;
+    h->lastq_span = sp;
     h->lastq_goals = goals != nullptr;
-    h->lastq_rows[0] = o.s_row0;
-    h->lastq_rows[1] = o.s_step;
-    h->lastq_rows[2] = o.s_rows;
     h->lastq_epoch = h->epoch;
     q_copy_result(h, C, out);
     if (want_detail) {
@@ -1428,51 +1467,47 @@ static int plan_internal(f1l_handle h, const double pose[4], const double* opp, 
 
 int f1l_plan(f1l_handle h, const double pose[4], const double* opp, int n_opp, int update_prev,
              f1l_plan_result* out) {
-    return plan_internal(h, pose, opp, n_opp, nullptr, 0, 0, 0, update_prev, out);
+    return plan_internal(h, pose, opp, n_opp, nullptr, 0, Shard{}, false, update_prev, out);
 }
 
 int f1l_plan_shard(f1l_handle h, const double pose[4], const double* opp, int n_opp, int c_begin,
                    int c_end, f1l_plan_result* out) {
     // with peers attached (f1l_xchg_attach) every rank returns the GLOBAL winner
-    return plan_internal(h, pose, opp, n_opp, nullptr, 0, c_begin, c_end, 0, out, true);
+    return plan_internal(h, pose, opp, n_opp, nullptr, 0, Shard{c_begin, c_end, 0, 1}, true, 0, out);
 }
 
 int f1l_plan_rows(f1l_handle h, const double pose[4], const double* opp, int n_opp, int row_begin,
                   int row_step, int update_prev, f1l_plan_result* out) {
     if (row_step < 1) return F1L_ERR_INVALID_ARG;
-    if (row_step == 1) return plan_internal(h, pose, opp, n_opp, nullptr, 0, 0, 0, update_prev, out, true);
-    return plan_internal(h, pose, opp, n_opp, nullptr, 0, 0, 0, update_prev, out, true, row_begin, row_step);
+    return plan_internal(h, pose, opp, n_opp, nullptr, 0, Shard{0, 0, row_begin, row_step}, true,
+                         update_prev, out);
 }
 
 int f1l_select_candidate(f1l_handle h, int idx, float cost, int update_prev, f1l_plan_result* out) {
     if (!h || !out) return F1L_ERR_INVALID_ARG;
     // the sampler context, goal centres / explicit goals of the last query must still be current
-    if (h->lastq_epoch != h->epoch || idx < 0 || idx >= h->lastq_C) return F1L_ERR_INVALID_ARG;
+    if (h->lastq_epoch != h->epoch || idx < 0 || idx >= h->lastq_span.C) return F1L_ERR_INVALID_ARG;
     CK(cudaSetDevice(h->device));
     cudaStream_t st = h->stream;
-    const int M = h->cfg.n_samples, C = h->lastq_C;
+    const int M = h->cfg.n_samples;
     unsigned long long* hkey = (unsigned long long*)h->h_in.p;   // pinned staging
     uint32_t cb;
     memcpy(&cb, &cost, 4);
     const uint32_t ord = (cb & 0x80000000u) ? ~cb : (cb | 0x80000000u);   // float_orderable
     *hkey = ((unsigned long long)ord << 32) | (unsigned)idx;
-    const PipeScratch& sc = h->q_scratch;
-    CK(cudaMemcpyAsync(sc.best.p, hkey, 8, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(h->q_scratch.best.p, hkey, 8, cudaMemcpyHostToDevice, st));
+    PipeIn in;
+    in.S = 1;
+    in.goals = h->lastq_goals ? (const float4*)h->q_goals.p : nullptr;
+    in.span = h->lastq_span;
     BatchOut o = q_result_out(h, out->best_traj_map != nullptr);
     o.prev_out = update_prev ? (float*)h->prev.p : nullptr;
-    o.s_row0 = h->lastq_rows[0];
-    o.s_step = h->lastq_rows[1];
-    o.s_rows = h->lastq_rows[2];
-    const SelectArgs se = select_args(h, track_view(h), lut_view(h), eval_params(h),
-                                      (const QueryCtx*)sc.ctx.p, (const Centre*)sc.centres.p,
-                                      h->lastq_goals ? (const float4*)h->q_goals.p : nullptr, C, 0,
-                                      (const unsigned long long*)sc.best.p, 1, o);
-    eval_bucket_of(M).select<<<1, SELECT_THREADS, 0, st>>>(se);
+    eval_bucket_of(M).select<<<1, SELECT_THREADS, 0, st>>>(select_args(h, in, h->q_scratch, o));
     h->launches += 1;
     CK(cudaGetLastError());
     CK(cudaStreamSynchronize(st));
     if (update_prev) { h->has_prev = 1; h->prev_m = M; }
-    q_copy_result(h, C, out);
+    q_copy_result(h, in.span.C, out);
     return F1L_OK;
 }
 
@@ -1535,7 +1570,7 @@ int f1l_xchg_detach(f1l_handle h) {
 int f1l_plan_goals(f1l_handle h, const double pose[4], const double* goals, int n_goals,
                    const double* opp, int n_opp, int update_prev, f1l_plan_result* out) {
     if (!goals || n_goals <= 0) return F1L_ERR_INVALID_ARG;
-    return plan_internal(h, pose, opp, n_opp, goals, n_goals, 0, 0, update_prev, out);
+    return plan_internal(h, pose, opp, n_opp, goals, n_goals, Shard{}, false, update_prev, out);
 }
 
 int f1l_generate(f1l_handle h, const double* goals, int n_goals, float* states, float* params,
@@ -1543,28 +1578,20 @@ int f1l_generate(f1l_handle h, const double* goals, int n_goals, float* states, 
     if (!h || !goals || n_goals <= 0 || !states) return F1L_ERR_INVALID_ARG;
     CK(cudaSetDevice(h->device));
     const int C = n_goals, M = h->cfg.n_samples;
-    std::vector<float> g4(4 * (size_t)C);
-    for (int c = 0; c < C; ++c) {
-        g4[4 * c] = (float)goals[3 * c];
-        g4[4 * c + 1] = (float)goals[3 * c + 1];
-        g4[4 * c + 2] = (float)goals[3 * c + 2];
-        g4[4 * c + 3] = 0.0f;
-    }
-    ENS(h->q_goals, (size_t)C * 16);
-    ENS(h->q_states, (size_t)C * M * 16);
-    ENS(h->q_params, (size_t)C * 16);
-    ENS(h->q_flags, (size_t)C);
     cudaStream_t st = h->stream;
-    CK(cudaMemcpyAsync(h->q_goals.p, g4.data(), (size_t)C * 16, cudaMemcpyHostToDevice, st));
+    const Stage t[] = {{&h->q_states, nullptr, states, (size_t)M * 16},
+                       {&h->q_params, nullptr, params, 16},
+                       {&h->q_flags, nullptr, flags, 1}};
+    if (const int r = stage_in(h, st, t, 0, C); r != F1L_OK) return r;
+    std::vector<float> g4;   // outlives the copy: the call ends in a synchronise
+    if (const int r = upload_goals(h, goals, C, g4, st); r != F1L_OK) return r;
     const int wpc = 8;
     eval_bucket_of(M).generate<<<(C + wpc - 1) / wpc, wpc * 32, 0, st>>>(
-        lut_view(h), eval_params(h), (const float4*)h->q_goals.p, C, (float4*)h->q_states.p,
-        (float4*)h->q_params.p, (uint8_t*)h->q_flags.p);
+        lut_view(h), eval_params(h), (const float4*)h->q_goals.p, C, (float4*)t[0].dev(),
+        (float4*)t[1].dev(), (uint8_t*)t[2].dev());
     h->launches += 1;
     CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(states, h->q_states.p, (size_t)C * M * 16, cudaMemcpyDeviceToHost, st));
-    if (params) CK(cudaMemcpyAsync(params, h->q_params.p, (size_t)C * 16, cudaMemcpyDeviceToHost, st));
-    if (flags) CK(cudaMemcpyAsync(flags, h->q_flags.p, (size_t)C, cudaMemcpyDeviceToHost, st));
+    if (const int r = stage_out(h, st, t, 0, C); r != F1L_OK) return r;
     CK(cudaStreamSynchronize(st));
     return F1L_OK;
 }
@@ -1574,43 +1601,45 @@ int f1l_generate(f1l_handle h, const double* goals, int n_goals, float* states, 
 // select kernel overwrites them in place with each scenario's best trajectory.  That is safe:
 // eval_kernel reads a scenario's path in its prologue, and select_kernel writes it in a later
 // kernel on the same stream.
-static int plan_batch_dev_internal(f1l_handle h, const double* poses_dev, const double* opp_dev,
-                                   const int32_t* n_opp_dev, int S, int max_opp, float* prev_theta_dev,
-                                   uint8_t* has_prev_dev, int update_prev, int32_t* best_idx_dev,
-                                   float* best_cost_dev, float* best_traj_dev, float* costs_dev,
-                                   uint8_t* flags_dev, double* steer_speed_dev, void* stream) {
-    if (!h || !poses_dev || S <= 0) return F1L_ERR_INVALID_ARG;
-    if (max_opp > 0 && !opp_dev) return F1L_ERR_INVALID_ARG;
-    if ((update_prev || has_prev_dev) && !prev_theta_dev) return F1L_ERR_INVALID_ARG;
-    CK(cudaSetDevice(h->device));
-    if (h->nL * h->nW <= 0) return F1L_ERR_NO_GOALS;
-    if (const int r = h->b_scratch.reserve(h, S); r != F1L_OK) return r;
-    PipeIn in;
-    in.poses = poses_dev;
-    in.opp = max_opp > 0 ? opp_dev : nullptr;
-    in.n_opp = n_opp_dev;
+// The arguments of a batch call over the whole goal grid, checked; device or host pointers alike
+static int batch_args(f1l_handle h, const double* poses, const double* opp, const int32_t* n_opp, int S,
+                      int max_opp, float* prev_theta, uint8_t* has_prev, int update_prev, int32_t* best_idx,
+                      float* best_cost, float* best_traj, float* costs, uint8_t* flags, double* steer_speed,
+                      PipeIn& in, BatchOut& o) {
+    if (!h || !poses || S <= 0) return F1L_ERR_INVALID_ARG;
+    if (max_opp > 0 && !opp) return F1L_ERR_INVALID_ARG;
+    if ((update_prev || has_prev) && !prev_theta) return F1L_ERR_INVALID_ARG;
+    if (const int r = make_span(h, 0, Shard{}, false, in.span); r != F1L_OK) return r;
+    in.poses = poses;
+    in.opp = max_opp > 0 ? opp : nullptr;
+    in.n_opp = n_opp;
     in.S = S;
     in.max_opp = max_opp;
-    in.prev_theta = prev_theta_dev;
+    in.prev_theta = prev_theta;
     in.prev_stride = h->cfg.n_samples;
-    in.prev_valid = has_prev_dev;
-    BatchOut o;
-    o.best_idx = best_idx_dev;
-    o.best_cost = best_cost_dev;
-    o.best_traj = (float4*)best_traj_dev;
-    o.costs = costs_dev;
-    o.flags = flags_dev;
-    o.steer_speed = steer_speed_dev;
-    o.prev_out = update_prev ? prev_theta_dev : nullptr;
-    o.prev_valid_out = update_prev ? has_prev_dev : nullptr;
-    return launch_pipeline(h, (cudaStream_t)stream, in, h->b_scratch, o, h->timing != 0);
+    in.prev_valid = has_prev;
+    o.best_idx = best_idx;
+    o.best_cost = best_cost;
+    o.best_traj = (float4*)best_traj;
+    o.costs = costs;
+    o.flags = flags;
+    o.steer_speed = steer_speed;
+    o.prev_out = update_prev ? prev_theta : nullptr;
+    o.prev_valid_out = update_prev ? has_prev : nullptr;
+    return F1L_OK;
+}
+
+static int plan_batch_dev_internal(f1l_handle h, const PipeIn& in, const BatchOut& o, cudaStream_t stream) {
+    CK(cudaSetDevice(h->device));
+    if (const int r = h->b_scratch.reserve(h, in.S); r != F1L_OK) return r;
+    return launch_pipeline(h, stream, in, h->b_scratch, o, h->timing != 0);
 }
 
 int f1l_plan_batch_dev(f1l_handle h, const double* poses_dev, const double* opp_dev,
                        const int32_t* n_opp_dev, int S, int max_opp, int32_t* best_idx_dev,
                        float* best_cost_dev, float* best_traj_dev, float* costs_dev,
                        uint8_t* flags_dev, double* steer_speed_dev, void* stream) {
-    return plan_batch_dev_internal(h, poses_dev, opp_dev, n_opp_dev, S, max_opp, nullptr, nullptr, 0,
+    return f1l_plan_batch_prev_dev(h, poses_dev, opp_dev, n_opp_dev, S, max_opp, nullptr, nullptr, 0,
                                    best_idx_dev, best_cost_dev, best_traj_dev, costs_dev, flags_dev,
                                    steer_speed_dev, stream);
 }
@@ -1620,22 +1649,18 @@ int f1l_plan_batch_prev_dev(f1l_handle h, const double* poses_dev, const double*
                             uint8_t* has_prev_dev, int update_prev, int32_t* best_idx_dev,
                             float* best_cost_dev, float* best_traj_dev, float* costs_dev,
                             uint8_t* flags_dev, double* steer_speed_dev, void* stream) {
-    return plan_batch_dev_internal(h, poses_dev, opp_dev, n_opp_dev, S, max_opp, prev_theta_dev,
-                                   has_prev_dev, update_prev, best_idx_dev, best_cost_dev, best_traj_dev,
-                                   costs_dev, flags_dev, steer_speed_dev, stream);
+    PipeIn in;
+    BatchOut o;
+    const int r = batch_args(h, poses_dev, opp_dev, n_opp_dev, S, max_opp, prev_theta_dev, has_prev_dev,
+                             update_prev, best_idx_dev, best_cost_dev, best_traj_dev, costs_dev, flags_dev,
+                             steer_speed_dev, in, o);
+    return r != F1L_OK ? r : plan_batch_dev_internal(h, in, o, (cudaStream_t)stream);
 }
 
-static int plan_batch_internal(f1l_handle h, const double* poses, const double* opp, const int32_t* n_opp,
-                               int S, int max_opp, float* prev_theta, uint8_t* has_prev, int update_prev,
-                               int32_t* best_idx, float* best_cost, float* best_traj, float* costs,
-                               uint8_t* flags, double* steer_speed) {
-    if (!h || !poses || S <= 0) return F1L_ERR_INVALID_ARG;
-    if (max_opp > 0 && !opp) return F1L_ERR_INVALID_ARG;
-    if ((update_prev || has_prev) && !prev_theta) return F1L_ERR_INVALID_ARG;
+// `in` and `o` hold host pointers: each chunk is copied in, planned and copied back on a slot stream
+static int plan_batch_internal(f1l_handle h, const PipeIn& in, const BatchOut& o) {
     CK(cudaSetDevice(h->device));
-    const int C = h->nL * h->nW;
-    if (C <= 0) return F1L_ERR_NO_GOALS;
-    const int M = h->cfg.n_samples;
+    const int S = in.S, C = in.span.C, M = h->cfg.n_samples;
     // chunked 3-stream pipeline: H2D(i+1) | kernels(i) | D2H(i-1)
     // 8192-scenario chunks (0.23 M candidates: 1 ms of kernels against ~30 us of launches) for
     // large batches; smaller batches are cut into about eight chunks, down to 1024 scenarios.  The
@@ -1654,59 +1679,33 @@ static int plan_batch_internal(f1l_handle h, const double* poses, const double* 
         PipeSlot& p = h->pipe[slot];
         cudaStream_t st = p.stream;
         CK(cudaStreamSynchronize(st));  // slot buffers free again (grow-only ensure below)
-        ENS(p.poses, (size_t)n * 32);
-        if (max_opp > 0) ENS(p.opp, (size_t)n * max_opp * 24);
-        if (n_opp) ENS(p.nopp, (size_t)n * 4);
         if (const int r = p.scratch.reserve(h, n); r != F1L_OK) return r;
-        if (best_idx) ENS(p.idx, (size_t)n * 4);
-        if (best_cost) ENS(p.cost, (size_t)n * 4);
-        if (best_traj) ENS(p.traj, (size_t)n * M * 16);
-        if (costs) ENS(p.costs, (size_t)n * C * 4);
-        if (flags) ENS(p.flags, (size_t)n * C);
-        if (steer_speed) ENS(p.ss, (size_t)n * 16);
-        if (prev_theta) ENS(p.prev, (size_t)n * M * 4);
-        if (has_prev) ENS(p.pvalid, (size_t)n);
-        CK(cudaMemcpyAsync(p.poses.p, poses + 4 * (size_t)s0, (size_t)n * 32, cudaMemcpyHostToDevice, st));
-        if (max_opp > 0)
-            CK(cudaMemcpyAsync(p.opp.p, opp + 3 * (size_t)max_opp * s0, (size_t)n * max_opp * 24,
-                               cudaMemcpyHostToDevice, st));
-        if (n_opp) CK(cudaMemcpyAsync(p.nopp.p, n_opp + s0, (size_t)n * 4, cudaMemcpyHostToDevice, st));
-        if (prev_theta)
-            CK(cudaMemcpyAsync(p.prev.p, prev_theta + (size_t)M * s0, (size_t)n * M * 4, cudaMemcpyHostToDevice, st));
-        if (has_prev) CK(cudaMemcpyAsync(p.pvalid.p, has_prev + s0, (size_t)n, cudaMemcpyHostToDevice, st));
-        BatchOut o;
-        o.best_idx = best_idx ? (int32_t*)p.idx.p : nullptr;
-        o.best_cost = best_cost ? (float*)p.cost.p : nullptr;
-        o.best_traj = best_traj ? (float4*)p.traj.p : nullptr;
-        o.costs = costs ? (float*)p.costs.p : nullptr;
-        o.flags = flags ? (uint8_t*)p.flags.p : nullptr;
-        o.steer_speed = steer_speed ? (double*)p.ss.p : nullptr;
-        // in place on the slot's copies, as in plan_batch_dev_internal
-        o.prev_out = update_prev ? (float*)p.prev.p : nullptr;
-        o.prev_valid_out = update_prev && has_prev ? (uint8_t*)p.pvalid.p : nullptr;
-        PipeIn in;
-        in.poses = (const double*)p.poses.p;
-        in.opp = max_opp > 0 ? (const double*)p.opp.p : nullptr;
-        in.n_opp = n_opp ? (const int32_t*)p.nopp.p : nullptr;
-        in.S = n;
-        in.max_opp = max_opp;
-        in.prev_theta = prev_theta ? (const float*)p.prev.p : nullptr;
-        in.prev_stride = M;
-        in.prev_valid = has_prev ? (const uint8_t*)p.pvalid.p : nullptr;
-        int r = launch_pipeline(h, st, in, p.scratch, o, false);
+        // the chunk's arrays: the previous paths travel in and, with update_prev, back out
+        const Stage t[B_ARRAYS] = {
+            {&p.buf[B_POSES], in.poses, nullptr, 32},
+            {&p.buf[B_OPP], in.opp, nullptr, (size_t)in.max_opp * 24},
+            {&p.buf[B_NOPP], in.n_opp, nullptr, 4},
+            {&p.buf[B_IDX], nullptr, o.best_idx, 4},
+            {&p.buf[B_COST], nullptr, o.best_cost, 4},
+            {&p.buf[B_TRAJ], nullptr, o.best_traj, (size_t)M * 16},
+            {&p.buf[B_COSTS], nullptr, o.costs, (size_t)C * 4},
+            {&p.buf[B_FLAGS], nullptr, o.flags, (size_t)C},
+            {&p.buf[B_SS], nullptr, o.steer_speed, 16},
+            {&p.buf[B_PREV], in.prev_theta, o.prev_out, (size_t)M * 4},
+            {&p.buf[B_PVALID], in.prev_valid, o.prev_valid_out, 1},
+        };
+        if (const int r = stage_in(h, st, t, s0, n); r != F1L_OK) return r;
+        // the chunk is a batch call of n scenarios on the slot's copies (updated in place)
+        PipeIn din;
+        BatchOut dout;
+        int r = batch_args(h, (const double*)t[B_POSES].dev(), (const double*)t[B_OPP].dev(),
+                           (const int32_t*)t[B_NOPP].dev(), n, in.max_opp, (float*)t[B_PREV].dev(),
+                           (uint8_t*)t[B_PVALID].dev(), o.prev_out != nullptr, (int32_t*)t[B_IDX].dev(),
+                           (float*)t[B_COST].dev(), (float*)t[B_TRAJ].dev(), (float*)t[B_COSTS].dev(),
+                           (uint8_t*)t[B_FLAGS].dev(), (double*)t[B_SS].dev(), din, dout);
+        if (r == F1L_OK) r = launch_pipeline(h, st, din, p.scratch, dout, false);
+        if (r == F1L_OK) r = stage_out(h, st, t, s0, n);
         if (r != F1L_OK) return r;
-        if (best_idx) CK(cudaMemcpyAsync(best_idx + s0, p.idx.p, (size_t)n * 4, cudaMemcpyDeviceToHost, st));
-        if (best_cost) CK(cudaMemcpyAsync(best_cost + s0, p.cost.p, (size_t)n * 4, cudaMemcpyDeviceToHost, st));
-        if (best_traj)
-            CK(cudaMemcpyAsync(best_traj + 4 * (size_t)M * s0, p.traj.p, (size_t)n * M * 16,
-                               cudaMemcpyDeviceToHost, st));
-        if (costs) CK(cudaMemcpyAsync(costs + (size_t)C * s0, p.costs.p, (size_t)n * C * 4, cudaMemcpyDeviceToHost, st));
-        if (flags) CK(cudaMemcpyAsync(flags + (size_t)C * s0, p.flags.p, (size_t)n * C, cudaMemcpyDeviceToHost, st));
-        if (steer_speed) CK(cudaMemcpyAsync(steer_speed + 2 * (size_t)s0, p.ss.p, (size_t)n * 16, cudaMemcpyDeviceToHost, st));
-        if (update_prev) {
-            CK(cudaMemcpyAsync(prev_theta + (size_t)M * s0, p.prev.p, (size_t)n * M * 4, cudaMemcpyDeviceToHost, st));
-            if (has_prev) CK(cudaMemcpyAsync(has_prev + s0, p.pvalid.p, (size_t)n, cudaMemcpyDeviceToHost, st));
-        }
     }
     for (int i = 0; i < N_PIPE; ++i) CK(cudaStreamSynchronize(h->pipe[i].stream));
     return F1L_OK;
@@ -1715,7 +1714,7 @@ static int plan_batch_internal(f1l_handle h, const double* poses, const double* 
 int f1l_plan_batch(f1l_handle h, const double* poses, const double* opp, const int32_t* n_opp,
                    int S, int max_opp, int32_t* best_idx, float* best_cost, float* best_traj,
                    float* costs, uint8_t* flags, double* steer_speed) {
-    return plan_batch_internal(h, poses, opp, n_opp, S, max_opp, nullptr, nullptr, 0, best_idx, best_cost,
+    return f1l_plan_batch_prev(h, poses, opp, n_opp, S, max_opp, nullptr, nullptr, 0, best_idx, best_cost,
                                best_traj, costs, flags, steer_speed);
 }
 
@@ -1723,8 +1722,11 @@ int f1l_plan_batch_prev(f1l_handle h, const double* poses, const double* opp, co
                         int S, int max_opp, float* prev_theta, uint8_t* has_prev, int update_prev,
                         int32_t* best_idx, float* best_cost, float* best_traj, float* costs,
                         uint8_t* flags, double* steer_speed) {
-    return plan_batch_internal(h, poses, opp, n_opp, S, max_opp, prev_theta, has_prev, update_prev, best_idx,
-                               best_cost, best_traj, costs, flags, steer_speed);
+    PipeIn in;
+    BatchOut o;
+    const int r = batch_args(h, poses, opp, n_opp, S, max_opp, prev_theta, has_prev, update_prev, best_idx,
+                             best_cost, best_traj, costs, flags, steer_speed, in, o);
+    return r != F1L_OK ? r : plan_batch_internal(h, in, o);
 }
 
 // ---- closed-loop rollouts -----------------------------------------------------------------
@@ -1751,7 +1753,8 @@ int f1l_rollout_dev(f1l_handle h, const f1l_rollout_config* rc, const f1l_fleet*
         return F1L_ERR_INVALID_ARG;
     if (n_steps == 0) return F1L_OK;
     if (h->n < 2) return F1L_ERR_NO_TRACK;
-    if (h->nL * h->nW <= 0) return F1L_ERR_NO_GOALS;
+    PipeIn in;
+    if (const int r = make_span(h, 0, Shard{}, false, in.span); r != F1L_OK) return r;
     CK(cudaSetDevice(h->device));
     ENS(h->r_ss, (size_t)S * 16);
     ENS(h->r_cost, (size_t)S * 4);
@@ -1797,8 +1800,7 @@ int f1l_rollout_dev(f1l_handle h, const f1l_rollout_config* rc, const f1l_fleet*
     PPOut po{};
     po.nearest = (double*)sc.near4.p;
     po.nearest_i = (int32_t*)sc.near_i.p;
-    launch_pp(a.tr, st, fl->state, 4, S, -1.0, h->cfg.wheelbase, 0.0, 0, 0.0,
-              (unsigned long long*)sc.best.p, pp_slots(h), po, ctab_valid(h), h);
+    launch_pp(h, st, fl->state, 4, S, -1.0, h->cfg.wheelbase, 0.0, 0, 0.0, (unsigned long long*)sc.best.p, po);
     a.near_i = po.nearest_i;
     a.near4 = po.nearest;
     rollout_step_kernel<<<blocks, ROLLOUT_WARPS * 32, 0, st>>>(a);
@@ -1808,13 +1810,24 @@ int f1l_rollout_dev(f1l_handle h, const f1l_rollout_config* rc, const f1l_fleet*
     a.near4 = nullptr;
     a.steer_speed = (const double*)h->r_ss.p;
     a.best_cost = (const float*)h->r_cost.p;
+    // every step plans the fleet as f1l_plan_batch_prev_dev with update_prev does
+    in.poses = fl->state;
+    in.opp = a.opp;
+    in.n_opp = a.n_opp;
+    in.S = S;
+    in.max_opp = F1L_MAX_OPP;
+    in.prev_theta = fl->prev_theta;
+    in.prev_stride = h->cfg.n_samples;
+    in.prev_valid = fl->has_prev;
+    BatchOut o;
+    o.best_cost = (float*)h->r_cost.p;
+    o.steer_speed = (double*)h->r_ss.p;
+    o.prev_out = fl->prev_theta;
+    o.prev_valid_out = fl->has_prev;
     for (int k = 0; k < n_steps; ++k) {
         const size_t row = (size_t)k * S;
-        int32_t* best_idx = trace && trace->best_idx ? trace->best_idx + row : nullptr;
-        const int r = plan_batch_dev_internal(h, fl->state, a.opp, a.n_opp, S, F1L_MAX_OPP, fl->prev_theta,
-                                              fl->has_prev, 1, best_idx, (float*)h->r_cost.p, nullptr,
-                                              nullptr, nullptr, (double*)h->r_ss.p, stream);
-        if (r != F1L_OK) return r;
+        o.best_idx = trace && trace->best_idx ? trace->best_idx + row : nullptr;
+        if (const int r = plan_batch_dev_internal(h, in, o, st); r != F1L_OK) return r;
         a.tr_state = trace && trace->state ? trace->state + 4 * row : nullptr;
         a.tr_ss = trace && trace->steer_speed ? trace->steer_speed + 2 * row : nullptr;
         a.tr_status = trace && trace->status ? trace->status + row : nullptr;
@@ -1843,8 +1856,8 @@ int f1l_pure_pursuit_batch_dev(f1l_handle h, const double* poses_dev, int n_pose
     o.actuation = actuation_dev;
     o.status = status_dev;
     ENS(h->pp_key, (size_t)n_poses * 8);   // scan scratch (one call in flight per handle)
-    launch_pp(track_view(h), (cudaStream_t)stream, poses_dev, 3, n_poses, L, h->cfg.wheelbase,
-              h->cfg.max_reacquire, 0, 0.0, (unsigned long long*)h->pp_key.p, pp_slots(h), o, ctab_valid(h), h);
+    launch_pp(h, (cudaStream_t)stream, poses_dev, 3, n_poses, L, h->cfg.wheelbase, h->cfg.max_reacquire, 0,
+              0.0, (unsigned long long*)h->pp_key.p, o);
     h->launches += 2;
     CK(cudaGetLastError());
     return F1L_OK;
@@ -1856,26 +1869,17 @@ int f1l_pure_pursuit_batch(f1l_handle h, const double* poses, int n, double L, d
     if (!h || !poses || n <= 0) return F1L_ERR_INVALID_ARG;
     CK(cudaSetDevice(h->device));
     cudaStream_t st = h->stream;
-    ENS(h->m_in, (size_t)n * 24);
-    if (nearest) ENS(h->m_o0, (size_t)n * 32);
-    if (nearest_i) ENS(h->m_o1, (size_t)n * 4);
-    if (lookahead) ENS(h->m_o2, (size_t)n * 32);
-    if (lookahead_i) ENS(h->m_o3, (size_t)n * 4);
-    if (actuation) ENS(h->m_o4, (size_t)n * 16);
-    if (status) ENS(h->m_o5, (size_t)n * 4);
-    CK(cudaMemcpyAsync(h->m_in.p, poses, (size_t)n * 24, cudaMemcpyHostToDevice, st));
-    int r = f1l_pure_pursuit_batch_dev(
-        h, (const double*)h->m_in.p, n, L, nearest ? (double*)h->m_o0.p : nullptr,
-        nearest_i ? (int32_t*)h->m_o1.p : nullptr, lookahead ? (double*)h->m_o2.p : nullptr,
-        lookahead_i ? (int32_t*)h->m_o3.p : nullptr, actuation ? (double*)h->m_o4.p : nullptr,
-        status ? (int32_t*)h->m_o5.p : nullptr, st);
+    const Stage t[] = {{&h->m[0], poses, nullptr, 24},       {&h->m[1], nullptr, nearest, 32},
+                       {&h->m[2], nullptr, nearest_i, 4},    {&h->m[3], nullptr, lookahead, 32},
+                       {&h->m[4], nullptr, lookahead_i, 4},  {&h->m[5], nullptr, actuation, 16},
+                       {&h->m[6], nullptr, status, 4}};
+    int r = stage_in(h, st, t, 0, n);
+    if (r == F1L_OK)
+        r = f1l_pure_pursuit_batch_dev(h, (const double*)t[0].dev(), n, L, (double*)t[1].dev(),
+                                       (int32_t*)t[2].dev(), (double*)t[3].dev(), (int32_t*)t[4].dev(),
+                                       (double*)t[5].dev(), (int32_t*)t[6].dev(), st);
+    if (r == F1L_OK) r = stage_out(h, st, t, 0, n);
     if (r != F1L_OK) return r;
-    if (nearest) CK(cudaMemcpyAsync(nearest, h->m_o0.p, (size_t)n * 32, cudaMemcpyDeviceToHost, st));
-    if (nearest_i) CK(cudaMemcpyAsync(nearest_i, h->m_o1.p, (size_t)n * 4, cudaMemcpyDeviceToHost, st));
-    if (lookahead) CK(cudaMemcpyAsync(lookahead, h->m_o2.p, (size_t)n * 32, cudaMemcpyDeviceToHost, st));
-    if (lookahead_i) CK(cudaMemcpyAsync(lookahead_i, h->m_o3.p, (size_t)n * 4, cudaMemcpyDeviceToHost, st));
-    if (actuation) CK(cudaMemcpyAsync(actuation, h->m_o4.p, (size_t)n * 16, cudaMemcpyDeviceToHost, st));
-    if (status) CK(cudaMemcpyAsync(status, h->m_o5.p, (size_t)n * 4, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
     return F1L_OK;
 }
@@ -1890,8 +1894,8 @@ int f1l_front_axle_batch_dev(f1l_handle h, const double* poses_dev, int n_poses,
     o.nearest_i = nearest_i_dev;
     o.front = front_dev;
     ENS(h->pp_key, (size_t)n_poses * 8);
-    launch_pp(track_view(h), (cudaStream_t)stream, poses_dev, 4, n_poses, 0.0, wheelbase, 0.0, 1,
-              k_path, (unsigned long long*)h->pp_key.p, pp_slots(h), o, ctab_valid(h), h);
+    launch_pp(h, (cudaStream_t)stream, poses_dev, 4, n_poses, 0.0, wheelbase, 0.0, 1, k_path,
+              (unsigned long long*)h->pp_key.p, o);
     h->launches += 2;
     CK(cudaGetLastError());
     return F1L_OK;
@@ -1902,15 +1906,14 @@ int f1l_front_axle_batch(f1l_handle h, const double* poses, int n, double wheelb
     if (!h || !poses || n <= 0 || !front) return F1L_ERR_INVALID_ARG;
     CK(cudaSetDevice(h->device));
     cudaStream_t st = h->stream;
-    ENS(h->m_in, (size_t)n * 32);
-    ENS(h->m_o0, (size_t)n * 48);
-    if (nearest_i) ENS(h->m_o1, (size_t)n * 4);
-    CK(cudaMemcpyAsync(h->m_in.p, poses, (size_t)n * 32, cudaMemcpyHostToDevice, st));
-    int r = f1l_front_axle_batch_dev(h, (const double*)h->m_in.p, n, wheelbase, k_path,
-                                     (double*)h->m_o0.p, nearest_i ? (int32_t*)h->m_o1.p : nullptr, st);
+    const Stage t[] = {{&h->m[0], poses, nullptr, 32}, {&h->m[1], nullptr, front, 48},
+                       {&h->m[2], nullptr, nearest_i, 4}};
+    int r = stage_in(h, st, t, 0, n);
+    if (r == F1L_OK)
+        r = f1l_front_axle_batch_dev(h, (const double*)t[0].dev(), n, wheelbase, k_path, (double*)t[1].dev(),
+                                     (int32_t*)t[2].dev(), st);
+    if (r == F1L_OK) r = stage_out(h, st, t, 0, n);
     if (r != F1L_OK) return r;
-    CK(cudaMemcpyAsync(front, h->m_o0.p, (size_t)n * 48, cudaMemcpyDeviceToHost, st));
-    if (nearest_i) CK(cudaMemcpyAsync(nearest_i, h->m_o1.p, (size_t)n * 4, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
     return F1L_OK;
 }
@@ -1925,19 +1928,15 @@ int f1l_intersect_point_batch(f1l_handle h, const double* points, const double* 
         if (!(t_start[i] >= 0.0 && t_start[i] < (double)h->n)) return F1L_ERR_INVALID_ARG;
     CK(cudaSetDevice(h->device));
     cudaStream_t st = h->stream;
-    ENS(h->m_in, (size_t)n * 16);
-    ENS(h->m_in2, (size_t)n * 8);
-    ENS(h->m_o0, (size_t)n * 32);
-    ENS(h->m_o1, (size_t)n * 4);
-    CK(cudaMemcpyAsync(h->m_in.p, points, (size_t)n * 16, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(h->m_in2.p, t_start, (size_t)n * 8, cudaMemcpyHostToDevice, st));
+    const Stage t[] = {{&h->m[0], points, nullptr, 16}, {&h->m[1], t_start, nullptr, 8},
+                       {&h->m[2], nullptr, out, 32}, {&h->m[3], nullptr, out_i, 4}};
+    if (const int r = stage_in(h, st, t, 0, n); r != F1L_OK) return r;
     intersect_batch_kernel<<<(n + 63) / 64, 64, 0, st>>>(
-        track_view(h), (const double*)h->m_in.p, (const double*)h->m_in2.p, n, radius, wrap,
-        (double*)h->m_o0.p, (int32_t*)h->m_o1.p);
+        track_view(h), (const double*)t[0].dev(), (const double*)t[1].dev(), n, radius, wrap,
+        (double*)t[2].dev(), (int32_t*)t[3].dev());
     h->launches += 1;
     CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(out, h->m_o0.p, (size_t)n * 32, cudaMemcpyDeviceToHost, st));
-    CK(cudaMemcpyAsync(out_i, h->m_o1.p, (size_t)n * 4, cudaMemcpyDeviceToHost, st));
+    if (const int r = stage_out(h, st, t, 0, n); r != F1L_OK) return r;
     CK(cudaStreamSynchronize(st));
     return F1L_OK;
 }
@@ -1946,14 +1945,13 @@ int f1l_get_actuation_batch(f1l_handle h, const double* in, int n, double wheelb
     if (!h || !in || n <= 0 || !out) return F1L_ERR_INVALID_ARG;
     CK(cudaSetDevice(h->device));
     cudaStream_t st = h->stream;
-    ENS(h->m_in, (size_t)n * 56);
-    ENS(h->m_o0, (size_t)n * 16);
-    CK(cudaMemcpyAsync(h->m_in.p, in, (size_t)n * 56, cudaMemcpyHostToDevice, st));
-    actuation_batch_kernel<<<(n + 63) / 64, 64, 0, st>>>((const double*)h->m_in.p, n, wheelbase,
-                                                         (double*)h->m_o0.p);
+    const Stage t[] = {{&h->m[0], in, nullptr, 56}, {&h->m[1], nullptr, out, 16}};
+    if (const int r = stage_in(h, st, t, 0, n); r != F1L_OK) return r;
+    actuation_batch_kernel<<<(n + 63) / 64, 64, 0, st>>>((const double*)t[0].dev(), n, wheelbase,
+                                                         (double*)t[1].dev());
     h->launches += 1;
     CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(out, h->m_o0.p, (size_t)n * 16, cudaMemcpyDeviceToHost, st));
+    if (const int r = stage_out(h, st, t, 0, n); r != F1L_OK) return r;
     CK(cudaStreamSynchronize(st));
     return F1L_OK;
 }
@@ -2025,13 +2023,13 @@ int f1l_bind_host_numa(int device) {
 int f1l_measure_peaks(f1l_handle h, double* fp32_tflops, double* mufu_gops) {
     if (!h) return F1L_ERR_INVALID_ARG;
     CK(cudaSetDevice(h->device));
-    ENS(h->m_o0, (size_t)h->sm_count * 8 * 256 * 4);
+    ENS(h->m[0], (size_t)h->sm_count * 8 * 256 * 4);
     cudaStream_t st = h->stream;
     const int blocks = h->sm_count * 8, threads = 256, iters = 4096;
     float ms = 0.f;
     for (int rep = 0; rep < 3; ++rep) {
         CK(cudaEventRecord(h->ev[0], st));
-        ffma_peak_kernel<<<blocks, threads, 0, st>>>((float*)h->m_o0.p, iters, 1.0001f, 0.5f);
+        ffma_peak_kernel<<<blocks, threads, 0, st>>>((float*)h->m[0].p, iters, 1.0001f, 0.5f);
         CK(cudaEventRecord(h->ev[1], st));
         CK(cudaStreamSynchronize(st));
         CK(cudaEventElapsedTime(&ms, h->ev[0], h->ev[1]));
@@ -2041,7 +2039,7 @@ int f1l_measure_peaks(f1l_handle h, double* fp32_tflops, double* mufu_gops) {
         *fp32_tflops = 2.0 * PEAK_CHAINS * (double)iters * blocks * threads / (ms * 1e-3) / 1e12;
     for (int rep = 0; rep < 3; ++rep) {
         CK(cudaEventRecord(h->ev[0], st));
-        mufu_peak_kernel<<<blocks, threads, 0, st>>>((float*)h->m_o0.p, iters);
+        mufu_peak_kernel<<<blocks, threads, 0, st>>>((float*)h->m[0].p, iters);
         CK(cudaEventRecord(h->ev[1], st));
         CK(cudaStreamSynchronize(st));
         CK(cudaEventElapsedTime(&ms, h->ev[0], h->ev[1]));
@@ -2064,7 +2062,7 @@ int f1l_measure_peaks_ex(f1l_handle h, double* out, int n) {
     float ms = 0.f;
     for (int rep = 0; rep < 3; ++rep) {
         CK(cudaEventRecord(h->ev[0], st));
-        ffma2_peak_kernel<<<blocks, threads, 0, st>>>((float*)h->m_o0.p, iters, 1.0001f, 0.5f);
+        ffma2_peak_kernel<<<blocks, threads, 0, st>>>((float*)h->m[0].p, iters, 1.0001f, 0.5f);
         CK(cudaEventRecord(h->ev[1], st));
         CK(cudaStreamSynchronize(st));
         CK(cudaEventElapsedTime(&ms, h->ev[0], h->ev[1]));
@@ -2072,7 +2070,7 @@ int f1l_measure_peaks_ex(f1l_handle h, double* out, int n) {
     out[2] = 4.0 * PEAK_CHAINS * (double)iters * blocks * threads / (ms * 1e-3) / 1e12;
     for (int rep = 0; rep < 3; ++rep) {
         CK(cudaEventRecord(h->ev[0], st));
-        mixed_peak_kernel<<<blocks, threads, 0, st>>>((float*)h->m_o0.p, iters, 1.0001f, 0.5f);
+        mixed_peak_kernel<<<blocks, threads, 0, st>>>((float*)h->m[0].p, iters, 1.0001f, 0.5f);
         CK(cudaEventRecord(h->ev[1], st));
         CK(cudaStreamSynchronize(st));
         CK(cudaEventElapsedTime(&ms, h->ev[0], h->ev[1]));
