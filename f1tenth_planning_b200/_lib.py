@@ -69,6 +69,16 @@ class RolloutTraceBuffers(C.Structure):
                 ("progress", _vp)]
 
 
+class BatchCall(C.Structure):
+    """f1l_batch_call (include/f1l.h): every input and output of one batch call, host or device
+    pointers; None for an absent array."""
+    _fields_ = [("poses", _vp), ("opp", _vp), ("n_opp", _vp), ("n_scenarios", C.c_int32),
+                ("max_opp", C.c_int32), ("prev_theta", _vp), ("has_prev", _vp),
+                ("update_prev", C.c_int32), ("reserved", C.c_int32), ("weights", _vp),
+                ("best_idx", _vp), ("best_cost", _vp), ("best_traj", _vp), ("costs", _vp),
+                ("flags", _vp), ("steer_speed", _vp), ("terms", _vp)]
+
+
 # name -> (restype, argtypes); must list every symbol include/f1l.h declares
 SIGNATURES = {
     "f1l_default_config": (C.c_int, [C.POINTER(Config)]),
@@ -103,9 +113,13 @@ SIGNATURES = {
                                           _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "f1l_plan_batch_prev": (C.c_int, [_vp, _vp, _vp, _vp, C.c_int, C.c_int, _vp, _vp, C.c_int,
                                       _vp, _vp, _vp, _vp, _vp, _vp]),
+    "f1l_plan_batch_call_dev": (C.c_int, [_vp, C.POINTER(BatchCall), _vp]),
+    "f1l_plan_batch_call": (C.c_int, [_vp, C.POINTER(BatchCall)]),
     "f1l_default_rollout_config": (C.c_int, [C.POINTER(RolloutConfig)]),
     "f1l_rollout_dev": (C.c_int, [_vp, C.POINTER(RolloutConfig), C.POINTER(FleetBuffers), C.c_int,
                                   C.c_int, C.POINTER(RolloutTraceBuffers), _vp]),
+    "f1l_rollout_weights_dev": (C.c_int, [_vp, C.POINTER(RolloutConfig), C.POINTER(FleetBuffers), _vp,
+                                          C.c_int, C.c_int, C.POINTER(RolloutTraceBuffers), _vp]),
     "f1l_pure_pursuit_batch_dev": (C.c_int, [_vp, _vp, C.c_int, C.c_double, _vp, _vp, _vp, _vp,
                                              _vp, _vp, _vp]),
     "f1l_pure_pursuit_batch": (C.c_int, [_vp, _vp, C.c_int, C.c_double, _vp, _vp, _vp, _vp, _vp,

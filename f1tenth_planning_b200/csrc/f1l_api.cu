@@ -60,7 +60,8 @@ struct PipeScratch {
 };
 
 // The per-scenario arrays of a host-buffer batch chunk, in the order they are copied
-enum { B_POSES, B_OPP, B_NOPP, B_IDX, B_COST, B_TRAJ, B_COSTS, B_FLAGS, B_SS, B_PREV, B_PVALID, B_ARRAYS };
+enum { B_POSES, B_OPP, B_NOPP, B_IDX, B_COST, B_TRAJ, B_COSTS, B_FLAGS, B_SS, B_PREV, B_PVALID, B_W, B_TERMS,
+       B_ARRAYS };
 
 struct PipeSlot {
     cudaStream_t stream = nullptr;
@@ -372,7 +373,8 @@ typedef void (*generate_fn)(LutView, EvalParams, const float4*, int, float4*, fl
 // One compiled eval_kernel: the resident CTAs per SM its register budget is built for (MINB), and
 // its shared memory in front of the window table (EvalSmem::C_TAB).
 struct EvalBuild {
-    eval_fn fn;   // null: not built
+    eval_fn fn;     // null: not built
+    eval_fn fn_w;   // the same with per-scenario cost weights (null: not built)
     int minb;
     uint32_t smem_fixed;
     size_t smem_bytes(int nseg_pad) const {
@@ -386,22 +388,25 @@ struct EvalBuild {
 struct EvalBucket {
     int m_max, ipl, s, sg;
     EvalBuild nw4, nw7, nw8;
-    EvalBuild wide;   // 8 warps at two CTAs per SM (128 registers), large dense queries
+    EvalBuild wide;   // 8 warps at two CTAs per SM (128 registers), large dense queries (no
+                      // per-scenario weights: lone queries plan with the config's)
     select_fn select;
     generate_fn generate;
     const EvalBuild& build(int nw) const { return nw == 4 ? nw4 : (nw == 7 ? nw7 : nw8); }
 };
 
-template <int IPL, int S, int SG, int NW, int MINB>
+template <int IPL, int S, int SG, int NW, int MINB, bool WEIGHTS = true>
 EvalBuild eval_build() {
-    if constexpr (MINB == 0) return {nullptr, 0, 0};
-    else return {eval_kernel<IPL, S, SG, NW, MINB>, MINB, EvalSmem<S, SG, NW>::C_TAB};
+    if constexpr (MINB == 0) return {nullptr, nullptr, 0, 0};
+    else if constexpr (!WEIGHTS) return {eval_kernel<IPL, S, SG, NW, MINB, false>, nullptr, MINB, EvalSmem<S, SG, NW>::C_TAB};
+    else return {eval_kernel<IPL, S, SG, NW, MINB, false>, eval_kernel<IPL, S, SG, NW, MINB, true>, MINB,
+                 EvalSmem<S, SG, NW>::C_TAB};
 }
 template <int M_MAX, int IPL, int S, int SG, int MINB4, int MINB7, int MINB8, int MINB_WIDE>
 EvalBucket eval_bucket() {
     return {M_MAX, IPL, S, SG,
             eval_build<IPL, S, SG, 4, MINB4>(), eval_build<IPL, S, SG, 7, MINB7>(),
-            eval_build<IPL, S, SG, 8, MINB8>(), eval_build<IPL, S, SG, 8, MINB_WIDE>(),
+            eval_build<IPL, S, SG, 8, MINB8>(), eval_build<IPL, S, SG, 8, MINB_WIDE, false>(),
             select_kernel<IPL>, generate_kernel<IPL>};
 }
 
@@ -582,6 +587,7 @@ struct PipeIn {
     const float* prev_theta = nullptr;
     int prev_stride = 0;
     const uint8_t* prev_valid = nullptr;
+    const float* weights = nullptr;    // [S,5] cost weights per scenario (null: the config's)
     const XchgView* xc = nullptr;      // sharded single query: exchange the argmin with the peers
     int* work_next = nullptr;          // single query: device counter for the persistent-grid schedule
 };
@@ -693,7 +699,7 @@ int launch_pipeline(f1l_handle h, cudaStream_t stream, const PipeIn& in, PipeScr
     // build of the M > 128 shapes on two CTAs per SM (measured on config 5: 65 536 candidates
     // 471 -> 431 us, 32 768: 247 -> 234, 16 384: 134 -> 128, 8 192: 76 -> 100)
     constexpr int EVAL_WIDE_MIN = 4;
-    const bool wide = dyn && wpc == 8 && bucket.wide.fn &&
+    const bool wide = dyn && wpc == 8 && bucket.wide.fn && !in.weights &&
                       (long long)n_cand >= (long long)EVAL_WIDE_MIN * resident_ctas * wpc;
     if (wide) {
         build = &bucket.wide;
@@ -760,6 +766,7 @@ int launch_pipeline(f1l_handle h, cudaStream_t stream, const PipeIn& in, PipeScr
     ea.prev_theta = in.prev_theta;
     ea.prev_stride = in.prev_stride;
     ea.prev_valid = in.prev_valid;
+    ea.weights = in.weights;
     ea.C = sp.C;
     ea.c_begin = sp.c_begin;
     ea.c_end = sp.c_end;
@@ -792,7 +799,7 @@ int launch_pipeline(f1l_handle h, cudaStream_t stream, const PipeIn& in, PipeScr
     ea.stats = h->stats_on ? (unsigned long long*)h->stats.p : nullptr;
     const long long n_ctas = (long long)S * ea.ctas_per_scn;
     if (n_ctas > 0x7fffffffLL) return F1L_ERR_TOO_LARGE;
-    if (!sp.empty) build->fn<<<(unsigned)n_ctas, wpc * 32, smem, stream>>>(ea);
+    if (!sp.empty) (in.weights ? build->fn_w : build->fn)<<<(unsigned)n_ctas, wpc * 32, smem, stream>>>(ea);
     {
         const int info[8] = {bucket.ipl, bucket.s, bucket.sg, wpc, build->minb, ea.chunk, ea.ctas_per_scn, ea.item};
         for (int i = 0; i < 8; ++i) h->eval_info[i] = info[i];
@@ -1074,9 +1081,11 @@ int f1l_create(f1l_handle* out, int device, const f1l_config* cfg) {
         const int big = 226 * 1024;  // opt-in maximum is 227 KB per block INCLUDING static shared memory
         for (const EvalBucket& b : kEvalBuckets) {
             for (const EvalBuild* eb : {&b.nw4, &b.nw7, &b.nw8, &b.wide}) {
-                if (!eb->fn) continue;
-                cudaError_t e2 = cudaFuncSetAttribute(eb->fn, cudaFuncAttributeMaxDynamicSharedMemorySize, big);
-                if (e2 != cudaSuccess && e == cudaSuccess) e = e2;
+                for (eval_fn fn : {eb->fn, eb->fn_w}) {
+                    if (!fn) continue;
+                    cudaError_t e2 = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, big);
+                    if (e2 != cudaSuccess && e == cudaSuccess) e = e2;
+                }
             }
         }
     }
@@ -1602,30 +1611,29 @@ int f1l_generate(f1l_handle h, const double* goals, int n_goals, float* states, 
 // eval_kernel reads a scenario's path in its prologue, and select_kernel writes it in a later
 // kernel on the same stream.
 // The arguments of a batch call over the whole goal grid, checked; device or host pointers alike
-static int batch_args(f1l_handle h, const double* poses, const double* opp, const int32_t* n_opp, int S,
-                      int max_opp, float* prev_theta, uint8_t* has_prev, int update_prev, int32_t* best_idx,
-                      float* best_cost, float* best_traj, float* costs, uint8_t* flags, double* steer_speed,
-                      PipeIn& in, BatchOut& o) {
-    if (!h || !poses || S <= 0) return F1L_ERR_INVALID_ARG;
-    if (max_opp > 0 && !opp) return F1L_ERR_INVALID_ARG;
-    if ((update_prev || has_prev) && !prev_theta) return F1L_ERR_INVALID_ARG;
+static int batch_args(f1l_handle h, const f1l_batch_call* b, PipeIn& in, BatchOut& o) {
+    if (!h || !b || !b->poses || b->n_scenarios <= 0) return F1L_ERR_INVALID_ARG;
+    if (b->max_opp < 0 || b->max_opp > F1L_MAX_OPP || (b->max_opp > 0 && !b->opp)) return F1L_ERR_INVALID_ARG;
+    if ((b->update_prev || b->has_prev) && !b->prev_theta) return F1L_ERR_INVALID_ARG;
     if (const int r = make_span(h, 0, Shard{}, false, in.span); r != F1L_OK) return r;
-    in.poses = poses;
-    in.opp = max_opp > 0 ? opp : nullptr;
-    in.n_opp = n_opp;
-    in.S = S;
-    in.max_opp = max_opp;
-    in.prev_theta = prev_theta;
+    in.poses = b->poses;
+    in.opp = b->max_opp > 0 ? b->opp : nullptr;
+    in.n_opp = b->n_opp;
+    in.S = b->n_scenarios;
+    in.max_opp = b->max_opp;
+    in.prev_theta = b->prev_theta;
     in.prev_stride = h->cfg.n_samples;
-    in.prev_valid = has_prev;
-    o.best_idx = best_idx;
-    o.best_cost = best_cost;
-    o.best_traj = (float4*)best_traj;
-    o.costs = costs;
-    o.flags = flags;
-    o.steer_speed = steer_speed;
-    o.prev_out = update_prev ? prev_theta : nullptr;
-    o.prev_valid_out = update_prev ? has_prev : nullptr;
+    in.prev_valid = b->has_prev;
+    in.weights = b->weights;
+    o.best_idx = b->best_idx;
+    o.best_cost = b->best_cost;
+    o.best_traj = (float4*)b->best_traj;
+    o.costs = b->costs;
+    o.terms = b->terms;
+    o.flags = b->flags;
+    o.steer_speed = b->steer_speed;
+    o.prev_out = b->update_prev ? b->prev_theta : nullptr;
+    o.prev_valid_out = b->update_prev ? b->has_prev : nullptr;
     return F1L_OK;
 }
 
@@ -1633,6 +1641,13 @@ static int plan_batch_dev_internal(f1l_handle h, const PipeIn& in, const BatchOu
     CK(cudaSetDevice(h->device));
     if (const int r = h->b_scratch.reserve(h, in.S); r != F1L_OK) return r;
     return launch_pipeline(h, stream, in, h->b_scratch, o, h->timing != 0);
+}
+
+int f1l_plan_batch_call_dev(f1l_handle h, const f1l_batch_call* b, void* stream) {
+    PipeIn in;
+    BatchOut o;
+    const int r = batch_args(h, b, in, o);
+    return r != F1L_OK ? r : plan_batch_dev_internal(h, in, o, (cudaStream_t)stream);
 }
 
 int f1l_plan_batch_dev(f1l_handle h, const double* poses_dev, const double* opp_dev,
@@ -1649,12 +1664,10 @@ int f1l_plan_batch_prev_dev(f1l_handle h, const double* poses_dev, const double*
                             uint8_t* has_prev_dev, int update_prev, int32_t* best_idx_dev,
                             float* best_cost_dev, float* best_traj_dev, float* costs_dev,
                             uint8_t* flags_dev, double* steer_speed_dev, void* stream) {
-    PipeIn in;
-    BatchOut o;
-    const int r = batch_args(h, poses_dev, opp_dev, n_opp_dev, S, max_opp, prev_theta_dev, has_prev_dev,
-                             update_prev, best_idx_dev, best_cost_dev, best_traj_dev, costs_dev, flags_dev,
-                             steer_speed_dev, in, o);
-    return r != F1L_OK ? r : plan_batch_dev_internal(h, in, o, (cudaStream_t)stream);
+    const f1l_batch_call b = {poses_dev, opp_dev, n_opp_dev, S, max_opp, prev_theta_dev, has_prev_dev,
+                              update_prev, 0, nullptr, best_idx_dev, best_cost_dev, best_traj_dev,
+                              costs_dev, flags_dev, steer_speed_dev, nullptr};
+    return f1l_plan_batch_call_dev(h, &b, stream);
 }
 
 // `in` and `o` hold host pointers: each chunk is copied in, planned and copied back on a slot stream
@@ -1693,22 +1706,44 @@ static int plan_batch_internal(f1l_handle h, const PipeIn& in, const BatchOut& o
             {&p.buf[B_SS], nullptr, o.steer_speed, 16},
             {&p.buf[B_PREV], in.prev_theta, o.prev_out, (size_t)M * 4},
             {&p.buf[B_PVALID], in.prev_valid, o.prev_valid_out, 1},
+            {&p.buf[B_W], in.weights, nullptr, F1L_N_TERMS * 4},
+            {&p.buf[B_TERMS], nullptr, o.terms, (size_t)C * F1L_N_TERMS * 4},
         };
         if (const int r = stage_in(h, st, t, s0, n); r != F1L_OK) return r;
         // the chunk is a batch call of n scenarios on the slot's copies (updated in place)
+        f1l_batch_call d{};
+        d.poses = (const double*)t[B_POSES].dev();
+        d.opp = (const double*)t[B_OPP].dev();
+        d.n_opp = (const int32_t*)t[B_NOPP].dev();
+        d.n_scenarios = n;
+        d.max_opp = in.max_opp;
+        d.prev_theta = (float*)t[B_PREV].dev();
+        d.has_prev = (uint8_t*)t[B_PVALID].dev();
+        d.update_prev = o.prev_out != nullptr;
+        d.weights = (const float*)t[B_W].dev();
+        d.best_idx = (int32_t*)t[B_IDX].dev();
+        d.best_cost = (float*)t[B_COST].dev();
+        d.best_traj = (float*)t[B_TRAJ].dev();
+        d.costs = (float*)t[B_COSTS].dev();
+        d.flags = (uint8_t*)t[B_FLAGS].dev();
+        d.steer_speed = (double*)t[B_SS].dev();
+        d.terms = (float*)t[B_TERMS].dev();
         PipeIn din;
         BatchOut dout;
-        int r = batch_args(h, (const double*)t[B_POSES].dev(), (const double*)t[B_OPP].dev(),
-                           (const int32_t*)t[B_NOPP].dev(), n, in.max_opp, (float*)t[B_PREV].dev(),
-                           (uint8_t*)t[B_PVALID].dev(), o.prev_out != nullptr, (int32_t*)t[B_IDX].dev(),
-                           (float*)t[B_COST].dev(), (float*)t[B_TRAJ].dev(), (float*)t[B_COSTS].dev(),
-                           (uint8_t*)t[B_FLAGS].dev(), (double*)t[B_SS].dev(), din, dout);
+        int r = batch_args(h, &d, din, dout);
         if (r == F1L_OK) r = launch_pipeline(h, st, din, p.scratch, dout, false);
         if (r == F1L_OK) r = stage_out(h, st, t, s0, n);
         if (r != F1L_OK) return r;
     }
     for (int i = 0; i < N_PIPE; ++i) CK(cudaStreamSynchronize(h->pipe[i].stream));
     return F1L_OK;
+}
+
+int f1l_plan_batch_call(f1l_handle h, const f1l_batch_call* b) {
+    PipeIn in;
+    BatchOut o;
+    const int r = batch_args(h, b, in, o);
+    return r != F1L_OK ? r : plan_batch_internal(h, in, o);
 }
 
 int f1l_plan_batch(f1l_handle h, const double* poses, const double* opp, const int32_t* n_opp,
@@ -1722,11 +1757,9 @@ int f1l_plan_batch_prev(f1l_handle h, const double* poses, const double* opp, co
                         int S, int max_opp, float* prev_theta, uint8_t* has_prev, int update_prev,
                         int32_t* best_idx, float* best_cost, float* best_traj, float* costs,
                         uint8_t* flags, double* steer_speed) {
-    PipeIn in;
-    BatchOut o;
-    const int r = batch_args(h, poses, opp, n_opp, S, max_opp, prev_theta, has_prev, update_prev, best_idx,
-                             best_cost, best_traj, costs, flags, steer_speed, in, o);
-    return r != F1L_OK ? r : plan_batch_internal(h, in, o);
+    const f1l_batch_call b = {poses, opp, n_opp, S, max_opp, prev_theta, has_prev, update_prev, 0, nullptr,
+                              best_idx, best_cost, best_traj, costs, flags, steer_speed, nullptr};
+    return f1l_plan_batch_call(h, &b);
 }
 
 // ---- closed-loop rollouts -----------------------------------------------------------------
@@ -1743,6 +1776,12 @@ int f1l_default_rollout_config(f1l_rollout_config* rc) {
 
 int f1l_rollout_dev(f1l_handle h, const f1l_rollout_config* rc, const f1l_fleet* fl, int S,
                     int n_steps, const f1l_rollout_trace* trace, void* stream) {
+    return f1l_rollout_weights_dev(h, rc, fl, nullptr, S, n_steps, trace, stream);
+}
+
+int f1l_rollout_weights_dev(f1l_handle h, const f1l_rollout_config* rc, const f1l_fleet* fl,
+                            const float* weights_dev, int S, int n_steps, const f1l_rollout_trace* trace,
+                            void* stream) {
     if (!h || !rc || !fl) return F1L_ERR_INVALID_ARG;
     if (!fl->state || !fl->prev_theta || !fl->has_prev || !fl->status || !fl->progress ||
         !fl->track_i || !fl->track_s)
@@ -1810,7 +1849,7 @@ int f1l_rollout_dev(f1l_handle h, const f1l_rollout_config* rc, const f1l_fleet*
     a.near4 = nullptr;
     a.steer_speed = (const double*)h->r_ss.p;
     a.best_cost = (const float*)h->r_cost.p;
-    // every step plans the fleet as f1l_plan_batch_prev_dev with update_prev does
+    // every step plans the fleet as f1l_plan_batch_call_dev does with update_prev and these weights
     in.poses = fl->state;
     in.opp = a.opp;
     in.n_opp = a.n_opp;
@@ -1819,6 +1858,7 @@ int f1l_rollout_dev(f1l_handle h, const f1l_rollout_config* rc, const f1l_fleet*
     in.prev_theta = fl->prev_theta;
     in.prev_stride = h->cfg.n_samples;
     in.prev_valid = fl->has_prev;
+    in.weights = weights_dev;
     BatchOut o;
     o.best_cost = (float*)h->r_cost.p;
     o.steer_speed = (double*)h->r_ss.p;

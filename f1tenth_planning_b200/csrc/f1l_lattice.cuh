@@ -343,6 +343,7 @@ struct EvalArgs {
     const float* prev_theta; // previous path of scenario s at prev_theta + s * prev_stride, or null
     int prev_stride;         // 0: one [M] path for every scenario (single query), M: [S,M]
     const uint8_t* prev_valid; // [S]: scenario s has a previous path iff != 0 (null: every one has)
+    const float* weights;    // [S,5] cost weights of each scenario (the PW instances only)
     int C;                   // candidates per scenario
     int c_begin, c_end;      // evaluated range (of shard-local indices when row_step > 1)
     int row0, row_step;      // row-interleaved shard: local index v -> lookahead row
@@ -893,8 +894,10 @@ struct EvalSmem {
     static constexpr uint32_t W_SLABY = W_SLABX + SLAB * 4;
     static constexpr uint32_t W_BYTES = W_SLABY + SLAB * 4;
     static constexpr uint32_t C_OPP = NW * W_BYTES;                // [F1L_MAX_OPP] float4
-    static constexpr uint32_t C_GRID = C_OPP + F1L_MAX_OPP * 16;   // 3 float4: A, (fx, fy, ix0, iy0), (n_opp, has_grid, use_prev)
-    static constexpr uint32_t C_PREV = C_GRID + 48;                // [F1L_MAX_M] float
+    static constexpr uint32_t C_GRID = C_OPP + F1L_MAX_OPP * 16;   // 4 float4: A, (fx, fy, ix0, iy0),
+                                                                   // (n_opp, has_grid, use_prev, w4), (w0, w1, w2, w3)
+                                                                   // (the weights with PW only)
+    static constexpr uint32_t C_PREV = C_GRID + 64;                // [F1L_MAX_M] float
     static constexpr uint32_t C_TAB = C_PREV + F1L_MAX_M * 4;      // [ntab][2] float4
     static_assert(W_BYTES % 16 == 0, "per-warp block keeps 16-byte alignment");
 };
@@ -902,7 +905,11 @@ struct EvalSmem {
 // One CTA per (scenario, candidate chunk).  The CTA builds the scenario's raceline window once,
 // then its NW warps pull candidates of the chunk from a shared counter until it is exhausted
 // (warps that finish an early-exit candidate immediately take the next one).
-template <int IPL, int S, int SG, int NW, int MINB>
+// PW: the call has per-scenario cost weights (a.weights), which the candidate loop reads from the
+// CTA's shared memory.  Without them the instance takes the config's weights from the kernel
+// parameters, whose constant-bank operands cost no register: its schedule is the one it had before
+// per-scenario weights existed (shared-memory operands there made the batch instance 1.2 % slower).
+template <int IPL, int S, int SG, int NW, int MINB, bool PW>
 __global__ void __launch_bounds__(NW * 32, MINB) eval_kernel(EvalArgs a) {
     constexpr int GG = 32 / SG;
     using L = EvalSmem<S, SG, NW>;
@@ -977,13 +984,19 @@ __global__ void __launch_bounds__(NW * 32, MINB) eval_kernel(EvalArgs a) {
             sts128(cbase + L::C_OPP + tid * 16,
                    tid < q->n_opp ? q->opp[tid] : make_float4(1e9f, 1e9f, 1.0f, 0.0f));
         if (tid == 0) { s_next = cb + NW * a.item; s_work = 0ull; }
-        // per-scenario collision constants live in shared memory, not in registers, so that the
-        // candidate loop does not carry them through the deviation pass
+        // per-scenario collision constants (and with PW the cost weights) live in shared memory,
+        // not in registers, so that the candidate loop does not carry them through the deviation pass
         if (tid == 32 % (NW * 32)) {
+            float w4 = 0.0f;
+            if constexpr (PW) {
+                const float* w = a.weights + (size_t)s * F1L_N_TERMS;
+                w4 = w[4];
+                sts128(cbase + L::C_GRID + 48, make_float4(w[0], w[1], w[2], w[3]));
+            }
             sts128(cbase + L::C_GRID, make_float4(q->gA00, q->gA01, q->gA10, q->gA11));
             sts128(cbase + L::C_GRID + 16, make_float4(q->gfx, q->gfy, __int_as_float(q->gix), __int_as_float(q->giy)));
             sts128(cbase + L::C_GRID + 32, make_float4(__int_as_float(q->n_opp), __int_as_float(q->has_grid),
-                                                       __int_as_float((int)use_prev), 0.0f));
+                                                       __int_as_float((int)use_prev), w4));
         }
     }
     __syncthreads();
@@ -1134,6 +1147,16 @@ __global__ void __launch_bounds__(NW * 32, MINB) eval_kernel(EvalArgs a) {
             const float t_maxk = maxk;                         // :277
             const float t_meank = sumk * a.ep.inv_M;           // :284
             float t_sim = 0.0f;
+            if constexpr (PW) {
+                // the first three weighted terms now, so that only their sum lives through the
+                // collision tests (the operations and order of the one weighted sum below)
+                const float4 GW = lds128(cbase + L::C_GRID + 48);
+                partial = GW.x * t_len + GW.y * t_maxk + GW.z * t_meank;
+                if (lane == 0 && a.terms) {
+                    float* t = a.terms + cand * F1L_N_TERMS;
+                    t[0] = t_len; t[1] = t_maxk; t[2] = t_meank;
+                }
+            }
 
             // ---- similarity (lattice_planner.py:287-296), collision (SURVEY B.6) ----
             float sim = 0.0f;
@@ -1286,10 +1309,15 @@ __global__ void __launch_bounds__(NW * 32, MINB) eval_kernel(EvalArgs a) {
             hit_map = __any_sync(F1L_FULL, hit_map);
             if (hit_opp) flags |= F1L_FLAG_COLLIDE_OPP;
             if (hit_map) flags |= F1L_FLAG_COLLIDE_MAP;
-            partial = a.ep.w[0] * t_len + a.ep.w[1] * t_maxk + a.ep.w[2] * t_meank + a.ep.w[3] * t_sim;
-            if (lane == 0 && a.terms) {
-                float* t = a.terms + cand * F1L_N_TERMS;
-                t[0] = t_len; t[1] = t_maxk; t[2] = t_meank; t[3] = t_sim;
+            if constexpr (PW) {
+                partial = partial + lds32(cbase + L::C_GRID + 60) * t_sim;
+                if (lane == 0 && a.terms) a.terms[cand * F1L_N_TERMS + 3] = t_sim;
+            } else {
+                partial = a.ep.w[0] * t_len + a.ep.w[1] * t_maxk + a.ep.w[2] * t_meank + a.ep.w[3] * t_sim;
+                if (lane == 0 && a.terms) {
+                    float* t = a.terms + cand * F1L_N_TERMS;
+                    t[0] = t_len; t[1] = t_maxk; t[2] = t_meank; t[3] = t_sim;
+                }
             }
 
             // ---- raceline deviation: mean over samples of the nearest distance to the window
@@ -1408,7 +1436,7 @@ __global__ void __launch_bounds__(NW * 32, MINB) eval_kernel(EvalArgs a) {
             }
 
             if (!(flags & (F1L_FLAG_COLLIDE_OPP | F1L_FLAG_COLLIDE_MAP))) {
-                cost = partial + a.ep.w[4] * t_dev;
+                cost = partial + (PW ? lds32(cbase + L::C_GRID + 44) : a.ep.w[4]) * t_dev;
                 if (!isfinite(cost)) cost = CUDART_INF_F;
             }
         }

@@ -22,7 +22,7 @@ PlanDetail = namedtuple("PlanDetail", [
     defaults=[None])
 
 BatchPlan = namedtuple("BatchPlan", ["best_idx", "best_cost", "best_traj", "costs", "flags",
-                                     "steer_speed"])
+                                     "steer_speed", "terms"], defaults=[None])
 
 PurePursuitBatch = namedtuple("PurePursuitBatch", ["nearest", "nearest_i", "lookahead",
                                                    "lookahead_i", "actuation", "status"])
@@ -303,9 +303,18 @@ class Engine:
                                 and (has_prev is None or has_prev.flags.writeable)):
             raise ValueError("update_prev writes prev_theta / has_prev in place: they must be writeable")
 
+    def _check_dev_array(self, name, t, shape, dtype):
+        """A device array of a batch call must be a contiguous CUDA tensor of exactly this shape and
+        dtype on the engine's device: the library reads or writes it where it is."""
+        import torch
+        if not (isinstance(t, torch.Tensor) and t.is_cuda and t.device.index == self.device
+                and t.dtype == dtype and tuple(t.shape) == tuple(shape) and t.is_contiguous()):
+            raise ValueError("%s must be a contiguous %s CUDA tensor %s on cuda:%d"
+                             % (name, str(dtype).replace("torch.", ""), list(shape), self.device))
+
     def plan_batch(self, poses, opponents=None, n_opp=None, out=None, want_traj=True,
                    want_costs=True, want_flags=False, prev_theta=None, has_prev=None,
-                   update_prev=False):
+                   update_prev=False, weights=None, want_terms=False):
         """S independent scenarios with HOST buffers (numpy; pinned if allocated through
         ``pinned_empty``).  poses [S,4], opponents [S,K,3], n_opp [S].
 
@@ -315,10 +324,20 @@ class Engine:
         Scenario s then plans exactly as plan() after set_prev_path(prev_theta[s]) (or
         set_prev_path(None) where has_prev[s] is 0).  update_prev=True overwrites both arrays in
         place with this call's best trajectories' theta columns and ones, ready for the next
-        step.  The engine's own previous path (set_prev_path) is not used."""
+        step.  The engine's own previous path (set_prev_path) is not used.
+
+        Cost weights per scenario (f1l_plan_batch_call): weights [S,5] float (converted to
+        float32), scenario s then plans exactly as plan() after configure(weights=weights[s]);
+        None: every scenario uses the configured weights.  want_terms=True also returns the
+        unweighted per-term costs [S,C,5] (BatchPlan.terms), as plan_detailed's terms."""
         poses = _f64(poses).reshape(-1, 4)
         S = poses.shape[0]
         self._check_prev(S, prev_theta, has_prev, update_prev, False)
+        if weights is not None:
+            w = np.asarray(weights)
+            if w.shape != (S, N_TERMS) or w.dtype.kind != "f":
+                raise ValueError("weights must be a float array [%d, %d]" % (S, N_TERMS))
+            weights = np.ascontiguousarray(w, dtype=np.float32)
         K = 0
         if opponents is not None:
             opponents = _f64(opponents)
@@ -342,51 +361,52 @@ class Engine:
         flags = o.get("flags") if want_flags else None
         if want_flags and flags is None:
             flags = np.zeros((S, Cn), np.uint8)
+        terms = o.get("terms") if want_terms else None
+        if want_terms and terms is None:
+            terms = np.zeros((S, Cn, N_TERMS), np.float32)
+        if terms is not None and not (isinstance(terms, np.ndarray) and terms.dtype == np.float32
+                                      and terms.shape == (S, Cn, N_TERMS) and terms.flags.c_contiguous
+                                      and terms.flags.writeable):
+            raise ValueError("terms must be a writeable C-contiguous float32 array [%d, %d, %d]"
+                             % (S, Cn, N_TERMS))
         if S == 0:   # an empty batch is a valid (empty) answer, not an error
-            return BatchPlan(best_idx, best_cost, best_traj, costs, flags, steer_speed)
-        if prev_theta is None:
-            self._ck(self._L.f1l_plan_batch(self._h, _vp(poses), _vp(opponents), _vp(n_opp), S, K,
-                                            _vp(best_idx), _vp(best_cost), _vp(best_traj),
-                                            _vp(costs), _vp(flags), _vp(steer_speed)))
-        else:
-            self._ck(self._L.f1l_plan_batch_prev(self._h, _vp(poses), _vp(opponents), _vp(n_opp),
-                                                 S, K, _vp(prev_theta), _vp(has_prev),
-                                                 int(bool(update_prev)), _vp(best_idx),
-                                                 _vp(best_cost), _vp(best_traj), _vp(costs),
-                                                 _vp(flags), _vp(steer_speed)))
-        return BatchPlan(best_idx, best_cost, best_traj, costs, flags, steer_speed)
+            return BatchPlan(best_idx, best_cost, best_traj, costs, flags, steer_speed, terms)
+        b = _lib.BatchCall(_vp(poses), _vp(opponents), _vp(n_opp), S, K, _vp(prev_theta), _vp(has_prev),
+                           int(bool(update_prev)), 0, _vp(weights), _vp(best_idx), _vp(best_cost),
+                           _vp(best_traj), _vp(costs), _vp(flags), _vp(steer_speed), _vp(terms))
+        self._ck(self._L.f1l_plan_batch_call(self._h, C.byref(b)))
+        return BatchPlan(best_idx, best_cost, best_traj, costs, flags, steer_speed, terms)
 
     def plan_batch_dev(self, poses, opponents=None, n_opp=None, best_idx=None, best_cost=None,
                        best_traj=None, costs=None, flags=None, steer_speed=None, stream=None,
-                       prev_theta=None, has_prev=None, update_prev=False):
+                       prev_theta=None, has_prev=None, update_prev=False, weights=None, terms=None):
         """Same with torch CUDA tensors; enqueues on `stream` (default: torch's current stream)
         and does not synchronise.  prev_theta / has_prev / update_prev as for plan_batch, as
         contiguous CUDA tensors (float32 [S, n_samples], uint8 / bool [S]) updated in place on
-        the stream (f1l_plan_batch_prev_dev)."""
+        the stream.  weights: a contiguous float32 CUDA tensor [S,5] (None: the configured
+        weights); terms: a contiguous float32 CUDA tensor [S,C,5] that receives the per-term
+        costs (f1l_plan_batch_call_dev)."""
         import torch
         S = poses.shape[0]
         K = 0 if opponents is None else opponents.shape[1]
         self._check_prev(S, prev_theta, has_prev, update_prev, True)
+        if weights is not None:
+            self._check_dev_array("weights", weights, (S, N_TERMS), torch.float32)
+        if terms is not None:
+            self._check_dev_array("terms", terms, (S, self.n_candidates, N_TERMS), torch.float32)
         st = stream if stream is not None else torch.cuda.current_stream(poses.device).cuda_stream
-        if prev_theta is None:
-            self._ck(self._L.f1l_plan_batch_dev(self._h, _vp(poses), _vp(opponents), _vp(n_opp), S,
-                                                K, _vp(best_idx), _vp(best_cost), _vp(best_traj),
-                                                _vp(costs), _vp(flags), _vp(steer_speed),
-                                                C.c_void_p(st)))
-        else:
-            self._ck(self._L.f1l_plan_batch_prev_dev(self._h, _vp(poses), _vp(opponents),
-                                                     _vp(n_opp), S, K, _vp(prev_theta),
-                                                     _vp(has_prev), int(bool(update_prev)),
-                                                     _vp(best_idx), _vp(best_cost),
-                                                     _vp(best_traj), _vp(costs), _vp(flags),
-                                                     _vp(steer_speed), C.c_void_p(st)))
+        b = _lib.BatchCall(_vp(poses), _vp(opponents), _vp(n_opp), S, K, _vp(prev_theta), _vp(has_prev),
+                           int(bool(update_prev)), 0, _vp(weights), _vp(best_idx), _vp(best_cost),
+                           _vp(best_traj), _vp(costs), _vp(flags), _vp(steer_speed), _vp(terms))
+        self._ck(self._L.f1l_plan_batch_call_dev(self._h, C.byref(b), C.c_void_p(st)))
 
     # -- closed-loop rollouts ----------------------------------------------------------------
-    def fleet(self, poses, group=1):
+    def fleet(self, poses, group=1, weights=None):
         """A fleet of kinematic-bicycle cars at `poses` [S,4] (x, y, theta, v) on this engine's
-        device, raced in groups of `group` consecutive cars (rollout.Fleet, f1l_rollout_dev)."""
+        device, raced in groups of `group` consecutive cars, each planned with its row of
+        `weights` [S,5] (None: the configured weights) (rollout.Fleet, f1l_rollout_weights_dev)."""
         from .rollout import Fleet
-        return Fleet(self, poses, group)
+        return Fleet(self, poses, group, weights)
 
     # -- candidate sharding over peer memory -------------------------------------------------
     def export_peer_handle(self):

@@ -21,7 +21,7 @@ Additive (north-star) surface
     .plan_detailed(...) / .last           PlanDetail: best_idx, costs[C], terms[C,5], flags[C] ...
     .plan_batch(poses[S,4], opponents[S,K,3], n_opp[S][, prev_theta=[S,M], has_prev=[S],
                 update_prev=True])  per-scenario previous paths, carried in place step to step
-    .rollout(poses[S,4], n_steps, group=1, **kw)  closed-loop rollouts of a fleet on the device
+    .rollout(poses[S,4], n_steps, group=1, weights=None, **kw)  closed-loop rollouts of a fleet on the device
     .set_map(occupancy, origin, resolution), .set_goal_grid(lookaheads, widths)
 
 With no plug-ins registered every stage runs on the GPU.  A registered ``sample_func`` replaces
@@ -234,12 +234,13 @@ class LatticePlanner():
         self.last = d
         return d
 
-    def rollout(self, poses, n_steps, group=1, **kw):
+    def rollout(self, poses, n_steps, group=1, weights=None, **kw):
         """Closed-loop rollouts on the device for host users: the cars at `poses` [S,4] (x, y,
-        theta, v), raced in groups of `group` consecutive cars, advanced n_steps planning steps
+        theta, v), raced in groups of `group` consecutive cars, each planned with its row of
+        `weights` [S,5] (None: the configured weights), advanced n_steps planning steps
         (keywords as rollout.Fleet.run).  Returns the per-step RolloutTrace as numpy arrays and the
         final (state [S,4], status [S], progress [S])."""
-        fleet = self._sync().fleet(poses, group)
+        fleet = self._sync().fleet(poses, group, weights)
         tr = fleet.run(n_steps, trace=True, **kw)
         trace = type(tr)(*(t.cpu().numpy() for t in tr))
         return trace, (fleet.state.cpu().numpy(), fleet.status.cpu().numpy(), fleet.progress.cpu().numpy())
@@ -263,7 +264,9 @@ class LatticePlanner():
         of what plan() keeps from call to call: prev_theta [S,M] float32 (C-contiguous) and
         has_prev [S] bool / uint8.  With update_prev=True both are overwritten in place with this
         step's best trajectories' theta columns and ones, so a loop of S cars passes them back
-        unchanged on the next step.  Keywords go to Engine.plan_batch."""
+        unchanged on the next step.  weights [S,5] gives each scenario its own cost weights and
+        want_terms=True returns the per-term costs [S,C,5] as BatchPlan.terms.  Keywords go to
+        Engine.plan_batch."""
         return self._sync().plan_batch(poses, opponents, n_opp, **kw)
 
 

@@ -3,6 +3,7 @@ into races whose cars are each other's opponents, advanced T planning steps by t
 without leaving the GPU.
 
     fleet = engine.fleet(poses, group=4)       # poses [S,4] (x, y, theta, v), S % group == 0
+                                               # weights=[S,5]: cost weights per car
     tr = fleet.run(500, substeps=5, trace=True)
     fleet.status, fleet.progress               # F1L_CAR_* bits, metres along the raceline
 
@@ -34,12 +35,26 @@ def _poses_tensor(poses, device):
     return t.to(device=device, dtype=torch.float64).contiguous().clone()   # the fleet owns its state
 
 
+def _weights_tensor(weights, S, device):
+    import torch
+    if isinstance(weights, torch.Tensor):
+        t = weights.detach()
+    else:
+        import numpy as np
+        t = torch.from_numpy(np.array(weights, dtype=np.float64, copy=True))
+    if tuple(t.shape) != (S, _lib.N_TERMS) or not t.dtype.is_floating_point:
+        raise ValueError("weights must be a float array [%d, %d]" % (S, _lib.N_TERMS))
+    return t.to(device=device, dtype=torch.float32).contiguous().clone()
+
+
 class Fleet:
     """S cars on one Engine: state [S,4] f64, prev_theta [S,M] f32, has_prev [S] u8, status [S] u8,
     progress [S] f64, track_i [S] i32, track_s [S] f64 (f1l_fleet), all CUDA tensors on the
-    engine's device.  Races are the `group` consecutive cars [g*group, (g+1)*group)."""
+    engine's device.  Races are the `group` consecutive cars [g*group, (g+1)*group).  `weights` is
+    a float32 CUDA tensor [S,5] of cost weights per car, or None: every car uses the engine's
+    configured weights."""
 
-    def __init__(self, engine, poses, group=1):
+    def __init__(self, engine, poses, group=1, weights=None):
         import torch
         group = int(group)
         dev = torch.device("cuda", engine.device)
@@ -58,12 +73,14 @@ class Fleet:
         self.progress = torch.zeros(S, dtype=torch.float64, device=dev)
         self.track_i = torch.full((S,), -1, dtype=torch.int32, device=dev)
         self.track_s = torch.zeros(S, dtype=torch.float64, device=dev)
+        self.weights = None if weights is None else _weights_tensor(weights, S, dev)
 
     @property
     def n_cars(self):
         return self.state.shape[0]
 
     def _buffers(self):
+        import torch
         for name, dtype, shape in (("state", "float64", (self.n_cars, 4)),
                                    ("prev_theta", "float32", (self.n_cars, self.engine.n_samples)),
                                    ("has_prev", "uint8", (self.n_cars,)), ("status", "uint8", (self.n_cars,)),
@@ -74,6 +91,9 @@ class Fleet:
                     or tuple(t.shape) != shape or not t.is_contiguous()):
                 raise ValueError("fleet buffer %s must be a contiguous %s CUDA tensor %s on cuda:%d"
                                  % (name, dtype, list(shape), self.engine.device))
+        if self.weights is not None:
+            self.engine._check_dev_array("fleet weights", self.weights, (self.n_cars, _lib.N_TERMS),
+                                         torch.float32)
         return _lib.FleetBuffers(*(t.data_ptr() for t in (
             self.state, self.prev_theta, self.has_prev, self.status, self.progress, self.track_i,
             self.track_s)))
@@ -106,13 +126,14 @@ class Fleet:
             tb = _lib.RolloutTraceBuffers(*(t.data_ptr() for t in out))
         st = stream if stream is not None else torch.cuda.current_stream(dev).cuda_stream
         eng = self.engine
-        eng._ck(eng._L.f1l_rollout_dev(eng._h, C.byref(rc), C.byref(fl), S, n_steps,
-                                       C.byref(tb) if tb is not None else None, C.c_void_p(st)))
+        w = C.c_void_p(self.weights.data_ptr() if self.weights is not None else None)
+        eng._ck(eng._L.f1l_rollout_weights_dev(eng._h, C.byref(rc), C.byref(fl), w, S, n_steps,
+                                               C.byref(tb) if tb is not None else None, C.c_void_p(st)))
         return out
 
     def reset(self, cars, poses):
         """Put `cars` (indices) back on the road at `poses` [n,4] as fresh cars: no previous path,
-        status 0, progress 0, raceline tracking re-acquired on the next run()."""
+        status 0, progress 0, raceline tracking re-acquired on the next run().  Their weights stay."""
         import torch
         idx = torch.as_tensor(cars, dtype=torch.long).reshape(-1).to(self.state.device)
         if idx.numel() and (int(idx.min()) < 0 or int(idx.max()) >= self.n_cars):

@@ -307,6 +307,43 @@ int f1l_plan_batch_prev(f1l_handle h, const double* poses, const double* opp,
                         float* costs, uint8_t* flags, double* steer_speed);
 
 /*
+ * One batch call with every input and output in a struct: the previous paths of
+ * f1l_plan_batch_prev_dev, cost weights per scenario and the per-term costs.  The four batch
+ * calls above are this call with weights and terms NULL.
+ *   weights [S,F1L_N_TERMS] f32 or NULL (every scenario uses the config's weights): scenario s
+ *       gives bit-identically what f1l_plan gives on this handle after f1l_set_config with
+ *       weights = (double) weights[s], together with the previous-path rule of
+ *       f1l_plan_batch_prev_dev.  Weights are used as given, as the config's are: a non-finite
+ *       weighted sum makes the candidate's cost +inf.
+ *   terms [S,C,F1L_N_TERMS] f32 or NULL: the unweighted per-term costs, as f1l_plan_result.terms.
+ *       With prune_window = 1, requesting them makes collided candidates scan the raceline window
+ *       too (see f1l_config.prune_window).
+ * F1L_ERR_INVALID_ARG for a NULL handle, call or poses, n_scenarios <= 0, max_opp outside
+ * 0..F1L_MAX_OPP (or > 0 without opp), and update_prev or has_prev without prev_theta.
+ * `reserved` is ignored.
+ */
+typedef struct {
+    const double* poses;    /* [S,4] */
+    const double* opp;      /* [S,max_opp,3] or NULL */
+    const int32_t* n_opp;   /* [S] or NULL */
+    int32_t n_scenarios, max_opp;
+    float* prev_theta;      /* [S,M] or NULL, as f1l_plan_batch_prev_dev */
+    uint8_t* has_prev;      /* [S] or NULL */
+    int32_t update_prev, reserved;
+    const float* weights;   /* [S,F1L_N_TERMS] or NULL: every scenario uses the config's weights */
+    /* outputs, each nullable */
+    int32_t* best_idx; float* best_cost; float* best_traj; float* costs; uint8_t* flags;
+    double* steer_speed;
+    float* terms;           /* [S,C,F1L_N_TERMS] unweighted per-term costs, as f1l_plan_result.terms */
+} f1l_batch_call;
+
+/* Device buffers, caller's stream, no sync (as f1l_plan_batch_dev). */
+int f1l_plan_batch_call_dev(f1l_handle h, const f1l_batch_call* b, void* stream);
+/* Host buffers, through the chunked pipeline of f1l_plan_batch: weights travel with each chunk's
+ * inputs, terms come back with its outputs.  Synchronised before returning. */
+int f1l_plan_batch_call(f1l_handle h, const f1l_batch_call* b);
+
+/*
  * Closed-loop rollouts on the device: a fleet of S kinematic-bicycle cars advanced n_steps planning
  * steps.  Replaces the user loop around the planner -- plan, then step the vehicle
  * (lattice_planner.py:204-214 plus the gym step of examples/control/pure_pursuit.py:47-57, which
@@ -383,6 +420,13 @@ int f1l_default_rollout_config(f1l_rollout_config* rc);
  * handle.  Numpy users go through the Python layer (Fleet), which copies once per call. */
 int f1l_rollout_dev(f1l_handle h, const f1l_rollout_config* rc, const f1l_fleet* fleet,
                     int n_scenarios, int n_steps, const f1l_rollout_trace* trace, void* stream);
+
+/* The same with cost weights per car: every step plans car s with weights_dev[s] as
+ * f1l_plan_batch_call_dev does.  weights_dev [S,F1L_N_TERMS] f32 device buffer, read only, or
+ * NULL: f1l_rollout_dev. */
+int f1l_rollout_weights_dev(f1l_handle h, const f1l_rollout_config* rc, const f1l_fleet* fleet,
+                            const float* weights_dev, int n_scenarios, int n_steps,
+                            const f1l_rollout_trace* trace, void* stream);
 
 /*
  * Batched nearest_point + pure-pursuit lookahead over B poses on the uploaded track.
