@@ -12,6 +12,7 @@ MAX_M = 256
 FLAG_VALID, FLAG_COLLIDE_OPP, FLAG_COLLIDE_MAP, FLAG_NO_CENTRE = 1, 2, 4, 8
 CAR_HIT_MAP, CAR_HIT_CAR, CAR_NO_FEASIBLE = 1, 2, 4
 MAX_GROUP = 1 + MAX_OPP
+EVAL_LONE, EVAL_WEIGHTS = 1, 2   # f1l_debug_eval_choice flags
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 # F1L_LIB selects another build of the same library (A/B builds of kernel variants)
@@ -146,6 +147,8 @@ SIGNATURES = {
     "f1l_measure_peaks_ex": (C.c_int, [_vp, _dp, C.c_int]),
     "f1l_debug_query_ctx": (C.c_int, [_vp, _fp, _ip]),
     "f1l_debug_eval_plan": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _ip, C.c_int]),
+    "f1l_debug_eval_choice": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _ip, C.c_int]),
+    "f1l_debug_eval_builds": (C.c_int, [_ip, C.c_int]),
     "f1l_debug_pp_parts": (C.c_int, [C.c_int, C.c_int, C.c_int]),
 }
 

@@ -164,7 +164,7 @@ struct f1l_ctx {
     DevBuf xchg;
     XchgView xview = {0, 0, {nullptr}};
     // template instance / CTA plan of the last eval_kernel launch (f1l_last_eval_shape)
-    int eval_info[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+    int eval_info[10] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
     // the last single query, for f1l_select_candidate: its span, explicit goals?, epoch
     Span lastq_span;
     int lastq_goals = 0;
@@ -370,6 +370,10 @@ typedef void (*eval_fn)(EvalArgs);
 typedef void (*select_fn)(SelectArgs);
 typedef void (*generate_fn)(LutView, EvalParams, const float4*, int, float4*, float4*, uint8_t*);
 
+// dynamic shared memory an eval_kernel launch may use: the opt-in maximum is 227 KB per block
+// INCLUDING static shared memory
+constexpr int EVAL_SMEM_MAX = 226 * 1024;
+
 // One compiled eval_kernel: the resident CTAs per SM its register budget is built for (MINB), and
 // its shared memory in front of the window table (EvalSmem::C_TAB).
 struct EvalBuild {
@@ -413,6 +417,8 @@ EvalBucket eval_bucket() {
 // Every eval_kernel instance and its residency, one row per bucket (MINB 0: no such build).
 // NW = 7 (four resident CTAs of 7 warps at <= 72 registers) serves candidate counts that are a
 // small multiple of 7 -- the default 4x7 goal grid; everything else runs 8-warp CTAs (three at 80).
+// The M > 128 shapes have no 4- and 7-warp builds: their 72-register builds spill, so the launch
+// policy only ever runs them on 8 warps.
 // The M <= 104 shape on 4-warp CTAs (the batch regime of the 4x7 grid) runs FOUR CTAs per SM at
 // 125 registers instead of seven at 72 -- the deviation loop gets the schedule it wants (no spill,
 // 8.2 instead of 9.6 sub-partition cycles per (sample, segment) in isolation) and sixteen warps per
@@ -429,8 +435,8 @@ const EvalBucket kEvalBuckets[] = {
     eval_bucket<      64,   2,  8,  8,   7, 4, 3, 0>(),
     eval_bucket<     104,   4, 13,  8,   4, 4, 3, 0>(),
     eval_bucket<     128,   4, 16,  8,   7, 4, 3, 0>(),
-    eval_bucket<     208,   7, 13, 16,   7, 4, 3, 2>(),
-    eval_bucket<F1L_MAX_M,  8, 16, 16,   7, 4, 3, 2>(),
+    eval_bucket<     208,   7, 13, 16,   0, 0, 3, 2>(),
+    eval_bucket<F1L_MAX_M,  8, 16, 16,   0, 0, 3, 2>(),
 };
 
 const EvalBucket& eval_bucket_of(int M) {
@@ -455,16 +461,17 @@ CtaPlan plan_ctas(int n_cand, int S, int M, int sm_count, bool cubic) {
     // Newton solves: one 4-warp CTA per scenario whose warps pull the scenario's 4-candidate items.
     // Measured, not modelled (the wave model below counts CTAs and would always prefer the CTA with
     // more warps at equal residency): 10.84 ms on the bench workload against 11.19 for 7-warp CTAs.
+    const EvalBucket& bucket = eval_bucket_of(M);
     {
         const int full4 = ((n_cand + 3) / 4) * 4;
-        if (cubic && M <= 128 && full4 >= 4 * EVAL_ITEM && n_cand <= 256 &&
-            (long long)S >= 8LL * eval_bucket_of(M).nw4.minb * sm_count)
+        if (cubic && bucket.nw4.fn && full4 >= 4 * EVAL_ITEM && n_cand <= 256 &&
+            (long long)S >= 8LL * bucket.nw4.minb * sm_count)
             return CtaPlan{4, full4, 1};
     }
     const int nws[3] = {4, 7, 8};
     for (int nw : nws) {
-        if (nw != 8 && M > 128) continue;   // the 72-register builds of the M = 200 shapes spill
-        const int resident = eval_bucket_of(M).build(nw).minb * sm_count;
+        if (!bucket.build(nw).fn) continue;
+        const int resident = bucket.build(nw).minb * sm_count;
         const int full = ((n_cand + nw - 1) / nw) * nw;   // one CTA per scenario
         // chunk sizes worth a look: enough CTAs for ~8 waves (dense single queries), the smallest
         // chunk whose warps share Newton solves, and the whole scenario in one CTA
@@ -499,6 +506,57 @@ CtaPlan plan_ctas(int n_cand, int S, int M, int sm_count, bool cubic) {
         }
     }
     return best;
+}
+
+// The eval_kernel instance one pipeline launch runs, and its CTA plan
+struct EvalChoice {
+    const EvalBucket* bucket;
+    const EvalBuild* build;
+    int nw, chunk, ctas_per_scn, item;
+    bool persistent;   // one wave of CTAs pulling candidates from a device-wide counter
+    bool wide;         // build is bucket->wide
+    bool pw;           // per-scenario cost weights: build->fn_w
+    eval_fn fn() const { return pw ? build->fn_w : build->fn; }
+};
+
+// The whole instance choice of a pipeline launch (launch_pipeline, f1l_debug_eval_choice): the CTA
+// plan, the persistent grid and the wide build of a lone dense query, and the PW twin of a call
+// with per-scenario cost weights.  lone: a single query with a persistent-grid counter and a
+// non-empty span.
+EvalChoice choose_eval(int n_cand, int S, int M, int sm_count, bool cubic, bool lone, bool weights) {
+    const CtaPlan cp = plan_ctas(n_cand, S, M, sm_count, cubic);
+    EvalChoice c;
+    c.bucket = &eval_bucket_of(M);
+    c.build = &c.bucket->build(cp.nw);
+    c.nw = cp.nw;
+    c.chunk = cp.chunk;
+    c.ctas_per_scn = cp.ctas_per_scn;
+    // four candidates per warp at a time (shared Newton) when every warp has at least four
+    c.item = (cubic && cp.chunk >= 4 * cp.nw) ? EVAL_ITEM : 1;
+    c.pw = weights;
+    // A lone dense query that needs more than one wave of CTAs runs on a PERSISTENT grid instead: one
+    // wave of CTAs whose warps pull single candidates from a device-wide counter, far lookahead rows
+    // (the expensive candidates) first.  No wave quantisation, one window-table prologue per
+    // resident CTA, and the cheap early-exit candidates fill the tail.
+    long long resident = (long long)c.build->minb * sm_count;
+    c.persistent = lone && cp.nw != 4 && cp.ctas_per_scn > resident;
+    // ... and with at least EVAL_WIDE_MIN candidates per resident warp it runs the 128-register
+    // build of the M > 128 shapes on two CTAs per SM (measured on config 5: 65 536 candidates
+    // 471 -> 431 us, 32 768: 247 -> 234, 16 384: 134 -> 128, 8 192: 76 -> 100)
+    constexpr int EVAL_WIDE_MIN = 4;
+    c.wide = c.persistent && cp.nw == 8 && c.bucket->wide.fn && !weights &&
+             (long long)n_cand >= EVAL_WIDE_MIN * resident * cp.nw;
+    if (c.wide) {
+        c.build = &c.bucket->wide;
+        resident = (long long)c.build->minb * sm_count;
+    }
+    if (c.persistent) {
+        // single candidates per pull, unless every warp has at least four 4-candidate items to go
+        // through: then the shared Newton solve pays more than the coarser tail costs
+        c.item = (cubic && (long long)n_cand >= 16LL * resident * cp.nw) ? EVAL_ITEM : 1;
+        if (c.ctas_per_scn > resident) c.ctas_per_scn = (int)resident;
+    }
+    return c;
 }
 
 // owner of the constant-memory line-form table of each device (f1l_pp.cuh): the key of the handle
@@ -684,29 +742,12 @@ int launch_pipeline(f1l_handle h, cudaStream_t stream, const PipeIn& in, PipeScr
     if (nseg <= 0 || nseg > nsegs) nseg = nsegs;
     const int nseg_pad = (nseg + 31) & ~31;
     const int n_cand = sp.empty ? 1 : sp.c_end - sp.c_begin;
-    const CtaPlan cp = plan_ctas(n_cand, S, M, h->sm_count, ep.generator == 0);
-    const int wpc = cp.nw;
-    const EvalBucket& bucket = eval_bucket_of(M);
-    const EvalBuild* build = &bucket.build(wpc);
-    // A lone dense query that needs more than one wave of CTAs runs on a PERSISTENT grid instead: one
-    // wave of CTAs whose warps pull single candidates from a device-wide counter, far lookahead rows
-    // (the expensive candidates) first.  No wave quantisation, one window-table prologue per
-    // resident CTA, and the cheap early-exit candidates fill the tail.
-    int resident_ctas = build->minb * h->sm_count;
-    const bool dyn = S == 1 && wpc != 4 && in.work_next && !sp.empty &&
-                     (long long)cp.ctas_per_scn > resident_ctas;
-    // ... and with at least EVAL_WIDE_MIN candidates per resident warp it runs the 128-register
-    // build of the M > 128 shapes on two CTAs per SM (measured on config 5: 65 536 candidates
-    // 471 -> 431 us, 32 768: 247 -> 234, 16 384: 134 -> 128, 8 192: 76 -> 100)
-    constexpr int EVAL_WIDE_MIN = 4;
-    const bool wide = dyn && wpc == 8 && bucket.wide.fn && !in.weights &&
-                      (long long)n_cand >= (long long)EVAL_WIDE_MIN * resident_ctas * wpc;
-    if (wide) {
-        build = &bucket.wide;
-        resident_ctas = build->minb * h->sm_count;
-    }
-    const size_t smem = build->smem_bytes(nseg_pad);
-    if (smem > 226 * 1024) return F1L_ERR_TOO_LARGE;
+    const EvalChoice ec = choose_eval(n_cand, S, M, h->sm_count, ep.generator == 0,
+                                      S == 1 && in.work_next && !sp.empty, in.weights != nullptr);
+    if (!ec.fn()) return F1L_ERR_INVALID_ARG;   // the choice names an instance that is not built
+    const bool dyn = ec.persistent;
+    const size_t smem = ec.build->smem_bytes(nseg_pad);
+    if (smem > EVAL_SMEM_MAX) return F1L_ERR_TOO_LARGE;
 
     SampleArgs sa;
     sa.tr = track_view(h);
@@ -772,20 +813,11 @@ int launch_pipeline(f1l_handle h, cudaStream_t stream, const PipeIn& in, PipeScr
     ea.c_end = sp.c_end;
     ea.row0 = sp.row0;
     ea.row_step = sp.row_step;
-    ea.chunk = cp.chunk;
-    ea.ctas_per_scn = cp.ctas_per_scn;
-    // four candidates per warp at a time (shared Newton) when every warp has at least four
-    ea.item = (ep.generator == 0 && cp.chunk >= 4 * cp.nw) ? EVAL_ITEM : 1;
-    ea.work_next = nullptr;
-    ea.v_last = 0;
-    if (dyn) {
-        ea.work_next = in.work_next;
-        ea.v_last = sp.c_begin + sp.c_end - 1;
-        // single candidates per pull, unless every warp has at least four 4-candidate items to go
-        // through: then the shared Newton solve pays more than the coarser tail costs
-        ea.item = (ep.generator == 0 && (long long)n_cand >= 16LL * resident_ctas * wpc) ? EVAL_ITEM : 1;
-        ea.ctas_per_scn = cp.ctas_per_scn < resident_ctas ? cp.ctas_per_scn : resident_ctas;
-    }
+    ea.chunk = ec.chunk;
+    ea.ctas_per_scn = ec.ctas_per_scn;
+    ea.item = ec.item;
+    ea.work_next = dyn ? in.work_next : nullptr;
+    ea.v_last = dyn ? sp.c_begin + sp.c_end - 1 : 0;
     ea.inv_nW = 1.0f / (float)(h->nW > 0 ? h->nW : 1);
     ea.nseg_pad = nseg_pad;
     ea.costs = o.costs;
@@ -799,14 +831,16 @@ int launch_pipeline(f1l_handle h, cudaStream_t stream, const PipeIn& in, PipeScr
     ea.stats = h->stats_on ? (unsigned long long*)h->stats.p : nullptr;
     const long long n_ctas = (long long)S * ea.ctas_per_scn;
     if (n_ctas > 0x7fffffffLL) return F1L_ERR_TOO_LARGE;
-    if (!sp.empty) (in.weights ? build->fn_w : build->fn)<<<(unsigned)n_ctas, wpc * 32, smem, stream>>>(ea);
+    if (!sp.empty) ec.fn()<<<(unsigned)n_ctas, ec.nw * 32, smem, stream>>>(ea);
     {
-        const int info[8] = {bucket.ipl, bucket.s, bucket.sg, wpc, build->minb, ea.chunk, ea.ctas_per_scn, ea.item};
-        for (int i = 0; i < 8; ++i) h->eval_info[i] = info[i];
+        const EvalBucket& b = *ec.bucket;
+        const int info[10] = {b.ipl, b.s, b.sg, ec.nw, ec.build->minb, ea.chunk, ea.ctas_per_scn, ea.item,
+                              (int)ec.persistent, (int)ec.pw};
+        for (int i = 0; i < 10; ++i) h->eval_info[i] = info[i];
     }
     if (time_it) cudaEventRecord(ev[2], stream);
 
-    bucket.select<<<S, SELECT_THREADS, 0, stream>>>(select_args(h, in, sc, o));
+    ec.bucket->select<<<S, SELECT_THREADS, 0, stream>>>(select_args(h, in, sc, o));
     if (time_it) {
         cudaEventRecord(ev[3], stream);
         h->timed = 1;
@@ -941,14 +975,34 @@ int f1l_set_stats(f1l_handle h, int on) {
 
 int f1l_debug_eval_plan(int n_cand, int n_scenarios, int M, int sm_count, int generator,
                         int32_t* out, int n) {
-    if (!out || n < 4 || n_cand <= 0 || n_scenarios <= 0 || M < 2 || M > F1L_MAX_M || sm_count <= 0)
+    return f1l_debug_eval_choice(n_cand, n_scenarios, M, sm_count, generator, 0, out, n < 4 ? n : 4);
+}
+
+int f1l_debug_eval_choice(int n_cand, int n_scenarios, int M, int sm_count, int generator, int flags,
+                          int32_t* out, int n) {
+    if (!out || n < 4 || n_cand <= 0 || n_scenarios <= 0 || M < 2 || M > F1L_MAX_M || sm_count <= 0 ||
+        (flags & ~(F1L_EVAL_LONE | F1L_EVAL_WEIGHTS)) || ((flags & F1L_EVAL_LONE) && n_scenarios != 1))
         return F1L_ERR_INVALID_ARG;
-    const CtaPlan cp = plan_ctas(n_cand, n_scenarios, M, sm_count, generator == 0);
-    out[0] = cp.nw;
-    out[1] = cp.chunk;
-    out[2] = cp.ctas_per_scn;
-    out[3] = (generator == 0 && cp.chunk >= 4 * cp.nw) ? EVAL_ITEM : 1;
+    const EvalChoice c = choose_eval(n_cand, n_scenarios, M, sm_count, generator == 0,
+                                     (flags & F1L_EVAL_LONE) != 0, (flags & F1L_EVAL_WEIGHTS) != 0);
+    const EvalBucket& b = *c.bucket;
+    // minb 0: the choice names an instance that is not built (launch_pipeline refuses it)
+    const int v[13] = {c.nw, c.chunk, c.ctas_per_scn, c.item, b.m_max, b.ipl, b.s, b.sg,
+                       c.fn() ? c.build->minb : 0, (int)c.wide, (int)c.persistent, (int)c.pw,
+                       ((EVAL_SMEM_MAX - (int)c.build->smem_fixed) / 32 - EVAL_SEG_PAD) & ~31};
+    for (int i = 0; i < n && i < 13; ++i) out[i] = v[i];
     return F1L_OK;
+}
+
+int f1l_debug_eval_builds(int32_t* out, int n) {
+    const int rows = (int)(sizeof(kEvalBuckets) / sizeof(kEvalBuckets[0]));
+    if (!out || n < 8 * rows) return F1L_ERR_INVALID_ARG;
+    for (int r = 0; r < rows; ++r) {
+        const EvalBucket& b = kEvalBuckets[r];
+        const int v[8] = {b.m_max, b.ipl, b.s, b.sg, b.nw4.minb, b.nw7.minb, b.nw8.minb, b.wide.minb};
+        for (int i = 0; i < 8; ++i) out[8 * r + i] = v[i];
+    }
+    return rows;
 }
 
 int f1l_debug_pp_parts(int n_poses, int n_waypoints, int slots) {
@@ -958,7 +1012,7 @@ int f1l_debug_pp_parts(int n_poses, int n_waypoints, int slots) {
 
 int f1l_last_eval_shape(f1l_handle h, int32_t* out, int n) {
     if (!h || !out || n < 8) return F1L_ERR_INVALID_ARG;
-    for (int i = 0; i < 8; ++i) out[i] = h->eval_info[i];
+    for (int i = 0; i < n && i < 10; ++i) out[i] = h->eval_info[i];
     return F1L_OK;
 }
 
@@ -1078,12 +1132,11 @@ int f1l_create(f1l_handle* out, int device, const f1l_config* cfg) {
         cudaDeviceGetAttribute(&sm, cudaDevAttrMultiProcessorCount, device);
         if (sm > 0) h->sm_count = sm;
         // opt in to large dynamic shared memory for every eval instantiation
-        const int big = 226 * 1024;  // opt-in maximum is 227 KB per block INCLUDING static shared memory
         for (const EvalBucket& b : kEvalBuckets) {
             for (const EvalBuild* eb : {&b.nw4, &b.nw7, &b.nw8, &b.wide}) {
                 for (eval_fn fn : {eb->fn, eb->fn_w}) {
                     if (!fn) continue;
-                    cudaError_t e2 = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, big);
+                    cudaError_t e2 = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, EVAL_SMEM_MAX);
                     if (e2 != cudaSuccess && e == cudaSuccess) e = e2;
                 }
             }

@@ -521,12 +521,14 @@ class Engine:
 
     def last_eval_shape(self):
         """Template instance and CTA plan of the last eval_kernel launch (f1l_last_eval_shape):
-        dict with ipl, s, sg, nw, minb, chunk, ctas_per_scenario, item and the instance `name`."""
-        out = (C.c_int32 * 8)()
-        self._ck(self._L.f1l_last_eval_shape(self._h, out, 8))
-        keys = ("ipl", "s", "sg", "nw", "minb", "chunk", "ctas_per_scenario", "item")
+        dict with ipl, s, sg, nw, minb, chunk, ctas_per_scenario, item, persistent (the persistent
+        grid of a lone dense query), pw (per-scenario cost weights) and the instance `name`."""
+        out = (C.c_int32 * 10)()
+        self._ck(self._L.f1l_last_eval_shape(self._h, out, 10))
+        keys = ("ipl", "s", "sg", "nw", "minb", "chunk", "ctas_per_scenario", "item", "persistent", "pw")
         d = {k: int(v) for k, v in zip(keys, out)}
-        d["name"] = "eval_kernel<%d,%d,%d,%d,%d>" % tuple(out[:5])
+        d["name"] = "eval_kernel<%d,%d,%d,%d,%d,%s>%s" % (tuple(out[:5]) + ("true" if out[9] else "false",
+                                                                            " persistent" if out[8] else ""))
         return d
 
     def set_graph(self, on):

@@ -487,10 +487,12 @@ int f1l_set_stats(f1l_handle h, int on);
  * window length.  n >= 2. */
 int f1l_get_stats(f1l_handle h, uint64_t* out, int n);
 
-/* Which eval_kernel<IPL, S, SG, NW, MINB> instance the last f1l_plan* call launched and its CTA
- * plan: out[0..4] = IPL, S, SG, NW (warps per CTA), MINB (resident CTAs per SM asked of the
+/* Which eval_kernel<IPL, S, SG, NW, MINB, PW> instance the last f1l_plan* call launched and its
+ * CTA plan: out[0..4] = IPL, S, SG, NW (warps per CTA), MINB (resident CTAs per SM asked of the
  * compiler); out[5] = candidates per CTA, out[6] = CTAs per scenario, out[7] = candidates a warp
- * solves together (4 = shared Newton).  n >= 8.  Evidence for bench.py / profiles. */
+ * solves together (4 = shared Newton).  n >= 8.  With n >= 10 also out[8] = 1 on the persistent
+ * grid of a lone dense query and out[9] = PW (1: per-scenario cost weights).  Evidence for
+ * bench.py / profiles. */
 int f1l_last_eval_shape(f1l_handle h, int32_t* out, int n);
 
 /* Timing / evidence helpers: number of kernels launched by this handle so far, and the device
@@ -526,11 +528,29 @@ int f1l_measure_peaks_ex(f1l_handle h, double* out, int n);
 /* Host-side launch planning, callable without a device (tests of the host logic):
  * f1l_debug_eval_plan: the CTA plan of eval_kernel for n_scenarios queries of n_cand candidates
  * and M arc samples on sm_count SMs -- out[0] = warps per CTA, out[1] = candidates per CTA,
- * out[2] = CTAs per scenario, out[3] = candidates a warp solves together (n >= 4).
+ * out[2] = CTAs per scenario, out[3] = candidates a warp solves together (n >= 4).  This is the
+ * plan of a batch call without per-scenario weights; f1l_debug_eval_choice with flags 0 gives the
+ * same four entries.
+ * f1l_debug_eval_choice: the eval_kernel instance and CTA plan a pipeline launch chooses.  flags:
+ * F1L_EVAL_LONE for a single query (f1l_plan*, n_scenarios = 1: persistent grid and wide build
+ * allowed), F1L_EVAL_WEIGHTS for a call with per-scenario cost weights.  out[0..3] as above (on
+ * the persistent grid out[2] is its CTA count and out[3] the candidates per pull); with n >= 12
+ * also the bucket's out[4] = largest M, out[5] = IPL, out[6] = S, out[7] = SG, then out[8] = MINB
+ * of the chosen build (0: not built), out[9] = 1 for the wide build, out[10] = 1 for the
+ * persistent grid, out[11] = PW; with n >= 13 out[12] = the largest window (segments) the build's
+ * shared memory holds.
+ * f1l_debug_eval_builds: every row of the instance table, 8 entries each: largest M, IPL, S, SG,
+ * then MINB of the 4-, 7- and 8-warp builds and of the wide build (0: not built).  Every build
+ * but the wide one also has its PW twin.  Returns the number of rows (n >= 8 x rows).
  * f1l_debug_pp_parts: into how many parts pp_scan_kernel splits a track of n_waypoints for
  * n_poses poses when `slots` one-warp CTAs are resident on the device (> 0), or an error (< 0). */
+#define F1L_EVAL_LONE 1
+#define F1L_EVAL_WEIGHTS 2
 int f1l_debug_eval_plan(int n_cand, int n_scenarios, int M, int sm_count, int generator,
                         int32_t* out, int n);
+int f1l_debug_eval_choice(int n_cand, int n_scenarios, int M, int sm_count, int generator, int flags,
+                          int32_t* out, int n);
+int f1l_debug_eval_builds(int32_t* out, int n);
 int f1l_debug_pp_parts(int n_poses, int n_waypoints, int slots);
 
 /* Debug / test hook: the float32 per-query constants of the last f1l_plan* call, for
