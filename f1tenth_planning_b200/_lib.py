@@ -6,6 +6,8 @@ raises.
 import ctypes as C
 import os
 
+import numpy as np
+
 N_TERMS = 5
 MAX_OPP = 16
 MAX_M = 256
@@ -78,6 +80,89 @@ class BatchCall(C.Structure):
                 ("update_prev", C.c_int32), ("reserved", C.c_int32), ("weights", _vp),
                 ("best_idx", _vp), ("best_cost", _vp), ("best_traj", _vp), ("costs", _vp),
                 ("flags", _vp), ("steer_speed", _vp), ("terms", _vp)]
+
+
+# Arrays the library uses in place: name -> (accepted dtypes, shape, direction).  Shapes name S
+# scenarios or cars, K = max_opp, C candidates, M = n_samples, B poses.  INOUT is read and written
+# in place (by a batch call only with update_prev).
+IN, OUT, INOUT = "in", "out", "inout"
+
+BATCH_FIELDS = {   # the pointer fields of f1l_batch_call
+    "poses": (("float64",), ("S", 4), IN),
+    "opp": (("float64",), ("S", "K", 3), IN),
+    "n_opp": (("int32",), ("S",), IN),
+    "prev_theta": (("float32",), ("S", "M"), INOUT),
+    "has_prev": (("uint8", "bool"), ("S",), INOUT),
+    "weights": (("float32",), ("S", N_TERMS), IN),
+    "best_idx": (("int32",), ("S",), OUT),
+    "best_cost": (("float32",), ("S",), OUT),
+    "best_traj": (("float32",), ("S", "M", 4), OUT),
+    "costs": (("float32",), ("S", "C"), OUT),
+    "flags": (("uint8",), ("S", "C"), OUT),
+    "steer_speed": (("float64",), ("S", 2), OUT),
+    "terms": (("float32",), ("S", "C", N_TERMS), OUT),
+}
+
+FLEET_FIELDS = {   # f1l_fleet
+    "state": (("float64",), ("S", 4), INOUT),
+    "prev_theta": (("float32",), ("S", "M"), INOUT),
+    "has_prev": (("uint8",), ("S",), INOUT),
+    "status": (("uint8",), ("S",), INOUT),
+    "progress": (("float64",), ("S",), INOUT),
+    "track_i": (("int32",), ("S",), INOUT),
+    "track_s": (("float64",), ("S",), INOUT),
+}
+
+PP_FIELDS = {   # the outputs of f1l_pure_pursuit_batch, in argument order
+    "nearest": (("float64",), ("B", 4), OUT),
+    "nearest_i": (("int32",), ("B",), OUT),
+    "lookahead": (("float64",), ("B", 4), OUT),
+    "lookahead_i": (("int32",), ("B",), OUT),
+    "actuation": (("float64",), ("B", 2), OUT),
+    "status": (("int32",), ("B",), OUT),
+}
+
+
+def shape_of(row, dims):
+    """the shape of a field row with its sizes from `dims` (name -> size)"""
+    return tuple([dims.get(d, d) for d in row[1]])
+
+
+def zeros_or(a, row, dims):
+    """`a`, or zeros of the row's shape and first dtype when `a` is None"""
+    return np.zeros(shape_of(row, dims), row[0][0]) if a is None else a
+
+
+def check_array(name, a, shape, dtypes, where, writes=False):
+    """ValueError unless the library can use `a` in place: exactly this shape, one of `dtypes`, and
+    for where="host" a C-contiguous numpy array (writeable if `writes`), else a contiguous CUDA
+    tensor on device `where`."""
+    if where == "host":
+        if not (isinstance(a, np.ndarray) and a.dtype in dtypes and a.shape == shape
+                and a.flags.c_contiguous and (a.flags.writeable or not writes)):
+            raise ValueError("%s must be a %sC-contiguous %s numpy array %s"
+                             % (name, "writeable " if writes else "", " / ".join(dtypes), list(shape)))
+        return
+    import torch
+    if not (isinstance(a, torch.Tensor) and a.is_cuda and a.device.index == where
+            and str(a.dtype)[6:] in dtypes and a.shape == shape and a.is_contiguous()):
+        raise ValueError("%s must be a contiguous %s CUDA tensor %s on cuda:%d"
+                         % (name, " / ".join(dtypes), list(shape), where))
+
+
+def batch_call(arrays, where, dims, update_prev):
+    """BatchCall of `arrays` (BATCH_FIELDS name -> array or None) with sizes `dims` (S, K, C, M),
+    each given array checked against its row, on the host or device `where` (check_array)."""
+    if arrays.get("prev_theta") is None and (arrays.get("has_prev") is not None or update_prev):
+        raise ValueError("has_prev / update_prev need prev_theta")
+    b = BatchCall(n_scenarios=dims["S"], max_opp=dims["K"], update_prev=int(bool(update_prev)))
+    for name, a in arrays.items():
+        if a is not None:
+            row = BATCH_FIELDS[name]
+            check_array(name, a, shape_of(row, dims), row[0], where,
+                        row[2] == OUT or (row[2] == INOUT and update_prev))
+            setattr(b, name, a.ctypes.data if where == "host" else a.data_ptr())
+    return b
 
 
 # name -> (restype, argtypes); must list every symbol include/f1l.h declares

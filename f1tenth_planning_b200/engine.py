@@ -268,50 +268,6 @@ class Engine:
         return states, params, (flags & FLAG_VALID) != 0
 
     # -- batch ------------------------------------------------------------------------------
-    def _check_prev(self, S, prev_theta, has_prev, update_prev, is_dev):
-        """Validates the per-scenario previous paths of plan_batch / plan_batch_dev.  They are
-        read and, with update_prev, written in place, so anything that would need a copy (wrong
-        type, shape, dtype, layout or device) is a ValueError rather than a silent conversion."""
-        if prev_theta is None:
-            if has_prev is not None or update_prev:
-                raise ValueError("has_prev / update_prev need prev_theta")
-            return
-        shape = (S, self.n_samples)
-        if is_dev:
-            import torch
-            ok_type = isinstance(prev_theta, torch.Tensor) and prev_theta.is_cuda
-            if not (ok_type and prev_theta.dtype == torch.float32 and tuple(prev_theta.shape) == shape
-                    and prev_theta.is_contiguous() and prev_theta.device.index == self.device):
-                raise ValueError("prev_theta must be a contiguous float32 CUDA tensor [%d, %d] on "
-                                 "cuda:%d" % (S, self.n_samples, self.device))
-            if has_prev is not None and not (
-                    isinstance(has_prev, torch.Tensor) and has_prev.is_cuda
-                    and has_prev.dtype in (torch.uint8, torch.bool) and tuple(has_prev.shape) == (S,)
-                    and has_prev.is_contiguous() and has_prev.device == prev_theta.device):
-                raise ValueError("has_prev must be a contiguous uint8 / bool CUDA tensor [%d] on "
-                                 "prev_theta's device" % S)
-            return
-        if not (isinstance(prev_theta, np.ndarray) and prev_theta.dtype == np.float32
-                and prev_theta.shape == shape and prev_theta.flags.c_contiguous):
-            raise ValueError("prev_theta must be a C-contiguous float32 numpy array [%d, %d]"
-                             % (S, self.n_samples))
-        if has_prev is not None and not (
-                isinstance(has_prev, np.ndarray) and has_prev.dtype in (np.uint8, np.bool_)
-                and has_prev.shape == (S,) and has_prev.flags.c_contiguous):
-            raise ValueError("has_prev must be a contiguous uint8 / bool numpy array [%d]" % S)
-        if update_prev and not (prev_theta.flags.writeable
-                                and (has_prev is None or has_prev.flags.writeable)):
-            raise ValueError("update_prev writes prev_theta / has_prev in place: they must be writeable")
-
-    def _check_dev_array(self, name, t, shape, dtype):
-        """A device array of a batch call must be a contiguous CUDA tensor of exactly this shape and
-        dtype on the engine's device: the library reads or writes it where it is."""
-        import torch
-        if not (isinstance(t, torch.Tensor) and t.is_cuda and t.device.index == self.device
-                and t.dtype == dtype and tuple(t.shape) == tuple(shape) and t.is_contiguous()):
-            raise ValueError("%s must be a contiguous %s CUDA tensor %s on cuda:%d"
-                             % (name, str(dtype).replace("torch.", ""), list(shape), self.device))
-
     def plan_batch(self, poses, opponents=None, n_opp=None, out=None, want_traj=True,
                    want_costs=True, want_flags=False, prev_theta=None, has_prev=None,
                    update_prev=False, weights=None, want_terms=False):
@@ -332,50 +288,22 @@ class Engine:
         unweighted per-term costs [S,C,5] (BatchPlan.terms), as plan_detailed's terms."""
         poses = _f64(poses).reshape(-1, 4)
         S = poses.shape[0]
-        self._check_prev(S, prev_theta, has_prev, update_prev, False)
-        if weights is not None:
-            w = np.asarray(weights)
-            if w.shape != (S, N_TERMS) or w.dtype.kind != "f":
-                raise ValueError("weights must be a float array [%d, %d]" % (S, N_TERMS))
-            weights = np.ascontiguousarray(w, dtype=np.float32)
-        K = 0
-        if opponents is not None:
-            opponents = _f64(opponents)
-            K = opponents.shape[1]
-        if n_opp is not None:
-            n_opp = np.ascontiguousarray(n_opp, dtype=np.int32)
-        Cn, M = self.n_candidates, self.n_samples
+        opponents = None if opponents is None else _f64(opponents)
+        K = opponents.shape[1] if opponents is not None and opponents.ndim == 3 else 0
+        if weights is not None and np.asarray(weights).dtype.kind == "f":   # else rejected below
+            weights = np.ascontiguousarray(weights, dtype=np.float32)
+        a = dict(poses=poses, opp=opponents, prev_theta=prev_theta, has_prev=has_prev, weights=weights,
+                 n_opp=None if n_opp is None else np.ascontiguousarray(n_opp, dtype=np.int32))
+        dims = dict(S=S, K=K, C=self.n_candidates, M=self.n_samples)
         o = out or {}
-        best_idx = o.get("best_idx", None)
-        if best_idx is None:
-            best_idx = np.zeros(S, np.int32)
-        best_cost = o.get("best_cost") if o.get("best_cost") is not None else np.zeros(S, np.float32)
-        steer_speed = (o.get("steer_speed") if o.get("steer_speed") is not None
-                       else np.zeros((S, 2), np.float64))
-        best_traj = o.get("best_traj") if want_traj else None
-        if want_traj and best_traj is None:
-            best_traj = np.zeros((S, M, 4), np.float32)
-        costs = o.get("costs") if want_costs else None
-        if want_costs and costs is None:
-            costs = np.zeros((S, Cn), np.float32)
-        flags = o.get("flags") if want_flags else None
-        if want_flags and flags is None:
-            flags = np.zeros((S, Cn), np.uint8)
-        terms = o.get("terms") if want_terms else None
-        if want_terms and terms is None:
-            terms = np.zeros((S, Cn, N_TERMS), np.float32)
-        if terms is not None and not (isinstance(terms, np.ndarray) and terms.dtype == np.float32
-                                      and terms.shape == (S, Cn, N_TERMS) and terms.flags.c_contiguous
-                                      and terms.flags.writeable):
-            raise ValueError("terms must be a writeable C-contiguous float32 array [%d, %d, %d]"
-                             % (S, Cn, N_TERMS))
-        if S == 0:   # an empty batch is a valid (empty) answer, not an error
-            return BatchPlan(best_idx, best_cost, best_traj, costs, flags, steer_speed, terms)
-        b = _lib.BatchCall(_vp(poses), _vp(opponents), _vp(n_opp), S, K, _vp(prev_theta), _vp(has_prev),
-                           int(bool(update_prev)), 0, _vp(weights), _vp(best_idx), _vp(best_cost),
-                           _vp(best_traj), _vp(costs), _vp(flags), _vp(steer_speed), _vp(terms))
-        self._ck(self._L.f1l_plan_batch_call(self._h, C.byref(b)))
-        return BatchPlan(best_idx, best_cost, best_traj, costs, flags, steer_speed, terms)
+        for name, want in (("best_idx", True), ("best_cost", True), ("best_traj", want_traj),
+                           ("costs", want_costs), ("flags", want_flags), ("steer_speed", True),
+                           ("terms", want_terms)):
+            a[name] = _lib.zeros_or(o.get(name), _lib.BATCH_FIELDS[name], dims) if want else None
+        b = _lib.batch_call(a, "host", dims, update_prev)
+        if S:   # an empty batch is a valid (empty) answer, not an error
+            self._ck(self._L.f1l_plan_batch_call(self._h, C.byref(b)))
+        return BatchPlan(*(a[k] for k in BatchPlan._fields))
 
     def plan_batch_dev(self, poses, opponents=None, n_opp=None, best_idx=None, best_cost=None,
                        best_traj=None, costs=None, flags=None, steer_speed=None, stream=None,
@@ -387,17 +315,14 @@ class Engine:
         weights); terms: a contiguous float32 CUDA tensor [S,C,5] that receives the per-term
         costs (f1l_plan_batch_call_dev)."""
         import torch
-        S = poses.shape[0]
-        K = 0 if opponents is None else opponents.shape[1]
-        self._check_prev(S, prev_theta, has_prev, update_prev, True)
-        if weights is not None:
-            self._check_dev_array("weights", weights, (S, N_TERMS), torch.float32)
-        if terms is not None:
-            self._check_dev_array("terms", terms, (S, self.n_candidates, N_TERMS), torch.float32)
+        K = opponents.shape[1] if opponents is not None and opponents.ndim == 3 else 0
+        dims = dict(S=poses.shape[0], K=K, C=self.n_candidates, M=self.n_samples)
+        b = _lib.batch_call(dict(poses=poses, opp=opponents, n_opp=n_opp, prev_theta=prev_theta,
+                                 has_prev=has_prev, weights=weights, best_idx=best_idx,
+                                 best_cost=best_cost, best_traj=best_traj, costs=costs, flags=flags,
+                                 steer_speed=steer_speed, terms=terms),
+                            self.device, dims, update_prev)
         st = stream if stream is not None else torch.cuda.current_stream(poses.device).cuda_stream
-        b = _lib.BatchCall(_vp(poses), _vp(opponents), _vp(n_opp), S, K, _vp(prev_theta), _vp(has_prev),
-                           int(bool(update_prev)), 0, _vp(weights), _vp(best_idx), _vp(best_cost),
-                           _vp(best_traj), _vp(costs), _vp(flags), _vp(steer_speed), _vp(terms))
         self._ck(self._L.f1l_plan_batch_call_dev(self._h, C.byref(b), C.c_void_p(st)))
 
     # -- closed-loop rollouts ----------------------------------------------------------------
@@ -446,18 +371,14 @@ class Engine:
         poses = _f64(poses).reshape(-1, 3)
         B = poses.shape[0]
         o = out or {}
-        nearest = o.get("nearest") if o.get("nearest") is not None else np.zeros((B, 4))
-        nearest_i = o.get("nearest_i") if o.get("nearest_i") is not None else np.zeros(B, np.int32)
-        look = o.get("lookahead") if o.get("lookahead") is not None else np.zeros((B, 4))
-        look_i = o.get("lookahead_i") if o.get("lookahead_i") is not None else np.zeros(B, np.int32)
-        act = o.get("actuation") if o.get("actuation") is not None else np.zeros((B, 2))
-        status = o.get("status") if o.get("status") is not None else np.zeros(B, np.int32)
-        if B == 0:
-            return PurePursuitBatch(nearest, nearest_i, look, look_i, act, status)
-        self._ck(self._L.f1l_pure_pursuit_batch(self._h, _vp(poses), B, float(lookahead_distance),
-                                                _vp(nearest), _vp(nearest_i), _vp(look),
-                                                _vp(look_i), _vp(act), _vp(status)))
-        return PurePursuitBatch(nearest, nearest_i, look, look_i, act, status)
+        dims = {"B": B}
+        r = PurePursuitBatch(**{k: _lib.zeros_or(o.get(k), row, dims) for k, row in _lib.PP_FIELDS.items()})
+        for k, row in _lib.PP_FIELDS.items():
+            _lib.check_array(k, getattr(r, k), _lib.shape_of(row, dims), row[0], "host", writes=True)
+        if B:
+            self._ck(self._L.f1l_pure_pursuit_batch(self._h, _vp(poses), B, float(lookahead_distance),
+                                                    *map(_vp, r)))
+        return r
 
     def pure_pursuit_batch_dev(self, poses, lookahead_distance, nearest=None, nearest_i=None,
                                lookahead=None, lookahead_i=None, actuation=None, status=None,
@@ -485,6 +406,8 @@ class Engine:
         pts = _f64(points).reshape(-1, 2)
         t0 = _f64(t_start).ravel()
         n = pts.shape[0]
+        if t0.size != n:
+            raise ValueError("t_start must have one entry per point (%d)" % n)
         out = np.zeros((n, 4))
         out_i = np.zeros(n, np.int32)
         if n == 0:

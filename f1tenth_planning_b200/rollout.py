@@ -80,23 +80,13 @@ class Fleet:
         return self.state.shape[0]
 
     def _buffers(self):
-        import torch
-        for name, dtype, shape in (("state", "float64", (self.n_cars, 4)),
-                                   ("prev_theta", "float32", (self.n_cars, self.engine.n_samples)),
-                                   ("has_prev", "uint8", (self.n_cars,)), ("status", "uint8", (self.n_cars,)),
-                                   ("progress", "float64", (self.n_cars,)), ("track_i", "int32", (self.n_cars,)),
-                                   ("track_s", "float64", (self.n_cars,))):
-            t = getattr(self, name)
-            if (not t.is_cuda or t.device.index != self.engine.device or str(t.dtype) != "torch." + dtype
-                    or tuple(t.shape) != shape or not t.is_contiguous()):
-                raise ValueError("fleet buffer %s must be a contiguous %s CUDA tensor %s on cuda:%d"
-                                 % (name, dtype, list(shape), self.engine.device))
-        if self.weights is not None:
-            self.engine._check_dev_array("fleet weights", self.weights, (self.n_cars, _lib.N_TERMS),
-                                         torch.float32)
-        return _lib.FleetBuffers(*(t.data_ptr() for t in (
-            self.state, self.prev_theta, self.has_prev, self.status, self.progress, self.track_i,
-            self.track_s)))
+        dims, dev = {"S": self.n_cars, "M": self.engine.n_samples}, self.engine.device
+        for name, row in _lib.FLEET_FIELDS.items():
+            _lib.check_array("fleet " + name, getattr(self, name), _lib.shape_of(row, dims), row[0], dev)
+        if self.weights is not None:   # read as a batch call's weights
+            row = _lib.BATCH_FIELDS["weights"]
+            _lib.check_array("fleet weights", self.weights, _lib.shape_of(row, dims), row[0], dev)
+        return _lib.FleetBuffers(**{name: getattr(self, name).data_ptr() for name in _lib.FLEET_FIELDS})
 
     def run(self, n_steps, dt=0.01, substeps=1, max_steer=0.4189, max_accel=9.51, v_max=math.inf,
             trace=False, stream=None):
