@@ -72,6 +72,12 @@ class RolloutTraceBuffers(C.Structure):
                 ("progress", _vp)]
 
 
+class Vehicle(C.Structure):
+    """f1l_vehicle (include/f1l.h): the single-track model's parameters."""
+    _fields_ = [(n, C.c_double) for n in ("mu", "C_Sf", "C_Sr", "lf", "lr", "h", "m", "I", "max_steer_vel",
+                                          "v_switch", "v_kin")]
+
+
 class BatchCall(C.Structure):
     """f1l_batch_call (include/f1l.h): every input and output of one batch call, host or device
     pointers; None for an absent array."""
@@ -111,6 +117,10 @@ FLEET_FIELDS = {   # f1l_fleet
     "progress": (("float64",), ("S",), INOUT),
     "track_i": (("int32",), ("S",), INOUT),
     "track_s": (("float64",), ("S",), INOUT),
+}
+
+ST_FIELDS = {   # the single-track fleet's array beside f1l_fleet (f1l_rollout_st_dev's dyn_dev)
+    "dyn": (("float64",), ("S", 3), INOUT),
 }
 
 PP_FIELDS = {   # the outputs of f1l_pure_pursuit_batch, in argument order
@@ -206,6 +216,9 @@ SIGNATURES = {
                                   C.c_int, C.POINTER(RolloutTraceBuffers), _vp]),
     "f1l_rollout_weights_dev": (C.c_int, [_vp, C.POINTER(RolloutConfig), C.POINTER(FleetBuffers), _vp,
                                           C.c_int, C.c_int, C.POINTER(RolloutTraceBuffers), _vp]),
+    "f1l_default_vehicle": (C.c_int, [C.POINTER(Vehicle)]),
+    "f1l_rollout_st_dev": (C.c_int, [_vp, C.POINTER(RolloutConfig), C.POINTER(Vehicle), C.POINTER(FleetBuffers),
+                                     _vp, _vp, C.c_int, C.c_int, C.POINTER(RolloutTraceBuffers), _vp, _vp]),
     "f1l_pure_pursuit_batch_dev": (C.c_int, [_vp, _vp, C.c_int, C.c_double, _vp, _vp, _vp, _vp,
                                              _vp, _vp, _vp]),
     "f1l_pure_pursuit_batch": (C.c_int, [_vp, _vp, C.c_int, C.c_double, _vp, _vp, _vp, _vp, _vp,

@@ -1827,14 +1827,17 @@ int f1l_default_rollout_config(f1l_rollout_config* rc) {
     return F1L_OK;
 }
 
-int f1l_rollout_dev(f1l_handle h, const f1l_rollout_config* rc, const f1l_fleet* fl, int S,
-                    int n_steps, const f1l_rollout_trace* trace, void* stream) {
-    return f1l_rollout_weights_dev(h, rc, fl, nullptr, S, n_steps, trace, stream);
+int f1l_default_vehicle(f1l_vehicle* veh) {
+    if (!veh) return F1L_ERR_INVALID_ARG;
+    *veh = f1l_vehicle{1.0489, 4.718, 5.4562, 0.15875, 0.17145, 0.074, 3.74, 0.04712, 3.2, 7.319, 0.5};
+    return F1L_OK;
 }
 
-int f1l_rollout_weights_dev(f1l_handle h, const f1l_rollout_config* rc, const f1l_fleet* fl,
-                            const float* weights_dev, int S, int n_steps, const f1l_rollout_trace* trace,
-                            void* stream) {
+// every rollout entry point: veh == nullptr runs the kinematic bicycle, else the single-track model
+// on dyn (checked by the caller)
+static int rollout_internal(f1l_handle h, const f1l_rollout_config* rc, const f1l_vehicle* veh,
+                            const f1l_fleet* fl, double* dyn, const float* weights_dev, int S, int n_steps,
+                            const f1l_rollout_trace* trace, double* trace_dyn, void* stream) {
     if (!h || !rc || !fl) return F1L_ERR_INVALID_ARG;
     if (!fl->state || !fl->prev_theta || !fl->has_prev || !fl->status || !fl->progress ||
         !fl->track_i || !fl->track_s)
@@ -1884,6 +1887,11 @@ int f1l_rollout_weights_dev(f1l_handle h, const f1l_rollout_config* rc, const f1
     a.track_s = fl->track_s;
     a.opp = (double*)h->r_opp.p;
     a.n_opp = (int32_t*)h->r_nopp.p;
+    if (veh) {
+        a.dyn = dyn;
+        a.veh = *veh;
+    }
+    void (*const step)(RolloutArgs) = veh ? rollout_step_kernel<SingleTrack> : rollout_step_kernel<Kinematic>;
     const unsigned blocks = (unsigned)((a.n_races + ROLLOUT_WARPS - 1) / ROLLOUT_WARPS);
 
     // once per call: global nearest_point of every car (K1) for the cars to re-acquire, then the
@@ -1895,7 +1903,7 @@ int f1l_rollout_weights_dev(f1l_handle h, const f1l_rollout_config* rc, const f1
     launch_pp(h, st, fl->state, 4, S, -1.0, h->cfg.wheelbase, 0.0, 0, 0.0, (unsigned long long*)sc.best.p, po);
     a.near_i = po.nearest_i;
     a.near4 = po.nearest;
-    rollout_step_kernel<<<blocks, ROLLOUT_WARPS * 32, 0, st>>>(a);
+    step<<<blocks, ROLLOUT_WARPS * 32, 0, st>>>(a);
     h->launches += 3;
     CK(cudaGetLastError());
     a.near_i = nullptr;
@@ -1925,11 +1933,34 @@ int f1l_rollout_weights_dev(f1l_handle h, const f1l_rollout_config* rc, const f1
         a.tr_ss = trace && trace->steer_speed ? trace->steer_speed + 2 * row : nullptr;
         a.tr_status = trace && trace->status ? trace->status + row : nullptr;
         a.tr_progress = trace && trace->progress ? trace->progress + row : nullptr;
-        rollout_step_kernel<<<blocks, ROLLOUT_WARPS * 32, 0, st>>>(a);
+        a.tr_dyn = trace_dyn ? trace_dyn + 3 * row : nullptr;
+        step<<<blocks, ROLLOUT_WARPS * 32, 0, st>>>(a);
         h->launches += 1;
         CK(cudaGetLastError());
     }
     return F1L_OK;
+}
+
+int f1l_rollout_dev(f1l_handle h, const f1l_rollout_config* rc, const f1l_fleet* fl, int S,
+                    int n_steps, const f1l_rollout_trace* trace, void* stream) {
+    return rollout_internal(h, rc, nullptr, fl, nullptr, nullptr, S, n_steps, trace, nullptr, stream);
+}
+
+int f1l_rollout_weights_dev(f1l_handle h, const f1l_rollout_config* rc, const f1l_fleet* fl,
+                            const float* weights_dev, int S, int n_steps, const f1l_rollout_trace* trace,
+                            void* stream) {
+    return rollout_internal(h, rc, nullptr, fl, nullptr, weights_dev, S, n_steps, trace, nullptr, stream);
+}
+
+int f1l_rollout_st_dev(f1l_handle h, const f1l_rollout_config* rc, const f1l_vehicle* veh,
+                       const f1l_fleet* fl, double* dyn_dev, const float* weights_dev, int S, int n_steps,
+                       const f1l_rollout_trace* trace, double* trace_dyn_dev, void* stream) {
+    if (!veh || !dyn_dev) return F1L_ERR_INVALID_ARG;
+    for (const double p : {veh->mu, veh->C_Sf, veh->C_Sr, veh->lf, veh->lr, veh->m, veh->I, veh->max_steer_vel,
+                           veh->v_switch, veh->v_kin})
+        if (!(p > 0)) return F1L_ERR_INVALID_ARG;
+    if (!(veh->h >= 0)) return F1L_ERR_INVALID_ARG;
+    return rollout_internal(h, rc, veh, fl, dyn_dev, weights_dev, S, n_steps, trace, trace_dyn_dev, stream);
 }
 
 // ---- pure pursuit -------------------------------------------------------------------------

@@ -1,4 +1,4 @@
-// f1l_rollout.cuh -- K6: one closed-loop step of a fleet of kinematic-bicycle cars (f1l_rollout_dev).
+// f1l_rollout.cuh -- K6: one closed-loop step of a fleet of cars (f1l_rollout_dev, f1l_rollout_st_dev).
 //
 // After the batch pipeline (sampler -> eval -> select) has planned every car of the fleet, this
 // kernel turns each car's (steer, speed) command into motion, tests the new poses against the map
@@ -9,6 +9,10 @@
 // One warp per race of G <= 17 consecutive cars, one lane per car.  All lanes of a race go through
 // the substeps together, so the car-to-car tests and the opponent table take the other cars' poses
 // from __shfl_sync: no global-memory exchange between cars.
+//
+// Two instances, one per vehicle model: Kinematic (the rear-axle kinematic bicycle) and SingleTrack
+// (f1tenth_gym's dynamic single-track model, one RK4 step per substep, include/f1l.h).  They differ
+// only in the motion of a live car within a substep; everything else is the same code.
 #pragma once
 #include "f1l_common.cuh"
 #include "f1l_lattice.cuh"
@@ -45,7 +49,94 @@ struct RolloutArgs {
     double* tr_ss;           // [S,2] raw command
     uint8_t* tr_status;      // [S] after the step
     double* tr_progress;     // [S] after the step
+    // single-track model only (appended: the kinematic instance reads none of it)
+    double* dyn;             // [S,3] delta, yaw rate, slip angle
+    double* tr_dyn;          // [S,3] dyn at the start of the step, nullable
+    f1l_vehicle veh;
 };
+
+struct Kinematic { static constexpr bool single_track = false; };
+struct SingleTrack { static constexpr bool single_track = true; };
+
+// d/dt of q = (x, y, delta, v, psi, yaw rate, beta) with (sv, acc) held; tests/st_model.py restates
+// it operation for operation.  cf / cr / A1 / A2 / A3 / B1 depend on acc only (once per substep).
+struct StSubstep {
+    double sv, acc, cf, A1, A2, A3, B1;
+};
+
+__device__ __forceinline__ void st_deriv(const RolloutArgs& a, double L, double kr, double kb,
+                                         const StSubstep& u, const double q[7], double f[7]) {
+    const double d = q[2], v = q[3], psi = q[4], r = q[5], b = q[6];
+    f[2] = u.sv;
+    f[3] = u.acc;
+    if (fabs(v) < a.veh.v_kin) {
+        // kinematic form
+        double sd, cd;
+        sincos(d, &sd, &cd);
+        const double td = __ddiv_rn(sd, cd);
+        double sp, cp;
+        sincos(psi, &sp, &cp);
+        f[0] = fm(v, cp);
+        f[1] = fm(v, sp);
+        f[4] = fm(__ddiv_rn(v, L), td);
+        f[5] = fa(fm(__ddiv_rn(u.acc, L), td), fm(__ddiv_rn(v, fm(fm(L, cd), cd)), u.sv));
+        f[6] = 0.0;
+    } else {
+        double sp, cp;
+        sincos(fa(psi, b), &sp, &cp);
+        const double iv = __ddiv_rn(1.0, v);
+        f[0] = fm(v, cp);
+        f[1] = fm(v, sp);
+        f[4] = r;
+        f[5] = fm(kr, fs(fa(fm(u.A2, b), fm(u.A3, d)), fm(fm(u.A1, iv), r)));
+        f[6] = fs(fm(fs(fm(fm(fm(kb, u.A2), iv), iv), 1.0), r), fm(fm(kb, iv), fs(fm(u.B1, b), fm(u.cf, d))));
+    }
+}
+
+// one substep of a live single-track car: command -> (sv, acc), then one classical RK4 step
+__device__ __forceinline__ void st_substep(const RolloutArgs& a, double steer, double target, double& x,
+                                           double& y, double& th, double& v, double& dl, double& r,
+                                           double& b) {
+    const f1l_vehicle& p = a.veh;
+    const double g = 9.81;
+    const double L = fa(p.lf, p.lr);
+    const double kr = __ddiv_rn(fm(p.mu, p.m), fm(p.I, L));
+    const double kb = __ddiv_rn(p.mu, L);
+    const double dt = a.dt;
+    StSubstep u;
+    u.sv = fmin(fmax(__ddiv_rn(fs(steer, dl), dt), -p.max_steer_vel), p.max_steer_vel);
+    const double a_pos = v > p.v_switch ? __ddiv_rn(fm(a.max_accel, p.v_switch), v) : a.max_accel;
+    u.acc = fmin(fmax(__ddiv_rn(fs(target, v), dt), -a.max_accel), a_pos);
+    const double Ff = fs(fm(g, p.lr), fm(u.acc, p.h)), Fr = fa(fm(g, p.lf), fm(u.acc, p.h));
+    u.cf = fm(p.C_Sf, Ff);
+    const double cr = fm(p.C_Sr, Fr);
+    u.A1 = fa(fm(fm(p.lf, p.lf), u.cf), fm(fm(p.lr, p.lr), cr));
+    u.A2 = fs(fm(p.lr, cr), fm(p.lf, u.cf));
+    u.A3 = fm(p.lf, u.cf);
+    u.B1 = fa(cr, u.cf);
+    const double q0[7] = {x, y, dl, v, th, r, b};
+    const double hdt = fm(0.5, dt), dt6 = __ddiv_rn(dt, 6.0);
+    double k[7], q[7], sum[7];
+    st_deriv(a, L, kr, kb, u, q0, k);
+#pragma unroll
+    for (int i = 0; i < 7; ++i) { sum[i] = k[i]; q[i] = fa(q0[i], fm(hdt, k[i])); }
+    st_deriv(a, L, kr, kb, u, q, k);
+#pragma unroll
+    for (int i = 0; i < 7; ++i) { sum[i] = fa(sum[i], fm(2.0, k[i])); q[i] = fa(q0[i], fm(hdt, k[i])); }
+    st_deriv(a, L, kr, kb, u, q, k);
+#pragma unroll
+    for (int i = 0; i < 7; ++i) { sum[i] = fa(sum[i], fm(2.0, k[i])); q[i] = fa(q0[i], fm(dt, k[i])); }
+    st_deriv(a, L, kr, kb, u, q, k);
+#pragma unroll
+    for (int i = 0; i < 7; ++i) sum[i] = fa(sum[i], k[i]);
+    x = fa(q0[0], fm(dt6, sum[0]));
+    y = fa(q0[1], fm(dt6, sum[1]));
+    dl = fa(q0[2], fm(dt6, sum[2]));
+    v = fa(q0[3], fm(dt6, sum[3]));
+    th = fa(q0[4], fm(dt6, sum[4]));
+    r = fa(q0[5], fm(dt6, sum[5]));
+    b = fa(q0[6], fm(dt6, sum[6]));
+}
 
 // the footprint's map predicate of collision_mode, in float64 in the map frame
 __device__ __forceinline__ bool rollout_map_hit(const RolloutArgs& a, double x, double y, double c,
@@ -79,7 +170,9 @@ __device__ __forceinline__ bool rollout_map_hit(const RolloutArgs& a, double x, 
     return hit;
 }
 
+template <class Model>
 __global__ void __launch_bounds__(ROLLOUT_WARPS * 32) rollout_step_kernel(RolloutArgs a) {
+    constexpr bool ST = Model::single_track;
     const int lane = threadIdx.x & 31;
     const int race = blockIdx.x * ROLLOUT_WARPS + (threadIdx.x >> 5);
     if (race >= a.n_races) return;   // warp-uniform
@@ -106,7 +199,19 @@ __global__ void __launch_bounds__(ROLLOUT_WARPS * 32) rollout_step_kernel(Rollou
         double target = 0.0;
         if (a.best_cost[car] < CUDART_INF_F) target = fmin(cmd_speed, a.v_max);
         else st |= F1L_CAR_NO_FEASIBLE;
+        double dl = 0.0, r = 0.0, b = 0.0;   // single-track: delta, yaw rate, slip angle
+        if constexpr (ST) {
+            dl = a.dyn[3 * (size_t)car];
+            r = a.dyn[3 * (size_t)car + 1];
+            b = a.dyn[3 * (size_t)car + 2];
+        }
         if (live) {
+            if constexpr (ST) {
+                if (a.tr_dyn) {
+                    double* o = a.tr_dyn + 3 * (size_t)car;
+                    o[0] = dl; o[1] = r; o[2] = b;
+                }
+            }
             if (a.tr_state) {
                 double2* o = reinterpret_cast<double2*>(a.tr_state + 4 * (size_t)car);
                 o[0] = make_double2(x, y);
@@ -119,7 +224,10 @@ __global__ void __launch_bounds__(ROLLOUT_WARPS * 32) rollout_step_kernel(Rollou
         const double c_hl = a.hl, c_hw = a.hw;
         for (int k = 0; k < a.substeps; ++k) {
             if (st & (F1L_CAR_HIT_MAP | F1L_CAR_HIT_CAR)) {
-                v = 0.0;   // frozen: keeps its pose
+                v = 0.0;   // frozen: keeps its pose (and steering angle)
+                if constexpr (ST) { r = 0.0; b = 0.0; }
+            } else if constexpr (ST) {
+                st_substep(a, steer, target, x, y, th, v, dl, r, b);
             } else {
                 v = fa(v, fmin(fmax(fs(target, v), -dv), dv));
                 x = fa(x, fm(fm(v, cos(th)), a.dt));
@@ -135,7 +243,10 @@ __global__ void __launch_bounds__(ROLLOUT_WARPS * 32) rollout_step_kernel(Rollou
                 const double cj = __shfl_sync(F1L_FULL, c, j), sj = __shfl_sync(F1L_FULL, s, j);
                 if (j != lane && sat_collide(fs(xj, x), fs(yj, y), c, s, cj, sj, c_hl, c_hw)) st |= F1L_CAR_HIT_CAR;
             }
-            if (st & (F1L_CAR_HIT_MAP | F1L_CAR_HIT_CAR)) v = 0.0;
+            if (st & (F1L_CAR_HIT_MAP | F1L_CAR_HIT_CAR)) {
+                v = 0.0;
+                if constexpr (ST) { r = 0.0; b = 0.0; }
+            }
         }
         // raceline progress: nearest segment in a 32-segment window starting 4 behind the tracked
         // one, cyclic over the n-1 segments, first minimum in window order (nearest_point's own
@@ -165,6 +276,10 @@ __global__ void __launch_bounds__(ROLLOUT_WARPS * 32) rollout_step_kernel(Rollou
             double2* o = reinterpret_cast<double2*>(a.state + 4 * (size_t)car);
             o[0] = make_double2(x, y);
             o[1] = make_double2(th, v);
+            if constexpr (ST) {
+                double* d = a.dyn + 3 * (size_t)car;
+                d[0] = dl; d[1] = r; d[2] = b;
+            }
             a.status[car] = (uint8_t)st;
             a.progress[car] = prog;
             a.track_i[car] = ti;

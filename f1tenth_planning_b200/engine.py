@@ -326,12 +326,14 @@ class Engine:
         self._ck(self._L.f1l_plan_batch_call_dev(self._h, C.byref(b), C.c_void_p(st)))
 
     # -- closed-loop rollouts ----------------------------------------------------------------
-    def fleet(self, poses, group=1, weights=None):
+    def fleet(self, poses, group=1, weights=None, vehicle=None):
         """A fleet of kinematic-bicycle cars at `poses` [S,4] (x, y, theta, v) on this engine's
         device, raced in groups of `group` consecutive cars, each planned with its row of
-        `weights` [S,5] (None: the configured weights) (rollout.Fleet, f1l_rollout_weights_dev)."""
+        `weights` [S,5] (None: the configured weights) (rollout.Fleet, f1l_rollout_weights_dev).
+        With a rollout.Vehicle the cars follow the dynamic single-track model instead
+        (f1l_rollout_st_dev)."""
         from .rollout import Fleet
-        return Fleet(self, poses, group, weights)
+        return Fleet(self, poses, group, weights, vehicle)
 
     # -- candidate sharding over peer memory -------------------------------------------------
     def export_peer_handle(self):

@@ -344,7 +344,8 @@ int f1l_plan_batch_call_dev(f1l_handle h, const f1l_batch_call* b, void* stream)
 int f1l_plan_batch_call(f1l_handle h, const f1l_batch_call* b);
 
 /*
- * Closed-loop rollouts on the device: a fleet of S kinematic-bicycle cars advanced n_steps planning
+ * Closed-loop rollouts on the device: a fleet of S kinematic-bicycle cars (f1l_rollout_st_dev below:
+ * dynamic single-track cars) advanced n_steps planning
  * steps.  Replaces the user loop around the planner -- plan, then step the vehicle
  * (lattice_planner.py:204-214 plus the gym step of examples/control/pure_pursuit.py:47-57, which
  * is not part of the reference checkout) -- with no host synchronisation and no host copy inside
@@ -427,6 +428,58 @@ int f1l_rollout_dev(f1l_handle h, const f1l_rollout_config* rc, const f1l_fleet*
 int f1l_rollout_weights_dev(f1l_handle h, const f1l_rollout_config* rc, const f1l_fleet* fleet,
                             const float* weights_dev, int n_scenarios, int n_steps,
                             const f1l_rollout_trace* trace, void* stream);
+
+/*
+ * The dynamic single-track (ST) vehicle model of f1tenth_gym (CommonRoad's vehicle_dynamics_st),
+ * for rollouts whose cars understeer, slide and answer the steering late.  Defaults are
+ * f1tenth_gym's; max_steer, max_accel and v_max stay in f1l_rollout_config.
+ */
+typedef struct {
+    double mu;             /* surface friction coefficient, > 0 */
+    double C_Sf;           /* front cornering stiffness coefficient (1/rad), > 0 */
+    double C_Sr;           /* rear cornering stiffness coefficient (1/rad), > 0 */
+    double lf;             /* centre of gravity to front axle (m), > 0 */
+    double lr;             /* centre of gravity to rear axle (m), > 0 */
+    double h;              /* height of the centre of gravity (m), >= 0 */
+    double m;              /* mass (kg), > 0 */
+    double I;              /* yaw moment of inertia (kg m^2), > 0 */
+    double max_steer_vel;  /* steering rate limit (rad/s), > 0 */
+    double v_switch;       /* speed above which the acceleration limit falls as 1/v (m/s), > 0 */
+    double v_kin;          /* speed below which the kinematic form is used (m/s), > 0 */
+} f1l_vehicle;
+
+/* Defaults: mu 1.0489, C_Sf 4.718, C_Sr 5.4562, lf 0.15875, lr 0.17145, h 0.074, m 3.74,
+ * I 0.04712, max_steer_vel 3.2, v_switch 7.319, v_kin 0.5. */
+int f1l_default_vehicle(f1l_vehicle* veh);
+
+/*
+ * f1l_rollout_weights_dev with the ST model.  The fleet's state (x, y, psi, v) is unchanged and
+ * still what the planner reads (theta = psi, (x, y) the model's reference point, which the
+ * footprint, collision tests, progress and opponent table use as before).  dyn_dev [S,3] f64
+ * (steering angle delta, yaw rate, slip angle beta) is read and written in place; zeros for a car
+ * at rest.  Every rule of f1l_rollout_dev holds except step 3, which becomes, per substep:
+ *   sv = clamp((clamp(steer_cmd, +-max_steer) - delta) / dt, +-max_steer_vel);
+ *   a = clamp((target - v) / dt, -max_accel, a_pos), a_pos = max_accel * v_switch / v when
+ *   v > v_switch, else max_accel (f1tenth_gym's power limit);
+ *   with (sv, a) held, one classical RK4 step in float64 of (x, y, delta, v, psi, yaw rate, beta)
+ *   under f1tenth_gym's equations: the kinematic form when |v| < v_kin, else the dynamic one
+ *   (L = lf + lr, g = 9.81, load transfer through h).  psi is not wrapped.
+ * A frozen car keeps its pose and delta at v = yaw rate = beta = 0.
+ *
+ * The tyres are linear and never saturate, as in f1tenth_gym: there is no friction circle, so the
+ * model has no grip limit at high lateral acceleration.  RK4 is stable here only for a small
+ * enough dt: the fastest (yaw rate, beta) mode is at the lowest dynamic speed, v = v_kin, where
+ * with the defaults and dt = 0.01 it has dt * |lambda| = 2.27, inside RK4's real-axis limit of
+ * 2.785.  A larger dt or a smaller v_kin can make the integration diverge.
+ *
+ * trace_dyn_dev [T,S,3] f64 or NULL: dyn at the START of step k.  F1L_ERR_INVALID_ARG as
+ * f1l_rollout_dev, and for a null vehicle or dyn_dev, any of mu, C_Sf, C_Sr, lf, lr, m, I,
+ * max_steer_vel, v_switch, v_kin that is not positive (NaN included), or a negative or NaN h.
+ */
+int f1l_rollout_st_dev(f1l_handle h, const f1l_rollout_config* rc, const f1l_vehicle* veh,
+                       const f1l_fleet* fleet, double* dyn_dev, const float* weights_dev,
+                       int n_scenarios, int n_steps, const f1l_rollout_trace* trace,
+                       double* trace_dyn_dev, void* stream);
 
 /*
  * Batched nearest_point + pure-pursuit lookahead over B poses on the uploaded track.

@@ -5,7 +5,10 @@ device-resident loop cost.
     configuration (the cars start at bench.py's seeded scenario poses), --steps planning steps.
     Device time per step (CUDA events) of Fleet.run against f1l_plan_batch_prev_dev alone on the
     same fleet state (the races' opponents uploaded once, previous paths updated in place), and the
-    mean device time of rollout_step_kernel from a torch.profiler pass of its own.
+    mean device time of rollout_step_kernel from a torch.profiler pass of its own.  With
+    --vehicle st a fleet of dynamic single-track cars (rollout.Vehicle's defaults) at the same poses
+    is timed as a third arm, alternated with the others, and each model's rollout_step_kernel
+    instance gets a profiler pass of its own.
 (b) latency: 32 cars, --long-steps steps, wall time per step (host clock around calls that end in a
     device synchronise) of one Fleet.run call against the Python loop of the batch planner's
     device-resident test: plan_batch_dev + a kinematic bicycle in torch, one step at a time.
@@ -13,6 +16,7 @@ Arms alternate for --rounds rounds.  Prints one JSON line (and writes it to --ou
 name and power limit read in the same run.  Needs a CUDA device; there is no CPU fallback.
 
     python tools/rollout_bench.py --out rollout.json
+    python tools/rollout_bench.py --vehicle st --out rollout_st.json
 """
 import argparse
 import json
@@ -68,11 +72,14 @@ def main():
     ap.add_argument("--long-cars", type=int, default=32)
     ap.add_argument("--long-steps", type=int, default=500, help="(b) planning steps per timed call")
     ap.add_argument("--rounds", type=int, default=3)
+    ap.add_argument("--vehicle", choices=("kinematic", "st"), default="kinematic",
+                    help="st: also time (a) with the dynamic single-track model")
     ap.add_argument("--out", help="also write the JSON line to this file")
     args = ap.parse_args()
 
     import torch
     from f1tenth_planning_b200.engine import Engine
+    from f1tenth_planning_b200.rollout import Vehicle
     if not torch.cuda.is_available():
         raise RuntimeError("rollout_bench.py needs a CUDA device")
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -89,6 +96,10 @@ def main():
     # (a) the fleet's own steps against the planner alone on the same state
     fleet = eng.fleet(poses, group=G)
     fleet.run(2)   # warm-up: buffers, modules
+    fleets = {"fleet_run": fleet}
+    if args.vehicle == "st":
+        fleets["fleet_run_st"] = eng.fleet(poses, group=G, vehicle=Vehicle())
+        fleets["fleet_run_st"].run(2)
     opp, n_opp = race_opponents(torch, dev, fleet.state.cpu().numpy(), G)
     P = fleet.prev_theta.clone()
     V = fleet.has_prev.clone()
@@ -102,16 +113,22 @@ def main():
                                steer_speed=o_ss, prev_theta=P, has_prev=V, update_prev=True)
 
     plan_only()
-    ms_a = {"fleet_run": [], "plan_batch_prev_dev": []}
+    ms_a = {name: [] for name in fleets}
+    ms_a["plan_batch_prev_dev"] = []
     for _ in range(args.rounds):
-        ms_a["fleet_run"].append(event_ms(torch, lambda: fleet.run(T)) / T)
+        for name, f in fleets.items():
+            ms_a[name].append(event_ms(torch, lambda: f.run(T)) / T)
         ms_a["plan_batch_prev_dev"].append(event_ms(torch, plan_only) / T)
-    assert torch.isfinite(fleet.state).all()
+    for f in fleets.values():
+        assert torch.isfinite(f.state).all() and (f.dyn is None or torch.isfinite(f.dyn).all())
     from torch.profiler import profile, ProfilerActivity
-    with profile(activities=[ProfilerActivity.CUDA]) as prof:
-        fleet.run(T)
-        torch.cuda.synchronize(dev)
-    step_us = [e.device_time_total / e.count for e in prof.key_averages() if "rollout_step_kernel" in e.key]
+    step_us = {}
+    for name, f in fleets.items():   # one pass per model: the instances' names differ by template only
+        with profile(activities=[ProfilerActivity.CUDA]) as prof:
+            f.run(T)
+            torch.cuda.synchronize(dev)
+        us = [e.device_time_total / e.count for e in prof.key_averages() if "rollout_step_kernel" in e.key]
+        step_us[name] = us[0] if us else None
 
     # (b) one Fleet.run call against the Python loop with a torch bicycle
     Sb, Tb = args.long_cars, args.long_steps
@@ -146,7 +163,8 @@ def main():
         "a_workload": "%d cars in races of %d, bench.py ellipse + corridor, %d candidates, M=%d, %d steps"
                       % (S, G, eng.n_candidates, M, T),
         "a_device_ms_per_step": mean(ms_a), "a_device_ms_per_step_rounds": ms_a,
-        "a_step_kernel_us_profiler": step_us[0] if step_us else None,
+        "a_step_kernel_us_profiler": step_us["fleet_run"],
+        "a_step_kernel_us_profiler_st": step_us.get("fleet_run_st"),
         "b_workload": "%d cars, %d steps" % (Sb, Tb),
         "b_wall_ms_per_step": mean(ms_b), "b_wall_ms_per_step_rounds": ms_b,
         "card": card(local), "device_name": torch.cuda.get_device_name(dev),
