@@ -963,8 +963,12 @@ __global__ void __launch_bounds__(NW * 32, MINB) eval_kernel(EvalArgs a) {
                 const float avx = fmaf(cth, ax, sth * ay), avy = fmaf(cth, ay, -sth * ax);
                 const float dx = fmaf(cth, dxm, sth * dym), dy = fmaf(cth, dym, -sth * dxm);
                 const float l2 = fmaf(dx, dx, dy * dy);
-                const float il = rsqrtf(l2);
-                const float ux = dx * il, uy = dy * il;
+                // a zero-length segment (a repeated waypoint) is its point: any unit direction,
+                // h = 0.  (rsqrtf(0) would make the entry NaN, which the minima ignore, and the
+                // point would drop out of a window it ends.)
+                const bool point = !(l2 > 0.0f);
+                const float il = point ? 0.0f : rsqrtf(l2);
+                const float ux = point ? 1.0f : dx * il, uy = point ? 0.0f : dy * il;
                 T0 = make_float4(ux, uy, -uy, il);
                 const float hh = 0.5f * (l2 * il);
                 T1 = make_float4(-(fmaf(avx, ux, avy * uy) + hh) * EVAL_DEV_SCALE,
