@@ -123,6 +123,10 @@ ST_FIELDS = {   # the single-track fleet's array beside f1l_fleet (f1l_rollout_s
     "dyn": (("float64",), ("S", 3), INOUT),
 }
 
+MOTION_FIELDS = {   # the opponent velocities beside a batch call (f1l_plan_batch_motion*)
+    "opp_vel": (("float64",), ("S", "K", 2), IN),
+}
+
 PP_FIELDS = {   # the outputs of f1l_pure_pursuit_batch, in argument order
     "nearest": (("float64",), ("B", 4), OUT),
     "nearest_i": (("int32",), ("B",), OUT),
@@ -196,6 +200,7 @@ SIGNATURES = {
     "f1l_set_prev_path": (C.c_int, [_vp, _fp, C.c_int]),
     "f1l_clear_prev_path": (C.c_int, [_vp]),
     "f1l_plan": (C.c_int, [_vp, _vp, _vp, C.c_int, C.c_int, C.POINTER(PlanResult)]),
+    "f1l_plan_motion": (C.c_int, [_vp, _vp, _vp, _vp, C.c_int, C.c_double, C.c_int, C.POINTER(PlanResult)]),
     "f1l_plan_shard": (C.c_int, [_vp, _vp, _vp, C.c_int, C.c_int, C.c_int, C.POINTER(PlanResult)]),
     "f1l_plan_goals": (C.c_int, [_vp, _vp, _vp, C.c_int, _vp, C.c_int, C.c_int,
                                  C.POINTER(PlanResult)]),
@@ -211,6 +216,8 @@ SIGNATURES = {
                                       _vp, _vp, _vp, _vp, _vp, _vp]),
     "f1l_plan_batch_call_dev": (C.c_int, [_vp, C.POINTER(BatchCall), _vp]),
     "f1l_plan_batch_call": (C.c_int, [_vp, C.POINTER(BatchCall)]),
+    "f1l_plan_batch_motion_dev": (C.c_int, [_vp, C.POINTER(BatchCall), _vp, C.c_double, _vp]),
+    "f1l_plan_batch_motion": (C.c_int, [_vp, C.POINTER(BatchCall), _vp, C.c_double]),
     "f1l_default_rollout_config": (C.c_int, [C.POINTER(RolloutConfig)]),
     "f1l_rollout_dev": (C.c_int, [_vp, C.POINTER(RolloutConfig), C.POINTER(FleetBuffers), C.c_int,
                                   C.c_int, C.POINTER(RolloutTraceBuffers), _vp]),
@@ -219,6 +226,9 @@ SIGNATURES = {
     "f1l_default_vehicle": (C.c_int, [C.POINTER(Vehicle)]),
     "f1l_rollout_st_dev": (C.c_int, [_vp, C.POINTER(RolloutConfig), C.POINTER(Vehicle), C.POINTER(FleetBuffers),
                                      _vp, _vp, C.c_int, C.c_int, C.POINTER(RolloutTraceBuffers), _vp, _vp]),
+    "f1l_rollout_predict_dev": (C.c_int, [_vp, C.POINTER(RolloutConfig), C.POINTER(Vehicle),
+                                          C.POINTER(FleetBuffers), _vp, _vp, C.c_double, C.c_int, C.c_int,
+                                          C.POINTER(RolloutTraceBuffers), _vp, _vp]),
     "f1l_pure_pursuit_batch_dev": (C.c_int, [_vp, _vp, C.c_int, C.c_double, _vp, _vp, _vp, _vp,
                                              _vp, _vp, _vp]),
     "f1l_pure_pursuit_batch": (C.c_int, [_vp, _vp, C.c_int, C.c_double, _vp, _vp, _vp, _vp, _vp,
@@ -244,6 +254,7 @@ SIGNATURES = {
     "f1l_measure_peaks": (C.c_int, [_vp, _dp, _dp]),
     "f1l_measure_peaks_ex": (C.c_int, [_vp, _dp, C.c_int]),
     "f1l_debug_query_ctx": (C.c_int, [_vp, _fp, _ip]),
+    "f1l_debug_motion_ctx": (C.c_int, [_vp, _fp, C.c_int]),
     "f1l_debug_eval_plan": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _ip, C.c_int]),
     "f1l_debug_eval_choice": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _ip, C.c_int]),
     "f1l_debug_eval_builds": (C.c_int, [_ip, C.c_int]),

@@ -61,7 +61,7 @@ struct PipeScratch {
 
 // The per-scenario arrays of a host-buffer batch chunk, in the order they are copied
 enum { B_POSES, B_OPP, B_NOPP, B_IDX, B_COST, B_TRAJ, B_COSTS, B_FLAGS, B_SS, B_PREV, B_PVALID, B_W, B_TERMS,
-       B_ARRAYS };
+       B_VEL, B_ARRAYS };
 
 struct PipeSlot {
     cudaStream_t stream = nullptr;
@@ -105,6 +105,7 @@ struct f1l_ctx {
     unsigned long long epoch = 0;   // bumped by every upload / config change
     cudaGraphExec_t gexec = nullptr;
     unsigned long long gkey[2] = {~0ull, ~0ull};   // epoch and output mask of the captured graph
+    double gvmin = 0.0;                            // ... v_min of a captured moving-opponent query
     Span gspan;                                    // ... and its span
     int timed = 0;  // events of the last pipeline launch are valid
 #define F1L_EV_SLOTS 64
@@ -151,6 +152,8 @@ struct f1l_ctx {
     PipeScratch b_scratch;
     // rollout (f1l_rollout_dev) scratch: command, cost, the races' opponent table
     DevBuf r_ss, r_cost, r_opp, r_nopp;
+    DevBuf r_vel;   // the races' opponent velocities [S,F1L_MAX_OPP,2] (f1l_rollout_predict_dev)
+    DevBuf mo_dbg;  // k_t and (wx, wy) of the last moving-opponent single query (f1l_debug_motion_ctx)
     // batch pipeline (host-pointer API)
     PipeSlot pipe[N_PIPE];
     // device copies of the arrays of the one-shot host-buffer calls (pure pursuit, intersect, ...)
@@ -164,7 +167,7 @@ struct f1l_ctx {
     DevBuf xchg;
     XchgView xview = {0, 0, {nullptr}};
     // template instance / CTA plan of the last eval_kernel launch (f1l_last_eval_shape)
-    int eval_info[10] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
+    int eval_info[11] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
     // the last single query, for f1l_select_candidate: its span, explicit goals?, epoch
     Span lastq_span;
     int lastq_goals = 0;
@@ -376,13 +379,17 @@ constexpr int EVAL_SMEM_MAX = 226 * 1024;
 
 // One compiled eval_kernel: the resident CTAs per SM its register budget is built for (MINB), and
 // its shared memory in front of the window table (EvalSmem::C_TAB).
+// shared memory the MO twin stages in front of the window table (the opponent velocities and k_t)
+constexpr uint32_t EVAL_MO_SMEM = EvalSmem<1, 8, 1, true>::C_TAB - EvalSmem<1, 8, 1>::C_TAB;
+
 struct EvalBuild {
     eval_fn fn;     // null: not built
     eval_fn fn_w;   // the same with per-scenario cost weights (null: not built)
     int minb;
     uint32_t smem_fixed;
-    size_t smem_bytes(int nseg_pad) const {
-        return smem_fixed + (size_t)(nseg_pad + EVAL_SEG_PAD) * (2 * sizeof(float4));
+    eval_fn fn_m = nullptr;   // fn_w's twin with moving opponents (null: not built)
+    size_t smem_bytes(int nseg_pad, bool mo = false) const {
+        return smem_fixed + (mo ? EVAL_MO_SMEM : 0) + (size_t)(nseg_pad + EVAL_SEG_PAD) * (2 * sizeof(float4));
     }
 };
 
@@ -404,7 +411,7 @@ EvalBuild eval_build() {
     if constexpr (MINB == 0) return {nullptr, nullptr, 0, 0};
     else if constexpr (!WEIGHTS) return {eval_kernel<IPL, S, SG, NW, MINB, false>, nullptr, MINB, EvalSmem<S, SG, NW>::C_TAB};
     else return {eval_kernel<IPL, S, SG, NW, MINB, false>, eval_kernel<IPL, S, SG, NW, MINB, true>, MINB,
-                 EvalSmem<S, SG, NW>::C_TAB};
+                 EvalSmem<S, SG, NW>::C_TAB, eval_kernel<IPL, S, SG, NW, MINB, true, true>};
 }
 template <int M_MAX, int IPL, int S, int SG, int MINB4, int MINB7, int MINB8, int MINB_WIDE>
 EvalBucket eval_bucket() {
@@ -516,14 +523,17 @@ struct EvalChoice {
     bool persistent;   // one wave of CTAs pulling candidates from a device-wide counter
     bool wide;         // build is bucket->wide
     bool pw;           // per-scenario cost weights: build->fn_w
-    eval_fn fn() const { return pw ? build->fn_w : build->fn; }
+    bool mo;           // moving opponents: build->fn_m (pw is set too)
+    eval_fn fn() const { return mo ? build->fn_m : (pw ? build->fn_w : build->fn); }
 };
 
 // The whole instance choice of a pipeline launch (launch_pipeline, f1l_debug_eval_choice): the CTA
 // plan, the persistent grid and the wide build of a lone dense query, and the PW twin of a call
 // with per-scenario cost weights.  lone: a single query with a persistent-grid counter and a
-// non-empty span.
-EvalChoice choose_eval(int n_cand, int S, int M, int sm_count, bool cubic, bool lone, bool weights) {
+// non-empty span.  motion: the MO twin of the PW instance, chosen as for a call with weights.
+EvalChoice choose_eval(int n_cand, int S, int M, int sm_count, bool cubic, bool lone, bool weights,
+                       bool motion = false) {
+    weights = weights || motion;
     const CtaPlan cp = plan_ctas(n_cand, S, M, sm_count, cubic);
     EvalChoice c;
     c.bucket = &eval_bucket_of(M);
@@ -534,6 +544,7 @@ EvalChoice choose_eval(int n_cand, int S, int M, int sm_count, bool cubic, bool 
     // four candidates per warp at a time (shared Newton) when every warp has at least four
     c.item = (cubic && cp.chunk >= 4 * cp.nw) ? EVAL_ITEM : 1;
     c.pw = weights;
+    c.mo = motion;
     // A lone dense query that needs more than one wave of CTAs runs on a PERSISTENT grid instead: one
     // wave of CTAs whose warps pull single candidates from a device-wide counter, far lookahead rows
     // (the expensive candidates) first.  No wave quantisation, one window-table prologue per
@@ -648,6 +659,11 @@ struct PipeIn {
     const float* weights = nullptr;    // [S,5] cost weights per scenario (null: the config's)
     const XchgView* xc = nullptr;      // sharded single query: exchange the argmin with the peers
     int* work_next = nullptr;          // single query: device counter for the persistent-grid schedule
+    // moving opponents: velocities [S,max_opp,2] (null without opponents), the ego's v_min
+    bool motion = false;
+    const double* opp_vel = nullptr;
+    double v_min = 1.0;
+    float* mo_ctx = nullptr;           // debug copy of scenario 0's k_t and velocities (nullable)
 };
 
 // The span of a query over the explicit goals (n_goals > 0) or the goal grid (n_goals 0), with the
@@ -743,10 +759,10 @@ int launch_pipeline(f1l_handle h, cudaStream_t stream, const PipeIn& in, PipeScr
     const int nseg_pad = (nseg + 31) & ~31;
     const int n_cand = sp.empty ? 1 : sp.c_end - sp.c_begin;
     const EvalChoice ec = choose_eval(n_cand, S, M, h->sm_count, ep.generator == 0,
-                                      S == 1 && in.work_next && !sp.empty, in.weights != nullptr);
+                                      S == 1 && in.work_next && !sp.empty, in.weights != nullptr, in.motion);
     if (!ec.fn()) return F1L_ERR_INVALID_ARG;   // the choice names an instance that is not built
     const bool dyn = ec.persistent;
-    const size_t smem = ec.build->smem_bytes(nseg_pad);
+    const size_t smem = ec.build->smem_bytes(nseg_pad, ec.mo);
     if (smem > EVAL_SMEM_MAX) return F1L_ERR_TOO_LARGE;
 
     SampleArgs sa;
@@ -829,14 +845,18 @@ int launch_pipeline(f1l_handle h, cudaStream_t stream, const PipeIn& in, PipeScr
     ea.headings = o.headings;
     ea.best = best;
     ea.stats = h->stats_on ? (unsigned long long*)h->stats.p : nullptr;
+    ea.opp_vel = in.motion ? in.opp_vel : nullptr;
+    ea.vel_stride = in.max_opp;
+    ea.v_min = in.v_min;
+    ea.mo_ctx = in.motion ? in.mo_ctx : nullptr;
     const long long n_ctas = (long long)S * ea.ctas_per_scn;
     if (n_ctas > 0x7fffffffLL) return F1L_ERR_TOO_LARGE;
     if (!sp.empty) ec.fn()<<<(unsigned)n_ctas, ec.nw * 32, smem, stream>>>(ea);
     {
         const EvalBucket& b = *ec.bucket;
-        const int info[10] = {b.ipl, b.s, b.sg, ec.nw, ec.build->minb, ea.chunk, ea.ctas_per_scn, ea.item,
-                              (int)ec.persistent, (int)ec.pw};
-        for (int i = 0; i < 10; ++i) h->eval_info[i] = info[i];
+        const int info[11] = {b.ipl, b.s, b.sg, ec.nw, ec.build->minb, ea.chunk, ea.ctas_per_scn, ea.item,
+                              (int)ec.persistent, (int)ec.pw, (int)ec.mo};
+        for (int i = 0; i < 11; ++i) h->eval_info[i] = info[i];
     }
     if (time_it) cudaEventRecord(ev[2], stream);
 
@@ -904,7 +924,16 @@ struct QInput {
     double pose[4];
     int32_t n_opp, pad;
     double opp[3 * F1L_MAX_OPP];
+    double opp_vel[2 * F1L_MAX_OPP];   // f1l_plan_motion
 };
+static_assert(sizeof(QInput) <= 1024, "QInput fits the pinned staging block");
+
+// the checks every moving-opponent entry point makes on v_min and the velocity pointer
+int check_motion(int n_opp, const double* opp_vel, double v_min) {
+    if (!std::isfinite(v_min) || !(v_min > 0.0)) return F1L_ERR_INVALID_ARG;
+    if (n_opp > 0 && !opp_vel) return F1L_ERR_INVALID_ARG;
+    return F1L_OK;
+}
 
 }  // namespace
 
@@ -1012,7 +1041,7 @@ int f1l_debug_pp_parts(int n_poses, int n_waypoints, int slots) {
 
 int f1l_last_eval_shape(f1l_handle h, int32_t* out, int n) {
     if (!h || !out || n < 8) return F1L_ERR_INVALID_ARG;
-    for (int i = 0; i < n && i < 10; ++i) out[i] = h->eval_info[i];
+    for (int i = 0; i < n && i < 11; ++i) out[i] = h->eval_info[i];
     return F1L_OK;
 }
 
@@ -1134,7 +1163,7 @@ int f1l_create(f1l_handle* out, int device, const f1l_config* cfg) {
         // opt in to large dynamic shared memory for every eval instantiation
         for (const EvalBucket& b : kEvalBuckets) {
             for (const EvalBuild* eb : {&b.nw4, &b.nw7, &b.nw8, &b.wide}) {
-                for (eval_fn fn : {eb->fn, eb->fn_w}) {
+                for (eval_fn fn : {eb->fn, eb->fn_w, eb->fn_m}) {
                     if (!fn) continue;
                     cudaError_t e2 = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, EVAL_SMEM_MAX);
                     if (e2 != cudaSuccess && e == cudaSuccess) e = e2;
@@ -1379,11 +1408,18 @@ int f1l_clear_prev_path(f1l_handle h) {
 }
 
 // ---- single query -------------------------------------------------------------------------
+// opp_vel / v_min: moving opponents (f1l_plan_motion; motion false: static)
 static int plan_internal(f1l_handle h, const double pose[4], const double* opp, int n_opp,
                          const double* goals, int n_goals, const Shard& shard, bool exchange,
-                         int update_prev, f1l_plan_result* out) {
+                         int update_prev, f1l_plan_result* out, bool motion = false,
+                         const double* opp_vel = nullptr, double v_min = 1.0) {
     if (!h || !pose || !out) return F1L_ERR_INVALID_ARG;
     if (n_opp < 0 || n_opp > F1L_MAX_OPP || (n_opp > 0 && !opp)) return F1L_ERR_INVALID_ARG;
+    if (motion) {
+        if (const int r = check_motion(n_opp, opp_vel, v_min); r != F1L_OK) return r;
+        for (int k = 0; k < 2 * n_opp; ++k)
+            if (!std::isfinite(opp_vel[k])) return F1L_ERR_INVALID_ARG;
+    }
     if (h->n < 2) return F1L_ERR_NO_TRACK;
     CK(cudaSetDevice(h->device));
     exchange = exchange && h->xview.world > 1;
@@ -1400,7 +1436,9 @@ static int plan_internal(f1l_handle h, const double pose[4], const double* opp, 
     hin->n_opp = n_opp;
     hin->pad = 0;
     if (n_opp) memcpy(hin->opp, opp, (size_t)n_opp * 3 * sizeof(double));
+    if (motion && n_opp) memcpy(hin->opp_vel, opp_vel, (size_t)n_opp * 2 * sizeof(double));
     ENS(h->q_in, sizeof(QInput));
+    if (motion) ENS(h->mo_dbg, (1 + 2 * F1L_MAX_OPP) * sizeof(float));
     if (const int r = h->q_scratch.reserve(h, 1); r != F1L_OK) return r;
     ENS(h->prev, F1L_MAX_M * sizeof(float));
     // detail block layout (every region 16-byte aligned)
@@ -1454,6 +1492,12 @@ static int plan_internal(f1l_handle h, const double pose[4], const double* opp, 
     in.max_opp = F1L_MAX_OPP;
     in.prev_theta = h->has_prev ? (const float*)h->prev.p : nullptr;
     in.work_next = (int*)((char*)h->q_scratch.best.p + 8);   // behind the one argmin key
+    if (motion) {
+        in.motion = true;
+        in.opp_vel = din->opp_vel;
+        in.v_min = v_min;
+        in.mo_ctx = (float*)h->mo_dbg.p;
+    }
     // H2D of the input block, the three kernels, D2H of the detail block.  The similarity term
     // reads the previous path while select overwrites it: eval reads it before select runs
     // (stream order), so one buffer suffices.
@@ -1480,8 +1524,10 @@ static int plan_internal(f1l_handle h, const double pose[4], const double* opp, 
                                         (out->goals ? 4u : 0u) | (out->params ? 8u : 0u) |
                                         (out->states ? 16u : 0u) | (out->headings ? 32u : 0u) |
                                         (update_prev ? 64u : 0u) | (h->has_prev ? 128u : 0u) |
-                                        (exchange ? 512u : 0u) | (out->best_traj_map ? 1024u : 0u);
-        if (!h->gexec || h->gkey[0] != h->epoch || h->gkey[1] != mask || memcmp(&h->gspan, &sp, sizeof(Span))) {
+                                        (exchange ? 512u : 0u) | (out->best_traj_map ? 1024u : 0u) |
+                                        (motion ? 2048u : 0u);
+        if (!h->gexec || h->gkey[0] != h->epoch || h->gkey[1] != mask || memcmp(&h->gspan, &sp, sizeof(Span)) ||
+            (motion && h->gvmin != v_min)) {
             if (h->gexec) { cudaGraphExecDestroy(h->gexec); h->gexec = nullptr; }
             const int64_t launches0 = h->launches;
             cudaGraph_t graph = nullptr;
@@ -1497,6 +1543,7 @@ static int plan_internal(f1l_handle h, const double pose[4], const double* opp, 
             h->gkey[0] = h->epoch;
             h->gkey[1] = mask;
             h->gspan = sp;
+            h->gvmin = motion ? v_min : 0.0;
         }
         CK(cudaGraphLaunch(h->gexec, st));
         h->launches += 3;
@@ -1530,6 +1577,19 @@ static int plan_internal(f1l_handle h, const double pose[4], const double* opp, 
 int f1l_plan(f1l_handle h, const double pose[4], const double* opp, int n_opp, int update_prev,
              f1l_plan_result* out) {
     return plan_internal(h, pose, opp, n_opp, nullptr, 0, Shard{}, false, update_prev, out);
+}
+
+int f1l_plan_motion(f1l_handle h, const double pose[4], const double* opp, const double* opp_vel, int n_opp,
+                    double v_min, int update_prev, f1l_plan_result* out) {
+    return plan_internal(h, pose, opp, n_opp, nullptr, 0, Shard{}, false, update_prev, out, true, opp_vel, v_min);
+}
+
+int f1l_debug_motion_ctx(f1l_handle h, float* out, int n) {
+    if (!h || !out || n < 1 + 2 * F1L_MAX_OPP || !h->mo_dbg.p) return F1L_ERR_INVALID_ARG;
+    CK(cudaSetDevice(h->device));
+    CK(cudaStreamSynchronize(h->stream));
+    CK(cudaMemcpy(out, h->mo_dbg.p, (1 + 2 * F1L_MAX_OPP) * sizeof(float), cudaMemcpyDeviceToHost));
+    return F1L_OK;
 }
 
 int f1l_plan_shard(f1l_handle h, const double pose[4], const double* opp, int n_opp, int c_begin,
@@ -1703,6 +1763,24 @@ int f1l_plan_batch_call_dev(f1l_handle h, const f1l_batch_call* b, void* stream)
     return r != F1L_OK ? r : plan_batch_dev_internal(h, in, o, (cudaStream_t)stream);
 }
 
+// the moving-opponent fields of a batch call's pipeline, checked
+static int motion_args(const f1l_batch_call* b, const double* opp_vel, double v_min, PipeIn& in) {
+    if (const int r = check_motion(b->max_opp, opp_vel, v_min); r != F1L_OK) return r;
+    in.motion = true;
+    in.opp_vel = b->max_opp > 0 ? opp_vel : nullptr;
+    in.v_min = v_min;
+    return F1L_OK;
+}
+
+int f1l_plan_batch_motion_dev(f1l_handle h, const f1l_batch_call* b, const double* opp_vel_dev, double v_min,
+                              void* stream) {
+    PipeIn in;
+    BatchOut o;
+    int r = batch_args(h, b, in, o);
+    if (r == F1L_OK) r = motion_args(b, opp_vel_dev, v_min, in);
+    return r != F1L_OK ? r : plan_batch_dev_internal(h, in, o, (cudaStream_t)stream);
+}
+
 int f1l_plan_batch_dev(f1l_handle h, const double* poses_dev, const double* opp_dev,
                        const int32_t* n_opp_dev, int S, int max_opp, int32_t* best_idx_dev,
                        float* best_cost_dev, float* best_traj_dev, float* costs_dev,
@@ -1761,6 +1839,7 @@ static int plan_batch_internal(f1l_handle h, const PipeIn& in, const BatchOut& o
             {&p.buf[B_PVALID], in.prev_valid, o.prev_valid_out, 1},
             {&p.buf[B_W], in.weights, nullptr, F1L_N_TERMS * 4},
             {&p.buf[B_TERMS], nullptr, o.terms, (size_t)C * F1L_N_TERMS * 4},
+            {&p.buf[B_VEL], in.opp_vel, nullptr, (size_t)in.max_opp * 16},
         };
         if (const int r = stage_in(h, st, t, s0, n); r != F1L_OK) return r;
         // the chunk is a batch call of n scenarios on the slot's copies (updated in place)
@@ -1784,6 +1863,7 @@ static int plan_batch_internal(f1l_handle h, const PipeIn& in, const BatchOut& o
         PipeIn din;
         BatchOut dout;
         int r = batch_args(h, &d, din, dout);
+        if (r == F1L_OK && in.motion) r = motion_args(&d, (const double*)t[B_VEL].dev(), in.v_min, din);
         if (r == F1L_OK) r = launch_pipeline(h, st, din, p.scratch, dout, false);
         if (r == F1L_OK) r = stage_out(h, st, t, s0, n);
         if (r != F1L_OK) return r;
@@ -1797,6 +1877,22 @@ int f1l_plan_batch_call(f1l_handle h, const f1l_batch_call* b) {
     BatchOut o;
     const int r = batch_args(h, b, in, o);
     return r != F1L_OK ? r : plan_batch_internal(h, in, o);
+}
+
+int f1l_plan_batch_motion(f1l_handle h, const f1l_batch_call* b, const double* opp_vel, double v_min) {
+    PipeIn in;
+    BatchOut o;
+    int r = batch_args(h, b, in, o);
+    if (r == F1L_OK) r = motion_args(b, opp_vel, v_min, in);
+    if (r != F1L_OK) return r;
+    // a NaN velocity would silently clear a collision: every velocity in use must be finite
+    for (int s = 0; s < b->n_scenarios; ++s) {
+        int k_n = b->n_opp ? b->n_opp[s] : b->max_opp;
+        k_n = k_n < 0 ? 0 : (k_n > b->max_opp ? b->max_opp : k_n);
+        for (int k = 0; k < 2 * k_n; ++k)
+            if (!std::isfinite(opp_vel[2 * (size_t)s * b->max_opp + k])) return F1L_ERR_INVALID_ARG;
+    }
+    return plan_batch_internal(h, in, o);
 }
 
 int f1l_plan_batch(f1l_handle h, const double* poses, const double* opp, const int32_t* n_opp,
@@ -1835,10 +1931,13 @@ int f1l_default_vehicle(f1l_vehicle* veh) {
 
 // every rollout entry point: veh == nullptr runs the kinematic bicycle, else the single-track model
 // on dyn (checked by the caller)
+// predict: every step plans against the opponents' constant-velocity prediction (v_min checked)
 static int rollout_internal(f1l_handle h, const f1l_rollout_config* rc, const f1l_vehicle* veh,
                             const f1l_fleet* fl, double* dyn, const float* weights_dev, int S, int n_steps,
-                            const f1l_rollout_trace* trace, double* trace_dyn, void* stream) {
+                            const f1l_rollout_trace* trace, double* trace_dyn, void* stream,
+                            bool predict = false, double v_min = 1.0) {
     if (!h || !rc || !fl) return F1L_ERR_INVALID_ARG;
+    if (predict && (!std::isfinite(v_min) || !(v_min > 0.0))) return F1L_ERR_INVALID_ARG;
     if (!fl->state || !fl->prev_theta || !fl->has_prev || !fl->status || !fl->progress ||
         !fl->track_i || !fl->track_s)
         return F1L_ERR_INVALID_ARG;
@@ -1855,6 +1954,7 @@ static int rollout_internal(f1l_handle h, const f1l_rollout_config* rc, const f1
     ENS(h->r_cost, (size_t)S * 4);
     ENS(h->r_opp, (size_t)S * F1L_MAX_OPP * 24);
     ENS(h->r_nopp, (size_t)S * 4);
+    if (predict) ENS(h->r_vel, (size_t)S * F1L_MAX_OPP * 16);
     PipeScratch& sc = h->b_scratch;   // every step's pipeline reserves it for the same S: no realloc
     if (const int r = sc.reserve(h, S); r != F1L_OK) return r;
     cudaStream_t st = (cudaStream_t)stream;
@@ -1891,6 +1991,7 @@ static int rollout_internal(f1l_handle h, const f1l_rollout_config* rc, const f1
         a.dyn = dyn;
         a.veh = *veh;
     }
+    a.opp_vel = predict ? (double*)h->r_vel.p : nullptr;
     void (*const step)(RolloutArgs) = veh ? rollout_step_kernel<SingleTrack> : rollout_step_kernel<Kinematic>;
     const unsigned blocks = (unsigned)((a.n_races + ROLLOUT_WARPS - 1) / ROLLOUT_WARPS);
 
@@ -1920,6 +2021,11 @@ static int rollout_internal(f1l_handle h, const f1l_rollout_config* rc, const f1
     in.prev_stride = h->cfg.n_samples;
     in.prev_valid = fl->has_prev;
     in.weights = weights_dev;
+    if (predict) {
+        in.motion = true;
+        in.opp_vel = a.opp_vel;
+        in.v_min = v_min;
+    }
     BatchOut o;
     o.best_cost = (float*)h->r_cost.p;
     o.steer_speed = (double*)h->r_ss.p;
@@ -1952,15 +2058,30 @@ int f1l_rollout_weights_dev(f1l_handle h, const f1l_rollout_config* rc, const f1
     return rollout_internal(h, rc, nullptr, fl, nullptr, weights_dev, S, n_steps, trace, nullptr, stream);
 }
 
-int f1l_rollout_st_dev(f1l_handle h, const f1l_rollout_config* rc, const f1l_vehicle* veh,
-                       const f1l_fleet* fl, double* dyn_dev, const float* weights_dev, int S, int n_steps,
-                       const f1l_rollout_trace* trace, double* trace_dyn_dev, void* stream) {
+static int check_vehicle(const f1l_vehicle* veh, const double* dyn_dev) {
     if (!veh || !dyn_dev) return F1L_ERR_INVALID_ARG;
     for (const double p : {veh->mu, veh->C_Sf, veh->C_Sr, veh->lf, veh->lr, veh->m, veh->I, veh->max_steer_vel,
                            veh->v_switch, veh->v_kin})
         if (!(p > 0)) return F1L_ERR_INVALID_ARG;
     if (!(veh->h >= 0)) return F1L_ERR_INVALID_ARG;
+    return F1L_OK;
+}
+
+int f1l_rollout_st_dev(f1l_handle h, const f1l_rollout_config* rc, const f1l_vehicle* veh,
+                       const f1l_fleet* fl, double* dyn_dev, const float* weights_dev, int S, int n_steps,
+                       const f1l_rollout_trace* trace, double* trace_dyn_dev, void* stream) {
+    if (const int r = check_vehicle(veh, dyn_dev); r != F1L_OK) return r;
     return rollout_internal(h, rc, veh, fl, dyn_dev, weights_dev, S, n_steps, trace, trace_dyn_dev, stream);
+}
+
+int f1l_rollout_predict_dev(f1l_handle h, const f1l_rollout_config* rc, const f1l_vehicle* veh,
+                            const f1l_fleet* fl, double* dyn_dev, const float* weights_dev, double v_min,
+                            int S, int n_steps, const f1l_rollout_trace* trace, double* trace_dyn_dev,
+                            void* stream) {
+    if (veh)
+        if (const int r = check_vehicle(veh, dyn_dev); r != F1L_OK) return r;
+    return rollout_internal(h, rc, veh, fl, veh ? dyn_dev : nullptr, weights_dev, S, n_steps, trace,
+                            veh ? trace_dyn_dev : nullptr, stream, true, v_min);
 }
 
 // ---- pure pursuit -------------------------------------------------------------------------

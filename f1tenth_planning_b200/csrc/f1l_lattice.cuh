@@ -368,6 +368,12 @@ struct EvalArgs {
                              // candidate from this device-wide counter (null: the CTA's own chunk)
     int v_last;              // with work_next: the walk is reversed, v -> v_last - v (far lookahead
                              // rows, the expensive candidates, first; the cheap ones fill the tail)
+    // moving opponents (the MO instances only)
+    const double* opp_vel;   // [S,vel_stride,2] map-frame opponent velocities (vx, vy), m/s, finite
+    int vel_stride;          // opponent slots per scenario in opp_vel
+    double v_min;            // the ego is timed at max(pose speed, v_min) along its candidate
+    float* mo_ctx;           // [1 + 2 F1L_MAX_OPP] k_t and the vehicle-frame (wx, wy) of scenario 0,
+                             // written by its first CTA (debug, nullable)
 };
 
 // Peer-memory exchange of a candidate-sharded query (SURVEY 8e: the one exchange step of the
@@ -883,7 +889,7 @@ __device__ __forceinline__ float halve_min_sqrt_sum(float (&v)[N], int lane_in_g
 // one 64-bit load yields a packed pair of samples -- then the CTA-wide part: opponents | grid
 // constants | previous path | window table (run-time length, last).  Everything sits at a
 // compile-time offset from two addresses, the CTA's base and the warp's block.
-template <int S, int SG, int NW>
+template <int S, int SG, int NW, bool MO = false>
 struct EvalSmem {
     static constexpr int PCAP = S * SG;
     static constexpr int SROWS = (S + 1) / 2;
@@ -898,7 +904,8 @@ struct EvalSmem {
                                                                    // (n_opp, has_grid, use_prev, w4), (w0, w1, w2, w3)
                                                                    // (the weights with PW only)
     static constexpr uint32_t C_PREV = C_GRID + 64;                // [F1L_MAX_M] float
-    static constexpr uint32_t C_TAB = C_PREV + F1L_MAX_M * 4;      // [ntab][2] float4
+    static constexpr uint32_t C_VEL = C_PREV + F1L_MAX_M * 4;      // MO: [F1L_MAX_OPP] (wx, wy), k_t
+    static constexpr uint32_t C_TAB = C_VEL + (MO ? F1L_MAX_OPP * 8 + 16 : 0);   // [ntab][2] float4
     static_assert(W_BYTES % 16 == 0, "per-warp block keeps 16-byte alignment");
 };
 
@@ -909,10 +916,17 @@ struct EvalSmem {
 // CTA's shared memory.  Without them the instance takes the config's weights from the kernel
 // parameters, whose constant-bank operands cost no register: its schedule is the one it had before
 // per-scenario weights existed (shared-memory operands there made the batch instance 1.2 % slower).
-template <int IPL, int S, int SG, int NW, int MINB, bool PW>
+// MO (PW instances only): the opponents move at constant velocity.  Opponent k's centre at time t
+// is o_k + w_k t (vehicle frame, heading kept); the ego reaches sample i of a candidate of length
+// s_f at t_i = i * s_f * k_t, k_t = 1 / ((M - 1) v_e), v_e = max(pose speed, v_min).  The prologue
+// stages k_t and the w_k next to the opponents; the prune, the broad phase and the narrow phase
+// test the predicted centres.  With every velocity zero the flags are those of the PW instance,
+// and a call without weights gives the config's weights as every scenario's row.
+template <int IPL, int S, int SG, int NW, int MINB, bool PW, bool MO = false>
 __global__ void __launch_bounds__(NW * 32, MINB) eval_kernel(EvalArgs a) {
+    static_assert(!MO || PW, "the moving-opponent instances are twins of the PW instances");
     constexpr int GG = 32 / SG;
-    using L = EvalSmem<S, SG, NW>;
+    using L = EvalSmem<S, SG, NW, MO>;
     extern __shared__ __align__(16) unsigned char ev_smem[];
     __shared__ int s_next;
     __shared__ unsigned long long s_work;   // deviation pass: candidates << 40 | (candidate, segment) pairs
@@ -987,15 +1001,45 @@ __global__ void __launch_bounds__(NW * 32, MINB) eval_kernel(EvalArgs a) {
         if (tid < F1L_MAX_OPP)   // unused slots: an opponent far away
             sts128(cbase + L::C_OPP + tid * 16,
                    tid < q->n_opp ? q->opp[tid] : make_float4(1e9f, 1e9f, 1.0f, 0.0f));
+        if constexpr (MO) {
+            // velocities rotated into the vehicle frame with the pose's float64 cos / sin, as the
+            // sampler rotates the positions (unused slots: at rest)
+            const bool dbg = a.mo_ctx && blockIdx.x == 0;
+            if (tid < F1L_MAX_OPP) {
+                float wx = 0.0f, wy = 0.0f;
+                if (tid < q->n_opp) {
+                    const double* vel = a.opp_vel + 2 * ((size_t)s * a.vel_stride + tid);
+                    double sth, cth;
+                    sincos(q->th, &sth, &cth);
+                    wx = (float)fa(fm(cth, vel[0]), fm(sth, vel[1]));
+                    wy = (float)fs(fm(cth, vel[1]), fm(sth, vel[0]));
+                }
+                sts32(cbase + L::C_VEL + tid * 8, wx);
+                sts32(cbase + L::C_VEL + tid * 8 + 4, wy);
+                if (dbg) { a.mo_ctx[1 + 2 * tid] = wx; a.mo_ctx[2 + 2 * tid] = wy; }
+            }
+            if (tid == F1L_MAX_OPP % (NW * 32)) {
+                const double ve = fmax(q->vel, a.v_min);
+                const float k_t = (float)__ddiv_rn(1.0, fm((double)(M - 1), ve));
+                sts32(cbase + L::C_VEL + F1L_MAX_OPP * 8, k_t);
+                if (dbg) a.mo_ctx[0] = k_t;
+            }
+        }
         if (tid == 0) { s_next = cb + NW * a.item; s_work = 0ull; }
         // per-scenario collision constants (and with PW the cost weights) live in shared memory,
         // not in registers, so that the candidate loop does not carry them through the deviation pass
         if (tid == 32 % (NW * 32)) {
             float w4 = 0.0f;
             if constexpr (PW) {
-                const float* w = a.weights + (size_t)s * F1L_N_TERMS;
-                w4 = w[4];
-                sts128(cbase + L::C_GRID + 48, make_float4(w[0], w[1], w[2], w[3]));
+                // (a moving-opponent call without weights: the config's as the scenario's row)
+                if (MO && !a.weights) {
+                    w4 = a.ep.w[4];
+                    sts128(cbase + L::C_GRID + 48, make_float4(a.ep.w[0], a.ep.w[1], a.ep.w[2], a.ep.w[3]));
+                } else {
+                    const float* w = a.weights + (size_t)s * F1L_N_TERMS;
+                    w4 = w[4];
+                    sts128(cbase + L::C_GRID + 48, make_float4(w[0], w[1], w[2], w[3]));
+                }
             }
             sts128(cbase + L::C_GRID, make_float4(q->gA00, q->gA01, q->gA10, q->gA11));
             sts128(cbase + L::C_GRID + 16, make_float4(q->gfx, q->gfy, __int_as_float(q->gix), __int_as_float(q->giy)));
@@ -1198,11 +1242,24 @@ __global__ void __launch_bounds__(NW * 32, MINB) eval_kernel(EvalArgs a) {
             // candidate-level opponent pruning: every point of a curve of length s_f from the
             // origin to (ex, ey) lies within s_f/2 of the chord's midpoint, so an opponent
             // farther than s_f/2 + 2 r_circ from it cannot pass the per-sample broad phase.
+            // MO: the ego reaches sample i at t_i = fm(i, dt).  Over [0, T], T = t_{M-1}, an
+            // opponent's centre stays within |w| T / 2 of o + w T / 2: the reach grows by that
+            // much, with 0.1 % + 1 mm of slack over the FP32 rounding of the predicted centres.
+            float dt = 0.0f;
+            if constexpr (MO) dt = fm(sp.sf, lds32(cbase + L::C_VEL + F1L_MAX_OPP * 8));
             unsigned opp_mask;
             {
                 const float4 o = lds128(cbase + L::C_OPP + (lane & (F1L_MAX_OPP - 1)) * 16);
-                const float mx = o.x - 0.5f * ex, my = o.y - 0.5f * ey;
-                const float reach = 0.5f * sp.sf + a.ep.reach_pad;
+                float mx = o.x - 0.5f * ex, my = o.y - 0.5f * ey;
+                float reach = 0.5f * sp.sf + a.ep.reach_pad;
+                if constexpr (MO) {
+                    float wx, wy;
+                    unpack2(lds64(cbase + L::C_VEL + (lane & (F1L_MAX_OPP - 1)) * 8), wx, wy);
+                    const float hT = 0.5f * fm((float)(M - 1), dt);
+                    mx = fmaf(wx, hT, mx);
+                    my = fmaf(wy, hT, my);
+                    reach = fmaf(hT, sqrtf(fmaf(wx, wx, wy * wy)), reach) * 1.001f + 1e-3f;
+                }
                 opp_mask = __ballot_sync(F1L_FULL, lane < n_opp && fmaf(mx, mx, my * my) <= reach * reach);
             }
             if (use_prev) {   // uniform
@@ -1221,19 +1278,40 @@ __global__ void __launch_bounds__(NW * 32, MINB) eval_kernel(EvalArgs a) {
             // the broad-phase radius from the first sample cannot pass any per-sample test.  (1 %
             // and 1 mm of slack over the quadrature; only provably negative tests are skipped,
             // the flags stay as they were.)
-            float lane_R2 = -1.0f;
+            // MO: over the lane's times [t_a, t_b] the opponent stays within |w| (t_b - t_a) / 2 of
+            // its centre at (t_a + t_b) / 2 (same slack as the prune).
+            float lane_R2 = -1.0f, lane_R = 0.0f;
             if (opp_mask && nown > 0) {
                 const float R = fmaf(1.01f * (float)(IPL - 1), __fdividef(sp.sf, (float)(M - 1)), a.ep.reach_pad);
                 lane_R2 = R * R;
+                lane_R = R;
             }
             for (unsigned m = opp_mask; m; m &= m - 1) {   // uniform; mostly empty
-                const float4 o = lds128(cbase + L::C_OPP + (__ffs(m) - 1) * 16);
-                const float ux = o.x - x[0], uy = o.y - y[0];
-                if (fmaf(ux, ux, uy * uy) <= lane_R2) {
+                const int k = __ffs(m) - 1;
+                const float4 o = lds128(cbase + L::C_OPP + k * 16);
+                float wx = 0.0f, wy = 0.0f;
+                float ux = o.x - x[0], uy = o.y - y[0];
+                float R2 = lane_R2;
+                if constexpr (MO) {
+                    unpack2(lds64(cbase + L::C_VEL + k * 8), wx, wy);
+                    const float ta = fm((float)(lane * IPL), dt), tb = fm((float)(lane * IPL + IPL - 1), dt);
+                    const float tm = 0.5f * (ta + tb), hs = 0.5f * (tb - ta);
+                    ux = fmaf(wx, tm, ux);
+                    uy = fmaf(wy, tm, uy);
+                    const float Rm = fmaf(hs, sqrtf(fmaf(wx, wx, wy * wy)), lane_R) * 1.001f + 1e-3f;
+                    R2 = lane_R2 < 0.0f ? -1.0f : Rm * Rm;
+                }
+                if (fmaf(ux, ux, uy * uy) <= R2) {
 #pragma unroll
                     for (int j = 0; j < IPL; ++j) {
                         if (j < nown) {
-                            const float tx = fs(o.x, x[j]), ty = fs(o.y, y[j]);
+                            float cx = o.x, cy = o.y;   // the opponent's centre when the ego is at sample i
+                            if constexpr (MO) {
+                                const float t = fm((float)(lane * IPL + j), dt);
+                                cx = fa(o.x, fm(wx, t));
+                                cy = fa(o.y, fm(wy, t));
+                            }
+                            const float tx = fs(cx, x[j]), ty = fs(cy, y[j]);
                             const float d2 = fa(fm(tx, tx), fm(ty, ty));
                             if (d2 <= a.ep.rc2 && sat_collide(tx, ty, cs[j], sn[j], o.z, o.w, hl, hw))
                                 hit_opp = true;

@@ -53,6 +53,9 @@ struct RolloutArgs {
     double* dyn;             // [S,3] delta, yaw rate, slip angle
     double* tr_dyn;          // [S,3] dyn at the start of the step, nullable
     f1l_vehicle veh;
+    // prediction (f1l_rollout_predict_dev, nullable): the next step's opponent velocities
+    // [S,F1L_MAX_OPP,2], map frame, in the order of `opp`
+    double* opp_vel;
 };
 
 struct Kinematic { static constexpr bool single_track = false; };
@@ -183,8 +186,14 @@ __global__ void __launch_bounds__(ROLLOUT_WARPS * 32) rollout_step_kernel(Rollou
     double th = a.state[4 * (size_t)car + 2], v = a.state[4 * (size_t)car + 3];
     int ti = a.track_i[car];
     double ts = a.track_s[car];
+    unsigned st_end = 0;   // prediction: the car's status and slip angle after this pass
+    double beta = 0.0;
 
     if (!a.steer_speed) {
+        if (a.opp_vel) {
+            st_end = a.status[car];
+            if constexpr (ST) beta = a.dyn[3 * (size_t)car + 2];
+        }
         // initial pass of a call: re-acquire lost cars on the whole raceline
         if (ti < 0) {
             ti = a.near_i[car];
@@ -287,15 +296,31 @@ __global__ void __launch_bounds__(ROLLOUT_WARPS * 32) rollout_step_kernel(Rollou
             if (a.tr_status) a.tr_status[car] = (uint8_t)st;
             if (a.tr_progress) a.tr_progress[car] = prog;
         }
+        st_end = st;
+        beta = b;
+    }
+    // the car's velocity as its opponents predict it: along the heading (kinematic) or the course
+    // psi + beta (single-track); a frozen car stands
+    double vx = 0.0, vy = 0.0;
+    if (a.opp_vel && !(st_end & (F1L_CAR_HIT_MAP | F1L_CAR_HIT_CAR))) {
+        double sc, cc;
+        sincos(ST ? fa(th, beta) : th, &sc, &cc);
+        vx = fm(v, cc);
+        vy = fm(v, sc);
     }
     // the next step's opponents of this car: the other cars of its race in race order
     int k = 0;
     for (int j = 0; j < G; ++j) {   // uniform
         const double xj = __shfl_sync(F1L_FULL, x, j), yj = __shfl_sync(F1L_FULL, y, j);
         const double tj = __shfl_sync(F1L_FULL, th, j);
+        const double vxj = __shfl_sync(F1L_FULL, vx, j), vyj = __shfl_sync(F1L_FULL, vy, j);
         if (live && j != lane) {
             double* o = a.opp + 3 * ((size_t)car * F1L_MAX_OPP + k);
             o[0] = xj; o[1] = yj; o[2] = tj;
+            if (a.opp_vel) {
+                double* ov = a.opp_vel + 2 * ((size_t)car * F1L_MAX_OPP + k);
+                ov[0] = vxj; ov[1] = vyj;
+            }
             ++k;
         }
     }

@@ -49,6 +49,15 @@ def _vp(a):
     return C.c_void_p(a.data_ptr())
 
 
+def _motion_array(opponent_velocities, where, dims):
+    """the opponent velocities of a batch call, checked against MOTION_FIELDS (host: float64 numpy,
+    converted; device: the tensor as given)"""
+    row = _lib.MOTION_FIELDS["opp_vel"]
+    v = _f64(opponent_velocities) if where == "host" else opponent_velocities
+    _lib.check_array("opponent_velocities", v, _lib.shape_of(row, dims), row[0], where)
+    return v
+
+
 class Engine:
     """Owns an f1l_handle.  Config keywords are the fields of f1l_config (include/f1l.h)."""
 
@@ -205,23 +214,44 @@ class Engine:
             raise ValueError("at most %d opponents" % MAX_OPP)
         return (o, o.shape[0]) if o.shape[0] else (None, 0)
 
+    @staticmethod
+    def _vel(opponent_velocities, k):
+        """opponent velocities [k,2] float64 (vx, vy) m/s, map frame, for k opponents"""
+        v = _f64(opponent_velocities).reshape(-1, 2)
+        if v.shape[0] != k:
+            raise ValueError("opponent_velocities must be [%d,2] (one (vx, vy) per opponent)" % k)
+        return v
+
     @property
     def n_samples(self):
         return self._n_samples
 
     def plan(self, pose, opponent_poses=None, update_prev=True, detail=True, want_states=False,
-             shard=None, want_headings=False, rows=None, want_map=False):
+             shard=None, want_headings=False, rows=None, want_map=False, opponent_velocities=None,
+             v_min=1.0):
         """One query.  pose = (x, y, theta, velocity).  Dense-sweep sharding across GPUs:
         shard = (c_begin, c_end) evaluates a candidate range only, rows = (row_begin, row_step)
         the lookahead rows row_begin, row_begin + row_step, ... (balanced across ranks).  With
         attach_peers() both are collective and return the global winner on every rank (and
-        rows= then honours update_prev: every rank stores the same previous path)."""
+        rows= then honours update_prev: every rank stores the same previous path).
+
+        opponent_velocities [K,2] (vx, vy) m/s, map frame: plan against the opponents'
+        constant-velocity prediction, the ego timed at max(pose velocity, v_min) (f1l_plan_motion).
+        Not with shard= or rows=."""
         pose = _f64(pose).ravel()
         if pose.size != 4:
             raise ValueError("pose must be (x, y, theta, velocity)")
         opp, k = self._opp(opponent_poses)
+        if opponent_velocities is not None:
+            if shard is not None or rows is not None:
+                raise ValueError("opponent_velocities cannot be combined with shard= or rows=")
+            vel = self._vel(opponent_velocities, k)
         res, bufs = self._result(self.n_candidates, detail, want_states, want_headings, want_map)
-        if rows is not None:
+        if opponent_velocities is not None:
+            code = self._L.f1l_plan_motion(self._h, pose.ctypes.data, opp.ctypes.data if k else None,
+                                           vel.ctypes.data if k else None, k, float(v_min),
+                                           int(bool(update_prev)), C.byref(res))
+        elif rows is not None:
             code = self._L.f1l_plan_rows(self._h, pose.ctypes.data, opp.ctypes.data if k else None,
                                          k, int(rows[0]), int(rows[1]),
                                          int(bool(update_prev) and self.peer_world > 1), C.byref(res))
@@ -270,7 +300,8 @@ class Engine:
     # -- batch ------------------------------------------------------------------------------
     def plan_batch(self, poses, opponents=None, n_opp=None, out=None, want_traj=True,
                    want_costs=True, want_flags=False, prev_theta=None, has_prev=None,
-                   update_prev=False, weights=None, want_terms=False):
+                   update_prev=False, weights=None, want_terms=False, opponent_velocities=None,
+                   v_min=1.0):
         """S independent scenarios with HOST buffers (numpy; pinned if allocated through
         ``pinned_empty``).  poses [S,4], opponents [S,K,3], n_opp [S].
 
@@ -285,7 +316,11 @@ class Engine:
         Cost weights per scenario (f1l_plan_batch_call): weights [S,5] float (converted to
         float32), scenario s then plans exactly as plan() after configure(weights=weights[s]);
         None: every scenario uses the configured weights.  want_terms=True also returns the
-        unweighted per-term costs [S,C,5] (BatchPlan.terms), as plan_detailed's terms."""
+        unweighted per-term costs [S,C,5] (BatchPlan.terms), as plan_detailed's terms.
+
+        opponent_velocities [S,K,2] float64 (vx, vy) m/s, map frame: every scenario plans against
+        its opponents' constant-velocity prediction as plan(..., opponent_velocities, v_min)
+        (f1l_plan_batch_motion)."""
         poses = _f64(poses).reshape(-1, 4)
         S = poses.shape[0]
         opponents = None if opponents is None else _f64(opponents)
@@ -301,19 +336,25 @@ class Engine:
                            ("terms", want_terms)):
             a[name] = _lib.zeros_or(o.get(name), _lib.BATCH_FIELDS[name], dims) if want else None
         b = _lib.batch_call(a, "host", dims, update_prev)
-        if S:   # an empty batch is a valid (empty) answer, not an error
+        if opponent_velocities is not None:
+            vel = _motion_array(opponent_velocities, "host", dims)
+            if S:
+                self._ck(self._L.f1l_plan_batch_motion(self._h, C.byref(b), vel.ctypes.data, float(v_min)))
+        elif S:   # an empty batch is a valid (empty) answer, not an error
             self._ck(self._L.f1l_plan_batch_call(self._h, C.byref(b)))
         return BatchPlan(*(a[k] for k in BatchPlan._fields))
 
     def plan_batch_dev(self, poses, opponents=None, n_opp=None, best_idx=None, best_cost=None,
                        best_traj=None, costs=None, flags=None, steer_speed=None, stream=None,
-                       prev_theta=None, has_prev=None, update_prev=False, weights=None, terms=None):
+                       prev_theta=None, has_prev=None, update_prev=False, weights=None, terms=None,
+                       opponent_velocities=None, v_min=1.0):
         """Same with torch CUDA tensors; enqueues on `stream` (default: torch's current stream)
         and does not synchronise.  prev_theta / has_prev / update_prev as for plan_batch, as
         contiguous CUDA tensors (float32 [S, n_samples], uint8 / bool [S]) updated in place on
         the stream.  weights: a contiguous float32 CUDA tensor [S,5] (None: the configured
         weights); terms: a contiguous float32 CUDA tensor [S,C,5] that receives the per-term
-        costs (f1l_plan_batch_call_dev)."""
+        costs (f1l_plan_batch_call_dev).  opponent_velocities: a contiguous float64 CUDA tensor
+        [S,K,2] as plan_batch's (f1l_plan_batch_motion_dev); its values must be finite."""
         import torch
         K = opponents.shape[1] if opponents is not None and opponents.ndim == 3 else 0
         dims = dict(S=poses.shape[0], K=K, C=self.n_candidates, M=self.n_samples)
@@ -323,7 +364,12 @@ class Engine:
                                  steer_speed=steer_speed, terms=terms),
                             self.device, dims, update_prev)
         st = stream if stream is not None else torch.cuda.current_stream(poses.device).cuda_stream
-        self._ck(self._L.f1l_plan_batch_call_dev(self._h, C.byref(b), C.c_void_p(st)))
+        if opponent_velocities is not None:
+            vel = _motion_array(opponent_velocities, self.device, dims)
+            self._ck(self._L.f1l_plan_batch_motion_dev(self._h, C.byref(b), C.c_void_p(vel.data_ptr()),
+                                                       float(v_min), C.c_void_p(st)))
+        else:
+            self._ck(self._L.f1l_plan_batch_call_dev(self._h, C.byref(b), C.c_void_p(st)))
 
     # -- closed-loop rollouts ----------------------------------------------------------------
     def fleet(self, poses, group=1, weights=None, vehicle=None):
@@ -494,6 +540,13 @@ class Engine:
         i = np.zeros(6, np.int32)
         self._ck(self._L.f1l_debug_query_ctx(self._h, _ptr(f, _fp), _ptr(i, _ip)))
         return f, i
+
+    def debug_motion_ctx(self):
+        """(k_t, [16,2] vehicle-frame opponent velocities) of the last moving-opponent plan()
+        (f1l_debug_motion_ctx), float32 as the kernel uses them"""
+        f = np.zeros(1 + 2 * MAX_OPP, np.float32)
+        self._ck(self._L.f1l_debug_motion_ctx(self._h, _ptr(f, _fp), f.size))
+        return f[0], f[1:].reshape(MAX_OPP, 2)
 
 
 _fp_weights = {}

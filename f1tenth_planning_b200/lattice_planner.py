@@ -186,10 +186,12 @@ class LatticePlanner():
 
     # -- planning -------------------------------------------------------------------------------
     def plan_detailed(self, pose_x, pose_y, pose_theta, velocity, waypoints=None,
-                      opponent_poses=None, want_states=False, want_map=False):
+                      opponent_poses=None, want_states=False, want_map=False, opponent_velocities=None):
         """Full result of one query as a PlanDetail (see engine.PlanDetail).  want_map adds
         ``best_traj_map`` [M,4] = (X, Y, v, Theta), the best trajectory in the map frame with a
-        speed column (what a map-frame tracker consumes, SURVEY B.8)."""
+        speed column (what a map-frame tracker consumes, SURVEY B.8).  opponent_velocities [K,2]
+        (vx, vy) m/s, map frame: plan against the opponents' constant-velocity prediction
+        (Engine.plan; not with a user sampler or a row shard)."""
         if waypoints is not None:
             self.waypoints = waypoints
         eng = self._sync()
@@ -198,7 +200,12 @@ class LatticePlanner():
         custom_select = self.selection_func is not None and self.selection_func is not np.argmin
         plugins = custom_cost or custom_select
         need_states = want_states or custom_cost
-        if self.sample_func is not None:
+        if opponent_velocities is not None and (self.sample_func is not None or self._shard is not None):
+            raise ValueError("opponent_velocities cannot be combined with a user sampler or a row shard")
+        if opponent_velocities is not None:
+            d = eng.plan(pose, opponent_poses, want_states=need_states, want_map=want_map and not plugins,
+                         opponent_velocities=opponent_velocities)
+        elif self.sample_func is not None:
             goal_grid = np.asarray(self.sample(pose_x, pose_y, pose_theta, velocity, self.waypoints),
                                    dtype=np.float64).reshape(-1, 3)
             d = eng.plan_goals(pose, goal_grid, opponent_poses, want_states=need_states,
@@ -248,13 +255,15 @@ class LatticePlanner():
         final = (fleet.state.cpu().numpy(), fleet.status.cpu().numpy(), fleet.progress.cpu().numpy())
         return trace, final + ((fleet.dyn.cpu().numpy(),) if vehicle is not None else ())
 
-    def plan(self, pose_x, pose_y, pose_theta, velocity, waypoints=None, opponent_poses=None):
+    def plan(self, pose_x, pose_y, pose_theta, velocity, waypoints=None, opponent_poses=None,
+             opponent_velocities=None):
         """lattice_planner.py:174-214 -> (steering_angle, speed, selected_traj [M,4]).
 
         selected_traj columns are (x, y, theta, |kappa|) in the vehicle frame like
         utils.sample_traj (utils/utils.py:285-295); the signed-curvature float32 trajectory,
         index, cost vector and flags are in ``self.last``."""
-        d = self.plan_detailed(pose_x, pose_y, pose_theta, velocity, waypoints, opponent_poses)
+        d = self.plan_detailed(pose_x, pose_y, pose_theta, velocity, waypoints, opponent_poses,
+                               opponent_velocities=opponent_velocities)
         traj = d.best_traj.astype(np.float64)
         traj[:, 3] = np.abs(traj[:, 3])
         return d.steer, d.speed, traj

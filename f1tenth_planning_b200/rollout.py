@@ -120,10 +120,13 @@ class Fleet:
         return _lib.FleetBuffers(**{name: getattr(self, name).data_ptr() for name in _lib.FLEET_FIELDS})
 
     def run(self, n_steps, dt=0.01, substeps=1, max_steer=0.4189, max_accel=9.51, v_max=math.inf,
-            trace=False, stream=None):
+            trace=False, stream=None, predict=False, v_min=1.0):
         """Advance every car n_steps planning steps on `stream` (default: torch's current stream)
         without synchronising.  Returns a RolloutTrace (SingleTrackTrace for a fleet with a
-        vehicle) of CUDA tensors with trace=True, else None."""
+        vehicle) of CUDA tensors with trace=True, else None.  predict=True: every planner sees its
+        opponents moving at their current velocity (along the heading, for single-track cars along
+        the course psi + slip angle; frozen cars stand) and times itself at max(v, v_min)
+        (f1l_rollout_predict_dev)."""
         import torch
         n_steps = int(n_steps)
         if n_steps < 0:
@@ -133,6 +136,8 @@ class Fleet:
         for name, val in (("dt", dt), ("max_steer", max_steer), ("max_accel", max_accel), ("v_max", v_max)):
             if not float(val) > 0:
                 raise ValueError("%s must be positive" % name)
+        if predict and not (math.isfinite(float(v_min)) and float(v_min) > 0):
+            raise ValueError("v_min must be finite and positive")
         rc = _lib.RolloutConfig(float(dt), int(substeps), self.group, float(max_steer), float(max_accel),
                                 float(v_max))
         veh = _vehicle_struct(self.vehicle) if self.vehicle is not None else None
@@ -153,7 +158,12 @@ class Fleet:
         eng = self.engine
         w = C.c_void_p(self.weights.data_ptr() if self.weights is not None else None)
         tbp = C.byref(tb) if tb is not None else None
-        if veh is None:
+        if predict:
+            eng._ck(eng._L.f1l_rollout_predict_dev(
+                eng._h, C.byref(rc), C.byref(veh) if veh is not None else None, C.byref(fl),
+                C.c_void_p(self.dyn.data_ptr() if veh is not None else None), w, float(v_min), S, n_steps, tbp,
+                C.c_void_p(out.dyn.data_ptr() if trace and veh is not None else None), C.c_void_p(st)))
+        elif veh is None:
             eng._ck(eng._L.f1l_rollout_weights_dev(eng._h, C.byref(rc), C.byref(fl), w, S, n_steps, tbp,
                                                    C.c_void_p(st)))
         else:

@@ -74,6 +74,15 @@ def random_opponents(track, idx, k, rng):
     return np.stack([x, y, th], axis=2)
 
 
+def opponent_velocities(track, opp, rng, lo=2.0, hi=8.0):
+    """[..., 2] map-frame velocities (vx, vy) of opponents `opp` [..., 3]: a speed drawn from
+    U(lo, hi) m/s along each opponent's heading.  (`track` is taken for symmetry with the other
+    scenario builders.)"""
+    opp = np.asarray(opp, dtype=np.float64)
+    v = rng.uniform(lo, hi, size=opp.shape[:-1])
+    return np.stack([v * np.cos(opp[..., 2]), v * np.sin(opp[..., 2])], axis=-1)
+
+
 def scenario_batch(track, s, k, seed):
     rng = np.random.default_rng(seed)
     poses, idx = random_poses(track, s, rng)

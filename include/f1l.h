@@ -196,6 +196,22 @@ typedef struct {
 int f1l_plan(f1l_handle h, const double pose[4], const double* opp, int n_opp,
              int update_prev, f1l_plan_result* out);
 
+/*
+ * f1l_plan against MOVING opponents: opponent k, at opp[k] = (x, y, theta) now, moves at the
+ * constant map-frame velocity opp_vel[k] = (vx, vy) m/s and keeps its heading: its centre at time
+ * t is (x + vx t, y + vy t).  The ego is timed along each candidate at v_e = max(pose[3], v_min):
+ * sample i of M on a candidate of length s_f is reached at t_i = i s_f / ((M - 1) v_e), and every
+ * sample's footprint is tested against the opponents' footprints at t_i.  In float32 as the
+ * kernel computes it: k_t = (float)(1 / ((M - 1) v_e)) and the velocities rotated into the vehicle
+ * frame (wx, wy) in float64, then per candidate dt = s_f * k_t and per sample t_i = (float)i * dt,
+ * centre (ox + wx t_i, oy + wy t_i), each operation rounded on its own.  With every velocity zero
+ * the result is bit-identical to f1l_plan.  v_min must be finite and > 0 (a car at rest would
+ * otherwise never arrive anywhere); opp_vel [n_opp,2] f64 may be NULL only when n_opp = 0, and
+ * every velocity must be finite (a NaN would clear a collision): else F1L_ERR_INVALID_ARG.
+ */
+int f1l_plan_motion(f1l_handle h, const double pose[4], const double* opp, const double* opp_vel,
+                    int n_opp, double v_min, int update_prev, f1l_plan_result* out);
+
 /* Same, but only candidates [c_begin, c_end) are evaluated (candidate sharding of one dense
  * query across GPUs; best_idx is still the global index).  Without attached peers the result is
  * the winner of the shard; with f1l_xchg_attach it is the winner over all ranks' shards. */
@@ -342,6 +358,17 @@ int f1l_plan_batch_call_dev(f1l_handle h, const f1l_batch_call* b, void* stream)
 /* Host buffers, through the chunked pipeline of f1l_plan_batch: weights travel with each chunk's
  * inputs, terms come back with its outputs.  Synchronised before returning. */
 int f1l_plan_batch_call(f1l_handle h, const f1l_batch_call* b);
+/* The batch call against moving opponents (f1l_plan_motion's prediction per scenario): opp_vel
+ * [S,max_opp,2] f64 map-frame velocities of b->opp's opponents, v_min as f1l_plan_motion.  Scenario
+ * s is bit-identical to f1l_plan_motion on the same inputs (with b->weights: after f1l_set_config
+ * with those weights).  F1L_ERR_INVALID_ARG for a non-finite or non-positive v_min, or opp_vel
+ * NULL with max_opp > 0.  _dev: device buffers, caller's stream, no sync; every velocity of an
+ * opponent in use must be finite (not checked).  Host version: through the chunked pipeline,
+ * opp_vel travelling with each chunk's inputs; a non-finite velocity of an opponent in use is
+ * F1L_ERR_INVALID_ARG. */
+int f1l_plan_batch_motion_dev(f1l_handle h, const f1l_batch_call* b, const double* opp_vel_dev,
+                              double v_min, void* stream);
+int f1l_plan_batch_motion(f1l_handle h, const f1l_batch_call* b, const double* opp_vel, double v_min);
 
 /*
  * Closed-loop rollouts on the device: a fleet of S kinematic-bicycle cars (f1l_rollout_st_dev below:
@@ -482,6 +509,20 @@ int f1l_rollout_st_dev(f1l_handle h, const f1l_rollout_config* rc, const f1l_veh
                        double* trace_dyn_dev, void* stream);
 
 /*
+ * Rollouts whose planners predict their opponents: as f1l_rollout_st_dev (veh != NULL, dyn_dev its
+ * state) or f1l_rollout_weights_dev (veh NULL: kinematic bicycle; dyn_dev, trace_dyn_dev ignored),
+ * but every step plans through f1l_plan_batch_motion_dev with v_min.  The step kernel writes the
+ * next step's opponent velocities next to the opponent table (a [S,F1L_MAX_OPP,2] table the handle
+ * owns): v (cos theta, sin theta) for a kinematic car, v (cos(psi + beta), sin(psi + beta)) for a
+ * single-track car with slip angle beta, 0 for a frozen car.  F1L_ERR_INVALID_ARG as those calls,
+ * and for a non-finite or non-positive v_min.
+ */
+int f1l_rollout_predict_dev(f1l_handle h, const f1l_rollout_config* rc, const f1l_vehicle* veh,
+                            const f1l_fleet* fleet, double* dyn_dev, const float* weights_dev,
+                            double v_min, int n_scenarios, int n_steps, const f1l_rollout_trace* trace,
+                            double* trace_dyn_dev, void* stream);
+
+/*
  * Batched nearest_point + pure-pursuit lookahead over B poses on the uploaded track.
  * Replaces nearest_point (utils/utils.py:37-67), intersect_point (:69-151), get_actuation
  * (:153-161) and PurePursuitPlanner._get_current_waypoint / plan (pure_pursuit.py:56-122).
@@ -544,8 +585,9 @@ int f1l_get_stats(f1l_handle h, uint64_t* out, int n);
  * CTA plan: out[0..4] = IPL, S, SG, NW (warps per CTA), MINB (resident CTAs per SM asked of the
  * compiler); out[5] = candidates per CTA, out[6] = CTAs per scenario, out[7] = candidates a warp
  * solves together (4 = shared Newton).  n >= 8.  With n >= 10 also out[8] = 1 on the persistent
- * grid of a lone dense query and out[9] = PW (1: per-scenario cost weights).  Evidence for
- * bench.py / profiles. */
+ * grid of a lone dense query and out[9] = PW (1: per-scenario cost weights); with n >= 11
+ * out[10] = MO (1: the moving-opponent twin of the PW instance, f1l_plan_motion and friends).
+ * Evidence for bench.py / profiles. */
 int f1l_last_eval_shape(f1l_handle h, int32_t* out, int n);
 
 /* Timing / evidence helpers: number of kernels launched by this handle so far, and the device
@@ -611,6 +653,11 @@ int f1l_debug_pp_parts(int n_poses, int n_waypoints, int slots);
  * A01 A10 A11 fx fy; then 16 opponents x (x, y, cos, sin) in the vehicle frame.  out_i[6]: grid
  * ix0, iy0, nearest segment, window start, window length, opponent count. */
 int f1l_debug_query_ctx(f1l_handle h, float* out_f, int32_t* out_i);
+
+/* Debug / test hook: the float32 motion constants of the last f1l_plan_motion call, for
+ * teacher-forced collision checks: out[0] = k_t, out[1 + 2k], out[2 + 2k] = opponent k's velocity
+ * (wx, wy) in the vehicle frame (0 for unused slots).  n >= 1 + 2 F1L_MAX_OPP. */
+int f1l_debug_motion_ctx(f1l_handle h, float* out, int n);
 
 #ifdef __cplusplus
 }
